@@ -34,6 +34,12 @@ cpu_baseline  the UNMODIFIED reference `model.py` class on the host cores (oracl
 parity  the CPU arm's users + more users scored by a float64 evaluation of the oracle, against the CUDA path's lists
 
 `--impl reference` times that CPU arm alone and prints the same JSON line with "impl": "reference".
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step, so that two builds can be compared output for
+output (the inputs are seeded: the same arguments give the same inputs): eval mode `scores.npy` (float32, raw pre-sigmoid scores)
+and `ids.npy` (float64) of the headline step's top-k lists [users_per_step, k]; train mode `loss.npy` and `grad.<parameter>.npy`
+(float32) of the C3 step, taken from the step mode the line reports as `step_mode`: the CUDA-graph replay when it gave the eager
+step's loss, else the eager step.
 """
 from __future__ import annotations
 
@@ -71,6 +77,23 @@ def load_peaks():
         return dict(hbm=d.get("hbm_gbs", 6650.0), tf_burst=d.get("bf16_tflops", 1590.0),
                     tf_sust=d.get("bf16_tflops_sustained", d.get("bf16_tflops", 1590.0)), which="measured")
     return dict(hbm=6650.0, tf_burst=1590.0, tf_sust=1400.0, which="fallback")
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """`--dump-outputs`: one DIR/<name>.npy per array; floats of up to 32 bits as float32, everything else (float64, integers:
+    exact up to 2^53) as float64."""
+    import torch
+    arrays = {k: v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float32 if v.dtype.kind == "f" and v.itemsize <= 4 else np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def synth_histories(users, pois, hist, seed=0):
@@ -288,8 +311,9 @@ def make_eval(cfg, dev, n_users, seed_hist=2):
 
 
 def time_eval(m, hist_np, cfg, ups, steps, warmup, precision, rank, world, local, dev, lib, sample_clocks=False, e2e=True,
-              parity_users=64):
-    """Device-resident timing (+ e2e through topk_host) of `steps` steps of `ups` users; returns a dict of raw results."""
+              parity_users=64, keep_last=False):
+    """Device-resident timing (+ e2e through topk_host) of `steps` steps of `ups` users; returns a dict of raw results
+    (`keep_last`: "last" = host copies of the (score, id) lists the last timed step returned)."""
     import torch
     import torch.distributed as dist
     from poi_recommendation_models_b200.distributed import ShardedRanker
@@ -333,7 +357,7 @@ def time_eval(m, hist_np, cfg, ups, steps, warmup, precision, rank, world, local
         dist.all_reduce(t_local, op=dist.ReduceOp.MAX)
     total_ms = float(t_local.item())
     res = {"ranker": ranker, "users_per_s": ups * steps / (total_ms / 1000.0), "ms_per_step": total_ms / steps, "kern_ms": kern_ms,
-           "launches": launches, "clocks": clocks, "ups": ups}
+           "launches": launches, "clocks": clocks, "ups": ups, "last": (out[0].cpu(), out[1].cpu()) if keep_last else None}
     # ---- N > 1: rank 0 re-scores users of the last step alone, over the whole catalogue, and compares bit for bit ------------
     if world > 1 and parity_users:
         pn = {"users": 0, "identical": 0}
@@ -412,17 +436,15 @@ def roofline_of(res, cfg, peaks, eff):
 # ----------------------------------------------------------------------------------------------------------------------
 # C3: BPR-style training step
 # ----------------------------------------------------------------------------------------------------------------------
-def train_c3(args, dev, lib, peaks, rank, world, steps, warmup, full=False):
-    """BASELINE config C3: BPR-style training forward + backward on (user, pos, neg) triples — 4,096 triples = 8,192
-    (history row, target) pairs, history 128, D = hid = 64; every row has its own history, positives are in the history
-    (live mask), negatives are not.  Step = pair forward (tcgen05), -log sigmoid(s+ - s-), hand-written backward of every
-    parameter (tcgen05 tile kernel + sorted-segment embedding-row reduce).  Data parallel over triples with N > 1 (+ gradient
-    all-reduce): weak scaling.  Returns the block for the JSON line."""
+C3_SHAPE = (40000, 128, 64, 64, 4096)  # POIs, history, D, hid, triples
+
+
+def c3_problem(dev, rank=0):
+    """C3's seeded model (in train mode) and this rank's 2 x 4,096 (history row, target) pairs: positives first, then
+    negatives.  Returns (model, hist, tgt, hreg, treg, ll, region count)."""
     import torch
-    import torch.distributed as dist
-    from poi_recommendation_models_b200 import model as M, ops, synthetic
-    from poi_recommendation_models_b200.distributed import allreduce_gradients
-    N, H, D, hid, T = 40000, 128, 64, 64, 4096
+    from poi_recommendation_models_b200 import model as M, synthetic
+    N, H, D, hid, T = C3_SHAPE
     coords, region, R = synthetic.make_catalog(N, seed=0)
     torch.manual_seed(1)
     m = M.NAIS_region_distance_Embedding(N, D, hid, BETA, R, 1)
@@ -442,7 +464,22 @@ def train_c3(args, dev, lib, peaks, rank, world, steps, warmup, full=False):
     reg = torch.from_numpy(region).to(dev)
     c = torch.from_numpy(coords).to(dev)
     ll = (c[tgt][:, None, :] - c[hist]).abs().float().contiguous()
-    hreg, treg = reg[hist], reg[tgt]
+    return m, hist, tgt, reg[hist], reg[tgt], ll, R
+
+
+def train_c3(args, dev, lib, peaks, rank, world, steps, warmup, full=False, dump_dir=None):
+    """BASELINE config C3: BPR-style training forward + backward on (user, pos, neg) triples — 4,096 triples = 8,192
+    (history row, target) pairs, history 128, D = hid = 64; every row has its own history, positives are in the history
+    (live mask), negatives are not.  Step = pair forward (tcgen05), -log sigmoid(s+ - s-), hand-written backward of every
+    parameter (tcgen05 tile kernel + sorted-segment embedding-row reduce).  Data parallel over triples with N > 1 (+ gradient
+    all-reduce): weak scaling.  Returns the block for the JSON line; `dump_dir`: rank 0 writes the loss and the gradients of
+    the last timed step of the step mode the block reports (`dump_outputs`)."""
+    import torch
+    import torch.distributed as dist
+    from poi_recommendation_models_b200 import ops
+    from poi_recommendation_models_b200.distributed import allreduce_gradients
+    N, H, D, hid, T = C3_SHAPE
+    m, hist, tgt, hreg, treg, ll, R = c3_problem(dev, rank)
 
     def step():
         m.zero_grad(set_to_none=True)
@@ -474,7 +511,14 @@ def train_c3(args, dev, lib, peaks, rank, world, steps, warmup, full=False):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item()) / n_s, int(lib.nais_launch_count() - l0) // n_s, r
 
+    def outputs(loss_):  # what a step hands its caller, copied before the next step overwrites it
+        if not dump_dir:
+            return None
+        return {"loss": loss_.detach().clone(),
+                **{"grad." + n: p.grad.detach().clone() for n, p in m.named_parameters() if p.grad is not None}}
+
     ms, launches, loss = timed(step, warmup, steps)
+    last = outputs(loss)
     step_host_ms = host_ms[0]
     eager_ms, mode = ms, "eager (one Python-level call chain per step)"
     # The eager step is ~60 launches and the host needs about as long to enqueue them as the device to run them (host_enqueue_ms_
@@ -509,11 +553,14 @@ def train_c3(args, dev, lib, peaks, rank, world, steps, warmup, full=False):
         same = abs(float(g_loss.detach()) - float(loss.detach())) <= 1e-6 * abs(float(loss.detach()))
         if same:
             ms, loss, mode = g_ms, g_loss, "CUDA graph replay of the captured step (torch.cuda.graph), one launch per step"
+            last = outputs(g_loss)
         else:
             mode = f"eager (graph replay gave another loss: {float(g_loss.detach())})"
     except Exception as e:  # capture is an optimisation of the measurement loop, never a requirement
         mode = f"eager (CUDA graph capture failed: {type(e).__name__}: {str(e)[:120]})"
         torch.cuda.synchronize()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, last)
     cells = 2 * T * H
     F = flops_per_cell(D, hid)
     blk = {"metric": "bpr_train_triples_per_sec", "value": T * world / (ms / 1000.0), "unit": "triples/s", "ms_per_step": ms,
@@ -831,7 +878,7 @@ def c1_block(dev, lib, no_cpu=False):
 
 
 def run_train(args, dev, lib, peaks, rank, world):
-    blk = train_c3(args, dev, lib, peaks, rank, world, args.steps, args.warmup, full=True)
+    blk = train_c3(args, dev, lib, peaks, rank, world, args.steps, args.warmup, full=True, dump_dir=args.dump_outputs)
     if rank == 0:
         line = {"metric": blk["metric"], "value": blk["value"], "unit": blk["unit"], "n_gpus": world, "steps": args.steps,
                 "warmup": args.warmup, "ms_per_step": blk["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -860,7 +907,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-blocks", action="store_true", help="headline workload only: skip the value_exact / c4 / train_c3 blocks")
     ap.add_argument("--no-presort", action="store_true", help="train: keep the backward's id sorts inside the backward call (A/B of ops.PRESORT_IN_FORWARD)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (impl ours)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     cfg = WORKLOADS[args.config]
 
     rank = int(os.environ.get("RANK", "0"))
@@ -896,7 +946,10 @@ def main():
     ups = min(ups, U)
     n_batches = min(args.steps + args.warmup, max(1, U // ups))
     m, hist_np = make_eval(cfg, dev, n_batches * ups)
-    res = time_eval(m, hist_np, cfg, ups, args.steps, args.warmup, args.precision, rank, world, local, dev, lib, sample_clocks=True)
+    res = time_eval(m, hist_np, cfg, ups, args.steps, args.warmup, args.precision, rank, world, local, dev, lib, sample_clocks=True,
+                    keep_last=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"scores": res["last"][0], "ids": res["last"][1]})
     prec_base = args.precision[:-7] if args.precision.endswith("_onecta") else args.precision  # "_onecta": one CTA per SM instead of CTA pairs, same math
     eff, choice = prec_base, None
     if prec_base == "tc_auto":  # the device-side gate picked MIX or SPLIT (no host sync inside the timed regions)

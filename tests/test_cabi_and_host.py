@@ -85,9 +85,20 @@ def test_ops_refuse_cpu_tensors():
         m(torch.zeros(2, 3, dtype=torch.long), torch.zeros(2, dtype=torch.long))
 
 
-def test_state_dict_keys_and_init_match_reference_classes():
-    if not ref_shim.reference_available():
-        pytest.skip("/root/reference not present")
+def test_state_dict_keys_and_init_match_reference_classes(golden_dir):
+    # tests/golden/scorer_<variant>.npz holds parameter sets the reference class of each of the five variants loaded with
+    # strict=True (make_golden.py): the drop-in class must declare exactly those keys and shapes
+    for variant in orc.VARIANTS:
+        z = np.load(os.path.join(golden_dir, f"scorer_{variant}.npz"))
+        sd = {k[len("reference_sd."):]: torch.from_numpy(z[k]) for k in z.files if k.startswith("reference_sd.")}
+        N, D, hid, beta, R = int(z["N"]), int(z["D"]), int(z["hid"]), float(z["beta"]), int(z["R"])
+        cls = M.CLASSES[variant]
+        b = cls(N, D, hid, beta) if variant == "basic" else cls(N, D, hid, beta, R) if variant == "region" else cls(N, D, hid, beta, R, 1)
+        assert {k: tuple(v.shape) for k, v in b.state_dict().items()} == {k: tuple(v.shape) for k, v in sd.items()}, variant
+        b.load_state_dict(sd, strict=True)
+        assert b.item_num == N and b.beta == beta
+    if not ref_shim.reference_available():  # the key order and the seeded initial values need the reference classes themselves
+        return
     ref = ref_shim.load_reference("model")
     cases = [("NAIS_basic", (50, 16, 8, 0.5)), ("NAIS_regionEmbedding", (50, 16, 8, 0.5, 7)),
              ("NAIS_region_distance_Embedding", (50, 16, 8, 0.5, 7, 1)), ("NAIS_distance_Embedding", (50, 16, 8, 0.5, 7, 1)),
@@ -134,7 +145,17 @@ def test_lat_lon_pairs_equals_latlon_mat_lookup():
     assert torch.equal(PB.lat_lon_pairs(coords, tgt, hist, device="cpu"), ref)
 
 
-def test_metrics_bit_identical_to_reference():
+def test_metrics_bit_identical_to_reference(golden_dir):
+    # the values the reference's eval_metrics.py returned for its own recommended lists (tests/golden/validation_*.npz rows:
+    # precision, recall, hit rate on the validation positives, then on the test positives, one column per k)
+    for name in ("validation_rd.npz", "validation_basic.npz", "validation_region.npz"):
+        z = np.load(os.path.join(golden_dir, name))
+        rec = z["rec"].tolist()
+        for j, part in enumerate(("val", "test")):
+            flat, ptr = z[part + "_flat"], z[part + "_ptr"]
+            positive = [flat[ptr[u]:ptr[u + 1]].tolist() for u in range(int(z["U"]))]
+            for c, fn in enumerate((PM.precision_at_k, PM.recall_at_k, PM.hitrate_at_k)):
+                assert [fn(positive, rec, k) for k in z["k_list"].tolist()] == z["metrics"][3 * j + c].tolist(), (name, part, c)
     rng = np.random.default_rng(3)
     U = 200
     actual = [rng.choice(500, rng.integers(0, 6), replace=False).tolist() for _ in range(U)]
