@@ -133,8 +133,9 @@ typedef struct NaisParams {
  * row; NaisCatalog conventions).  Per-cell arrays (act_mask) are indexed cell(row r of segment s, item h) =
  * seg_cell_offsets[s] + (r - row_offsets[s]) * H_s + h.  The work decomposition is host-known: tile t covers rows
  * tile_row0[t] .. of segment tile_seg[t], at most min(16, 128 / H_s) rows (1 row when H_s > 128), never crossing a segment;
- * segments without history or without rows have no tile (a host loop over the segments builds these arrays: INTEGRATION.md).  NAIS_DIST_KM and dropout are
- * dense-layout only. */
+ * segments without history or without rows have no tile (a host loop over the segments builds these arrays: INTEGRATION.md).  NAIS_DIST_KM
+ * forms dist_km per cell from the same centred coordinates (haversine, cos(latitude) = cos(center_lat + centred lat); NaisCatalog
+ * conventions).  Dropout is dense-layout only. */
 typedef struct NaisPairs {
   const int64_t* hist; /* dense [B,H] / segmented [nnz]: history POI ids */
   const int64_t* tgt;  /* [B]   target POI ids */
@@ -151,8 +152,10 @@ typedef struct NaisPairs {
   const int64_t* tile_row0;        /* [n_tiles] */
   int64_t n_tiles;
   int64_t n_cells;                 /* seg_cell_offsets[n_seg] (host copy: sizes the backward workspace and act_mask) */
-  const float* hist_coords;        /* [nnz,2] centred (lat, lon) of every history item (LATLON) */
-  const float* tgt_coords;         /* [B,2]   centred (lat, lon) of every target (LATLON) */
+  const float* hist_coords;        /* [nnz,2] centred (lat, lon) of every history item (LATLON, KM) */
+  const float* tgt_coords;         /* [B,2]   centred (lat, lon) of every target (LATLON, KM) */
+  float center_lat;                /* segmented KM: the (lat, lon) that was subtracted from the coordinates */
+  float center_lon;
 } NaisPairs;
 
 /* Gradients of nais_pairs_backward.  Dense tables must be zero-filled by the caller; the library writes each touched
@@ -273,7 +276,7 @@ NAIS_API int nais_sample_batch(const int64_t* seg_offsets, const int64_t* hist, 
  * whose gradient is zero does not move, so stepping only the touched rows IS the dense step).  For every table with a
  * non-NULL `sum_*` pointer (the optimizer's `state['sum']`, same shape as the table) the summed row gradient g is applied
  * in place instead of being written to NaisGrads:  sum += g*g ;  param -= lr * g / (sqrt(sum) + eps).  The parameter
- * tables are the ones NaisParams points to (they ARE written).  One branch only. */
+ * tables are the ones NaisParams points to (they ARE written).  Two branches only in the disentangled layout (see below). */
 typedef struct NaisAdagrad {
   float lr, eps;
   float* sum_hist_poi[2];
@@ -291,8 +294,14 @@ NAIS_API int nais_pairs_backward_adagrad(const NaisParams* p, const NaisPairs* b
  * NULL (the batch mean of nn.BCELoss); log terms clamped at -100 and the gradient's denominator at 1e-12 like torch.
  * Embedding tables: row-sparse Adagrad as in nais_pairs_backward_adagrad (`tables`).  MLP / distance-layer parameters: dense
  * Adagrad on the optimizer's state['sum'] tensors in `dense`:  sum += g*g ;  param += -lr * (g / (sqrt(sum) + eps))  (torch's
- * update with weight_decay = lr_decay = 0).  Every parameter NaisParams points to IS written.  One branch only.
- * loss: device float[1]; score (optional): device float[B], the pre-sigmoid scores of the forward. */
+ * update with weight_decay = lr_decay = 0).  Every parameter NaisParams points to IS written.
+ * loss: device float[1]; score (optional): device float[B], the pre-sigmoid scores of the forward.
+ *
+ * Two branches (nais_pairs_backward_adagrad, nais_pairs_train_step, nais_train_users): accepted for the disentangled layout only —
+ * branch[0].w_reg == 0 and branch[1].w_poi == 0, so every table belongs to exactly one branch and one row-sparse step per id list IS
+ * the dense step — with NAIS_DIST_NONE or NAIS_DIST_KM; any other two-branch input is NAIS_ERR_MODE.  Branch 0's tables go in
+ * NaisAdagrad slot [0], branch 1's region table in sum_reg[1]; the sum_region_* / sum_dist_embed fields below are required
+ * (NAIS_ERR_NULL) exactly then.  embed_distance: only row 0 is read (dist_buckets == 1), so only row 0 moves. */
 typedef struct NaisDenseAdagrad {
   float lr, eps;
   float* sum_w1;
@@ -300,6 +309,10 @@ typedef struct NaisDenseAdagrad {
   float* sum_w2;
   float* sum_dist_w; /* NULL unless NAIS_DIST_LATLON */
   float* sum_dist_b;
+  float* sum_region_w1;  /* disentangled layout: region_attn_layer1.weight / .bias, region_attn_layer2.weight */
+  float* sum_region_b1;
+  float* sum_region_w2;
+  float* sum_dist_embed; /* disentangled layout: [D], row 0 of embed_distance's state */
 } NaisDenseAdagrad;
 NAIS_API size_t nais_pairs_train_step_workspace_bytes(const NaisParams* p, const NaisPairs* batch);
 NAIS_API int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
@@ -313,7 +326,8 @@ NAIS_API int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, 
  * entry_region / entry_coords are the region id / centred (lat, lon) of every CSR entry (region[indices], coords[indices]; NULL
  * when the variant has no region table / distance lanes).  host_indptr [n_rows + 1] and host_users are HOST arrays (read during
  * the call; a user id outside [0, n_rows) is an argument error).
- * User i samples with seed + host_users[i].  losses: device float[n_users] (0 for a user without history).  One branch only.
+ * User i samples with seed + host_users[i].  losses: device float[n_users] (0 for a user without history).  Two branches: as
+ * nais_pairs_train_step.  entry_coords / poi_coords are needed for NAIS_DIST_KM as for NAIS_DIST_LATLON.
  * Streams: what depends on the batch only (segment structure, sampler, the id sorts of the backward) is enqueued ONE USER AHEAD on
  * a library-owned preparation stream (one per device, created on first use) into the other half of the workspace, so the chain
  * of dependent launches per optimizer step is forward -> BCE -> backward -> Adagrad; the preparation stream starts after the work
@@ -324,6 +338,13 @@ NAIS_API int nais_train_users(const NaisParams* p, const int64_t* host_indptr, i
                               const float* entry_coords, const int32_t* poi_region, const float* poi_coords, const int64_t* host_users,
                               int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables, const NaisDenseAdagrad* dense,
                               float* losses, void* workspace, size_t workspace_bytes, nais_stream_t stream);
+/* nais_train_users for coordinates centred on (center_lat, center_lon): the (lat, lon) that was subtracted from entry_coords /
+ * poi_coords (NaisCatalog conventions).  NAIS_DIST_KM needs it for cos(latitude); nais_train_users is this call with (0, 0). */
+NAIS_API int nais_train_users_centred(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
+                                      const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region,
+                                      const float* poi_coords, const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed,
+                                      const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* losses, void* workspace,
+                                      size_t workspace_bytes, float center_lat, float center_lon, nais_stream_t stream);
 
 /* Workspace for nais_fullrank_topk / nais_fullrank_scores: n_users and nnz = offsets[n_users] are host-known. */
 NAIS_API size_t nais_fullrank_workspace_bytes(const NaisParams* p, int32_t n_users, int64_t nnz, int64_t poi_begin,

@@ -39,7 +39,8 @@ class NaisPairs(C.Structure):
     _fields_ = [("hist", C.c_void_p), ("tgt", C.c_void_p), ("hreg", C.c_void_p), ("treg", C.c_void_p),
                 ("aux", C.c_void_p), ("B", C.c_int64), ("H", C.c_int32), ("n_seg", C.c_int32), ("seg_offsets", C.c_void_p),
                 ("row_offsets", C.c_void_p), ("seg_cell_offsets", C.c_void_p), ("tile_seg", C.c_void_p), ("tile_row0", C.c_void_p),
-                ("n_tiles", C.c_int64), ("n_cells", C.c_int64), ("hist_coords", C.c_void_p), ("tgt_coords", C.c_void_p)]
+                ("n_tiles", C.c_int64), ("n_cells", C.c_int64), ("hist_coords", C.c_void_p), ("tgt_coords", C.c_void_p),
+                ("center_lat", C.c_float), ("center_lon", C.c_float)]
 
 
 class NaisGrads(C.Structure):
@@ -56,7 +57,8 @@ class NaisAdagrad(C.Structure):
 
 class NaisDenseAdagrad(C.Structure):
     _fields_ = [("lr", C.c_float), ("eps", C.c_float), ("sum_w1", C.c_void_p), ("sum_b1", C.c_void_p), ("sum_w2", C.c_void_p),
-                ("sum_dist_w", C.c_void_p), ("sum_dist_b", C.c_void_p)]
+                ("sum_dist_w", C.c_void_p), ("sum_dist_b", C.c_void_p), ("sum_region_w1", C.c_void_p), ("sum_region_b1", C.c_void_p),
+                ("sum_region_w2", C.c_void_p), ("sum_dist_embed", C.c_void_p)]
 
 
 class NaisCatalog(C.Structure):
@@ -85,6 +87,10 @@ SYMBOLS = {
     "nais_train_users": (C.c_int, [C.POINTER(NaisParams), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_int32, C.c_int32, C.c_uint64, C.POINTER(NaisAdagrad), C.POINTER(NaisDenseAdagrad),
                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "nais_train_users_centred": (C.c_int, [C.POINTER(NaisParams), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_uint64, C.POINTER(NaisAdagrad),
+                                           C.POINTER(NaisDenseAdagrad), C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float,
+                                           C.c_void_p]),
     "nais_rows_adagrad_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
     "nais_rows_adagrad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_float, C.c_float, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -78,6 +78,19 @@ def lat_lon_pairs(place_coords, target_pois, history_pois, device=None):
     return torch.from_numpy(ll).to(device or _device())
 
 
+def dist_km_pairs(place_coords, target_pois, history_pois, device=None):
+    """km[b,h] = great-circle km between target_b and history_h (powerLaw.dist in float64, cast to float32): the `target_distance`
+    argument of NAIS_region_distance_disentangled_Embedding (model.py:497-504) for a dense [B,H] batch."""
+    from .powerlaw import dist
+    c = np.asarray(place_coords, dtype=np.float64)
+    t = np.asarray(target_pois, dtype=np.int64)
+    h = np.asarray(history_pois, dtype=np.int64)
+    if h.ndim == 1:
+        h = np.broadcast_to(h, (len(t), len(h)))
+    km = dist((c[t][:, None, 0], c[t][:, None, 1]), (c[h][..., 0], c[h][..., 1])).astype(np.float32)
+    return torch.from_numpy(np.ascontiguousarray(km)).to(device or _device())
+
+
 class DeviceBatcher:
     """Training batches built ON THE DEVICE (SURVEY.md §8 f1): same batch layout as `get_NAIS_batch_region`
     (batches.py:67-108: shuffled positives, targets interleaved [p, n..n], labels [1, 0..0], history repeated per target)
@@ -128,7 +141,7 @@ class DeviceBatcher:
         fields = {k: st[k] for k in ("seg_offsets", "row_offsets", "seg_cell_offsets", "tile_seg", "tile_row0", "n_seg", "B", "n_tiles",
                                      "n_cells", "max_hist", "host_row_offsets")}
         return ops.SegmentedPairs(hist=hist, hreg=self.region[hist], hist_coords=self.coords32[hist].contiguous(), tgt=tgt, treg=treg,
-                                  tgt_coords=tcoords, label=label, **fields)
+                                  tgt_coords=tcoords, label=label, center=self.center, **fields)
 
     def batch(self, uid: int, negative_num: int):
         """-> (user_history [B,H], train_data [B], train_label [B], user_history_region [B,H], train_data_region [B],

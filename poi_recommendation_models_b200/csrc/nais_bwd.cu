@@ -167,7 +167,7 @@ __global__ void __launch_bounds__(NT, (NKB * DB <= 1) ? 2 : 1) pairs_bwd_kernel(
             g0 = sigmoidf_exact(fmaf(a1, __ldg(p.dist_w + 1), fmaf(a0, __ldg(p.dist_w + 0), __ldg(p.dist_b + 0))));
             g1 = sigmoidf_exact(fmaf(a1, __ldg(p.dist_w + 3), fmaf(a0, __ldg(p.dist_w + 2), __ldg(p.dist_b + 1))));
           } else if (valid && p.dist_mode == NAIS_DIST_KM) {
-            l0 = A.b.aux[cidx];
+            l0 = pair_km(A.b, cidx, hidx, row0 + r);
             g0 = l0 * km_c;
           }
           g[cell] = g0;
@@ -1014,13 +1014,15 @@ static int launch_bwd_tile(const BwdArgs& A, int D, int grid, cudaStream_t strea
 // one-call training step forks them before its forward so they run next to it); phase 2: the rest, on lists sorted by phase 1
 // (same p, b, g, opt, ws).  phase 4: join the sort streams of a phase-1 call to `stream` (the forward of the autograd path ends with
 // it, so that nothing enqueued on `stream` later — or the caller's allocator — can overtake the sorts); phase 3: phase 2 after such
-// a join (no wait of its own for the long list).  One branch in phases 1 - 4.
+// a join (no wait of its own for the long list).  Phases 1 - 4 and the fused optimizer take one branch or the disentangled layout
+// (pairs_disentangled: each id list belongs to one branch, so a row-sparse step per list IS the dense step); branch 0 sorts lists
+// 0 / 1, branch 1 list 2.  `dense`: one DenseAdagradLaunch per branch, each enqueued behind that branch's param_reduce — branch 1's
+// holds embed_distance, whose gradient is complete only after branch 1's param_reduce (both branches read it).
 int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score_parts, const float* row_sum,
                      const unsigned long long* act_mask, const float* dscore, const NaisGrads& g, const NaisAdagrad* opt, void* ws,
                      size_t ws_bytes, cudaStream_t stream, int phase, const DenseAdagradLaunch* dense) {
   if (pairs_n_cells(b) + b.B >= 0x7fffffffLL) return NAIS_ERR_SHAPE;
-  if (phase && p.n_branch != 1) return NAIS_ERR_MODE;
-  if (opt && p.n_branch != 1) return NAIS_ERR_MODE;  // two branches share tables: two sparse steps != one dense step
+  if ((phase || opt) && p.n_branch != 1 && !pairs_disentangled(p)) return NAIS_ERR_MODE;
   const BwdLayout L = bwd_layout(p, b);
   if (ws_bytes < L.total) return NAIS_ERR_WORKSPACE;
   char* base = reinterpret_cast<char*>(ws);
@@ -1075,10 +1077,7 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
         cudaStreamWaitEvent(stream, ev, 0);
       }
     }
-    if (phase == 1 || phase == 4) {
-      cudaError_t e1 = cudaGetLastError();
-      return e1 == cudaSuccess ? 0 : (int)e1;
-    }
+    if (phase == 1 || phase == 4) continue;
     // ---- 2. the tile kernel ------------------------------------------------------------------------------------------------
     BwdArgs A;
     A.p = p;
@@ -1148,7 +1147,8 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
       NAIS_COUNT_LAUNCH(1);
       // the one-call training step's dense Adagrad of these tensors needs nothing else: right behind them, next to the table reduces
       if (dense) {
-        const int rd = launch_dense_adagrad(dense->param, dense->sum, dense->grad, dense->n, dense->lr, dense->eps, pstream);
+        const DenseAdagradLaunch& da = dense[bi];
+        const int rd = launch_dense_adagrad(da.param, da.sum, da.grad, da.n, da.lr, da.eps, pstream);
         if (rd) dense_rc = rd;
       }
       cudaEventRecord(side->pjoin, pstream);
@@ -1167,6 +1167,10 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return (int)e;
     if (dense_rc) return dense_rc;
+  }
+  if (phase == 1 || phase == 4) {
+    cudaError_t e1 = cudaGetLastError();
+    return e1 == cudaSuccess ? 0 : (int)e1;
   }
   return 0;
 }

@@ -106,8 +106,8 @@ static int check_pairs(const NaisParams* p, const NaisPairs* b) {
     if (b->n_seg < 1 || b->n_tiles < 0 || b->n_cells < 0) return NAIS_ERR_SHAPE;
     if (!b->row_offsets || !b->seg_cell_offsets || (b->n_tiles && (!b->tile_seg || !b->tile_row0))) return NAIS_ERR_NULL;
     if (b->aux) return NAIS_ERR_MODE;
-    if (p->dist_mode == NAIS_DIST_KM || p->dropout_p > 0.f) return NAIS_ERR_MODE;
-    if (p->dist_mode == NAIS_DIST_LATLON && (!b->hist_coords || !b->tgt_coords)) return NAIS_ERR_NULL;
+    if (p->dropout_p > 0.f) return NAIS_ERR_MODE;
+    if (p->dist_mode != NAIS_DIST_NONE && (!b->hist_coords || !b->tgt_coords)) return NAIS_ERR_NULL;
     return 0;
   }
   if (p->dist_mode != NAIS_DIST_NONE && !b->aux) return NAIS_ERR_NULL;
@@ -353,7 +353,7 @@ int nais_pairs_backward_adagrad(const NaisParams* p, const NaisPairs* batch, con
   rc = check_pairs(p, batch);
   if (rc) return rc;
   if (!grads || !opt) return NAIS_ERR_NULL;
-  if (p->n_branch != 1) return NAIS_ERR_MODE;
+  if (p->n_branch != 1 && !pairs_disentangled(*p)) return NAIS_ERR_MODE;
   if (!(opt->lr >= 0.f) || !(opt->eps >= 0.f)) return NAIS_ERR_MODE;
   if (batch->B == 0) return 0;
   if (!score_parts || !row_sum || !dscore || !workspace) return NAIS_ERR_NULL;
@@ -367,24 +367,29 @@ int nais_pairs_backward_adagrad(const NaisParams* p, const NaisPairs* batch, con
 namespace {
 inline size_t ts_al(size_t x) { return (x + 255) / 256 * 256; }
 struct TrainStepLayout {
-  size_t score, row_sum, parts, dscore, mask, gw1, gb1, gw2, gdw, gdb, bwd, total;
+  size_t score, row_sum, parts, dscore, mask, gw1[2], gb1[2], gw2[2], gdw, gdb, gde, bwd, total;
 };
 TrainStepLayout train_step_layout(const NaisParams& p, const NaisPairs& b) {
   TrainStepLayout L;
   const int64_t B = b.B, cells = pairs_n_cells(b);
-  const NaisBranch& br = p.branch[0];
-  const int lanes = p.dist_mode == NAIS_DIST_LATLON ? 2 : 0, ldw = br.w_poi + br.w_reg + lanes;
+  const int lanes = p.dist_mode == NAIS_DIST_LATLON ? 2 : 0;
   size_t o = 0;
   L.score = o, o += ts_al((size_t)B * 4);
-  L.row_sum = o, o += ts_al((size_t)B * 4);
-  L.parts = o, o += ts_al((size_t)B * 4);
+  L.row_sum = o, o += ts_al((size_t)p.n_branch * B * 4);
+  L.parts = o, o += ts_al((size_t)p.n_branch * B * 4);
   L.dscore = o, o += ts_al((size_t)B * 4);
   L.mask = o, o += ts_al((size_t)cells * 8);
-  L.gw1 = o, o += ts_al((size_t)p.hid * ldw * 4);
-  L.gb1 = o, o += ts_al((size_t)p.hid * 4);
-  L.gw2 = o, o += ts_al((size_t)p.hid * 4);
+  for (int bi = 0; bi < 2; ++bi) {  // per-branch MLP gradient scratch (branch 1: the disentangled layout's region MLP)
+    const NaisBranch& br = p.branch[bi];
+    const int ldw = br.w_poi + br.w_reg + lanes;
+    const bool on = bi < p.n_branch;
+    L.gw1[bi] = o, o += on ? ts_al((size_t)p.hid * ldw * 4) : 0;
+    L.gb1[bi] = o, o += on ? ts_al((size_t)p.hid * 4) : 0;
+    L.gw2[bi] = o, o += on ? ts_al((size_t)p.hid * 4) : 0;
+  }
   L.gdw = o, o += 256;
   L.gdb = o, o += 256;
+  L.gde = o, o += p.dist_mode == NAIS_DIST_KM ? ts_al((size_t)MAXD * 4) : 0;  // embed_distance row 0 (param_reduce writes D of a branch)
   L.bwd = o, o += ts_al(pairs_bwd_workspace_bytes(p, b));
   L.total = o;
   return L;
@@ -392,16 +397,21 @@ TrainStepLayout train_step_layout(const NaisParams& p, const NaisPairs& b) {
 }  // namespace
 
 size_t nais_pairs_train_step_workspace_bytes(const NaisParams* p, const NaisPairs* batch) {
-  if (check_params(p) || !batch || batch->B < 0 || (!batch->seg_offsets && batch->H < 1) || p->n_branch != 1) return 0;
+  if (check_params(p) || !batch || batch->B < 0 || (!batch->seg_offsets && batch->H < 1)) return 0;
+  if (p->n_branch != 1 && !pairs_disentangled(*p)) return 0;
   return train_step_layout(*p, *batch).total;
 }
 
 static int check_train_state(const NaisParams* p, const NaisAdagrad* tables, const NaisDenseAdagrad* dense) {
   if (!tables || !dense) return NAIS_ERR_NULL;
-  if (p->n_branch != 1 || p->dist_mode == NAIS_DIST_KM) return NAIS_ERR_MODE;
+  const bool two = pairs_disentangled(*p);
+  if (p->n_branch != 1 && !two) return NAIS_ERR_MODE;
+  if (p->n_branch == 1 && p->dist_mode == NAIS_DIST_KM) return NAIS_ERR_MODE;
   if (!(tables->lr >= 0.f) || !(tables->eps >= 0.f) || !(dense->lr >= 0.f) || !(dense->eps >= 0.f)) return NAIS_ERR_MODE;
   if (!dense->sum_w1 || !dense->sum_b1 || !dense->sum_w2) return NAIS_ERR_NULL;
   if (p->dist_mode == NAIS_DIST_LATLON && (!dense->sum_dist_w || !dense->sum_dist_b)) return NAIS_ERR_NULL;
+  if (two && (!dense->sum_region_w1 || !dense->sum_region_b1 || !dense->sum_region_w2)) return NAIS_ERR_NULL;
+  if (two && p->dist_mode == NAIS_DIST_KM && !dense->sum_dist_embed) return NAIS_ERR_NULL;
   return 0;
 }
 
@@ -440,13 +450,16 @@ static int train_step_impl(const NaisParams* p, const NaisPairs* batch, const fl
   // the gradient scratch of the MLP / distance layer (also tells the backward which lists it needs)
   NaisGrads g;
   memset(&g, 0, sizeof(g));
-  g.w1[0] = F(L.gw1);
-  g.b1[0] = F(L.gb1);
-  g.w2[0] = F(L.gw2);
+  for (int bi = 0; bi < p->n_branch; ++bi) {
+    g.w1[bi] = F(L.gw1[bi]);
+    g.b1[bi] = F(L.gb1[bi]);
+    g.w2[bi] = F(L.gw2[bi]);
+  }
   if (p->dist_mode == NAIS_DIST_LATLON) {
     g.dist_w = F(L.gdw);
     g.dist_b = F(L.gdb);
   }
+  if (p->dist_mode == NAIS_DIST_KM) g.dist_embed = F(L.gde);
   // the id sorts of the backward depend on the batch only: forked onto side streams now, they run next to the forward
   if (part != 2) {
     rc = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, g, tables, base + L.bwd, workspace_bytes - L.bwd, st, 1);
@@ -470,16 +483,27 @@ static int train_step_impl(const NaisParams* p, const NaisPairs* batch, const fl
   // backward: MLP / distance-layer gradients to scratch, tables stepped in place
   // (the dense Adagrad of the MLP / distance-layer tensors rides behind the kernel that finishes their gradients, next to the
   // table reduces: one launch less on the step's chain of dependent launches)
+  // (two branches: branch 1's launch also steps row 0 of embed_distance, whose gradient both branches' param_reduce add up)
   const NaisBranch& br = p->branch[0];
   const int lanes = p->dist_mode == NAIS_DIST_LATLON ? 2 : 0, ldw = br.w_poi + br.w_reg + lanes;
-  const DenseAdagradLaunch da = {{const_cast<float*>(br.w1), const_cast<float*>(br.b1), const_cast<float*>(br.w2),
-                                  lanes ? const_cast<float*>(p->dist_w) : nullptr, lanes ? const_cast<float*>(p->dist_b) : nullptr},
-                                 {dense->sum_w1, dense->sum_b1, dense->sum_w2, dense->sum_dist_w, dense->sum_dist_b},
-                                 {g.w1[0], g.b1[0], g.w2[0], g.dist_w, g.dist_b},
-                                 {p->hid * ldw, p->hid, p->hid, 4, 2},
-                                 dense->lr, dense->eps};
+  DenseAdagradLaunch da[2] = {{{const_cast<float*>(br.w1), const_cast<float*>(br.b1), const_cast<float*>(br.w2),
+                                lanes ? const_cast<float*>(p->dist_w) : nullptr, lanes ? const_cast<float*>(p->dist_b) : nullptr},
+                               {dense->sum_w1, dense->sum_b1, dense->sum_w2, dense->sum_dist_w, dense->sum_dist_b},
+                               {g.w1[0], g.b1[0], g.w2[0], g.dist_w, g.dist_b},
+                               {p->hid * ldw, p->hid, p->hid, 4, 2},
+                               dense->lr, dense->eps}};
+  if (p->n_branch == 2) {
+    const NaisBranch& r = p->branch[1];
+    const bool km = p->dist_mode == NAIS_DIST_KM;
+    da[1] = {{const_cast<float*>(r.w1), const_cast<float*>(r.b1), const_cast<float*>(r.w2), km ? const_cast<float*>(p->dist_embed) : nullptr,
+              nullptr},
+             {dense->sum_region_w1, dense->sum_region_b1, dense->sum_region_w2, dense->sum_dist_embed, nullptr},
+             {g.w1[1], g.b1[1], g.w2[1], g.dist_embed, nullptr},
+             {p->hid * (r.w_poi + r.w_reg), p->hid, p->hid, r.w_poi + r.w_reg, 0},
+             dense->lr, dense->eps};
+  }
   return launch_pairs_bwd(*p, *batch, F(L.parts), F(L.row_sum), mask, F(L.dscore), g, tables, base + L.bwd, workspace_bytes - L.bwd, st,
-                          part == 2 ? 3 : 2, &da);
+                          part == 2 ? 3 : 2, da);
 }
 
 // ---- nais_train_users: the reference's one-user-per-step schedule, a list of users per call ---------------------------------------
@@ -547,7 +571,7 @@ cudaStream_t prep_stream() {
 }  // namespace
 
 size_t nais_train_users_workspace_bytes(const NaisParams* p, int32_t max_hist, int32_t num_ng) {
-  if (check_params(p) || p->n_branch != 1 || max_hist < 1 || num_ng < 0) return 0;
+  if (check_params(p) || (p->n_branch != 1 && !pairs_disentangled(*p)) || max_hist < 1 || num_ng < 0) return 0;
   return 2 * users_layout(*p, max_hist, num_ng).total;  // two users in flight: one being prepared, one being stepped
 }
 
@@ -555,6 +579,15 @@ int nais_train_users(const NaisParams* p, const int64_t* host_indptr, int64_t n_
                      const float* entry_coords, const int32_t* poi_region, const float* poi_coords, const int64_t* host_users,
                      int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* losses,
                      void* workspace, size_t workspace_bytes, nais_stream_t stream) {
+  return nais_train_users_centred(p, host_indptr, n_rows, indices, entry_region, entry_coords, poi_region, poi_coords, host_users, n_users,
+                                  num_ng, seed, tables, dense, losses, workspace, workspace_bytes, 0.f, 0.f, stream);
+}
+
+int nais_train_users_centred(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
+                             const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region, const float* poi_coords,
+                             const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables,
+                             const NaisDenseAdagrad* dense, float* losses, void* workspace, size_t workspace_bytes, float center_lat,
+                             float center_lon, nais_stream_t stream) {
   int rc = check_params(p);
   if (rc) return rc;
   rc = check_train_state(p, tables, dense);
@@ -562,7 +595,9 @@ int nais_train_users(const NaisParams* p, const int64_t* host_indptr, int64_t n_
   if (n_users < 0 || num_ng < 0) return NAIS_ERR_SHAPE;
   if (n_users == 0) return 0;
   if (!host_indptr || !indices || !host_users || !losses || !workspace) return NAIS_ERR_NULL;
-  const bool need_reg = p->branch[0].w_reg > 0, need_co = p->dist_mode == NAIS_DIST_LATLON;
+  bool need_reg = false;
+  for (int i = 0; i < p->n_branch; ++i) need_reg |= p->branch[i].w_reg > 0;
+  const bool need_co = p->dist_mode != NAIS_DIST_NONE;
   if ((need_reg && (!entry_region || !poi_region)) || (need_co && (!entry_coords || !poi_coords))) return NAIS_ERR_NULL;
   if (!aligned16(workspace)) return NAIS_ERR_ALIGN;
   int max_hist = 0;
@@ -633,6 +668,8 @@ int nais_train_users(const NaisParams* p, const int64_t* host_indptr, int64_t n_
     b.n_cells = (int64_t)R * H;
     b.hist_coords = need_co ? entry_coords + 2 * a : nullptr;
     b.tgt_coords = need_co ? reinterpret_cast<float*>(base + L.tco) : nullptr;
+    b.center_lat = center_lat;
+    b.center_lon = center_lon;
     ub.label = reinterpret_cast<float*>(base + L.label);
     ub.step = base + L.step;
   };

@@ -295,7 +295,7 @@ __global__ void __launch_bounds__(NT, 2) pairs_fwd_kernel(const __grid_constant_
             pair_latlon(A.b, cidx, hidx, row0 + r, l0, l1);
             dist_lanes(p, l0, l1, g0, g1);
           } else if (valid && p.dist_mode == NAIS_DIST_KM) {
-            float km = A.b.aux[cidx];
+            const float km = pair_km(A.b, cidx, hidx, row0 + r);
             g0 = km * (p.dist_buckets == 1 ? km_c : km_coef(p, D, km));
           }
           s.g[cell] = g0;

@@ -30,6 +30,11 @@ struct PairTile {
   int64_t cell0;    // index of (row0, h = 0) in the per-cell arrays (aux, act_mask, dq positions): cell (r, h) = cell0 + r*H + h
 };
 
+// The disentangled two-branch layout (include/nais_b200.h): branch 0 owns the POI tables, branch 1 the region table, so no id list is
+// in both branches; the fused optimizer paths take it with NAIS_DIST_NONE or NAIS_DIST_KM.
+__host__ __device__ inline bool pairs_disentangled(const NaisParams& p) {
+  return p.n_branch == 2 && p.branch[0].w_reg == 0 && p.branch[1].w_poi == 0 && p.dist_mode != NAIS_DIST_LATLON;
+}
 __host__ __device__ inline bool pairs_segmented(const NaisPairs& b) { return b.seg_offsets != nullptr; }
 __host__ __device__ inline int64_t pairs_n_cells(const NaisPairs& b) { return pairs_segmented(b) ? b.n_cells : b.B * (int64_t)b.H; }
 __host__ __device__ inline int64_t pairs_n_tiles(const NaisPairs& b) {
@@ -74,6 +79,16 @@ __device__ __forceinline__ void pair_latlon(const NaisPairs& b, int64_t cidx, in
     l0 = fabsf(__ldg(b.tgt_coords + row * 2) - __ldg(b.hist_coords + hidx * 2));
     l1 = fabsf(__ldg(b.tgt_coords + row * 2 + 1) - __ldg(b.hist_coords + hidx * 2 + 1));
   }
+}
+
+// dist_km of one cell (NAIS_DIST_KM): the dense layout reads the tensor the caller built (powerLaw.dist, model.py:497-504), the
+// segmented layout forms the haversine distance from the centred fp32 coordinates like the full-rank path (nais_fp32.cu)
+__device__ __forceinline__ float pair_km(const NaisPairs& b, int64_t cidx, int64_t hidx, int64_t row) {
+  if (b.aux) return __ldg(b.aux + cidx);
+  const float tla = __ldg(b.tgt_coords + row * 2), tlo = __ldg(b.tgt_coords + row * 2 + 1);
+  const float hla = __ldg(b.hist_coords + hidx * 2), hlo = __ldg(b.hist_coords + hidx * 2 + 1);
+  const float d2r = 0.017453292519943295f;
+  return dist_km_f(tla, tlo, hla, hlo, cosf((b.center_lat + tla) * d2r), cosf((b.center_lat + hla) * d2r));
 }
 
 // ---- software pipelining of a tile's inputs (the two-threads-per-cell tcgen05 pair kernels): Ampere-style cp.async into shared

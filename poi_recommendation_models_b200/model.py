@@ -92,7 +92,8 @@ class _NAISBase(nn.Module):
         `state['sum']` move.  With the reference's `weight_decay = 0` (run.py:833) this IS the dense step (SURVEY.md §7
         'Dense Adagrad semantic'); other settings raise.  The MLP / dist-layer parameters go through `optimizer.step()` as
         usual.  Returns the loss (same value `loss_func(forward(...), label)` gives).  `hist` may be an ops.SegmentedPairs
-        (many users in one step; tgt / hreg / treg / aux then stay None).  `row_weight` [B]: the loss becomes
+        (many users in one step; tgt / hreg / treg / aux then stay None).  Every class takes the one-call path, the two-branch
+        disentangled one included (its embed_distance moves in row 0, the only row its forward reads).  `row_weight` [B]: the loss becomes
         sum_b row_weight[b] * BCE_b instead of the batch mean — e.g. 1 / rows(user of b) makes a multi-user step the sum of the
         reference's per-user mean losses (run.py:251)."""
         if not isinstance(optimizer, torch.optim.Adagrad):
@@ -121,7 +122,7 @@ class _NAISBase(nn.Module):
         # plain Adagrad on every parameter.  `one_call=False` on the model keeps the op-by-op path below (the parity tests compare).
         dense = {n: t for n, t in P.items() if n not in ops._TABLES}
         dgroups = [group_of.get(id(t)) for t in dense.values()]
-        if (getattr(self, "one_call", True) and isinstance(pp, str) and self.variant != "disentangled" and type(self.loss_func) is nn.BCELoss
+        if (getattr(self, "one_call", True) and isinstance(pp, str) and type(self.loss_func) is nn.BCELoss
                 and self.loss_func.reduction == "mean" and self.loss_func.weight is None and all(g is not None for g in dgroups)
                 and all(g["weight_decay"] == 0 and g["lr_decay"] == 0 and not g.get("maximize", False) for g in dgroups)
                 and len({(g["lr"], g["eps"]) for g in dgroups}) == 1 and all(t.dtype == torch.float32 for t in P.values())):
@@ -156,11 +157,12 @@ class _NAISBase(nn.Module):
         positive, forward, BCELoss, backward, Adagrad step — for a whole list of users in ONE library call (`nais_train_users`):
         the same optimizer steps in the same order as `for u in uids: fused_adagrad_step(optimizer, *batcher.multi_user_batch([u],
         negative_num, seed + u))`, bit for bit, without the per-user Python work.  `batcher`: a batches.DeviceBatcher over the
-        train matrix.  Returns the per-user losses [len(uids)] on the device."""
+        train matrix.  Every class without dropout in train mode, the disentangled one included.  Returns the per-user losses
+        [len(uids)] on the device."""
         if not isinstance(optimizer, torch.optim.Adagrad):
             raise RuntimeError("train_users needs torch.optim.Adagrad (run.py:225)")
-        if self.variant == "disentangled" or type(self.loss_func) is not nn.BCELoss or self.loss_func.reduction != "mean":
-            raise RuntimeError("train_users: one-branch variants with the reference's mean BCELoss")
+        if type(self.loss_func) is not nn.BCELoss or self.loss_func.reduction != "mean":
+            raise RuntimeError("train_users: the reference's mean BCELoss")
         if self._dropout_on_l1 and self.training and self.drop.p > 0:
             raise RuntimeError("train_users: dropout variants go through fused_adagrad_step (a fresh dropout seed per step)")
         P = self._params()
@@ -175,11 +177,12 @@ class _NAISBase(nn.Module):
         (lr_t, eps_t), (lr_d, eps_d) = next(iter(tg)), next(iter(dg))
         sums = {n: optimizer.state[t]["sum"] for n, t in P.items()}
         optimizer.zero_grad(set_to_none=True)
-        has_reg, has_ll = "embed_region.weight" in P, "dist_layer.weight" in P
+        has_reg, has_co = "embed_region.weight" in P, "dist_layer.weight" in P or self.variant == "disentangled"
         losses = ops.train_users(self.variant, float(self.beta), P, sums, sums, lr_t, eps_t, lr_d, eps_d, batcher.indptr, batcher.indices,
-                                 batcher.entry_region if has_reg else None, batcher.entry_coords if has_ll else None,
-                                 batcher.region32 if has_reg else None, batcher.coords32 if has_ll else None, uids, negative_num, seed,
-                                 getattr(self, "pairs_precision", "auto") if isinstance(getattr(self, "pairs_precision", "auto"), str) else "auto")
+                                 batcher.entry_region if has_reg else None, batcher.entry_coords if has_co else None,
+                                 batcher.region32 if has_reg else None, batcher.coords32 if has_co else None, uids, negative_num, seed,
+                                 getattr(self, "pairs_precision", "auto") if isinstance(getattr(self, "pairs_precision", "auto"), str) else "auto",
+                                 center=batcher.center)
         n_steps = int(sum(1 for u in np.asarray(uids).reshape(-1) if batcher.indptr[int(u) + 1] > batcher.indptr[int(u)]))
         for t in P.values():
             optimizer.state[t]["step"] += n_steps

@@ -178,7 +178,8 @@ def build_params(variant: str, P: Dict[str, torch.Tensor], beta: float, keep: Li
 class SegmentedPairs:
     """A multi-user training batch in the segmented layout of NaisPairs (include/nais_b200.h): the rows of a segment (= a
     user) share ONE stored history — no [B,H] repeat (batches.py:97), no materialised [B,H,2] distance tensor (run.py:239-247:
-    the kernels form |dlat|,|dlon| from centred coordinates).  Built by `segment_structure` + `sample_batch`
+    the kernels form |dlat|,|dlon|, or the haversine km of the disentangled model, from centred coordinates; `center` is the
+    (lat, lon) that was subtracted from them).  Built by `segment_structure` + `sample_batch`
     (batches.DeviceBatcher.multi_user_batch) or by hand."""
     hist: torch.Tensor                 # [nnz] int64 history POI ids, segment after segment
     hreg: Optional[torch.Tensor]       # [nnz] int64
@@ -198,6 +199,7 @@ class SegmentedPairs:
     n_cells: int
     max_hist: int
     host_row_offsets: Optional[object] = None  # numpy copy (per-user loss weights etc.)
+    center: Tuple[float, float] = (0.0, 0.0)
 
 
 def _upload_packed(arrays, device):
@@ -276,6 +278,7 @@ def _pairs_struct(hist, tgt, hreg, treg, aux, keep) -> NaisPairs:
         b.seg_offsets, b.row_offsets, b.seg_cell_offsets = _ptr(sp.seg_offsets), _ptr(sp.row_offsets), _ptr(sp.seg_cell_offsets)
         b.tile_seg, b.tile_row0, b.n_tiles, b.n_cells = _ptr(sp.tile_seg), _ptr(sp.tile_row0), sp.n_tiles, sp.n_cells
         b.hist_coords, b.tgt_coords = _ptr(sp.hist_coords), _ptr(sp.tgt_coords)
+        b.center_lat, b.center_lon = float(sp.center[0]), float(sp.center[1])
         keep.append(sp)
         return b
 
@@ -539,29 +542,23 @@ def pairs_backward_adagrad(variant: str, beta: float, P: Dict[str, torch.Tensor]
     """Backward of `pairs_score` with the embedding tables stepped in place by a row-sparse Adagrad fused into the
     sorted-segment reduce (nais_pairs_backward_adagrad; replaces run.py:252-254 for `embed_*`): `sums[name]` is the
     optimizer's `state['sum']` of table `name`; P[name] and sums[name] of every touched row are updated, nothing dense is
-    written.  Returns the gradients of the remaining (MLP / dist layer) parameters."""
-    from ._lib import NaisAdagrad
+    written.  Returns the gradients of the remaining (MLP / dist layer / embed_distance) parameters."""
     dev = _need_cuda(hist, tgt, dscore, *P.values())
     lib = _lib.load()
     keep: List[torch.Tensor] = []
     with torch.cuda.device(dev):
         p = build_params(variant, P, beta, keep, drop[0], drop[1], _fwd_bwd(drop[2])[1])
-        if p.n_branch != 1:
-            raise RuntimeError("fused Adagrad: one-branch variants only")
         b = _pairs_struct(hist, tgt, hreg, treg, aux, keep)
         G = {n: _grad_buffer(n, t, int(b.B)) for n, t in P.items() if n not in _TABLES}
         g = NaisGrads()
         g.w1[0], g.b1[0], g.w2[0] = (G["attn_layer1.weight"].data_ptr(), G["attn_layer1.bias"].data_ptr(), G["attn_layer2.weight"].data_ptr())
         if "dist_layer.weight" in G:
             g.dist_w, g.dist_b = G["dist_layer.weight"].data_ptr(), G["dist_layer.bias"].data_ptr()
-        o = NaisAdagrad()
-        o.lr, o.eps = float(lr), float(eps)
-        for name, field in zip(_TABLES, (o.sum_hist_poi, o.sum_tgt_poi, o.sum_reg)):
-            if name in P:
-                st = sums[name]
-                if st.dtype != torch.float32 or not st.is_contiguous() or st.shape != P[name].shape or not P[name].is_contiguous():
-                    raise RuntimeError(f"fused Adagrad: {name} and its state must be contiguous float32 of the same shape")
-                field[0] = st.data_ptr()
+        if variant == "disentangled":
+            g.w1[1], g.b1[1], g.w2[1] = (G["region_attn_layer1.weight"].data_ptr(), G["region_attn_layer1.bias"].data_ptr(),
+                                         G["region_attn_layer2.weight"].data_ptr())
+            g.dist_embed = G["embed_distance.weight"].data_ptr()
+        o = _table_adagrad(P, sums, lr, eps)
         ws_bytes = lib.nais_pairs_backward_workspace_bytes(C.byref(p), C.byref(b))
         ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)
         ds = _f32(dscore)
@@ -584,8 +581,6 @@ def pairs_train_step(variant: str, beta: float, P: Dict[str, torch.Tensor], tabl
     keep: List[torch.Tensor] = []
     with torch.cuda.device(dev):
         p = build_params(variant, P, beta, keep, drop[0], drop[1], drop[2])
-        if p.n_branch != 1:
-            raise RuntimeError("fused train step: one-branch variants only")
         b = _pairs_struct(hist, tgt, hreg, treg, aux, keep)
         o, d = _adagrad_structs(P, table_sums, dense_sums, lr_tables, eps_tables, lr_dense, eps_dense)
         lab = _f32(label)
@@ -600,20 +595,32 @@ def pairs_train_step(variant: str, beta: float, P: Dict[str, torch.Tensor], tabl
     return loss, score
 
 
-def _adagrad_structs(P, table_sums, dense_sums, lr_tables, eps_tables, lr_dense, eps_dense):
-    from ._lib import NaisAdagrad, NaisDenseAdagrad
+def _table_adagrad(P, table_sums, lr, eps):
+    """NaisAdagrad of the embedding tables: branch 0's slots, except the disentangled model's region table, which belongs to its
+    branch 1 (include/nais_b200.h)."""
+    from ._lib import NaisAdagrad
     o = NaisAdagrad()
-    o.lr, o.eps = float(lr_tables), float(eps_tables)
-    for name, field in zip(_TABLES, (o.sum_hist_poi, o.sum_tgt_poi, o.sum_reg)):
+    o.lr, o.eps = float(lr), float(eps)
+    reg_slot = 1 if "region_attn_layer1.weight" in P else 0
+    for name, field, slot in zip(_TABLES, (o.sum_hist_poi, o.sum_tgt_poi, o.sum_reg), (0, 0, reg_slot)):
         if name in P:
             st = table_sums[name]
             if st.dtype != torch.float32 or not st.is_contiguous() or st.shape != P[name].shape or not P[name].is_contiguous():
                 raise RuntimeError(f"fused Adagrad: {name} and its state must be contiguous float32 of the same shape")
-            field[0] = st.data_ptr()
+            field[slot] = st.data_ptr()
+    return o
+
+
+def _adagrad_structs(P, table_sums, dense_sums, lr_tables, eps_tables, lr_dense, eps_dense):
+    from ._lib import NaisDenseAdagrad
+    o = _table_adagrad(P, table_sums, lr_tables, eps_tables)
     d = NaisDenseAdagrad()
     d.lr, d.eps = float(lr_dense), float(eps_dense)
+    # (embed_distance: the kernels read and step row 0 only, so the state's row 0 — the start of the tensor — is what they get)
     for name, attr in (("attn_layer1.weight", "sum_w1"), ("attn_layer1.bias", "sum_b1"), ("attn_layer2.weight", "sum_w2"),
-                       ("dist_layer.weight", "sum_dist_w"), ("dist_layer.bias", "sum_dist_b")):
+                       ("dist_layer.weight", "sum_dist_w"), ("dist_layer.bias", "sum_dist_b"),
+                       ("region_attn_layer1.weight", "sum_region_w1"), ("region_attn_layer1.bias", "sum_region_b1"),
+                       ("region_attn_layer2.weight", "sum_region_w2"), ("embed_distance.weight", "sum_dist_embed")):
         if name in P:
             st = dense_sums[name]
             if st.dtype != torch.float32 or not st.is_contiguous() or st.shape != P[name].shape or not P[name].is_contiguous():
@@ -625,11 +632,11 @@ def _adagrad_structs(P, table_sums, dense_sums, lr_tables, eps_tables, lr_dense,
 def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sums, dense_sums, lr_tables, eps_tables, lr_dense,
                 eps_dense, host_indptr, indices: torch.Tensor, entry_region: Optional[torch.Tensor],
                 entry_coords: Optional[torch.Tensor], poi_region: Optional[torch.Tensor], poi_coords: Optional[torch.Tensor],
-                users, num_ng: int, seed: int, pairs_precision: str = "auto") -> torch.Tensor:
+                users, num_ng: int, seed: int, pairs_precision: str = "auto", center: Tuple[float, float] = (0.0, 0.0)) -> torch.Tensor:
     """nais_train_users: the reference's schedule, one optimizer step per user (run.py:227-255), for a list of users in ONE library
     call — per user the device sampler over his CSR slice + the one-call training step, ~15 launches and no host work in between.
-    `host_indptr` / `users`: numpy int64 (host).  Updates every tensor of `P` and the optimizer sums in place; returns the
-    per-user losses [n] (device)."""
+    `host_indptr` / `users`: numpy int64 (host).  `center`: the (lat, lon) subtracted from `entry_coords` / `poi_coords`.  Updates
+    every tensor of `P` and the optimizer sums in place; returns the per-user losses [n] (device)."""
     import numpy as np
     dev = _need_cuda(indices, entry_region, entry_coords, poi_region, poi_coords, *P.values())
     lib = _lib.load()
@@ -640,8 +647,6 @@ def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sum
         raise IndexError("train_users: user id outside the train matrix")
     with torch.cuda.device(dev):
         p = build_params(variant, P, beta, keep, 0.0, 0, pairs_precision)
-        if p.n_branch != 1:
-            raise RuntimeError("train_users: one-branch variants only")
         o, d = _adagrad_structs(P, table_sums, dense_sums, lr_tables, eps_tables, lr_dense, eps_dense)
         if indices.dtype != torch.int64 or not indices.is_contiguous():
             raise RuntimeError("train_users: `indices` must be contiguous int64 (the CSR of the train matrix)")
@@ -653,9 +658,10 @@ def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sum
         losses = torch.empty(max(hu.size, 1), device=dev, dtype=torch.float32)
         ws_bytes = lib.nais_train_users_workspace_bytes(C.byref(p), max(max_hist, 1), int(num_ng))
         ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)
-        _lib.check(lib.nais_train_users(C.byref(p), hp.ctypes.data, int(hp.size) - 1, indices.data_ptr(), _ptr(er), _ptr(ec), _ptr(pr), _ptr(pc),
-                                        hu.ctypes.data, int(hu.size), int(num_ng), int(seed) & (2 ** 64 - 1), C.byref(o), C.byref(d),
-                                        losses.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "nais_train_users")
+        _lib.check(lib.nais_train_users_centred(C.byref(p), hp.ctypes.data, int(hp.size) - 1, indices.data_ptr(), _ptr(er), _ptr(ec), _ptr(pr),
+                                                _ptr(pc), hu.ctypes.data, int(hu.size), int(num_ng), int(seed) & (2 ** 64 - 1), C.byref(o),
+                                                C.byref(d), losses.data_ptr(), ws.data_ptr(), ws_bytes, float(center[0]), float(center[1]),
+                                                _stream()), "nais_train_users_centred")
         _poll_bad_index(dev)
     return losses[: hu.size]
 
