@@ -975,7 +975,7 @@ size_t pairs_bwd_workspace_bytes(const NaisParams& p, const NaisPairs& b) { retu
 // streams forked from / joined to the caller's stream with events.  One pool per device, created on first use; the mutex is
 // held while a call ENQUEUES its work (cudaStreamWaitEvent binds to the record that precedes it at call time).
 struct SideStreams {
-  cudaStream_t s[3] = {nullptr, nullptr, nullptr};  // [0], [1]: lists 1, 2; [2]: the long list's sort when it is forked ahead (phase 1), then param_reduce
+  cudaStream_t s[3] = {nullptr, nullptr, nullptr};  // [0], [1]: lists 1, 2; [2]: the long list's sort when it is forked ahead (BWD_SORTS), then param_reduce
   cudaEvent_t fork = nullptr, join[2] = {nullptr, nullptr}, sorted0 = nullptr, pjoin = nullptr;  // pjoin: param_reduce (+ dense Adagrad) on s[2]
   bool ok = false;
 };
@@ -1010,19 +1010,15 @@ static int launch_bwd_tile(const BwdArgs& A, int D, int grid, cudaStream_t strea
   return (int)cudaGetLastError();
 }
 
-// phase 0: the whole backward.  phase 1: only the id sorts, ALL of them on side streams (they do not depend on the gradients: the
-// one-call training step forks them before its forward so they run next to it); phase 2: the rest, on lists sorted by phase 1
-// (same p, b, g, opt, ws).  phase 4: join the sort streams of a phase-1 call to `stream` (the forward of the autograd path ends with
-// it, so that nothing enqueued on `stream` later — or the caller's allocator — can overtake the sorts); phase 3: phase 2 after such
-// a join (no wait of its own for the long list).  Phases 1 - 4 and the fused optimizer take one branch or the disentangled layout
-// (pairs_disentangled: each id list belongs to one branch, so a row-sparse step per list IS the dense step); branch 0 sorts lists
-// 0 / 1, branch 1 list 2.  `dense`: one DenseAdagradLaunch per branch, each enqueued behind that branch's param_reduce — branch 1's
-// holds embed_distance, whose gradient is complete only after branch 1's param_reduce (both branches read it).
+// `phase`: see BwdPhase (the forward of the autograd path ends with BWD_JOIN_SORTS).  The split phases and the fused optimizer take
+// pairs_fused_layout (disentangled: each id list belongs to one branch, so a row-sparse step per list IS the dense step); branch 0
+// sorts lists 0 / 1, branch 1 list 2.  `dense`: one DenseAdagradLaunch per branch, each enqueued behind that branch's param_reduce —
+// branch 1's holds embed_distance, whose gradient is complete only after branch 1's param_reduce (both branches read it).
 int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score_parts, const float* row_sum,
                      const unsigned long long* act_mask, const float* dscore, const NaisGrads& g, const NaisAdagrad* opt, void* ws,
-                     size_t ws_bytes, cudaStream_t stream, int phase, const DenseAdagradLaunch* dense) {
+                     size_t ws_bytes, cudaStream_t stream, BwdPhase phase, const DenseAdagradLaunch* dense) {
   if (pairs_n_cells(b) + b.B >= 0x7fffffffLL) return NAIS_ERR_SHAPE;
-  if ((phase || opt) && p.n_branch != 1 && !pairs_disentangled(p)) return NAIS_ERR_MODE;
+  if ((phase != BWD_ALL || opt) && !pairs_fused_layout(p)) return NAIS_ERR_MODE;
   const BwdLayout L = bwd_layout(p, b);
   if (ws_bytes < L.total) return NAIS_ERR_WORKSPACE;
   char* base = reinterpret_cast<char*>(ws);
@@ -1049,7 +1045,7 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
                           br.w_poi > 0 && (g.tgt_poi[bi] || (opt && opt->sum_tgt_poi[bi])),
                           br.w_reg > 0 && (g.reg[bi] || (opt && opt->sum_reg[bi]))};
     // ---- 1. sort the ids (they do not depend on the gradients; stable radix sort: equal ids keep cell order) ----------------
-    if (phase < 2 && (want[0] || want[1] || want[2])) {
+    if ((phase == BWD_ALL || phase == BWD_SORTS) && (want[0] || want[1] || want[2])) {
       const int64_t n_thr = n_cells > b.B ? n_cells : b.B;
       make_keys_kernel<<<(unsigned)((n_thr + 255) / 256), 256, 0, stream>>>(
           b, p.item_num, p.region_num, want[0] ? I(L.kin[0]) : nullptr, U(L.vin[0]), want[1] ? I(L.kin[1]) : nullptr, U(L.vin[1]),
@@ -1058,7 +1054,7 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
       cudaEventRecord(side->fork, stream);
       for (int t = 2; t >= 0; --t) {  // (the caller's stream last: the side streams are busy while it sorts the long list)
         if (!want[t]) continue;
-        cudaStream_t sort_stream = t ? side->s[t - 1] : (phase == 1 ? side->s[2] : stream);
+        cudaStream_t sort_stream = t ? side->s[t - 1] : (phase == BWD_SORTS ? side->s[2] : stream);
         if (sort_stream != stream) cudaStreamWaitEvent(sort_stream, side->fork, 0);
         const int n_rows = t == 2 ? p.region_num : p.item_num;
         int bits = 1;  // keys are 0 .. n_rows (n_rows = the "drop" key of an out-of-range id)
@@ -1066,10 +1062,10 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
         size_t cb = L.cub_bytes;
         cub::DeviceRadixSort::SortPairs(base + L.cub[t], cb, I(L.kin[t]), I(L.kout[t]), U(L.vin[t]), U(L.vout[t]), (int)n_of[t], 0, bits,
                                         sort_stream);
-        if (phase == 1 && t == 0) cudaEventRecord(side->sorted0, side->s[2]);
+        if (phase == BWD_SORTS && t == 0) cudaEventRecord(side->sorted0, side->s[2]);
       }
     }
-    if (phase == 4) {
+    if (phase == BWD_JOIN_SORTS) {
       for (int t = 0; t < 3; ++t) {
         if (!want[t]) continue;
         cudaEvent_t ev = t ? side->join[t - 1] : side->sorted0;
@@ -1077,7 +1073,7 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
         cudaStreamWaitEvent(stream, ev, 0);
       }
     }
-    if (phase == 1 || phase == 4) continue;
+    if (phase == BWD_SORTS || phase == BWD_JOIN_SORTS) continue;
     // ---- 2. the tile kernel ------------------------------------------------------------------------------------------------
     BwdArgs A;
     A.p = p;
@@ -1153,7 +1149,7 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
       }
       cudaEventRecord(side->pjoin, pstream);
     }
-    if (phase == 2 && want[0]) cudaStreamWaitEvent(stream, side->sorted0, 0);  // the long list was sorted on a side stream
+    if (phase == BWD_AFTER_SORTS && want[0]) cudaStreamWaitEvent(stream, side->sorted0, 0);  // the long list was sorted on a side stream
     if (want[0]) seg(0, 0, br.w_poi, p.item_num, dest(g.hist_poi[bi], br.hist_poi, opt ? opt->sum_hist_poi[bi] : nullptr, g.remap_hist_poi[bi]));
     if (want[1]) seg(1, 0, br.w_poi, p.item_num, dest(g.tgt_poi[bi], br.tgt_poi, opt ? opt->sum_tgt_poi[bi] : nullptr, g.remap_tgt_poi[bi]));
     // (history-side and target-side region rows are one table in every variant: hist_reg == tgt_reg)
@@ -1168,7 +1164,7 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
     if (e != cudaSuccess) return (int)e;
     if (dense_rc) return dense_rc;
   }
-  if (phase == 1 || phase == 4) {
+  if (phase == BWD_SORTS || phase == BWD_JOIN_SORTS) {
     cudaError_t e1 = cudaGetLastError();
     return e1 == cudaSuccess ? 0 : (int)e1;
   }

@@ -24,7 +24,7 @@ int choose_splits(int n_users, int64_t range);
 size_t pairs_bwd_workspace_bytes(const NaisParams& p, const NaisPairs& b);
 int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score_parts, const float* row_sum,
                      const unsigned long long* act_mask, const float* dscore, const NaisGrads& g, const NaisAdagrad* opt, void* ws,
-                     size_t ws_bytes, cudaStream_t stream, int phase = 0, const DenseAdagradLaunch* dense = nullptr);
+                     size_t ws_bytes, cudaStream_t stream, BwdPhase phase = BWD_ALL, const DenseAdagradLaunch* dense = nullptr);
 bool pairs_tc_bwd_supported(const NaisParams& p, const NaisPairs& b);
 size_t rows_adagrad_workspace_bytes(int64_t n, int w);
 int launch_rows_adagrad(const int32_t* keys, const float* rows, int64_t n, int w, int n_rows, float* grad_out, float* param, float* sum,
@@ -219,6 +219,21 @@ static bool device_is_sm100() {
   return device_info().major == 10;
 }
 
+// The pair forward for (p, b): the tcgen05 kernel where the shape has it on an sm_100 device, unless NAIS_PAIRS_FP32 asks for the
+// FP32 kernel; NAIS_PAIRS_TC forces tcgen05 and is NAIS_ERR_SHAPE where it is not available.
+static int choose_pairs_fwd(const NaisParams& p, const NaisPairs& b, bool* tc) {
+  const bool tc_ok = pairs_tc_supported(p, b) && device_is_sm100();
+  if (p.pairs_precision == NAIS_PAIRS_TC && !tc_ok) return NAIS_ERR_SHAPE;
+  *tc = p.pairs_precision != NAIS_PAIRS_FP32 && tc_ok;
+  return 0;
+}
+
+// tcgen05 contraction (fp16 two-term splits, fp32-grade products; writes act_mask when given) or the FP32 kernel
+static int launch_chosen_fwd(bool tc, const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts,
+                             unsigned long long* act_mask, cudaStream_t stream) {
+  return tc ? launch_pairs_fwd_tc(p, b, score, row_sum, parts, act_mask, stream) : launch_pairs_fwd(p, b, score, row_sum, parts, stream);
+}
+
 size_t nais_rows_adagrad_workspace_bytes(int64_t n, int32_t w) {
   if (n < 0 || w < 1 || w > 128) return 0;
   return rows_adagrad_workspace_bytes(n, w);
@@ -254,10 +269,11 @@ int nais_pairs_dispatch(const NaisParams* p, const NaisPairs* batch, int32_t* fw
   if (batch->B < 0 || (!batch->seg_offsets && batch->H < 1)) return NAIS_ERR_SHAPE;
   NaisPairs b = *batch;
   if (b.B == 0) b.B = 1;  // the choice does not depend on the row count
-  const bool f_ok = pairs_tc_supported(*p, b) && device_is_sm100(), b_ok = pairs_tc_bwd_supported(*p, b);
-  if (p->pairs_precision == NAIS_PAIRS_TC && !f_ok) return NAIS_ERR_SHAPE;  // (a forced tcgen05 backward reports its own shape error)
-  *fwd_tc = (p->pairs_precision != NAIS_PAIRS_FP32 && f_ok) ? 1 : 0;
-  *bwd_tc = (p->pairs_precision != NAIS_PAIRS_FP32 && b_ok) ? 1 : 0;
+  bool f_tc = false;
+  rc = choose_pairs_fwd(*p, b, &f_tc);  // (a forced tcgen05 backward reports its own shape error)
+  if (rc) return rc;
+  *fwd_tc = f_tc ? 1 : 0;
+  *bwd_tc = (p->pairs_precision != NAIS_PAIRS_FP32 && pairs_tc_bwd_supported(*p, b)) ? 1 : 0;
   return 0;
 }
 
@@ -269,12 +285,11 @@ int nais_pairs_forward(const NaisParams* p, const NaisPairs* batch, float* score
   if (rc) return rc;
   if (batch->B && !score) return NAIS_ERR_NULL;
   if (batch->B == 0) return 0;
-  const bool tc_ok = pairs_tc_supported(*p, *batch) && device_is_sm100();
-  if (p->pairs_precision == NAIS_PAIRS_TC && !tc_ok) return NAIS_ERR_SHAPE;
-  if (p->pairs_precision != NAIS_PAIRS_FP32 && tc_ok)  // tcgen05 contraction (fp16 two-term splits): fp32-grade products
-    return launch_pairs_fwd_tc(*p, *batch, score, row_sum, score_parts, reinterpret_cast<unsigned long long*>(act_mask),
-                               static_cast<cudaStream_t>(stream));
-  return launch_pairs_fwd(*p, *batch, score, row_sum, score_parts, static_cast<cudaStream_t>(stream));
+  bool tc = false;
+  rc = choose_pairs_fwd(*p, *batch, &tc);
+  if (rc) return rc;
+  return launch_chosen_fwd(tc, *p, *batch, score, row_sum, score_parts, reinterpret_cast<unsigned long long*>(act_mask),
+                           static_cast<cudaStream_t>(stream));
 }
 
 size_t nais_pairs_backward_workspace_bytes(const NaisParams* p, const NaisPairs* batch) {
@@ -314,17 +329,16 @@ int nais_pairs_forward_presort(const NaisParams* p, const NaisPairs* batch, cons
   if (!bwd_workspace) return NAIS_ERR_NULL;
   if (!aligned16(bwd_workspace)) return NAIS_ERR_ALIGN;
   if (bwd_workspace_bytes < pairs_bwd_workspace_bytes(*p, *batch)) return NAIS_ERR_WORKSPACE;
-  const bool tc_ok = pairs_tc_supported(*p, *batch) && device_is_sm100();
-  if (p->pairs_precision == NAIS_PAIRS_TC && !tc_ok) return NAIS_ERR_SHAPE;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, *grads, nullptr, bwd_workspace, bwd_workspace_bytes, st, 1);
+  bool tc = false;
+  rc = choose_pairs_fwd(*p, *batch, &tc);
   if (rc) return rc;
-  if (p->pairs_precision != NAIS_PAIRS_FP32 && tc_ok)
-    rc = launch_pairs_fwd_tc(*p, *batch, score, row_sum, score_parts, reinterpret_cast<unsigned long long*>(act_mask), st);
-  else
-    rc = launch_pairs_fwd(*p, *batch, score, row_sum, score_parts, st);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  rc = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, *grads, nullptr, bwd_workspace, bwd_workspace_bytes, st, BWD_SORTS);
+  if (rc) return rc;
+  rc = launch_chosen_fwd(tc, *p, *batch, score, row_sum, score_parts, reinterpret_cast<unsigned long long*>(act_mask), st);
   // (also after a failed forward launch: the caller may release the workspace as soon as this returns)
-  const int rj = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, *grads, nullptr, bwd_workspace, bwd_workspace_bytes, st, 4);
+  const int rj = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, *grads, nullptr, bwd_workspace, bwd_workspace_bytes, st,
+                                  BWD_JOIN_SORTS);
   return rc ? rc : rj;
 }
 
@@ -342,7 +356,7 @@ int nais_pairs_backward_presorted(const NaisParams* p, const NaisPairs* batch, c
   if (!aligned16(workspace)) return NAIS_ERR_ALIGN;
   if (workspace_bytes < pairs_bwd_workspace_bytes(*p, *batch)) return NAIS_ERR_WORKSPACE;
   return launch_pairs_bwd(*p, *batch, score_parts, row_sum, reinterpret_cast<const unsigned long long*>(act_mask), dscore, *grads,
-                          nullptr, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), 3);
+                          nullptr, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), BWD_AFTER_JOIN);
 }
 
 int nais_pairs_backward_adagrad(const NaisParams* p, const NaisPairs* batch, const float* score_parts, const float* row_sum,
@@ -353,7 +367,7 @@ int nais_pairs_backward_adagrad(const NaisParams* p, const NaisPairs* batch, con
   rc = check_pairs(p, batch);
   if (rc) return rc;
   if (!grads || !opt) return NAIS_ERR_NULL;
-  if (p->n_branch != 1 && !pairs_disentangled(*p)) return NAIS_ERR_MODE;
+  if (!pairs_fused_layout(*p)) return NAIS_ERR_MODE;
   if (!(opt->lr >= 0.f) || !(opt->eps >= 0.f)) return NAIS_ERR_MODE;
   if (batch->B == 0) return 0;
   if (!score_parts || !row_sum || !dscore || !workspace) return NAIS_ERR_NULL;
@@ -398,14 +412,14 @@ TrainStepLayout train_step_layout(const NaisParams& p, const NaisPairs& b) {
 
 size_t nais_pairs_train_step_workspace_bytes(const NaisParams* p, const NaisPairs* batch) {
   if (check_params(p) || !batch || batch->B < 0 || (!batch->seg_offsets && batch->H < 1)) return 0;
-  if (p->n_branch != 1 && !pairs_disentangled(*p)) return 0;
+  if (!pairs_fused_layout(*p)) return 0;
   return train_step_layout(*p, *batch).total;
 }
 
 static int check_train_state(const NaisParams* p, const NaisAdagrad* tables, const NaisDenseAdagrad* dense) {
   if (!tables || !dense) return NAIS_ERR_NULL;
+  if (!pairs_fused_layout(*p)) return NAIS_ERR_MODE;
   const bool two = pairs_disentangled(*p);
-  if (p->n_branch != 1 && !two) return NAIS_ERR_MODE;
   if (p->n_branch == 1 && p->dist_mode == NAIS_DIST_KM) return NAIS_ERR_MODE;
   if (!(tables->lr >= 0.f) || !(tables->eps >= 0.f) || !(dense->lr >= 0.f) || !(dense->eps >= 0.f)) return NAIS_ERR_MODE;
   if (!dense->sum_w1 || !dense->sum_b1 || !dense->sum_w2) return NAIS_ERR_NULL;
@@ -415,10 +429,15 @@ static int check_train_state(const NaisParams* p, const NaisAdagrad* tables, con
   return 0;
 }
 
+// What one train_step_impl call enqueues: the whole step; only the id sorts of its backward (on the side streams, joined to `st`:
+// nais_train_users runs them for the NEXT user on its preparation stream); or the step on lists sorted by a STEP_SORTS call (same
+// arguments).
+enum StepPart { STEP_ALL = 0, STEP_SORTS = 1, STEP_AFTER_SORTS = 2 };
+
 // the launches of one optimizer step (arguments already checked)
 static int train_step_impl(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
                            const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace,
-                           size_t workspace_bytes, cudaStream_t st, int part = 0);
+                           size_t workspace_bytes, cudaStream_t st, StepPart part = STEP_ALL);
 
 int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
                           const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace,
@@ -437,11 +456,9 @@ int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, const flo
                          static_cast<cudaStream_t>(stream));
 }
 
-// part 0: the whole step.  part 1: only the id sorts of its backward (on the side streams, joined to `st`: nais_train_users runs
-// them for the NEXT user on its preparation stream); part 2: the step on lists sorted by a part-1 call (same arguments).
 static int train_step_impl(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
                            const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace,
-                           size_t workspace_bytes, cudaStream_t st, int part) {
+                           size_t workspace_bytes, cudaStream_t st, StepPart part) {
   int rc;
   const TrainStepLayout L = train_step_layout(*p, *batch);
   if (workspace_bytes < L.total) return NAIS_ERR_WORKSPACE;
@@ -461,18 +478,19 @@ static int train_step_impl(const NaisParams* p, const NaisPairs* batch, const fl
   }
   if (p->dist_mode == NAIS_DIST_KM) g.dist_embed = F(L.gde);
   // the id sorts of the backward depend on the batch only: forked onto side streams now, they run next to the forward
-  if (part != 2) {
-    rc = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, g, tables, base + L.bwd, workspace_bytes - L.bwd, st, 1);
+  if (part != STEP_AFTER_SORTS) {
+    rc = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, g, tables, base + L.bwd, workspace_bytes - L.bwd, st, BWD_SORTS);
     if (rc) return rc;
   }
-  if (part == 1) return launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, g, tables, base + L.bwd, workspace_bytes - L.bwd, st, 4);
+  if (part == STEP_SORTS)
+    return launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, g, tables, base + L.bwd, workspace_bytes - L.bwd, st,
+                            BWD_JOIN_SORTS);
   // forward
-  const bool tc_ok = pairs_tc_supported(*p, *batch) && device_is_sm100();
-  if (p->pairs_precision == NAIS_PAIRS_TC && !tc_ok) return NAIS_ERR_SHAPE;
-  const bool fwd_tc = p->pairs_precision != NAIS_PAIRS_FP32 && tc_ok;
+  bool fwd_tc = false;
+  rc = choose_pairs_fwd(*p, *batch, &fwd_tc);
+  if (rc) return rc;
   unsigned long long* mask = (fwd_tc && p->hid <= 64) ? reinterpret_cast<unsigned long long*>(base + L.mask) : nullptr;
-  rc = fwd_tc ? launch_pairs_fwd_tc(*p, *batch, F(L.score), F(L.row_sum), F(L.parts), mask, st)
-              : launch_pairs_fwd(*p, *batch, F(L.score), F(L.row_sum), F(L.parts), st);
+  rc = launch_chosen_fwd(fwd_tc, *p, *batch, F(L.score), F(L.row_sum), F(L.parts), mask, st);
   if (rc) return rc;
   if (score_out) {
     cudaError_t e = cudaMemcpyAsync(score_out, F(L.score), (size_t)batch->B * 4, cudaMemcpyDeviceToDevice, st);
@@ -503,7 +521,7 @@ static int train_step_impl(const NaisParams* p, const NaisPairs* batch, const fl
              dense->lr, dense->eps};
   }
   return launch_pairs_bwd(*p, *batch, F(L.parts), F(L.row_sum), mask, F(L.dscore), g, tables, base + L.bwd, workspace_bytes - L.bwd, st,
-                          part == 2 ? 3 : 2, da);
+                          part == STEP_AFTER_SORTS ? BWD_AFTER_JOIN : BWD_AFTER_SORTS, da);
 }
 
 // ---- nais_train_users: the reference's one-user-per-step schedule, a list of users per call ---------------------------------------
@@ -571,7 +589,7 @@ cudaStream_t prep_stream() {
 }  // namespace
 
 size_t nais_train_users_workspace_bytes(const NaisParams* p, int32_t max_hist, int32_t num_ng) {
-  if (check_params(p) || (p->n_branch != 1 && !pairs_disentangled(*p)) || max_hist < 1 || num_ng < 0) return 0;
+  if (check_params(p) || !pairs_fused_layout(*p) || max_hist < 1 || num_ng < 0) return 0;
   return 2 * users_layout(*p, max_hist, num_ng).total;  // two users in flight: one being prepared, one being stepped
 }
 
@@ -688,7 +706,7 @@ int nais_train_users_centred(const NaisParams* p, const int64_t* host_indptr, in
                                 reinterpret_cast<float*>(base + L.label), need_reg ? const_cast<int64_t*>(ub.b.treg) : nullptr,
                                 need_co ? const_cast<float*>(ub.b.tgt_coords) : nullptr, ps);
     if (r) return r;
-    return train_step_impl(p, &ub.b, ub.label, nullptr, tables, dense, nullptr, nullptr, ub.step, L.total - L.step, ps, 1);
+    return train_step_impl(p, &ub.b, ub.label, nullptr, tables, dense, nullptr, nullptr, ub.step, L.total - L.step, ps, STEP_SORTS);
   };
   // users with a history, in order; the others only get a zero loss
   int next = 0;
@@ -724,7 +742,7 @@ int nais_train_users_centred(const NaisParams* p, const int64_t* host_indptr, in
     UserBatch ub;
     buffers(cur, cur_slot, ub);
     cudaStreamWaitEvent(st, prepared[cur_slot], 0);
-    rc = train_step_impl(p, &ub.b, ub.label, nullptr, tables, dense, losses + cur, nullptr, ub.step, L.total - L.step, st, 2);
+    rc = train_step_impl(p, &ub.b, ub.label, nullptr, tables, dense, losses + cur, nullptr, ub.step, L.total - L.step, st, STEP_AFTER_SORTS);
     if (rc) return bail(rc);
     cudaEventRecord(stepped[cur_slot], st);
     ++done;

@@ -62,6 +62,16 @@ struct DenseAdagradLaunch {
   float lr, eps;
 };
 
+// What one launch_pairs_bwd call enqueues (nais_bwd.cu).  The id sorts depend on the batch only, so a caller may fork them ahead:
+enum BwdPhase : int {
+  BWD_ALL = 0,         // the whole backward
+  BWD_SORTS = 1,       // only the id sorts, ALL of them on side streams (the one-call training step forks them before its forward)
+  BWD_AFTER_SORTS = 2, // the rest, on lists sorted by a BWD_SORTS call (same p, b, g, opt, ws)
+  BWD_AFTER_JOIN = 3,  // BWD_AFTER_SORTS after a BWD_JOIN_SORTS (no wait of its own for the long list)
+  BWD_JOIN_SORTS = 4,  // join the sort streams of a BWD_SORTS call to `stream` (so that nothing enqueued on `stream` later — or
+                       // the caller's allocator — can overtake the sorts)
+};
+
 // Device address (current device) of the library's 4-byte bad-index word (nais_capi.cu); every launcher passes it to its kernel.
 int* bad_index_flag();
 // An id as the kernels use it: inside [0, n) or replaced by 0 with the bad-index word set (include/nais_b200.h,

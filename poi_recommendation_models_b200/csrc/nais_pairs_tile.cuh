@@ -35,6 +35,8 @@ struct PairTile {
 __host__ __device__ inline bool pairs_disentangled(const NaisParams& p) {
   return p.n_branch == 2 && p.branch[0].w_reg == 0 && p.branch[1].w_poi == 0 && p.dist_mode != NAIS_DIST_LATLON;
 }
+// The layouts the split backward phases and the fused optimizer take: one branch, or the disentangled two.
+inline bool pairs_fused_layout(const NaisParams& p) { return p.n_branch == 1 || pairs_disentangled(p); }
 __host__ __device__ inline bool pairs_segmented(const NaisPairs& b) { return b.seg_offsets != nullptr; }
 __host__ __device__ inline int64_t pairs_n_cells(const NaisPairs& b) { return pairs_segmented(b) ? b.n_cells : b.B * (int64_t)b.H; }
 __host__ __device__ inline int64_t pairs_n_tiles(const NaisPairs& b) {

@@ -177,7 +177,7 @@ class _NAISBase(nn.Module):
         (lr_t, eps_t), (lr_d, eps_d) = next(iter(tg)), next(iter(dg))
         sums = {n: optimizer.state[t]["sum"] for n, t in P.items()}
         optimizer.zero_grad(set_to_none=True)
-        has_reg, has_co = "embed_region.weight" in P, "dist_layer.weight" in P or self.variant == "disentangled"
+        has_reg, has_co = "embed_region.weight" in P, ops.VARIANT_DIST[self.variant][0] != ops.DIST_NONE
         losses = ops.train_users(self.variant, float(self.beta), P, sums, sums, lr_t, eps_t, lr_d, eps_d, batcher.indptr, batcher.indices,
                                  batcher.entry_region if has_reg else None, batcher.entry_coords if has_co else None,
                                  batcher.region32 if has_reg else None, batcher.coords32 if has_co else None, uids, negative_num, seed,

@@ -12,24 +12,43 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import torch
 
 from . import _lib
-from ._lib import (DIST_KM, DIST_LATLON, DIST_NONE, PAIRS_PRECISIONS, PRECISIONS, NaisBranch, NaisCatalog, NaisGrads,
-                   NaisPairs, NaisParams, NaisUsers)
+from ._lib import (DIST_KM, DIST_LATLON, DIST_NONE, PAIRS_PRECISIONS, PRECISIONS, NaisAdagrad, NaisBranch, NaisCatalog,
+                   NaisDenseAdagrad, NaisGrads, NaisPairs, NaisParams, NaisUsers)
 
-# parameter names per variant, in the reference's state_dict naming (SURVEY.md §5 checkpoint row)
-VARIANT_PARAMS: Dict[str, Tuple[str, ...]] = {
-    "basic": ("embed_history.weight", "embed_target.weight", "attn_layer1.weight", "attn_layer1.bias", "attn_layer2.weight"),
-    "region": ("embed_history.weight", "embed_target.weight", "embed_region.weight", "attn_layer1.weight",
-               "attn_layer1.bias", "attn_layer2.weight"),
+# Every parameter of a variant as (name, role, branch), in the reference's state_dict order (SURVEY.md §5 checkpoint row): autograd
+# returns the gradients by this position.  The role names the slot of the C structs (include/nais_b200.h) on that branch:
+#   "hist_poi" / "tgt_poi"  embedding table: NaisBranch.<role>, NaisGrads.<role>[branch], NaisAdagrad.sum_<role>[branch]
+#   "reg"                   region table: NaisBranch.hist_reg and .tgt_reg, NaisGrads.reg[branch], NaisAdagrad.sum_reg[branch]
+#   "w1" / "b1" / "w2"      attention MLP: NaisBranch.<role>, NaisGrads.<role>[branch], NaisDenseAdagrad.sum_<role> (branch 0)
+#                           or sum_region_<role> (branch 1)
+#   "dist_w" / "dist_b" / "dist_embed"  distance term, one for both branches: NaisParams / NaisGrads.<role>,
+#                           NaisDenseAdagrad.sum_<role>
+_HIST, _TGT = ("embed_history.weight", "hist_poi", 0), ("embed_target.weight", "tgt_poi", 0)
+_MLP = (("attn_layer1.weight", "w1", 0), ("attn_layer1.bias", "b1", 0), ("attn_layer2.weight", "w2", 0))
+_DIST_LAYER = (("dist_layer.weight", "dist_w", 0), ("dist_layer.bias", "dist_b", 0))
+VARIANT_SLOTS: Dict[str, Tuple[Tuple[str, str, int], ...]] = {
+    "basic": (_HIST, _TGT) + _MLP,
+    "region": (_HIST, _TGT, ("embed_region.weight", "reg", 0)) + _MLP,
     # embed_distance.weight exists in this class but is never read by its forward (model.py:204,270-276)
-    "region_distance": ("embed_history.weight", "embed_target.weight", "embed_region.weight",
-                        "attn_layer1.weight", "attn_layer1.bias", "attn_layer2.weight", "dist_layer.weight",
-                        "dist_layer.bias"),
-    "distance": ("embed_history.weight", "embed_target.weight", "attn_layer1.weight", "attn_layer1.bias",
-                 "attn_layer2.weight", "dist_layer.weight", "dist_layer.bias"),
-    "disentangled": ("embed_history.weight", "embed_target.weight", "embed_region.weight", "embed_distance.weight",
-                     "attn_layer1.weight", "attn_layer1.bias", "attn_layer2.weight", "region_attn_layer1.weight",
-                     "region_attn_layer1.bias", "region_attn_layer2.weight"),
+    "region_distance": (_HIST, _TGT, ("embed_region.weight", "reg", 0)) + _MLP + _DIST_LAYER,
+    "distance": (_HIST, _TGT) + _MLP + _DIST_LAYER,
+    # branch 1 scores the region table with its own MLP; the reference only ever reads row 0 of embed_distance (model.py:497-498)
+    "disentangled": (_HIST, _TGT, ("embed_region.weight", "reg", 1), ("embed_distance.weight", "dist_embed", 0)) + _MLP
+                    + (("region_attn_layer1.weight", "w1", 1), ("region_attn_layer1.bias", "b1", 1), ("region_attn_layer2.weight", "w2", 1)),
 }
+_TABLE_ROLES = frozenset(("hist_poi", "tgt_poi", "reg"))
+_SHARED_ROLES = frozenset(("dist_w", "dist_b", "dist_embed"))
+VARIANT_PARAMS: Dict[str, Tuple[str, ...]] = {v: tuple(n for n, _, _ in s) for v, s in VARIANT_SLOTS.items()}
+_TABLES = tuple(dict.fromkeys(n for s in VARIANT_SLOTS.values() for n, role, _ in s if role in _TABLE_ROLES))
+# gradients param_reduce_kernel writes in full (csrc/nais_bwd.cu): no zero fill needed; every other tensor has rows / entries the
+# backward does not touch (untouched table rows, the rows of embed_distance past row 0)
+_FULLY_WRITTEN = {n for s in VARIANT_SLOTS.values() for n, role, _ in s if role in ("w1", "b1", "w2", "dist_w", "dist_b")}
+_N_BRANCH = {v: 1 + max(bi for _, _, bi in s) for v, s in VARIANT_SLOTS.items()}
+# the optimizer-state field of each parameter: (name, NaisAdagrad field, branch) of the tables, (name, NaisDenseAdagrad field, None)
+# of the rest
+_ADAGRAD_FIELDS = {(v, tables): tuple((n, "sum_" + role, bi) if tables else (n, ("sum_region_" if bi else "sum_") + role, None)
+                                      for n, role, bi in s if (role in _TABLE_ROLES) == tables)
+                   for v, s in VARIANT_SLOTS.items() for tables in (True, False)}
 VARIANT_DIST = {"basic": (DIST_NONE, 0.0), "region": (DIST_NONE, 0.0), "region_distance": (DIST_LATLON, 100.0),
                 "distance": (DIST_LATLON, 1000.0), "disentangled": (DIST_KM, 0.0)}
 
@@ -93,6 +112,11 @@ def _poll_bad_index(dev: torch.device) -> None:
     if st["calls"] % _POLL_EVERY != 1 and _POLL_EVERY > 1:
         return
     check_indices(dev, sync=len(st["inflight"]) >= _POLL_SLOTS - 1)
+    _enqueue_poll(st)
+
+
+def _enqueue_poll(st: dict) -> None:
+    """nais_poll_bad_index into the next pinned slot on the current stream, and an event that tells when the slot is valid."""
     slot = st["next"]
     st["next"] = (slot + 1) % _POLL_SLOTS
     _lib.check(_lib.load().nais_poll_bad_index(st["buf"].data_ptr() + 4 * slot, _stream()), "nais_poll_bad_index")
@@ -114,12 +138,7 @@ def check_indices(dev=None, sync: bool = False) -> None:
             st = _poll_state(torch.device("cuda", d))
         if sync and not torch.cuda.is_current_stream_capturing():
             with torch.cuda.device(d):
-                slot = st["next"]
-                st["next"] = (slot + 1) % _POLL_SLOTS
-                _lib.check(_lib.load().nais_poll_bad_index(st["buf"].data_ptr() + 4 * slot, _stream()), "nais_poll_bad_index")
-                ev = torch.cuda.Event()
-                ev.record()
-                st["inflight"].append((slot, ev))
+                _enqueue_poll(st)
         q = st["inflight"]
         while q and (sync or q[0][1].query()):
             slot, ev = q.pop(0)
@@ -135,43 +154,70 @@ def build_params(variant: str, P: Dict[str, torch.Tensor], beta: float, keep: Li
                  dropout_p: float = 0.0, dropout_seed: int = 0, pairs_precision: str = "auto") -> NaisParams:
     """NaisParams for a reference-shaped parameter dict.  Contiguous copies are appended to `keep` to stay alive.
     `pairs_precision`: "auto" (tcgen05 pair kernels where the shape has them), "fp32", "tc" (NAIS_PAIRS_*)."""
-    def g(name):
-        t = _f32(P[name].detach())
-        keep.append(t)
-        return t
-
     p = NaisParams()
     mode, scale = VARIANT_DIST[variant]
-    eh, et = g("embed_history.weight"), g("embed_target.weight")
-    w1, b1, w2 = g("attn_layer1.weight"), g("attn_layer1.bias"), g("attn_layer2.weight")
-    p.item_num = eh.shape[0]
-    p.hid = w1.shape[0]
     p.dist_mode, p.dist_scale, p.beta = mode, scale, float(beta)
-    p.dist_buckets, p.dist_bucket_km, p.region_num, p.n_branch = 1, 1.0, 0, 1
+    p.dist_buckets, p.dist_bucket_km, p.region_num, p.n_branch = 1, 1.0, 0, _N_BRANCH[variant]
     p.dropout_p, p.dropout_seed = float(dropout_p), int(dropout_seed)
     p.pairs_precision = PAIRS_PRECISIONS[pairs_precision]
     b0 = p.branch[0]
-    b0.hist_poi, b0.tgt_poi, b0.w_poi, b0.w_reg = eh.data_ptr(), et.data_ptr(), eh.shape[1], 0
-    b0.w1, b0.b1, b0.w2 = w1.data_ptr(), b1.data_ptr(), w2.data_ptr()
-    if variant in ("region", "region_distance"):
-        er = g("embed_region.weight")
-        b0.hist_reg = b0.tgt_reg = er.data_ptr()
-        b0.w_reg, p.region_num = er.shape[1], er.shape[0]
-    if mode == DIST_LATLON:
-        p.dist_w, p.dist_b = g("dist_layer.weight").data_ptr(), g("dist_layer.bias").data_ptr()
-    if variant == "disentangled":
-        er, ed = g("embed_region.weight"), g("embed_distance.weight")
-        rw1, rb1, rw2 = g("region_attn_layer1.weight"), g("region_attn_layer1.bias"), g("region_attn_layer2.weight")
-        p.n_branch, p.region_num = 2, er.shape[0]
-        b1_ = p.branch[1]
-        b1_.hist_reg = b1_.tgt_reg = er.data_ptr()
-        b1_.w_poi, b1_.w_reg = 0, er.shape[1]
-        b1_.w1, b1_.b1, b1_.w2 = rw1.data_ptr(), rb1.data_ptr(), rw2.data_ptr()
-        p.dist_embed, p.dist_buckets = ed.data_ptr(), 1  # the reference only ever reads bucket 0 (model.py:497-498)
+    b0_tensors = {}
+    for name, role, bi in VARIANT_SLOTS[variant]:
+        t = _f32(P[name].detach())
+        keep.append(t)
+        if role in _SHARED_ROLES:
+            setattr(p, role, t.data_ptr())
+            continue
+        br = p.branch[1] if bi else b0
+        if role == "reg":
+            br.hist_reg = br.tgt_reg = t.data_ptr()
+            br.w_reg, p.region_num = t.shape[1], t.shape[0]
+        else:
+            setattr(br, role, t.data_ptr())
+        if bi == 0:
+            b0_tensors[role] = t
+    eh, w1, b1, w2 = b0_tensors["hist_poi"], b0_tensors["w1"], b0_tensors["b1"], b0_tensors["w2"]
+    p.item_num, p.hid = eh.shape[0], w1.shape[0]
+    b0.w_poi = eh.shape[1]
     w_in = b0.w_poi + b0.w_reg + (2 if mode == DIST_LATLON else 0)
     if w1.shape[1] != w_in or b1.numel() != p.hid or w2.numel() != p.hid:
         raise RuntimeError(f"attn_layer shapes do not match the variant: w1 {tuple(w1.shape)}, expected [*, {w_in}]")
     return p
+
+
+def _grads_struct(variant: str, grads: Dict[str, int], remaps: Optional[Dict[str, int]] = None) -> NaisGrads:
+    """NaisGrads with the slot of every parameter in `grads` (name -> device address of its gradient) set; every other slot stays
+    NULL, so the backward skips it.  A table in `remaps` (name -> address of its int32 remap) gets row-compacted gradients:
+    its `grads` entry is then the address of the touched rows (NaisGrads::remap_*)."""
+    g = NaisGrads()
+    for name, role, bi in VARIANT_SLOTS[variant]:
+        ptr = grads.get(name)
+        if ptr is None:
+            continue
+        if role in _SHARED_ROLES:
+            setattr(g, role, ptr)
+        else:
+            getattr(g, role)[bi] = ptr
+        if remaps and name in remaps:
+            getattr(g, "remap_" + role)[bi] = remaps[name]
+    return g
+
+
+def _adagrad_struct(variant: str, P: Dict[str, torch.Tensor], sums: Dict[str, torch.Tensor], lr: float, eps: float, tables: bool):
+    """NaisAdagrad of the embedding tables (`tables`) or NaisDenseAdagrad of the other parameters, from the optimizer's
+    `state['sum']` of each (`sums`: name -> tensor).  (embed_distance: the kernels read and step row 0 only, so the state's
+    row 0 — the start of the tensor — is what they get.)"""
+    s = NaisAdagrad() if tables else NaisDenseAdagrad()
+    s.lr, s.eps = float(lr), float(eps)
+    for name, field, bi in _ADAGRAD_FIELDS[variant, tables]:
+        st = sums[name]
+        if st.dtype != torch.float32 or not st.is_contiguous() or st.shape != P[name].shape or not P[name].is_contiguous():
+            raise RuntimeError(f"fused Adagrad: {name} and its state must be contiguous float32 of the same shape")
+        if bi is None:
+            setattr(s, field, st.data_ptr())
+        else:
+            getattr(s, field)[bi] = st.data_ptr()
+    return s
 
 
 @dataclass
@@ -313,21 +359,56 @@ def pairs_dispatch(p: NaisParams, b: NaisPairs) -> Tuple[bool, bool]:
 PRESORT_IN_FORWARD = True
 
 
-def _table_grads_skeleton(variant: str, ptr: int) -> NaisGrads:
-    """The NaisGrads of a dense-table backward with every wanted table pointer set to `ptr` — what nais_pairs_forward_presort
-    reads (NULL-ness only) to know which id lists the backward of `pairs_backward_raw(tables=True)` will reduce."""
-    g = NaisGrads()
-    g.hist_poi[0] = g.tgt_poi[0] = ptr
-    if variant in ("region", "region_distance"):
-        g.reg[0] = ptr
-    return g
+class _PairCall:
+    """What every pair entry point of the library does around its call: the device guard, the NaisParams (and the NaisPairs of
+    `batch` = (hist, tgt, hreg, treg, aux)) with their contiguous copies kept alive, the workspace, the return-code check and,
+    once the call is enqueued, the bad-index poll.  `with _PairCall(...) as c: c.launch(entry, ...)`."""
+
+    def __init__(self, dev: torch.device, variant: str, beta: float, P: Dict[str, torch.Tensor], precision: str, drop=(0.0, 0),
+                 batch=None):
+        self.dev, self.variant, self.lib, self.keep = dev, variant, _lib.load(), []
+        self._guard = torch.cuda.device(dev)
+        self._args = (beta, P, drop, precision, batch)
+
+    def __enter__(self) -> "_PairCall":
+        beta, P, drop, precision, batch = self._args
+        self._guard.__enter__()
+        try:
+            self.p = build_params(self.variant, P, beta, self.keep, drop[0], drop[1], precision)
+            self.b = None if batch is None else _pairs_struct(*batch, self.keep)
+        except BaseException:
+            self._guard.__exit__(None, None, None)
+            raise
+        self.structs = (C.byref(self.p),) if self.b is None else (C.byref(self.p), C.byref(self.b))
+        return self
+
+    def __exit__(self, exc_type, exc, tb) -> None:
+        try:
+            if exc_type is None:
+                _poll_bad_index(self.dev)
+        finally:
+            self._guard.__exit__(exc_type, exc, tb)
+
+    def query(self, entry: str, *args) -> int:
+        """lib.<entry>(p[, b], *args): a workspace size."""
+        return getattr(self.lib, entry)(*self.structs, *args)
+
+    def launch(self, entry: str, *args, ws_bytes: Optional[int] = None, ws: Optional[torch.Tensor] = None, tail=()):
+        """lib.<entry>(p[, b], *args[, workspace, ws_bytes], *tail, stream), raising on a non-zero return code.  A workspace of
+        `ws_bytes` is allocated unless `ws` is given; returns it."""
+        if ws_bytes is not None:
+            ws = torch.empty(max(ws_bytes, 16), device=self.dev, dtype=torch.uint8) if ws is None else ws
+            args += (ws.data_ptr(), ws_bytes)
+        _lib.check(getattr(self.lib, entry)(*self.structs, *args, *tail, _stream()), entry)
+        return ws
 
 
-def _forward_launch(lib, p: NaisParams, b: NaisPairs, dev, want_mask: bool = True, presort_variant: Optional[str] = None):
+def _forward_launch(c: _PairCall, want_mask: bool = True, presort: bool = False):
     """nais_pairs_forward -> (score, row_sum, parts, act_mask, presorted workspace): act_mask is the ReLU pattern the tcgen05
-    forward saves for the tcgen05 backward (int64 [B*H]; None when the FP32 forward runs or hid > 64).  With `presort_variant`
+    forward saves for the tcgen05 backward (int64 [B*H]; None when the FP32 forward runs or hid > 64).  With `presort`
     (one-branch variants) the call is nais_pairs_forward_presort and the last element is the backward workspace holding the
     sorted id lists for nais_pairs_backward_presorted; else None."""
+    p, b, dev = c.p, c.b, c.dev
     B = b.B
     score = torch.empty(B, device=dev, dtype=torch.float32)
     row_sum = torch.empty(p.n_branch, B, device=dev, dtype=torch.float32)
@@ -335,29 +416,29 @@ def _forward_launch(lib, p: NaisParams, b: NaisPairs, dev, want_mask: bool = Tru
     mask = None
     if want_mask and B and p.n_branch == 1 and p.hid <= 64 and pairs_dispatch(p, b)[0]:
         mask = torch.empty(b.n_cells if b.seg_offsets else B * b.H, device=dev, dtype=torch.int64)
+    outs = (score.data_ptr(), row_sum.data_ptr(), parts.data_ptr(), _ptr(mask))
     # (the backward tiles exist for D, hid <= 128: a wider forward-only shape keeps the plain call)
-    if presort_variant is not None and B and p.n_branch == 1 and p.hid <= 128 and p.branch[0].w_poi + p.branch[0].w_reg <= 128:
-        ws_bytes = lib.nais_pairs_backward_workspace_bytes(C.byref(p), C.byref(b))
+    if presort and B and p.n_branch == 1 and p.hid <= 128 and p.branch[0].w_poi + p.branch[0].w_reg <= 128:
+        ws_bytes = c.query("nais_pairs_backward_workspace_bytes")
         ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)
-        g = _table_grads_skeleton(presort_variant, ws.data_ptr())
-        _lib.check(lib.nais_pairs_forward_presort(C.byref(p), C.byref(b), C.byref(g), score.data_ptr(), row_sum.data_ptr(),
-                                                  parts.data_ptr(), _ptr(mask), ws.data_ptr(), ws_bytes, _stream()),
-                   "nais_pairs_forward_presort")
+        # (the forward reads only which table slots are set: they tell it which id lists the coming backward reduces)
+        g = _grads_struct(c.variant, {n: ws.data_ptr() for n in VARIANT_PARAMS[c.variant] if n in _TABLES})
+        c.launch("nais_pairs_forward_presort", C.byref(g), *outs, ws_bytes=ws_bytes, ws=ws)
         return score, row_sum, parts, mask, ws
-    _lib.check(lib.nais_pairs_forward(C.byref(p), C.byref(b), score.data_ptr(), row_sum.data_ptr(), parts.data_ptr(), _ptr(mask),
-                                      _stream()), "nais_pairs_forward")
+    c.launch("nais_pairs_forward", *outs)
     return score, row_sum, parts, mask, None
 
 
-# gradients param_reduce_kernel writes in full (csrc/nais_bwd.cu): no zero fill needed; every other tensor has rows / entries the
-# backward does not touch (untouched table rows, embed_distance of the one-branch variants)
-_FULLY_WRITTEN = {"attn_layer1.weight", "attn_layer1.bias", "attn_layer2.weight", "dist_layer.weight", "dist_layer.bias",
-                  "region_attn_layer1.weight", "region_attn_layer1.bias", "region_attn_layer2.weight"}
+def _grad_buffers(P: Dict[str, torch.Tensor], n_rows: int, tables: bool) -> Dict[str, torch.Tensor]:
+    """The dense float32 gradient of every parameter (`tables=False`: but the embedding tables) for a batch of `n_rows` rows."""
+    def buf(name, t):
+        mk = torch.empty_like if (name in _FULLY_WRITTEN and n_rows > 0) else torch.zeros_like  # (an empty batch launches nothing)
+        return mk(t, dtype=torch.float32, memory_format=torch.contiguous_format)
+    return {n: buf(n, t) for n, t in P.items() if tables or n not in _TABLES}
 
 
-def _grad_buffer(name: str, t: torch.Tensor, n_rows: int = 1) -> torch.Tensor:
-    mk = torch.empty_like if (name in _FULLY_WRITTEN and n_rows > 0) else torch.zeros_like  # (an empty batch launches nothing)
-    return mk(t, dtype=torch.float32, memory_format=torch.contiguous_format)
+def _addresses(G: Dict[str, torch.Tensor]) -> Dict[str, int]:
+    return {n: t.data_ptr() for n, t in G.items()}
 
 
 def _fwd_bwd(pairs_precision):
@@ -373,17 +454,11 @@ class _PairsFunction(torch.autograd.Function):
         names = VARIANT_PARAMS[variant]
         P = dict(zip(names, params))
         dev = _need_cuda(hist, tgt, hreg, treg, aux, *params)
-        lib = _lib.load()
-        keep: List[torch.Tensor] = []
-        with torch.cuda.device(dev):
-            p = build_params(variant, P, beta, keep, drop[0], drop[1], _fwd_bwd(drop[2])[0])
-            b = _pairs_struct(hist, tgt, hreg, treg, aux, keep)
-            need_bwd = any(t.requires_grad for t in params) and (len(drop) < 4 or bool(drop[3]))  # drop[3]: grad mode at the call
-            # (the forward and the backward must agree on the pair kernels' precision for the lists / workspace to match)
-            presort = need_bwd and PRESORT_IN_FORWARD and _fwd_bwd(drop[2])[0] == _fwd_bwd(drop[2])[1]
-            score, row_sum, parts, mask, ws = _forward_launch(lib, p, b, dev, want_mask=need_bwd,
-                                                              presort_variant=variant if presort else None)
-            _poll_bad_index(dev)
+        need_bwd = any(t.requires_grad for t in params) and (len(drop) < 4 or bool(drop[3]))  # drop[3]: grad mode at the call
+        # (the forward and the backward must agree on the pair kernels' precision for the lists / workspace to match)
+        presort = need_bwd and PRESORT_IN_FORWARD and _fwd_bwd(drop[2])[0] == _fwd_bwd(drop[2])[1]
+        with _PairCall(dev, variant, beta, P, _fwd_bwd(drop[2])[0], drop, (hist, tgt, hreg, treg, aux)) as c:
+            score, row_sum, parts, mask, ws = _forward_launch(c, want_mask=need_bwd, presort=presort)
         ctx.presorted_ws = ws  # (not an input or an output: rides on ctx; used once)
         ctx.variant, ctx.beta, ctx.drop = variant, beta, drop
         ctx.seg = hist if isinstance(hist, SegmentedPairs) else None  # (not a tensor: rides on ctx)
@@ -420,39 +495,16 @@ def pairs_backward_raw(variant: str, beta: float, P: Dict[str, torch.Tensor], hi
     rows for untouched table rows).  `tables=False` skips the embedding tables (no sort, no segment reduce): the attention-MLP /
     dist-layer gradients only.  `presorted_ws`: the workspace nais_pairs_forward_presort left for this batch (`tables=True`)."""
     dev = _need_cuda(hist, tgt, dscore, *P.values())
-    lib = _lib.load()
-    keep: List[torch.Tensor] = []
-    with torch.cuda.device(dev):
-        p = build_params(variant, P, beta, keep, drop[0], drop[1], _fwd_bwd(drop[2])[1])
-        b = _pairs_struct(hist, tgt, hreg, treg, aux, keep)
-        G = {n: _grad_buffer(n, t, int(b.B)) for n, t in P.items() if tables or n not in _TABLES}
-        g = NaisGrads()
-        if tables:
-            g.hist_poi[0], g.tgt_poi[0] = G["embed_history.weight"].data_ptr(), G["embed_target.weight"].data_ptr()
-        g.w1[0], g.b1[0], g.w2[0] = (G["attn_layer1.weight"].data_ptr(), G["attn_layer1.bias"].data_ptr(),
-                                     G["attn_layer2.weight"].data_ptr())
-        if variant in ("region", "region_distance") and tables:
-            g.reg[0] = G["embed_region.weight"].data_ptr()
-        if "dist_layer.weight" in G:
-            g.dist_w, g.dist_b = G["dist_layer.weight"].data_ptr(), G["dist_layer.bias"].data_ptr()
-        if variant == "disentangled":
-            if tables:
-                g.reg[1] = G["embed_region.weight"].data_ptr()
-            g.w1[1], g.b1[1], g.w2[1] = (G["region_attn_layer1.weight"].data_ptr(),
-                                         G["region_attn_layer1.bias"].data_ptr(),
-                                         G["region_attn_layer2.weight"].data_ptr())
-            g.dist_embed = G["embed_distance.weight"].data_ptr()
-        ws_bytes = lib.nais_pairs_backward_workspace_bytes(C.byref(p), C.byref(b))
+    with _PairCall(dev, variant, beta, P, _fwd_bwd(drop[2])[1], drop, (hist, tgt, hreg, treg, aux)) as c:
+        G = _grad_buffers(P, int(c.b.B), tables)
+        g = _grads_struct(variant, _addresses(G))
+        ws_bytes = c.query("nais_pairs_backward_workspace_bytes")
         ds = _f32(dscore)
-        if presorted_ws is not None and tables and p.n_branch == 1 and presorted_ws.numel() >= ws_bytes:
-            _lib.check(lib.nais_pairs_backward_presorted(C.byref(p), C.byref(b), parts.data_ptr(), row_sum.data_ptr(), _ptr(act_mask),
-                                                         ds.data_ptr(), C.byref(g), presorted_ws.data_ptr(), ws_bytes, _stream()),
-                       "nais_pairs_backward_presorted")
+        args = (parts.data_ptr(), row_sum.data_ptr(), _ptr(act_mask), ds.data_ptr(), C.byref(g))
+        if presorted_ws is not None and tables and c.p.n_branch == 1 and presorted_ws.numel() >= ws_bytes:
+            c.launch("nais_pairs_backward_presorted", *args, ws_bytes=ws_bytes, ws=presorted_ws)
         else:
-            ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)
-            _lib.check(lib.nais_pairs_backward(C.byref(p), C.byref(b), parts.data_ptr(), row_sum.data_ptr(), _ptr(act_mask),
-                                               ds.data_ptr(), C.byref(g), ws.data_ptr(), ws_bytes, _stream()), "nais_pairs_backward")
-        _poll_bad_index(dev)
+            c.launch("nais_pairs_backward", *args, ws_bytes=ws_bytes)
     return G
 
 
@@ -464,9 +516,6 @@ def pairs_score(variant: str, beta: float, params: Sequence[torch.Tensor], hist,
     tcgen05 forward / backward kernels where the shape has them (else the FP32 kernels), "fp32", "tc"."""
     return _PairsFunction.apply(variant, beta, (float(dropout_p), int(dropout_seed), pairs_precision, torch.is_grad_enabled()), hist, tgt, hreg, treg, aux,
                                 *params)
-
-
-_TABLES = ("embed_history.weight", "embed_target.weight", "embed_region.weight")
 
 
 def touched_rows(hist, tgt, hreg=None, treg=None) -> Dict[str, torch.Tensor]:
@@ -486,36 +535,25 @@ def pairs_backward_compact(variant: str, beta: float, P: Dict[str, torch.Tensor]
     dense gradients of the remaining (MLP / dist layer) parameters.  `remaps[name]`: a reusable int32 [table rows] scratch per
     table (only the touched entries are rewritten per call).  One-branch variants."""
     dev = _need_cuda(hist, tgt, dscore, *P.values())
-    lib = _lib.load()
-    keep: List[torch.Tensor] = []
-    with torch.cuda.device(dev):
-        p = build_params(variant, P, beta, keep, drop[0], drop[1], _fwd_bwd(drop[2])[1])
-        if p.n_branch != 1:
+    with _PairCall(dev, variant, beta, P, _fwd_bwd(drop[2])[1], drop, (hist, tgt, hreg, treg, aux)) as c:
+        if c.p.n_branch != 1:
             raise RuntimeError("row-compacted gradients: one-branch variants only")
-        b = _pairs_struct(hist, tgt, hreg, treg, aux, keep)
         ids = touched_rows(hist, tgt, hreg, treg)
-        G = {n: _grad_buffer(n, t, int(b.B)) for n, t in P.items() if n not in _TABLES}
-        g = NaisGrads()
-        g.w1[0], g.b1[0], g.w2[0] = (G["attn_layer1.weight"].data_ptr(), G["attn_layer1.bias"].data_ptr(), G["attn_layer2.weight"].data_ptr())
-        if "dist_layer.weight" in G:
-            g.dist_w, g.dist_b = G["dist_layer.weight"].data_ptr(), G["dist_layer.bias"].data_ptr()
-        sparse = {}
-        for name, gf, rf in (("embed_history.weight", g.hist_poi, g.remap_hist_poi), ("embed_target.weight", g.tgt_poi, g.remap_tgt_poi),
-                             ("embed_region.weight", g.reg, g.remap_reg)):
+        G = _grad_buffers(P, int(c.b.B), tables=False)
+        addr, remap_addr, sparse = _addresses(G), {}, {}
+        for name in _TABLES:
             if name not in P or name not in ids:
                 continue
             i_ = ids[name]
             rm = remaps[name]
             rm[i_] = torch.arange(i_.numel(), device=dev, dtype=torch.int32)
             rows = torch.empty(i_.numel(), P[name].shape[1], device=dev, dtype=torch.float32)
-            gf[0], rf[0] = rows.data_ptr(), rm.data_ptr()
+            addr[name], remap_addr[name] = rows.data_ptr(), rm.data_ptr()
             sparse[name] = (i_, rows)
-        ws_bytes = lib.nais_pairs_backward_workspace_bytes(C.byref(p), C.byref(b))
-        ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)
+        g = _grads_struct(variant, addr, remap_addr)
         ds = _f32(dscore)
-        _lib.check(lib.nais_pairs_backward(C.byref(p), C.byref(b), parts.data_ptr(), row_sum.data_ptr(), _ptr(act_mask), ds.data_ptr(),
-                                           C.byref(g), ws.data_ptr(), ws_bytes, _stream()), "nais_pairs_backward")
-        _poll_bad_index(dev)
+        c.launch("nais_pairs_backward", parts.data_ptr(), row_sum.data_ptr(), _ptr(act_mask), ds.data_ptr(), C.byref(g),
+                 ws_bytes=c.query("nais_pairs_backward_workspace_bytes"))
     return G, sparse
 
 
@@ -544,28 +582,13 @@ def pairs_backward_adagrad(variant: str, beta: float, P: Dict[str, torch.Tensor]
     optimizer's `state['sum']` of table `name`; P[name] and sums[name] of every touched row are updated, nothing dense is
     written.  Returns the gradients of the remaining (MLP / dist layer / embed_distance) parameters."""
     dev = _need_cuda(hist, tgt, dscore, *P.values())
-    lib = _lib.load()
-    keep: List[torch.Tensor] = []
-    with torch.cuda.device(dev):
-        p = build_params(variant, P, beta, keep, drop[0], drop[1], _fwd_bwd(drop[2])[1])
-        b = _pairs_struct(hist, tgt, hreg, treg, aux, keep)
-        G = {n: _grad_buffer(n, t, int(b.B)) for n, t in P.items() if n not in _TABLES}
-        g = NaisGrads()
-        g.w1[0], g.b1[0], g.w2[0] = (G["attn_layer1.weight"].data_ptr(), G["attn_layer1.bias"].data_ptr(), G["attn_layer2.weight"].data_ptr())
-        if "dist_layer.weight" in G:
-            g.dist_w, g.dist_b = G["dist_layer.weight"].data_ptr(), G["dist_layer.bias"].data_ptr()
-        if variant == "disentangled":
-            g.w1[1], g.b1[1], g.w2[1] = (G["region_attn_layer1.weight"].data_ptr(), G["region_attn_layer1.bias"].data_ptr(),
-                                         G["region_attn_layer2.weight"].data_ptr())
-            g.dist_embed = G["embed_distance.weight"].data_ptr()
-        o = _table_adagrad(P, sums, lr, eps)
-        ws_bytes = lib.nais_pairs_backward_workspace_bytes(C.byref(p), C.byref(b))
-        ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)
+    with _PairCall(dev, variant, beta, P, _fwd_bwd(drop[2])[1], drop, (hist, tgt, hreg, treg, aux)) as c:
+        G = _grad_buffers(P, int(c.b.B), tables=False)
+        g = _grads_struct(variant, _addresses(G))
+        o = _adagrad_struct(variant, P, sums, lr, eps, tables=True)
         ds = _f32(dscore)
-        _lib.check(lib.nais_pairs_backward_adagrad(C.byref(p), C.byref(b), parts.data_ptr(), row_sum.data_ptr(), _ptr(act_mask),
-                                                   ds.data_ptr(), C.byref(g), C.byref(o), ws.data_ptr(), ws_bytes, _stream()),
-                   "nais_pairs_backward_adagrad")
-        _poll_bad_index(dev)
+        c.launch("nais_pairs_backward_adagrad", parts.data_ptr(), row_sum.data_ptr(), _ptr(act_mask), ds.data_ptr(), C.byref(g),
+                 C.byref(o), ws_bytes=c.query("nais_pairs_backward_workspace_bytes"))
     return G
 
 
@@ -577,56 +600,17 @@ def pairs_train_step(variant: str, beta: float, P: Dict[str, torch.Tensor], tabl
     library call (8-12 launches).  Every tensor of `P` and every `state['sum']` in `table_sums` / `dense_sums` is updated in
     place.  Returns (loss [1] on the device, pre-sigmoid scores [B] or None)."""
     dev = _need_cuda(hist, tgt, label, *P.values())
-    lib = _lib.load()
-    keep: List[torch.Tensor] = []
-    with torch.cuda.device(dev):
-        p = build_params(variant, P, beta, keep, drop[0], drop[1], drop[2])
-        b = _pairs_struct(hist, tgt, hreg, treg, aux, keep)
-        o, d = _adagrad_structs(P, table_sums, dense_sums, lr_tables, eps_tables, lr_dense, eps_dense)
+    with _PairCall(dev, variant, beta, P, drop[2], drop, (hist, tgt, hreg, treg, aux)) as c:
+        o = _adagrad_struct(variant, P, table_sums, lr_tables, eps_tables, tables=True)
+        d = _adagrad_struct(variant, P, dense_sums, lr_dense, eps_dense, tables=False)
         lab = _f32(label)
         rw = None if row_weight is None else _f32(row_weight)
-        ws_bytes = lib.nais_pairs_train_step_workspace_bytes(C.byref(p), C.byref(b))
-        ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)
+        ws_bytes = c.query("nais_pairs_train_step_workspace_bytes")
         loss = torch.empty(1, device=dev, dtype=torch.float32)
-        score = torch.empty(int(b.B), device=dev, dtype=torch.float32) if want_score else None
-        _lib.check(lib.nais_pairs_train_step(C.byref(p), C.byref(b), lab.data_ptr(), _ptr(rw), C.byref(o), C.byref(d), loss.data_ptr(),
-                                             _ptr(score), ws.data_ptr(), ws_bytes, _stream()), "nais_pairs_train_step")
-        _poll_bad_index(dev)
+        score = torch.empty(int(c.b.B), device=dev, dtype=torch.float32) if want_score else None
+        c.launch("nais_pairs_train_step", lab.data_ptr(), _ptr(rw), C.byref(o), C.byref(d), loss.data_ptr(), _ptr(score),
+                 ws_bytes=ws_bytes)
     return loss, score
-
-
-def _table_adagrad(P, table_sums, lr, eps):
-    """NaisAdagrad of the embedding tables: branch 0's slots, except the disentangled model's region table, which belongs to its
-    branch 1 (include/nais_b200.h)."""
-    from ._lib import NaisAdagrad
-    o = NaisAdagrad()
-    o.lr, o.eps = float(lr), float(eps)
-    reg_slot = 1 if "region_attn_layer1.weight" in P else 0
-    for name, field, slot in zip(_TABLES, (o.sum_hist_poi, o.sum_tgt_poi, o.sum_reg), (0, 0, reg_slot)):
-        if name in P:
-            st = table_sums[name]
-            if st.dtype != torch.float32 or not st.is_contiguous() or st.shape != P[name].shape or not P[name].is_contiguous():
-                raise RuntimeError(f"fused Adagrad: {name} and its state must be contiguous float32 of the same shape")
-            field[slot] = st.data_ptr()
-    return o
-
-
-def _adagrad_structs(P, table_sums, dense_sums, lr_tables, eps_tables, lr_dense, eps_dense):
-    from ._lib import NaisDenseAdagrad
-    o = _table_adagrad(P, table_sums, lr_tables, eps_tables)
-    d = NaisDenseAdagrad()
-    d.lr, d.eps = float(lr_dense), float(eps_dense)
-    # (embed_distance: the kernels read and step row 0 only, so the state's row 0 — the start of the tensor — is what they get)
-    for name, attr in (("attn_layer1.weight", "sum_w1"), ("attn_layer1.bias", "sum_b1"), ("attn_layer2.weight", "sum_w2"),
-                       ("dist_layer.weight", "sum_dist_w"), ("dist_layer.bias", "sum_dist_b"),
-                       ("region_attn_layer1.weight", "sum_region_w1"), ("region_attn_layer1.bias", "sum_region_b1"),
-                       ("region_attn_layer2.weight", "sum_region_w2"), ("embed_distance.weight", "sum_dist_embed")):
-        if name in P:
-            st = dense_sums[name]
-            if st.dtype != torch.float32 or not st.is_contiguous() or st.shape != P[name].shape or not P[name].is_contiguous():
-                raise RuntimeError(f"fused Adagrad: {name} and its state must be contiguous float32 of the same shape")
-            setattr(d, attr, st.data_ptr())
-    return o, d
 
 
 def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sums, dense_sums, lr_tables, eps_tables, lr_dense,
@@ -639,15 +623,13 @@ def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sum
     every tensor of `P` and the optimizer sums in place; returns the per-user losses [n] (device)."""
     import numpy as np
     dev = _need_cuda(indices, entry_region, entry_coords, poi_region, poi_coords, *P.values())
-    lib = _lib.load()
-    keep: List[torch.Tensor] = []
     hp = np.ascontiguousarray(np.asarray(host_indptr, dtype=np.int64))
     hu = np.ascontiguousarray(np.asarray(users, dtype=np.int64))
     if hu.size and (hu.min() < 0 or hu.max() + 1 >= hp.size):
         raise IndexError("train_users: user id outside the train matrix")
-    with torch.cuda.device(dev):
-        p = build_params(variant, P, beta, keep, 0.0, 0, pairs_precision)
-        o, d = _adagrad_structs(P, table_sums, dense_sums, lr_tables, eps_tables, lr_dense, eps_dense)
+    with _PairCall(dev, variant, beta, P, pairs_precision) as c:
+        o = _adagrad_struct(variant, P, table_sums, lr_tables, eps_tables, tables=True)
+        d = _adagrad_struct(variant, P, dense_sums, lr_dense, eps_dense, tables=False)
         if indices.dtype != torch.int64 or not indices.is_contiguous():
             raise RuntimeError("train_users: `indices` must be contiguous int64 (the CSR of the train matrix)")
         er = None if entry_region is None else entry_region.to(torch.int64).contiguous()
@@ -656,13 +638,10 @@ def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sum
         pc = None if poi_coords is None else _f32(poi_coords)
         max_hist = int((hp[hu + 1] - hp[hu]).max()) if hu.size else 0
         losses = torch.empty(max(hu.size, 1), device=dev, dtype=torch.float32)
-        ws_bytes = lib.nais_train_users_workspace_bytes(C.byref(p), max(max_hist, 1), int(num_ng))
-        ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)
-        _lib.check(lib.nais_train_users_centred(C.byref(p), hp.ctypes.data, int(hp.size) - 1, indices.data_ptr(), _ptr(er), _ptr(ec), _ptr(pr),
-                                                _ptr(pc), hu.ctypes.data, int(hu.size), int(num_ng), int(seed) & (2 ** 64 - 1), C.byref(o),
-                                                C.byref(d), losses.data_ptr(), ws.data_ptr(), ws_bytes, float(center[0]), float(center[1]),
-                                                _stream()), "nais_train_users_centred")
-        _poll_bad_index(dev)
+        c.launch("nais_train_users_centred", hp.ctypes.data, int(hp.size) - 1, indices.data_ptr(), _ptr(er), _ptr(ec), _ptr(pr), _ptr(pc),
+                 hu.ctypes.data, int(hu.size), int(num_ng), int(seed) & (2 ** 64 - 1), C.byref(o), C.byref(d), losses.data_ptr(),
+                 ws_bytes=c.query("nais_train_users_workspace_bytes", max(max_hist, 1), int(num_ng)),
+                 tail=(float(center[0]), float(center[1])))
     return losses[: hu.size]
 
 
@@ -670,13 +649,8 @@ def pairs_forward_raw(variant: str, beta: float, P: Dict[str, torch.Tensor], his
     """(score[B], row_sum, parts, act_mask) of nais_pairs_forward without autograd bookkeeping (the fused train step keeps
     them for its backward; act_mask is None unless the tcgen05 forward ran)."""
     dev = _need_cuda(hist, tgt, *P.values())
-    lib = _lib.load()
-    keep: List[torch.Tensor] = []
-    with torch.cuda.device(dev):
-        p = build_params(variant, P, beta, keep, drop[0], drop[1], _fwd_bwd(drop[2])[0])
-        b = _pairs_struct(hist, tgt, hreg, treg, aux, keep)
-        score, row_sum, parts, mask, _ = _forward_launch(lib, p, b, dev)
-        _poll_bad_index(dev)
+    with _PairCall(dev, variant, beta, P, _fwd_bwd(drop[2])[0], drop, (hist, tgt, hreg, treg, aux)) as c:
+        score, row_sum, parts, mask, _ = _forward_launch(c)
     return score, row_sum, parts, mask
 
 
