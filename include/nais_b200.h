@@ -112,9 +112,11 @@ typedef struct NaisParams {
   float dist_bucket_km;    /* reserved (ignored) */
   float beta;              /* smoothing exponent of the softmax denominator (model.py:284-285) */
   /* Train-mode dropout on the attention hidden layer, relu(drop(W x + b)) (NAIS_basic / NAIS_regionEmbedding,
-   * model.py:71,162).  0 disables.  Element (pair b, history h, hidden k) is kept iff
-   * hi32(splitmix64(dropout_seed + ((b*H + h)*hid + k))) >= dropout_p * 2^32, kept values are scaled by 1/(1-p);
-   * forward and backward of one step must be given the same seed.  Pair API only. */
+   * model.py:71,162).  0 disables.  Element (cell, hidden k) is kept iff
+   * hi32(splitmix64(dropout_seed + (cell*hid + k))) >= dropout_p * 2^32, kept values are scaled by 1/(1-p), where cell is the
+   * per-cell index of NaisPairs (act_mask's): b*H + h in the dense layout, seg_cell_offsets[s] + (r - row_offsets[s])*H_s + h in
+   * the segmented one — so a one-segment batch draws the mask of the dense batch with the same rows.  Forward and backward of
+   * one step must be given the same seed.  Pair API only; one branch. */
   float dropout_p;
   uint64_t dropout_seed;
   int32_t pairs_precision; /* NAIS_PAIRS_* (pair API only) */
@@ -135,7 +137,7 @@ typedef struct NaisParams {
  * tile_row0[t] .. of segment tile_seg[t], at most min(16, 128 / H_s) rows (1 row when H_s > 128), never crossing a segment;
  * segments without history or without rows have no tile (a host loop over the segments builds these arrays: INTEGRATION.md).  NAIS_DIST_KM
  * forms dist_km per cell from the same centred coordinates (haversine, cos(latitude) = cos(center_lat + centred lat); NaisCatalog
- * conventions).  Dropout is dense-layout only. */
+ * conventions). */
 typedef struct NaisPairs {
   const int64_t* hist; /* dense [B,H] / segmented [nnz]: history POI ids */
   const int64_t* tgt;  /* [B]   target POI ids */
@@ -207,21 +209,24 @@ NAIS_API const char* nais_strerror(int code);
 NAIS_API uint64_t nais_launch_count(void);
 
 /* Which kernels the pair entry points run for (p, batch): *fwd_tc / *bwd_tc = 1 for the tcgen05 kernels, 0 for the FP32 CUDA-core
- * kernels (NaisParams::pairs_precision, the shape and the device decide; nothing is launched).  Returns 0 or NAIS_ERR_*. */
+ * kernels (NaisParams::pairs_precision, the shape and the device decide; nothing is launched).  With dropout_p > 0, *bwd_tc = 1
+ * holds for a backward given the forward's act_mask: without one, NAIS_PAIRS_AUTO runs the FP32 backward (which regenerates the
+ * mask) and NAIS_PAIRS_TC returns NAIS_ERR_NULL.  Returns 0 or NAIS_ERR_*. */
 NAIS_API int nais_pairs_dispatch(const NaisParams* p, const NaisPairs* batch, int32_t* fwd_tc, int32_t* bwd_tc);
 
 /* score[b] = attention_network(pairs)  (pre-sigmoid, model.py:246-297).  Saved for backward (each may be NULL):
  * row_sum[n_branch,B] = sum_h E_bh, score_parts[n_branch,B] = per-branch score (their sum over branches is score),
- * act_mask[B*H] = the ReLU pattern of attn_layer1: bit k of word (b*H + h) is set iff hidden unit k of that cell was active
- * (t_k > 0).  act_mask is written only by the tcgen05 forward with hid <= 64 (nais_pairs_dispatch: fwd_tc); the tcgen05
- * backward then takes the unit-step of ReLU from it instead of thresholding its own recomputed t (bf16 two-term splits:
- * ~1e-5 relative, enough to flip a unit that sits on the kink and move a gradient by one cell's whole contribution). */
+ * act_mask[cells] = the ReLU pattern of attn_layer1: bit k of word `cell` (b*H + h dense; NaisPairs) is set iff hidden unit k of
+ * that cell was active (t_k > 0) — with dropout, active AND kept.  act_mask is written only by the tcgen05 forward with
+ * hid <= 64 (nais_pairs_dispatch: fwd_tc); the tcgen05 backward then takes the unit-step of ReLU from it instead of thresholding
+ * its own recomputed t (bf16 two-term splits: ~1e-5 relative, enough to flip a unit that sits on the kink and move a gradient by
+ * one cell's whole contribution).  With dropout the tcgen05 backward NEEDS it: it draws no mask of its own. */
 NAIS_API int nais_pairs_forward(const NaisParams* p, const NaisPairs* batch, float* score, float* row_sum, float* score_parts,
                        uint64_t* act_mask, nais_stream_t stream);
 
 NAIS_API size_t nais_pairs_backward_workspace_bytes(const NaisParams* p, const NaisPairs* batch);
 /* Given dscore[B] = dL/dscore, write every parameter gradient.  score_parts / row_sum / act_mask are the forward's outputs
- * (act_mask: NULL unless the tcgen05 forward wrote it).
+ * (act_mask: NULL unless the tcgen05 forward wrote it; required by the tcgen05 backward with dropout, see nais_pairs_dispatch).
  * Streams: everything is ordered after the work already in `stream`, and `stream` is ordered after everything this call
  * enqueues, as for any other entry point — but the sort + reduce of the target-id and region-id lists and the reduce of the
  * per-CTA MLP-gradient partials run on three streams the library creates once per device (forked from / joined to `stream`
@@ -339,12 +344,22 @@ NAIS_API int nais_train_users(const NaisParams* p, const int64_t* host_indptr, i
                               int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables, const NaisDenseAdagrad* dense,
                               float* losses, void* workspace, size_t workspace_bytes, nais_stream_t stream);
 /* nais_train_users for coordinates centred on (center_lat, center_lon): the (lat, lon) that was subtracted from entry_coords /
- * poi_coords (NaisCatalog conventions).  NAIS_DIST_KM needs it for cos(latitude); nais_train_users is this call with (0, 0). */
+ * poi_coords (NaisCatalog conventions).  NAIS_DIST_KM needs it for cos(latitude); nais_train_users is this call with (0, 0).
+ * Both return NAIS_ERR_MODE for dropout_p > 0 (one seed for every step would repeat the mask): use nais_train_users_dropout. */
 NAIS_API int nais_train_users_centred(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
                                       const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region,
                                       const float* poi_coords, const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed,
                                       const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* losses, void* workspace,
                                       size_t workspace_bytes, float center_lat, float center_lon, nais_stream_t stream);
+/* nais_train_users_centred with train-mode dropout (NaisParams::dropout_p > 0): host_dropout_seeds is a HOST array of n_users
+ * seeds, the step of host_users[i] runs with dropout_seed = host_dropout_seeds[i] (entries of users without a history are
+ * ignored).  NULL with dropout_p > 0 is NAIS_ERR_NULL; with dropout_p == 0 the array is not read. */
+NAIS_API int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
+                                      const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region,
+                                      const float* poi_coords, const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed,
+                                      const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* losses, void* workspace,
+                                      size_t workspace_bytes, float center_lat, float center_lon, const uint64_t* host_dropout_seeds,
+                                      nais_stream_t stream);
 
 /* Workspace for nais_fullrank_topk / nais_fullrank_scores: n_users and nnz = offsets[n_users] are host-known. */
 NAIS_API size_t nais_fullrank_workspace_bytes(const NaisParams* p, int32_t n_users, int64_t nnz, int64_t poi_begin,

@@ -91,6 +91,10 @@ SYMBOLS = {
                                            C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_uint64, C.POINTER(NaisAdagrad),
                                            C.POINTER(NaisDenseAdagrad), C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float,
                                            C.c_void_p]),
+    "nais_train_users_dropout": (C.c_int, [C.POINTER(NaisParams), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_uint64, C.POINTER(NaisAdagrad),
+                                           C.POINTER(NaisDenseAdagrad), C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float,
+                                           C.c_void_p, C.c_void_p]),
     "nais_rows_adagrad_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
     "nais_rows_adagrad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_float, C.c_float, C.c_void_p, C.c_size_t, C.c_void_p]),

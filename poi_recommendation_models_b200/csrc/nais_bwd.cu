@@ -1040,6 +1040,9 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
     if (D > 128 || p.hid > 128) return NAIS_ERR_SHAPE;  // backward tiles: D, hid <= 128 in this version
     if (pairs_n_tiles(b) < 1) return 0;
     if (p.pairs_precision == NAIS_PAIRS_TC && !pairs_tc_bwd_supported(p, b)) return NAIS_ERR_SHAPE;
+    // the tcgen05 dropout backward takes the mask from the forward's act_mask (it regenerates nothing)
+    const bool tile_phase = phase != BWD_SORTS && phase != BWD_JOIN_SORTS;
+    if (p.pairs_precision == NAIS_PAIRS_TC && p.dropout_p > 0.f && !act_mask && tile_phase) return NAIS_ERR_NULL;
     // a table is processed if it has a gradient destination or a fused-optimizer state
     const bool want[3] = {br.w_poi > 0 && (g.hist_poi[bi] || (opt && opt->sum_hist_poi[bi])),
                           br.w_poi > 0 && (g.tgt_poi[bi] || (opt && opt->sum_tgt_poi[bi])),
@@ -1092,7 +1095,8 @@ int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score
     int rc;
     const int nkb = p.hid <= 64 ? 1 : 2, db = D <= 64 ? 1 : 2;
     A.bad = bad_index_flag();
-    const bool tc_ok = pairs_tc_bwd_supported(p, b);
+    A.drop_inv = p.dropout_p > 0.f ? 1.f / (1.f - p.dropout_p) : 1.f;
+    const bool tc_ok = pairs_tc_bwd_supported(p, b) && (p.dropout_p <= 0.f || A.act_mask);  // (else the FP32 kernel regenerates the mask)
     if (p.pairs_precision != NAIS_PAIRS_FP32 && tc_ok) rc = launch_pairs_bwd_tc(A, D, grid, stream);  // tcgen05 (bf16 two-term splits)
     else if (nkb == 1 && db == 1) rc = launch_bwd_tile<1, 1>(A, D, grid, stream);
     else if (nkb == 1) rc = launch_bwd_tile<1, 2>(A, D, grid, stream);

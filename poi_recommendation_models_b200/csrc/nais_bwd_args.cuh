@@ -25,6 +25,7 @@ struct BwdArgs {
   int part_stride;
   int64_t n_items;        // work items (tiles of rows: nais_pairs_tile.cuh)
   int* bad;               // the library's bad-index word (nais_common.cuh)
+  float drop_inv;         // 1 / (1 - dropout_p) (tcgen05 dropout backward; a kernel parameter, so no register holds it)
 };
 
 // layout of one CTA's parameter partial: w1 [hid][D+lanes] | b1 [hid] | w2 [hid] | dist_w[4] dist_b[2] km[1] pad[1]

@@ -106,7 +106,7 @@ static int check_pairs(const NaisParams* p, const NaisPairs* b) {
     if (b->n_seg < 1 || b->n_tiles < 0 || b->n_cells < 0) return NAIS_ERR_SHAPE;
     if (!b->row_offsets || !b->seg_cell_offsets || (b->n_tiles && (!b->tile_seg || !b->tile_row0))) return NAIS_ERR_NULL;
     if (b->aux) return NAIS_ERR_MODE;
-    if (p->dropout_p > 0.f) return NAIS_ERR_MODE;
+    if (p->dropout_p > 0.f && p->n_branch != 1) return NAIS_ERR_MODE;  // (the disentangled model has no dropout)
     if (p->dist_mode != NAIS_DIST_NONE && (!b->hist_coords || !b->tgt_coords)) return NAIS_ERR_NULL;
     return 0;
   }
@@ -606,11 +606,22 @@ int nais_train_users_centred(const NaisParams* p, const int64_t* host_indptr, in
                              const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables,
                              const NaisDenseAdagrad* dense, float* losses, void* workspace, size_t workspace_bytes, float center_lat,
                              float center_lon, nais_stream_t stream) {
+  if (p && p->dropout_p > 0.f) return NAIS_ERR_MODE;  // one seed for every step would repeat the mask: nais_train_users_dropout
+  return nais_train_users_dropout(p, host_indptr, n_rows, indices, entry_region, entry_coords, poi_region, poi_coords, host_users, n_users,
+                                  num_ng, seed, tables, dense, losses, workspace, workspace_bytes, center_lat, center_lon, nullptr, stream);
+}
+
+int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
+                             const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region, const float* poi_coords,
+                             const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables,
+                             const NaisDenseAdagrad* dense, float* losses, void* workspace, size_t workspace_bytes, float center_lat,
+                             float center_lon, const uint64_t* host_dropout_seeds, nais_stream_t stream) {
   int rc = check_params(p);
   if (rc) return rc;
   rc = check_train_state(p, tables, dense);
   if (rc) return rc;
   if (n_users < 0 || num_ng < 0) return NAIS_ERR_SHAPE;
+  if (p->dropout_p > 0.f && !host_dropout_seeds) return NAIS_ERR_NULL;
   if (n_users == 0) return 0;
   if (!host_indptr || !indices || !host_users || !losses || !workspace) return NAIS_ERR_NULL;
   bool need_reg = false;
@@ -741,8 +752,10 @@ int nais_train_users_centred(const NaisParams* p, const int64_t* host_indptr, in
     }
     UserBatch ub;
     buffers(cur, cur_slot, ub);
+    NaisParams pu = *p;  // (the id sorts of the preparation depend on the batch only, not on the dropout seed)
+    if (p->dropout_p > 0.f) pu.dropout_seed = host_dropout_seeds[cur];
     cudaStreamWaitEvent(st, prepared[cur_slot], 0);
-    rc = train_step_impl(p, &ub.b, ub.label, nullptr, tables, dense, losses + cur, nullptr, ub.step, L.total - L.step, st, STEP_AFTER_SORTS);
+    rc = train_step_impl(&pu, &ub.b, ub.label, nullptr, tables, dense, losses + cur, nullptr, ub.step, L.total - L.step, st, STEP_AFTER_SORTS);
     if (rc) return bail(rc);
     cudaEventRecord(stepped[cur_slot], st);
     ++done;

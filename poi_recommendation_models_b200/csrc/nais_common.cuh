@@ -146,6 +146,25 @@ __host__ __device__ __forceinline__ uint32_t dropout_threshold(float p) {
   const double t = (double)p * 4294967296.0;
   return t >= 4294967295.0 ? 0xFFFFFFFFu : (uint32_t)t;
 }
+constexpr uint64_t DROPOUT_GOLDEN = 0x9E3779B97F4A7C15ull;
+// dropout_bits(seed, idx) given z = seed + idx * DROPOUT_GOLDEN, so that a caller can hoist the per-cell part of z.  Bit-exact:
+// only the high half of the last product is formed (hi32(z * C) = umulhi(lo, C_lo) + lo * C_hi + hi * C_lo, mod 2^32), and the
+// final z ^= z >> 31 reaches the high half as h ^ (h >> 31).
+__host__ __device__ __forceinline__ uint32_t dropout_bits_z(uint64_t z) {
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z ^= z >> 27;
+  const uint32_t lo = (uint32_t)z, hi = (uint32_t)(z >> 32);
+  const uint32_t h = (uint32_t)(((uint64_t)lo * 0x133111EBu) >> 32) + lo * 0x94D049BBu + hi * 0x133111EBu;
+  return h ^ (h >> 31);
+}
+// Keep bits of N consecutive mask elements idx0 .. idx0 + N - 1 (bit i = element idx0 + i kept), z0 = seed + idx0 * DROPOUT_GOLDEN.
+template <int N>
+__host__ __device__ __forceinline__ uint32_t dropout_keep_bits(uint64_t z0, uint32_t thresh) {
+  uint32_t w = 0u;
+#pragma unroll
+  for (int i = 0; i < N; ++i) w |= (dropout_bits_z(z0 + (uint64_t)i * DROPOUT_GOLDEN) >= thresh ? 1u : 0u) << i;
+  return w;
+}
 
 __device__ __forceinline__ float sigmoidf_exact(float z) { return 1.0f / (1.0f + expf(-z)); }
 

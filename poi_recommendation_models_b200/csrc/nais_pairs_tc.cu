@@ -1,6 +1,7 @@
 // Pair forward (model.py:246-297) with the attention-MLP contraction on tcgen05 — the default of nais_pairs_forward
 // (NaisParams::pairs_precision = NAIS_PAIRS_AUTO) for one branch, D in {16, 32, 48, 64}, hid <= 128 (multiple of 16), lat/lon or
-// no distance mode, no dropout; everything else runs the FP32 kernel (nais_fp32.cu).
+// no distance mode; everything else runs the FP32 kernel (nais_fp32.cu).  Train-mode dropout is a compile-time parameter (kDrop): the
+// epilogue draws the keep bits of NaisParams::dropout_seed (the FP32 kernels' mask, bit for bit) and saves "active and kept" in act_mask.
 //
 // A training row has its own history, so unlike full-rank scoring there is no per-user operand to reuse: the GEMM is
 //     T[cell, k] = sum_d X[cell, d] * W[k, d],      X[cell, :] = q_cell (.) p_row       (M = 128 cells, N = hid, K = D)
@@ -34,6 +35,8 @@ struct Args {
   unsigned long long* act_mask;  // [cells] ReLU pattern per cell (hid <= 64) or NULL
   uint32_t tmem_cols;
   int* bad;  // the library's bad-index word (nais_common.cuh)
+  uint32_t drop_thresh;  // dropout: dropout_threshold(dropout_p) and 1 / (1 - dropout_p) (kernel parameters: read from the constant bank)
+  float drop_inv;
 };
 
 __device__ __forceinline__ float pow2_scale(float amax, int target_exp) {
@@ -46,7 +49,7 @@ __device__ __forceinline__ float pow2_scale(float amax, int target_exp) {
   return ldexpf(1.f, k);
 }
 
-template <int D>
+template <int D, bool kDrop>
 __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(const __grid_constant__ Args A) {
   extern __shared__ __align__(128) uint8_t smem[];
   const NaisParams& p = A.p;
@@ -264,6 +267,8 @@ __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(cons
       for (int c0 = 0; c0 < hid; c0 += 16) {
         uint32_t v[16];
         tmem_ld16(tlane + c0, v);
+        uint32_t keep = 0u;  // kDrop: keep bits of hidden units c0 .. c0 + 15 of this cell (independent of t: hashed while the load runs)
+        if constexpr (kDrop) keep = dropout_keep_bits<16>(p.dropout_seed + ((uint64_t)cidx * hid + c0) * DROPOUT_GOLDEN, A.drop_thresh);
         tmem_wait_ld16(v);
         uint32_t bits = 0u;
 #pragma unroll
@@ -271,6 +276,7 @@ __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(cons
           const int k = c0 + i;
           float t = fmaf(__uint_as_float(v[i]), inv, kc[k]);
           if (lanes) t = fmaf(kc[3 * hid + k], g1, fmaf(kc[2 * hid + k], g0, t));
+          if constexpr (kDrop) t = ((keep >> i) & 1u) ? t * A.drop_inv : 0.f;  // relu(drop(t)), model.py:71,162
           bits |= (t > 0.f ? 1u : 0u) << i;
           a = fmaf(kc[hid + k], fmaxf(t, 0.f), a);
         }
@@ -345,6 +351,7 @@ __device__ unsigned long long g_phase_clk[16];
 #define NAIS_PH(i)
 #endif
 
+template <bool kDrop>
 __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_constant__ Args A) {
   constexpr int D = 64, HIDC = 64, KC = D / 8, A_PLANE = KC * PT * 16, W_PLANE = KC * HIDC * 16;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -559,6 +566,9 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
       }
       __syncwarp();
     }
+    // kDrop: keep bits of this thread's 32 hidden units s0 .. s0 + 31 (they depend on (seed, cell, k) only: hashed while the MMAs run)
+    uint32_t keep = 0u;
+    if constexpr (kDrop) keep = dropout_keep_bits<32>(p.dropout_seed + ((uint64_t)c.cidx * HIDC + s0) * DROPOUT_GOLDEN, A.drop_thresh);
     mbar_wait(bar, phase);
     phase ^= 1u;
     tc_fence_after();
@@ -581,6 +591,7 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
         const float4 c4 = reinterpret_cast<const float4*>(kc)[s0 + c0 + i];
         float t = fmaf(__uint_as_float(v[i]), inv, c4.x);
         if (lanes) t = fmaf(c4.w, g1, fmaf(c4.z, g0, t));
+        if constexpr (kDrop) t = ((keep >> (c0 + i)) & 1u) ? t * A.drop_inv : 0.f;  // relu(drop(t)): a dropped unit is inactive in the saved pattern
         // t > 0  <=>  the sign bit of (0 - t) is set (IEEE: 0 - (+-0) = +0, so an exact zero counts as inactive like torch's
         // relu backward); shifted in from the right, un-reversed once below: 2 instructions per unit instead of 5
         bits = __funnelshift_l(__float_as_uint(0.f - t), bits, 1);
@@ -647,13 +658,14 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
   if (warp == 0) tmem_dealloc(tmem, 64u);
 }
 
+template <bool kDrop>
 static int launch2(const Args& A, int64_t n_items, int sms, cudaStream_t stream) {
   constexpr int D = 64, HIDC = 64;
   const size_t smem = 2 * (size_t)(D / 8) * PT * 16 + 2 * (size_t)(D / 8) * HIDC * 16 +
                       4096 + (4 * (size_t)HIDC + 2 * PMAXROWS * D + 2 * PT + 2 * PMAXROWS + 8 + 6 * PT + PT) * 4 +
                       (3 * (size_t)PT2 + PMAXROWS) * 8 + ((size_t)PT + PMAXROWS) * 8 + 16;
   static SmemAttrOnce attr;
-  cudaError_t e = attr(pairs_fwd_tc2_kernel, smem, true);
+  cudaError_t e = attr(pairs_fwd_tc2_kernel<kDrop>, smem, true);
   if (e != cudaSuccess) return (int)e;
   int per_sm = 3;
   const int by_smem = (int)((227 * 1024) / (smem + 1024));
@@ -661,18 +673,18 @@ static int launch2(const Args& A, int64_t n_items, int sms, cudaStream_t stream)
   if (per_sm < 1) return NAIS_ERR_SHAPE;
   const int64_t cap = (int64_t)sms * per_sm;
   const int grid = (int)(n_items < cap ? n_items : cap);
-  pairs_fwd_tc2_kernel<<<grid, PT2, smem, stream>>>(A);
+  pairs_fwd_tc2_kernel<kDrop><<<grid, PT2, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
 
-template <int D>
+template <int D, bool kDrop>
 static int launch(const Args& A, int hid, int64_t n_items, int sms, cudaStream_t stream) {
   const size_t smem = 2 * (size_t)(D / 8) * PT * 16 + 2 * (size_t)(D / 8) * hid * 16 +
                       (4 * (size_t)hid + PMAXROWS * D + 2 * PT + 2 * PMAXROWS + 8) * 4 + 16 + (size_t)PT * STG_STRIDE;
-  cudaError_t e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return (int)e;
   // Persistent grid: as many CTAs as can be co-resident — the kernel's register budget (3 per SM for D = 64, else 4), shared
   // memory, and TMEM (tmem_cols of the SM's 512 columns per CTA; a CTA beyond that would simply wait in tcgen05.alloc).
@@ -683,9 +695,22 @@ static int launch(const Args& A, int hid, int64_t n_items, int sms, cudaStream_t
   if (per_sm < 1) return NAIS_ERR_SHAPE;
   const int64_t cap = (int64_t)sms * per_sm;
   const int grid = (int)(n_items < cap ? n_items : cap);
-  pairs_fwd_tc_kernel<D><<<grid, PT, smem, stream>>>(A);
+  pairs_fwd_tc_kernel<D, kDrop><<<grid, PT, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
+}
+
+// `two`: two threads per cell (D = hid = 64, a cell's 32-column halves each lie in one table)
+template <bool kDrop>
+static int launch_shape(const Args& A, int D, bool two, int64_t n_items, int sms, cudaStream_t stream) {
+  if (two) return launch2<kDrop>(A, n_items, sms, stream);
+  switch (D) {
+    case 16: return launch<16, kDrop>(A, A.p.hid, n_items, sms, stream);
+    case 32: return launch<32, kDrop>(A, A.p.hid, n_items, sms, stream);
+    case 48: return launch<48, kDrop>(A, A.p.hid, n_items, sms, stream);
+    case 64: return launch<64, kDrop>(A, A.p.hid, n_items, sms, stream);
+    default: return NAIS_ERR_SHAPE;
+  }
 }
 
 }  // namespace ptc
@@ -695,7 +720,7 @@ bool pairs_tc_supported(const NaisParams& p, const NaisPairs& b) {
   const int D = p.branch[0].w_poi + p.branch[0].w_reg;
   if (D != 16 && D != 32 && D != 48 && D != 64) return false;
   if (p.hid < 16 || p.hid > 128 || (p.hid & 15)) return false;
-  if (p.dist_mode == NAIS_DIST_KM || p.dropout_p > 0.f) return false;
+  if (p.dist_mode == NAIS_DIST_KM) return false;
   return true;
 }
 
@@ -712,19 +737,15 @@ int launch_pairs_fwd_tc(const NaisParams& p, const NaisPairs& b, float* score, f
   A.parts = parts;
   A.act_mask = p.hid <= 64 ? act_mask : nullptr;
   A.bad = bad_index_flag();
+  A.drop_thresh = p.dropout_p > 0.f ? dropout_threshold(p.dropout_p) : 0u;
+  A.drop_inv = p.dropout_p > 0.f ? 1.f / (1.f - p.dropout_p) : 1.f;
   A.tmem_cols = p.hid <= 32 ? 32u : (p.hid <= 64 ? 64u : 128u);
   const int64_t n_items = pairs_n_tiles(b);
   if (n_items < 1) return 0;
   const int D = p.branch[0].w_poi + p.branch[0].w_reg;
-  if (D == 64 && p.hid == 64 && rows_vec4(p.branch[0], 4) && pair_gather_uniform(p.branch[0]))
-    return ptc::launch2(A, n_items, sms, stream);  // two threads per cell (a cell's 32-column halves each lie in one table)
-  switch (D) {
-    case 16: return ptc::launch<16>(A, p.hid, n_items, sms, stream);
-    case 32: return ptc::launch<32>(A, p.hid, n_items, sms, stream);
-    case 48: return ptc::launch<48>(A, p.hid, n_items, sms, stream);
-    case 64: return ptc::launch<64>(A, p.hid, n_items, sms, stream);
-    default: return NAIS_ERR_SHAPE;
-  }
+  const bool two = D == 64 && p.hid == 64 && rows_vec4(p.branch[0], 4) && pair_gather_uniform(p.branch[0]);
+  if (p.dropout_p > 0.f) return ptc::launch_shape<true>(A, D, two, n_items, sms, stream);
+  return ptc::launch_shape<false>(A, D, two, n_items, sms, stream);
 }
 
 }  // namespace nais

@@ -1,6 +1,8 @@
 // Backward of the pair scorer with all three contractions on tcgen05 — the default of nais_pairs_backward[_adagrad]
 // (NaisParams::pairs_precision = NAIS_PAIRS_AUTO) for one branch, hidden_size = 64, D in {32, 64}, lat/lon or no distance mode,
-// no dropout, 16-byte aligned table rows; everything else runs the FP32 kernel (nais_bwd.cu).
+// 16-byte aligned table rows; everything else runs the FP32 kernel (nais_bwd.cu).  Train-mode dropout (kDrop) draws nothing: with
+// m = the forward's saved "active and kept" bit, relu(drop(t)) = m relu(t) / (1-p), so m gives the recomputed logit, the dw2 term
+// and dt = m da v / (1-p) — the dropout backward needs act_mask (without it the FP32 kernel runs, which regenerates the mask).
 // It writes the SAME workspace as pairs_bwd_kernel (dq rows, dp rows, one parameter partial per CTA), so the deterministic
 // param_reduce and the sorted-segment embedding reduce that follow are shared.
 //
@@ -90,7 +92,7 @@ __device__ __forceinline__ void gather_segment(const NaisBranch& br, int it32, i
   __syncwarp();
 }
 
-template <int D>
+template <int D, bool kDrop>
 __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_constant__ BwdArgs A) {
   static_assert(D == 32 || D == 64, "segments of 32");
   extern __shared__ __align__(128) uint8_t smem[];
@@ -240,6 +242,8 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
       phase ^= 1u;
       tc_fence_after();
       // ---- epilogue 1: thread = cell = TMEM lane ----------------------------------------------------------------------------------------
+      unsigned long long amd = 0ull;  // kDrop: the forward's "active and kept" pattern (a dropped unit counts as t = 0)
+      if constexpr (kDrop) amd = valid ? __ldg(A.act_mask + cidx) : 0ull;
       float a = 0.f;
       for (int c0 = 0; c0 < HID; c0 += 16) {
         uint32_t v[16];
@@ -250,9 +254,11 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
           const int k = c0 + i;
           float t = __uint_as_float(v[i]) + kc[k];
           if (lanes) t = fmaf(kc[3 * HID + k], g1, fmaf(kc[2 * HID + k], g0, t));
+          if constexpr (kDrop) t = ((amd >> k) & 1ull) ? t : 0.f;
           a = fmaf(kc[HID + k], fmaxf(t, 0.f), a);
         }
       }
+      if constexpr (kDrop) a *= A.drop_inv;
       float dav = 0.f, gwv = 0.f;
       if (live) {
         const float S = rowv[r], sc = rowv[BWD_MAXROWS + r], G = rowv[2 * BWD_MAXROWS + r], Sb = rowv[3 * BWD_MAXROWS + r];
@@ -261,10 +267,11 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
         dav = G * (w * ssum - p.beta * (e / S) * sc);
         gwv = G * w;
       }
+      if constexpr (kDrop) dav *= A.drop_inv;  // d relu(drop(t)) / dt = m / (1-p)
       // unit step of ReLU: the forward's saved pattern when there is one (its t is accurate to ~2e-7; this kernel's recomputed t,
       // from bf16 two-term splits, only to ~1e-5 — a unit on the kink would flip and move the gradients by this cell's whole term)
-      const bool have_mask = A.act_mask != nullptr;
-      const unsigned long long am = (have_mask && valid) ? __ldg(A.act_mask + cidx) : 0ull;
+      const bool have_mask = kDrop || A.act_mask != nullptr;
+      const unsigned long long am = kDrop ? amd : (have_mask && valid) ? __ldg(A.act_mask + cidx) : 0ull;
       float dvv[HID];
       float dg0 = 0.f, dg1 = 0.f;
 #pragma unroll
@@ -278,6 +285,7 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
           const int k = c0 + i;
           float t = __uint_as_float(v[i]) + kc[k];
           if (lanes) t = fmaf(kc[3 * HID + k], g1, fmaf(kc[2 * HID + k], g0, t));
+          if constexpr (kDrop) t = ((am >> k) & 1ull) ? t : 0.f;
           dvv[k] = dav * fmaxf(t, 0.f);
           const bool on = have_mask ? ((am >> k) & 1ull) != 0ull : t > 0.f;
           dt[i] = on ? dav * kc[HID + k] : 0.f;
@@ -463,6 +471,7 @@ __device__ unsigned long long g_phase_clk[16];
 #define NAIS_PH(i)
 #endif
 
+template <bool kDrop>
 __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_constant__ BwdArgs A) {
   constexpr int D = 64;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -704,11 +713,12 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
           const float4 c4 = reinterpret_cast<const float4*>(kc)[s0 + c0 + i];
           float t = __uint_as_float(v[i]) + c4.x;
           if (lanes) t = fmaf(c4.w, g1, fmaf(c4.z, g0, t));
+          if constexpr (kDrop) t = ((am32 >> (c0 + i)) & 1u) ? t : 0.f;  // the forward's "active and kept" pattern
           tv[c0 + i] = t;
           ap = fmaf(c4.y, fmaxf(t, 0.f), ap);
         }
       }
-      asum[half * PT + cell] = ap;
+      asum[half * PT + cell] = kDrop ? ap * A.drop_inv : ap;
     }
     asm volatile("bar.sync %0, 64;" ::"r"(1 + qd) : "memory");  // the two warps of this lane quarter exchange their halves of a
     NAIS_PH(5)
@@ -721,7 +731,8 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
       dav = G * (w * ssum - p.beta * (e / S) * sc);
       gwv = G * w;
     }
-    const bool have_mask = A.act_mask != nullptr;
+    if constexpr (kDrop) dav *= A.drop_inv;  // d relu(drop(t)) / dt = m / (1-p)
+    const bool have_mask = kDrop || A.act_mask != nullptr;
     float dg0 = 0.f, dg1 = 0.f;
 #pragma unroll
     for (int c0 = 0; c0 < 32; c0 += 16) {
@@ -920,6 +931,7 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
   if (warp == 0) tmem_dealloc(tmem, TMEM_COLS);
 }
 
+template <bool kDrop>
 static int launch2(const BwdArgs& A, int grid, cudaStream_t stream) {
   constexpr int D = 64;
   constexpr size_t dt_region = (8 * 32 * STG_STRIDE > 2 * (HID / 8) * PT * 16) ? 8 * 32 * STG_STRIDE : 2 * (HID / 8) * PT * 16;
@@ -928,24 +940,31 @@ static int launch2(const BwdArgs& A, int grid, cudaStream_t stream) {
                           (3 * (size_t)PT + PT2 + BWD_MAXROWS) * 8 + ((size_t)PT + BWD_MAXROWS) * 8 + 4 * BWD_MAXROWS * 4 + 16;
   static_assert(2 * (smem + 1024) <= 228 * 1024, "two CTAs per SM");
   static SmemAttrOnce attr;
-  cudaError_t e = attr(pairs_bwd_tc2_kernel, smem, true);
+  cudaError_t e = attr(pairs_bwd_tc2_kernel<kDrop>, smem, true);
   if (e != cudaSuccess) return (int)e;
-  pairs_bwd_tc2_kernel<<<grid, PT2, smem, stream>>>(A);
+  pairs_bwd_tc2_kernel<kDrop><<<grid, PT2, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
 
-template <int D>
+template <int D, bool kDrop>
 static int launch(const BwdArgs& A, int grid, cudaStream_t stream) {
   constexpr size_t smem = 2 * (size_t)(D / 8 + 1) * PT * 16 + 2 * (size_t)(D / 8) * HID * 16 + 2 * (size_t)(HID / 8) * PT * 16 +
                           (4 * HID + 2 * BWD_MAXROWS * D + 4 * BWD_MAXROWS + 4 * HID + 32) * 4 + 16;
-  cudaError_t e = cudaFuncSetAttribute(pairs_bwd_tc_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(pairs_bwd_tc_kernel<D, kDrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  e = cudaFuncSetAttribute(pairs_bwd_tc_kernel<D>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  e = cudaFuncSetAttribute(pairs_bwd_tc_kernel<D, kDrop>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return (int)e;
-  pairs_bwd_tc_kernel<D><<<grid, PT, smem, stream>>>(A);
+  pairs_bwd_tc_kernel<D, kDrop><<<grid, PT, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
+}
+
+// D = 64: two threads per cell when each 32-column half of a row lies in one table (every shipped model class)
+template <bool kDrop>
+static int launch_shape(const BwdArgs& A, int D, int grid, cudaStream_t stream) {
+  if (D == 32) return launch<32, kDrop>(A, grid, stream);
+  return pair_gather_uniform(A.p.branch[A.bi]) ? launch2<kDrop>(A, grid, stream) : launch<64, kDrop>(A, grid, stream);
 }
 
 }  // namespace ptcb
@@ -955,17 +974,17 @@ bool pairs_tc_bwd_supported(const NaisParams& p, const NaisPairs& b) {
   const NaisBranch& br = p.branch[0];
   const int D = br.w_poi + br.w_reg;
   if (D != 32 && D != 64) return false;
-  if (p.dist_mode == NAIS_DIST_KM || p.dropout_p > 0.f) return false;
+  if (p.dist_mode == NAIS_DIST_KM) return false;
   if (!rows_vec4(br, 4)) return false;
   (void)b;
   return device_info().major == 10;
 }
 
-// grid <= 2 CTAs per SM (256 TMEM columns each); every CTA owns at least one tile (the caller passes min(n_items, grid))
+// grid <= 2 CTAs per SM (256 TMEM columns each); every CTA owns at least one tile (the caller passes min(n_items, grid)).  With
+// dropout A.act_mask must be the forward's pattern (launch_pairs_bwd runs the FP32 kernel instead when it is NULL).
 int launch_pairs_bwd_tc(const BwdArgs& A, int D, int grid, cudaStream_t stream) {
-  if (D == 32) return ptcb::launch<32>(A, grid, stream);
-  // D = 64: two threads per cell when each 32-column half of a row lies in one table (every shipped model class)
-  return pair_gather_uniform(A.p.branch[A.bi]) ? ptcb::launch2(A, grid, stream) : ptcb::launch<64>(A, grid, stream);
+  if (A.p.dropout_p > 0.f) return A.act_mask ? ptcb::launch_shape<true>(A, D, grid, stream) : NAIS_ERR_NULL;
+  return ptcb::launch_shape<false>(A, D, grid, stream);
 }
 
 }  // namespace nais

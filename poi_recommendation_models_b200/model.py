@@ -65,13 +65,17 @@ class _NAISBase(nn.Module):
         named = dict(self.named_parameters())
         return {n: named[n] for n in ops.VARIANT_PARAMS[self.variant]}
 
-    def _score(self, hist, tgt, hreg=None, treg=None, aux=None) -> torch.Tensor:
-        drop_p, seed = 0.0, 0
+    def _draw_dropout(self) -> Tuple[float, int]:
+        """(p, seed) of this call's dropout: relu(drop(attn_layer1(x))) in train mode (model.py:71,162) is fused, with a
+        counter-based mask; the seed comes from torch's CPU generator so torch.manual_seed makes a run reproducible (not the
+        reference's mask stream).  (0.0, 0) when no dropout applies."""
         if self._dropout_on_l1 and self.training and self.drop.p > 0:
-            # relu(drop(attn_layer1(x))) in train mode (model.py:71,162): fused, counter-based mask; the seed comes from
-            # torch's CPU generator so torch.manual_seed makes a run reproducible (not the reference's mask stream)
-            drop_p, seed = float(self.drop.p), int(torch.randint(0, 2 ** 62, (1,)).item())
-            self.last_dropout_seed = seed
+            self.last_dropout_seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+            return float(self.drop.p), self.last_dropout_seed
+        return 0.0, 0
+
+    def _score(self, hist, tgt, hreg=None, treg=None, aux=None) -> torch.Tensor:
+        drop_p, seed = self._draw_dropout()
         P = self._params()
         return ops.pairs_score(self.variant, float(self.beta), tuple(P.values()), hist, tgt, hreg, treg, aux, drop_p, seed,
                                getattr(self, "pairs_precision", "auto"))
@@ -79,9 +83,11 @@ class _NAISBase(nn.Module):
     def segmented_scores(self, batch: "ops.SegmentedPairs") -> torch.Tensor:
         """`attention_network` over a multi-user batch in the segmented layout (ops.SegmentedPairs: the rows of a user share
         one stored history, distances are formed in the kernel): pre-sigmoid scores [B], differentiable like the per-user
-        call.  One step over U users gives exactly the sum of the U single-user gradients (tests/test_gpu_segmented.py)."""
+        call.  One step over U users gives exactly the sum of the U single-user gradients (tests/test_gpu_segmented.py).  In train
+        mode the dropout classes apply dropout as `attention_network` does (the mask is indexed by the segmented cell)."""
+        drop_p, seed = self._draw_dropout()
         P = self._params()
-        return ops.pairs_score(self.variant, float(self.beta), tuple(P.values()), batch, None, None, None, None, 0.0, 0,
+        return ops.pairs_score(self.variant, float(self.beta), tuple(P.values()), batch, None, None, None, None, drop_p, seed,
                                getattr(self, "pairs_precision", "auto"))
 
     def fused_adagrad_step(self, optimizer: torch.optim.Adagrad, label, hist, tgt=None, hreg=None, treg=None, aux=None,
@@ -114,10 +120,7 @@ class _NAISBase(nn.Module):
             lr, eps = g["lr"], g["eps"]
             sums[name] = optimizer.state[P[name]]["sum"]
         pp = getattr(self, "pairs_precision", "auto")
-        drop = (0.0, 0, pp)
-        if self._dropout_on_l1 and self.training and self.drop.p > 0:
-            drop = (float(self.drop.p), int(torch.randint(0, 2 ** 62, (1,)).item()), pp)
-            self.last_dropout_seed = drop[1]
+        drop = (*self._draw_dropout(), pp)
         # ---- everything in one library call (nais_pairs_train_step) when the step is the reference's: mean / row-weighted BCE,
         # plain Adagrad on every parameter.  `one_call=False` on the model keeps the op-by-op path below (the parity tests compare).
         dense = {n: t for n, t in P.items() if n not in ops._TABLES}
@@ -157,14 +160,14 @@ class _NAISBase(nn.Module):
         positive, forward, BCELoss, backward, Adagrad step — for a whole list of users in ONE library call (`nais_train_users`):
         the same optimizer steps in the same order as `for u in uids: fused_adagrad_step(optimizer, *batcher.multi_user_batch([u],
         negative_num, seed + u))`, bit for bit, without the per-user Python work.  `batcher`: a batches.DeviceBatcher over the
-        train matrix.  Every class without dropout in train mode, the disentangled one included.  Returns the per-user losses
+        train matrix.  Every class, the disentangled one included.  In train mode the dropout classes draw one mask seed per
+        user with a history, in list order, as `torch.randint(0, 2**62, (n_steps,))`: torch's CPU generator gives the values of
+        n_steps single draws, so under the same `torch.manual_seed` the steps are the loop's.  Returns the per-user losses
         [len(uids)] on the device."""
         if not isinstance(optimizer, torch.optim.Adagrad):
             raise RuntimeError("train_users needs torch.optim.Adagrad (run.py:225)")
         if type(self.loss_func) is not nn.BCELoss or self.loss_func.reduction != "mean":
             raise RuntimeError("train_users: the reference's mean BCELoss")
-        if self._dropout_on_l1 and self.training and self.drop.p > 0:
-            raise RuntimeError("train_users: dropout variants go through fused_adagrad_step (a fresh dropout seed per step)")
         P = self._params()
         group_of = {id(p): g for g in optimizer.param_groups for p in g["params"]}
         groups = [group_of.get(id(t)) for t in P.values()]
@@ -176,14 +179,22 @@ class _NAISBase(nn.Module):
             raise RuntimeError("train_users: the tables / the MLP tensors must each share lr and eps")
         (lr_t, eps_t), (lr_d, eps_d) = next(iter(tg)), next(iter(dg))
         sums = {n: optimizer.state[t]["sum"] for n, t in P.items()}
+        hu = np.asarray(uids, dtype=np.int64).reshape(-1)
+        has_hist = np.asarray(batcher.indptr)[hu + 1] > np.asarray(batcher.indptr)[hu]
+        n_steps = int(has_hist.sum())
+        drop_p, drop_seeds = 0.0, None
+        if self._dropout_on_l1 and self.training and self.drop.p > 0 and n_steps:
+            drawn = torch.randint(0, 2 ** 62, (n_steps,))
+            drop_p, drop_seeds = float(self.drop.p), np.zeros(hu.size, dtype=np.uint64)
+            drop_seeds[has_hist] = drawn.numpy().astype(np.uint64)
+            self.last_dropout_seed = int(drawn[-1])
         optimizer.zero_grad(set_to_none=True)
         has_reg, has_co = "embed_region.weight" in P, ops.VARIANT_DIST[self.variant][0] != ops.DIST_NONE
         losses = ops.train_users(self.variant, float(self.beta), P, sums, sums, lr_t, eps_t, lr_d, eps_d, batcher.indptr, batcher.indices,
                                  batcher.entry_region if has_reg else None, batcher.entry_coords if has_co else None,
                                  batcher.region32 if has_reg else None, batcher.coords32 if has_co else None, uids, negative_num, seed,
                                  getattr(self, "pairs_precision", "auto") if isinstance(getattr(self, "pairs_precision", "auto"), str) else "auto",
-                                 center=batcher.center)
-        n_steps = int(sum(1 for u in np.asarray(uids).reshape(-1) if batcher.indptr[int(u) + 1] > batcher.indptr[int(u)]))
+                                 center=batcher.center, dropout_p=drop_p, dropout_seeds=drop_seeds)
         for t in P.values():
             optimizer.state[t]["step"] += n_steps
         self._plan_epoch = getattr(self, "_plan_epoch", 0) + 1

@@ -405,7 +405,8 @@ class _PairCall:
 
 def _forward_launch(c: _PairCall, want_mask: bool = True, presort: bool = False):
     """nais_pairs_forward -> (score, row_sum, parts, act_mask, presorted workspace): act_mask is the ReLU pattern the tcgen05
-    forward saves for the tcgen05 backward (int64 [B*H]; None when the FP32 forward runs or hid > 64).  With `presort`
+    forward saves for the tcgen05 backward (int64 [cells]; with dropout "active and kept"; None when the FP32 forward runs or
+    hid > 64).  With `presort`
     (one-branch variants) the call is nais_pairs_forward_presort and the last element is the backward workspace holding the
     sorted id lists for nais_pairs_backward_presorted; else None."""
     p, b, dev = c.p, c.b, c.dev
@@ -616,18 +617,26 @@ def pairs_train_step(variant: str, beta: float, P: Dict[str, torch.Tensor], tabl
 def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sums, dense_sums, lr_tables, eps_tables, lr_dense,
                 eps_dense, host_indptr, indices: torch.Tensor, entry_region: Optional[torch.Tensor],
                 entry_coords: Optional[torch.Tensor], poi_region: Optional[torch.Tensor], poi_coords: Optional[torch.Tensor],
-                users, num_ng: int, seed: int, pairs_precision: str = "auto", center: Tuple[float, float] = (0.0, 0.0)) -> torch.Tensor:
+                users, num_ng: int, seed: int, pairs_precision: str = "auto", center: Tuple[float, float] = (0.0, 0.0),
+                dropout_p: float = 0.0, dropout_seeds=None) -> torch.Tensor:
     """nais_train_users: the reference's schedule, one optimizer step per user (run.py:227-255), for a list of users in ONE library
     call — per user the device sampler over his CSR slice + the one-call training step, ~15 launches and no host work in between.
-    `host_indptr` / `users`: numpy int64 (host).  `center`: the (lat, lon) subtracted from `entry_coords` / `poi_coords`.  Updates
-    every tensor of `P` and the optimizer sums in place; returns the per-user losses [n] (device)."""
+    `host_indptr` / `users`: numpy int64 (host).  `center`: the (lat, lon) subtracted from `entry_coords` / `poi_coords`.
+    `dropout_p > 0`: train-mode dropout, the step of users[i] with mask seed `dropout_seeds[i]` (host, one per user; entries of
+    users without a history are ignored).  Updates every tensor of `P` and the optimizer sums in place; returns the per-user
+    losses [n] (device)."""
     import numpy as np
     dev = _need_cuda(indices, entry_region, entry_coords, poi_region, poi_coords, *P.values())
     hp = np.ascontiguousarray(np.asarray(host_indptr, dtype=np.int64))
     hu = np.ascontiguousarray(np.asarray(users, dtype=np.int64))
     if hu.size and (hu.min() < 0 or hu.max() + 1 >= hp.size):
         raise IndexError("train_users: user id outside the train matrix")
-    with _PairCall(dev, variant, beta, P, pairs_precision) as c:
+    ds = None
+    if dropout_p > 0:
+        ds = np.ascontiguousarray(np.asarray(dropout_seeds, dtype=np.uint64).reshape(-1))
+        if ds.size != hu.size:
+            raise RuntimeError("train_users: one dropout seed per user")
+    with _PairCall(dev, variant, beta, P, pairs_precision, (float(dropout_p), 0)) as c:
         o = _adagrad_struct(variant, P, table_sums, lr_tables, eps_tables, tables=True)
         d = _adagrad_struct(variant, P, dense_sums, lr_dense, eps_dense, tables=False)
         if indices.dtype != torch.int64 or not indices.is_contiguous():
@@ -638,10 +647,10 @@ def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sum
         pc = None if poi_coords is None else _f32(poi_coords)
         max_hist = int((hp[hu + 1] - hp[hu]).max()) if hu.size else 0
         losses = torch.empty(max(hu.size, 1), device=dev, dtype=torch.float32)
-        c.launch("nais_train_users_centred", hp.ctypes.data, int(hp.size) - 1, indices.data_ptr(), _ptr(er), _ptr(ec), _ptr(pr), _ptr(pc),
+        c.launch("nais_train_users_dropout", hp.ctypes.data, int(hp.size) - 1, indices.data_ptr(), _ptr(er), _ptr(ec), _ptr(pr), _ptr(pc),
                  hu.ctypes.data, int(hu.size), int(num_ng), int(seed) & (2 ** 64 - 1), C.byref(o), C.byref(d), losses.data_ptr(),
                  ws_bytes=c.query("nais_train_users_workspace_bytes", max(max_hist, 1), int(num_ng)),
-                 tail=(float(center[0]), float(center[1])))
+                 tail=(float(center[0]), float(center[1]), None if ds is None else ds.ctypes.data))
     return losses[: hu.size]
 
 
@@ -655,16 +664,22 @@ def pairs_forward_raw(variant: str, beta: float, P: Dict[str, torch.Tensor], his
 
 
 def dropout_keep_mask(seed: int, B: int, H: int, hid: int, p: float):
-    """The keep-mask the kernels use, on the host (numpy bool [B,H,hid]) — for tests / reproducing a step."""
+    """The keep-mask the kernels use for a dense [B,H] batch, on the host (numpy bool [B,H,hid]) — for tests / reproducing a step."""
+    return dropout_keep_mask_cells(seed, B * H, hid, p).reshape(B, H, hid)
+
+
+def dropout_keep_mask_cells(seed: int, n_cells: int, hid: int, p: float):
+    """The keep-mask of `n_cells` cells on the host (numpy bool [n_cells, hid]), indexed by the per-cell index of NaisPairs: b*H + h
+    for a dense batch, seg_cell_offsets[s] + (r - row_offsets[s]) * H_s + h for a segmented one (include/nais_b200.h)."""
     import numpy as np
-    idx = np.arange(B * H * hid, dtype=np.uint64)
+    idx = np.arange(n_cells * hid, dtype=np.uint64)
     with np.errstate(over="ignore"):
         z = np.uint64(seed) + idx * np.uint64(0x9E3779B97F4A7C15)
         z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
         z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
         z = z ^ (z >> np.uint64(31))
     t = min(int(float(np.float32(p)) * 4294967296.0), 0xFFFFFFFF)
-    return ((z >> np.uint64(32)) >= np.uint64(t)).reshape(B, H, hid)
+    return ((z >> np.uint64(32)) >= np.uint64(t)).reshape(n_cells, hid)
 
 
 # ----------------------------------------------------------------------------------------------------------------------
