@@ -434,6 +434,32 @@ NAIS_API int nais_hits_at_k(const int32_t* rec, int32_t n_users, int32_t k_rec, 
 NAIS_API int nais_powerlaw_logscore(const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin, int64_t poi_end, float a,
                            float b, float* out_logg, nais_stream_t stream);
 
+/* ---- geo re-ranking: the power-law mix of run.py:523-546 inside the full-rank top-k ----------------------------------------------
+ *   logG(u, j)  = sum_{h in history(u)} (ln a + b * ln max(0.01, d_km(h, j)))        (as nais_powerlaw_logscore)
+ *   M_u         = max_j logG(u, j) over the ranked candidates: the whole catalogue (every shard), minus the history when excluded
+ *   mixed(u, j) = (1 - alpha) * sigmoid(score(u, j)) + alpha * exp(logG(u, j) - M_u)
+ * The top-k is taken by `mixed` (desc, then id asc).  A history item that is not excluded includes its own h = j term (d = 0).
+ *
+ * nais_powerlaw_logmax writes out_logmax[n_users] = max over the candidates of [poi_begin, poi_end) (-inf for a user without
+ * candidates); the per-shard maxima of a range-sharded catalogue combine with a max.  It sums log G in the order of
+ * nais_powerlaw_logscore, so M_u equals the maximum of that output bit for bit.  Needs the coordinates of NaisCatalog and
+ * NaisUsers.  a <= 0 or a non-finite a / b -> NAIS_ERR_MODE.
+ *
+ * nais_fullrank_topk_geo_planned = nais_fullrank_topk_planned ranked by `mixed`: out_score (and the keys) hold mixed, not a
+ * pre-sigmoid score; the workspace is nais_fullrank_planned_workspace_bytes.  The tensor path runs the run-time-shape kernel
+ * (never the compile-time-shape or CTA-pair kernels); NAIS_PREC_FP32 takes a NULL plan.  a <= 0 or a non-finite a / b / alpha ->
+ * NAIS_ERR_MODE; geo, the coordinates or user_logmax missing -> NAIS_ERR_NULL (all checked before any CUDA call). */
+typedef struct NaisGeoMix {
+  float a, b, alpha;          /* power law a * d^b (a > 0) and the mixing weight (Args.powerlaw_weight) */
+  const float* user_logmax;   /* [n_users] device: M_u from nais_powerlaw_logmax over the whole ranked catalogue */
+} NaisGeoMix;
+NAIS_API int nais_powerlaw_logmax(const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin, int64_t poi_end, float a,
+                                  float b, int32_t exclude_history, float* out_logmax, nais_stream_t stream);
+NAIS_API int nais_fullrank_topk_geo_planned(const NaisParams* p, const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin,
+                                            int64_t poi_end, int32_t k, int32_t exclude_history, int32_t precision, const void* plan,
+                                            size_t plan_bytes, const NaisGeoMix* geo, uint64_t* out_keys, float* out_score,
+                                            int32_t* out_id, void* workspace, size_t workspace_bytes, nais_stream_t stream);
+
 /* Same scoring pass, but also writes every pre-sigmoid score: all_scores[n_users, poi_end-poi_begin] (history items are
  * scored with their own cell masked, like a training positive).  For parity checks of the fused path on small cases. */
 NAIS_API int nais_fullrank_scores(const NaisParams* p, const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin,

@@ -71,6 +71,10 @@ class NaisUsers(C.Structure):
                 ("n_users", C.c_int32)]
 
 
+class NaisGeoMix(C.Structure):
+    _fields_ = [("a", C.c_float), ("b", C.c_float), ("alpha", C.c_float), ("user_logmax", C.c_void_p)]
+
+
 # every symbol include/nais_b200.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "nais_abi_version": (C.c_int, []),
@@ -130,6 +134,12 @@ SYMBOLS = {
     "nais_fullrank_topk_planned": (C.c_int, [C.POINTER(NaisParams), C.POINTER(NaisCatalog), C.POINTER(NaisUsers), C.c_int64,
                                              C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "nais_powerlaw_logmax": (C.c_int, [C.POINTER(NaisCatalog), C.POINTER(NaisUsers), C.c_int64, C.c_int64, C.c_float, C.c_float,
+                                       C.c_int32, C.c_void_p, C.c_void_p]),
+    "nais_fullrank_topk_geo_planned": (C.c_int, [C.POINTER(NaisParams), C.POINTER(NaisCatalog), C.POINTER(NaisUsers), C.c_int64,
+                                                 C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t,
+                                                 C.POINTER(NaisGeoMix), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                                 C.c_void_p]),
     "nais_topk_merge_keys": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p]),
     "nais_poll_bad_index": (C.c_int, [C.c_void_p, C.c_void_p]),

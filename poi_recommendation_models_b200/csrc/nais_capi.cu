@@ -12,7 +12,7 @@ namespace nais {
 int launch_pairs_fwd(const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts, cudaStream_t stream);
 int launch_fullrank_fp32(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& users, int64_t poi_begin,
                          int64_t poi_end, int k, int exclude, float* out_score, int32_t* out_id, float* all_scores,
-                         void* ws, size_t ws_bytes, cudaStream_t stream);
+                         void* ws, size_t ws_bytes, cudaStream_t stream, const GeoMixArgs* geo = nullptr);
 int launch_topk_merge(const unsigned long long* in_keys, const float* in_score, const int32_t* in_id, int n_users,
                       int n_lists, int k, float* out_score, int32_t* out_id, cudaStream_t stream);
 int launch_topk_merge_keys_multi(const unsigned long long* keys, unsigned long long* scratch, int64_t user_stride, int64_t list_stride,
@@ -43,7 +43,8 @@ int fullrank_tc_prepare(const NaisParams& p, const NaisCatalog& cat, int64_t poi
                         size_t plan_bytes, cudaStream_t stream);
 int fullrank_tc_run(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& users, int64_t poi_begin, int64_t poi_end, int k,
                     int exclude, int precision, const void* plan, size_t plan_bytes, unsigned long long* out_keys, float* out_score,
-                    int32_t* out_id, float* all_scores, void* ws, size_t ws_bytes, cudaStream_t stream);
+                    int32_t* out_id, float* all_scores, void* ws, size_t ws_bytes, cudaStream_t stream,
+                    const GeoMixArgs* geo = nullptr);
 // nais_sampler.cu
 int launch_sample_batch(const int64_t* seg_offsets, const int64_t* hist, int n_seg, const int64_t* row_offsets, int num_ng, int item_num,
                         const int32_t* poi_region, const float* poi_coords, uint64_t seed, int max_hist, int64_t* tgt, float* label,
@@ -136,15 +137,15 @@ __global__ void fill_empty_topk_kernel(float* s, int32_t* id, size_t n) {
 // reference's Python set intersection (eval_metrics.py:40-42).
 // log of the power-law geographical score of powerLaw.py:85-92: G(u, j) = prod_{h in visited(u)} a * max(0.01, d(h, j))^b
 //   log G = sum_h (ln a + b * ln max(0.01, d_km(h, j)))      (a product of ~100 factors leaves fp32 / fp64 range; its log does not)
-// One thread per candidate, the user's history coordinates staged through shared memory in tiles of 256.
-__global__ void powerlaw_logscore_kernel(NaisCatalog cat, NaisUsers users, int64_t poi_begin, int64_t poi_end, float ln_a, float b,
-                                         float* __restrict__ out) {
+// One thread per candidate j (invalid threads compute a dummy), the user's history coordinates staged through shared memory in
+// tiles of 256; every thread of the block must call.  kHist: also report whether j is one of the user's history items.
+template <bool kHist>
+__device__ __forceinline__ float powerlaw_logg_block(const NaisCatalog& cat, const NaisUsers& users, int u, int64_t j, bool valid,
+                                                     float ln_a, float b, bool* in_hist) {
   __shared__ float s_la[256], s_lo[256], s_cos[256];
-  const int u = blockIdx.x;  // users on grid.x (no 65 535 limit), candidate blocks on grid.y
+  __shared__ int s_id[kHist ? 256 : 1];
   const int64_t hb = users.offsets[u];
   const int H = (int)(users.offsets[u + 1] - hb);
-  const int64_t j = poi_begin + (int64_t)blockIdx.y * blockDim.x + threadIdx.x;
-  const bool valid = j < poi_end;
   float cla = 0.f, clo = 0.f, ccos = 1.f;
   if (valid) {
     cla = __ldg(cat.coords + 2 * (j - cat.row_base));
@@ -152,6 +153,7 @@ __global__ void powerlaw_logscore_kernel(NaisCatalog cat, NaisUsers users, int64
     ccos = cosf((cat.center_lat + cla) * 0.017453292519943295f);
   }
   float acc = 0.f;
+  bool seen = false;
   for (int h0 = 0; h0 < H; h0 += 256) {
     __syncthreads();
     if (h0 + (int)threadIdx.x < H) {
@@ -159,15 +161,64 @@ __global__ void powerlaw_logscore_kernel(NaisCatalog cat, NaisUsers users, int64
       s_la[threadIdx.x] = la;
       s_lo[threadIdx.x] = lo;
       s_cos[threadIdx.x] = cosf((cat.center_lat + la) * 0.017453292519943295f);
+      if constexpr (kHist) s_id[threadIdx.x] = __ldg(users.items + hb + h0 + threadIdx.x);
     }
     __syncthreads();
     const int n = min(256, H - h0);
     for (int i = 0; i < n; ++i) {
-      const float d = fmaxf(0.01f, dist_km_f(cla, clo, s_la[i], s_lo[i], ccos, s_cos[i]));
-      acc += fmaf(b, logf(d), ln_a);
+      acc += powerlaw_log_term(dist_km_f(cla, clo, s_la[i], s_lo[i], ccos, s_cos[i]), ln_a, b);
+      if constexpr (kHist) seen = seen || (int64_t)s_id[i] == j;
     }
   }
+  if (in_hist) *in_hist = seen;
+  return acc;
+}
+
+__global__ void powerlaw_logscore_kernel(NaisCatalog cat, NaisUsers users, int64_t poi_begin, int64_t poi_end, float ln_a, float b,
+                                         float* __restrict__ out) {
+  const int u = blockIdx.x;  // users on grid.x (no 65 535 limit), candidate blocks on grid.y
+  const int64_t j = poi_begin + (int64_t)blockIdx.y * blockDim.x + threadIdx.x;
+  const bool valid = j < poi_end;
+  const float acc = powerlaw_logg_block<false>(cat, users, u, j, valid, ln_a, b, nullptr);
   if (valid) out[(size_t)u * (poi_end - poi_begin) + (j - poi_begin)] = acc;
+}
+
+// Atomic max of a float by its bit pattern: non-negative floats order like signed ints, negative ones reversed like unsigned
+// ints.  Exact, so the result does not depend on the order the blocks arrive in.
+__device__ __forceinline__ void atomic_max_float(float* addr, float v) {
+  if (v != v) return;
+  if (__float_as_int(v) >= 0) atomicMax(reinterpret_cast<int*>(addr), __float_as_int(v));
+  else atomicMin(reinterpret_cast<unsigned*>(addr), __float_as_uint(v));
+}
+
+__global__ void fill_float_kernel(float* out, int n, float v) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = v;
+}
+
+// M_u = max_j log G(u, j) over the candidates [poi_begin, poi_end) (minus the history when `exclude`), no [U, N] buffer:
+// blocks stride over the range, reduce in the block and fold into out[u] (filled with -inf first).
+__global__ void powerlaw_logmax_kernel(NaisCatalog cat, NaisUsers users, int64_t poi_begin, int64_t poi_end, float ln_a, float b,
+                                       int exclude, float* __restrict__ out) {
+  __shared__ float s_max[8];
+  const int u = blockIdx.x;
+  float m = -INFINITY;
+  for (int64_t j0 = poi_begin + (int64_t)blockIdx.y * blockDim.x; j0 < poi_end; j0 += (int64_t)gridDim.y * blockDim.x) {
+    const int64_t j = j0 + threadIdx.x;
+    const bool valid = j < poi_end;
+    bool in_hist = false;
+    const float acc = exclude ? powerlaw_logg_block<true>(cat, users, u, j, valid, ln_a, b, &in_hist)
+                              : powerlaw_logg_block<false>(cat, users, u, j, valid, ln_a, b, nullptr);
+    if (valid && !in_hist) m = fmaxf(m, acc);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < (int)(blockDim.x >> 5); ++w) m = fmaxf(m, s_max[w]);
+    if (m > -INFINITY) atomic_max_float(out + u, m);
+  }
 }
 
 __global__ void hits_at_k_kernel(const int32_t* __restrict__ rec, int n_users, int k_rec, const int64_t* __restrict__ po,
@@ -818,16 +869,28 @@ int nais_fullrank_prepare(const NaisParams* p, const NaisCatalog* cat, int64_t p
   return fullrank_tc_prepare(*p, *cat, poi_begin, poi_end, precision, plan, plan_bytes, static_cast<cudaStream_t>(stream));
 }
 
-int nais_fullrank_topk_planned(const NaisParams* p, const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin,
-                               int64_t poi_end, int32_t k, int32_t exclude_history, int32_t precision, const void* plan,
-                               size_t plan_bytes, uint64_t* out_keys, float* out_score, int32_t* out_id, void* workspace,
-                               size_t workspace_bytes, nais_stream_t stream) {
+// Geo re-ranking arguments (nais_fullrank_topk_geo_planned): checked before any CUDA call
+static int check_geo(const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin, int64_t poi_end, const NaisGeoMix* geo) {
+  if (!geo) return NAIS_ERR_NULL;
+  if (!(geo->a > 0.f) || !isfinite(geo->a) || !isfinite(geo->b) || !isfinite(geo->alpha)) return NAIS_ERR_MODE;
+  if (users->n_users > 0 && poi_end > poi_begin && (!cat->coords || !users->coords || !geo->user_logmax)) return NAIS_ERR_NULL;
+  return 0;
+}
+
+static int fullrank_topk_planned_impl(const NaisParams* p, const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin,
+                                      int64_t poi_end, int32_t k, int32_t exclude_history, int32_t precision, const void* plan,
+                                      size_t plan_bytes, const NaisGeoMix* geo, uint64_t* out_keys, float* out_score, int32_t* out_id,
+                                      void* workspace, size_t workspace_bytes, nais_stream_t stream) {
   int rc = check_fullrank(p, cat, users, poi_begin, poi_end, precision);
   if (rc) return rc;
   if (k < 1 || k > KCAP) return NAIS_ERR_SHAPE;
+  if (geo && (rc = check_geo(cat, users, poi_begin, poi_end, geo))) return rc;
   if (users->n_users == 0) return 0;
   if ((!out_score) != (!out_id) || (!out_score && !out_keys) || !workspace) return NAIS_ERR_NULL;
   if (!aligned16(workspace)) return NAIS_ERR_ALIGN;
+  GeoMixArgs gm = {};
+  if (geo) gm = GeoMixArgs{logf(geo->a), geo->b, geo->alpha, geo->user_logmax};
+  const GeoMixArgs* gp = geo ? &gm : nullptr;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   unsigned long long* keys = reinterpret_cast<unsigned long long*>(out_keys);
   const size_t n = (size_t)users->n_users * k;
@@ -844,7 +907,7 @@ int nais_fullrank_topk_planned(const NaisParams* p, const NaisCatalog* cat, cons
   }
   if ((precision & NAIS_PREC_MASK) != NAIS_PREC_FP32)
     return fullrank_tc_run(*p, *cat, *users, poi_begin, poi_end, k, exclude_history, precision, plan, plan_bytes, keys, out_score,
-                           out_id, nullptr, workspace, workspace_bytes, st);
+                           out_id, nullptr, workspace, workspace_bytes, st, gp);
   // FP32 kernel: no plan.  It writes score / id; keys (if wanted) are re-packed from them.
   float* sc = out_score;
   int32_t* id = out_id;
@@ -858,11 +921,28 @@ int nais_fullrank_topk_planned(const NaisParams* p, const NaisCatalog* cat, cons
     rest += head;
     rest_bytes -= head;
   }
-  rc = launch_fullrank_fp32(*p, *cat, *users, poi_begin, poi_end, k, exclude_history, sc, id, nullptr, rest, rest_bytes, st);
+  rc = launch_fullrank_fp32(*p, *cat, *users, poi_begin, poi_end, k, exclude_history, sc, id, nullptr, rest, rest_bytes, st, gp);
   if (rc || !keys) return rc;
   pack_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sc, id, n, keys);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
+}
+
+int nais_fullrank_topk_planned(const NaisParams* p, const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin,
+                               int64_t poi_end, int32_t k, int32_t exclude_history, int32_t precision, const void* plan,
+                               size_t plan_bytes, uint64_t* out_keys, float* out_score, int32_t* out_id, void* workspace,
+                               size_t workspace_bytes, nais_stream_t stream) {
+  return fullrank_topk_planned_impl(p, cat, users, poi_begin, poi_end, k, exclude_history, precision, plan, plan_bytes, nullptr, out_keys,
+                                    out_score, out_id, workspace, workspace_bytes, stream);
+}
+
+int nais_fullrank_topk_geo_planned(const NaisParams* p, const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin,
+                                   int64_t poi_end, int32_t k, int32_t exclude_history, int32_t precision, const void* plan,
+                                   size_t plan_bytes, const NaisGeoMix* geo, uint64_t* out_keys, float* out_score, int32_t* out_id,
+                                   void* workspace, size_t workspace_bytes, nais_stream_t stream) {
+  if (!geo) return NAIS_ERR_NULL;
+  return fullrank_topk_planned_impl(p, cat, users, poi_begin, poi_end, k, exclude_history, precision, plan, plan_bytes, geo, out_keys,
+                                    out_score, out_id, workspace, workspace_bytes, stream);
 }
 
 int nais_topk_merge_keys(const uint64_t* in_keys, int64_t user_stride, int64_t list_stride, int32_t n_users, int32_t n_lists,
@@ -953,6 +1033,26 @@ int nais_powerlaw_logscore(const NaisCatalog* cat, const NaisUsers* users, int64
   dim3 grid((unsigned)users->n_users, (unsigned)((poi_end - poi_begin + 255) / 256));
   powerlaw_logscore_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(*cat, *users, poi_begin, poi_end, logf(a), b, out_logg);
   NAIS_COUNT_LAUNCH(1);
+  return (int)cudaGetLastError();
+}
+
+int nais_powerlaw_logmax(const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin, int64_t poi_end, float a, float b,
+                         int32_t exclude_history, float* out_logmax, nais_stream_t stream) {
+  if (!cat || !users) return NAIS_ERR_NULL;
+  if (users->n_users < 0 || poi_begin < cat->row_base || poi_end < poi_begin || poi_end > cat->row_base + cat->n_rows) return NAIS_ERR_SHAPE;
+  if (!(a > 0.f) || !isfinite(a) || !isfinite(b)) return NAIS_ERR_MODE;
+  if (users->n_users == 0) return 0;
+  if (!out_logmax || !users->offsets) return NAIS_ERR_NULL;
+  if (poi_end > poi_begin && (!cat->coords || !users->coords || (exclude_history && !users->items))) return NAIS_ERR_NULL;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  fill_float_kernel<<<(users->n_users + 255) / 256, 256, 0, st>>>(out_logmax, users->n_users, -INFINITY);
+  NAIS_COUNT_LAUNCH(1);
+  if (poi_end > poi_begin) {
+    const int64_t blocks = (poi_end - poi_begin + 255) / 256;
+    dim3 grid((unsigned)users->n_users, (unsigned)(blocks < 64 ? blocks : 64));
+    powerlaw_logmax_kernel<<<grid, 256, 0, st>>>(*cat, *users, poi_begin, poi_end, logf(a), b, exclude_history ? 1 : 0, out_logmax);
+    NAIS_COUNT_LAUNCH(1);
+  }
   return (int)cudaGetLastError();
 }
 

@@ -190,4 +190,18 @@ __device__ __forceinline__ float dist_km_f(float lat1, float lon1, float lat2, f
   return 2.f * 6371.f * asinf(fminf(1.f, sqrtf(h)));
 }
 
+// One history item's term of the power-law log score log G(u, j) = sum_h (ln a + b * ln max(0.01, d_km(h, j)))
+// (powerLaw.py:85-92 in log space: a product of ~100 factors leaves the fp32 range, its log does not).  Every kernel that
+// forms log G adds these terms in history order, so their sums agree bit for bit.
+__device__ __forceinline__ float powerlaw_log_term(float km, float ln_a, float b) { return fmaf(b, logf(fmaxf(0.01f, km)), ln_a); }
+
+// Geo re-ranking (NaisGeoMix): mixed = (1 - alpha) * sigmoid(score) + alpha * exp(log G - M_u)
+struct GeoMixArgs {
+  float ln_a, b, alpha;
+  const float* user_logmax;  // [n_users] M_u
+};
+__device__ __forceinline__ float geo_mixed(float score, float logg, float logmax, float alpha) {
+  return (1.f - alpha) * sigmoidf_exact(score) + alpha * expf(logg - logmax);
+}
+
 }  // namespace nais

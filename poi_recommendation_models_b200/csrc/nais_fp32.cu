@@ -373,8 +373,12 @@ struct FullrankArgs {
   float* all_scores;  // optional [n_users, poi_end - poi_begin]
   int stage_p;        // 1: candidate vectors staged in smem (embed_size <= 128); 0: re-read from the tables (L1/L2) per history item
   int hc;             // history rows staged per chunk (HC, smaller when shared memory is tight)
+  GeoMixArgs geo;     // kGeo: rank by the power-law mix (nais_fullrank_topk_geo_planned)
 };
 
+// kGeo: every cell also adds its power-law term ln a + b ln max(0.01, d_km) to log G (in history order, as
+// nais_powerlaw_logscore), and the candidate is ranked by geo_mixed(score, log G, M_u) instead of its score.
+template <bool kGeo>
 __global__ void __launch_bounds__(NT, 2) fullrank_fp32_kernel(const __grid_constant__ FullrankArgs A) {
   extern __shared__ __align__(16) float smem[];
   const NaisParams& p = A.p;
@@ -416,12 +420,12 @@ __global__ void __launch_bounds__(NT, 2) fullrank_fp32_kernel(const __grid_const
     const bool jvalid = j < A.poi_end;
     const int64_t jl = j - A.cat.row_base;
     float cla = 0.f, clo = 0.f, ccos = 1.f;
-    if (jvalid && geo) {
+    if (jvalid && (geo || kGeo)) {
       cla = __ldg(A.cat.coords + jl * 2);
       clo = __ldg(A.cat.coords + jl * 2 + 1);
-      if (km_mode) ccos = cosf((A.cat.center_lat + cla) * 0.017453292519943295f);
+      if (km_mode || kGeo) ccos = cosf((A.cat.center_lat + cla) * 0.017453292519943295f);
     }
-    float score = 0.f;
+    float score = 0.f, logg = 0.f;
     bool excluded = false;
     for (int bi = 0; bi < p.n_branch; ++bi) {
       const NaisBranch& br = p.branch[bi];
@@ -453,7 +457,7 @@ __global__ void __launch_bounds__(NT, 2) fullrank_fp32_kernel(const __grid_const
         if (tid < hn) {
           const int64_t e = h_begin + h0 + tid;
           hid_s[tid] = __ldg(A.users.items + e);
-          if (geo) {
+          if (geo || kGeo) {
             hco[2 * tid] = __ldg(A.users.coords + 2 * e);
             hco[2 * tid + 1] = __ldg(A.users.coords + 2 * e + 1);
           }
@@ -490,6 +494,13 @@ __global__ void __launch_bounds__(NT, 2) fullrank_fp32_kernel(const __grid_const
           tile_logits(br, bi, p.hid, D, lanes, s, resident, DropCtx{0u, 1.f, 0ull, 0});
           if (tid < TC) {
             const bool m = (int64_t)hid_s[hh] != j;
+            if constexpr (kGeo) {
+              if (bi == 0) {  // every cell, the h = j one included; once per candidate, not per branch
+                const float hla = hco[2 * hh], hlo = hco[2 * hh + 1];
+                const float km = dist_km_f(cla, clo, hla, hlo, ccos, cosf((A.cat.center_lat + hla) * 0.017453292519943295f));
+                logg += powerlaw_log_term(km, A.geo.ln_a, A.geo.b);
+              }
+            }
             if (m) {
               float a = s.a[cell];
               if (km_mode) {  // logit += dist_km * sum_d embed_distance[bucket] (haversine from centred coordinates)
@@ -514,6 +525,7 @@ __global__ void __launch_bounds__(NT, 2) fullrank_fp32_kernel(const __grid_const
       if (tid < TC) score += sumES / powf(sumE, p.beta);
     }
     if (tid < TC) {
+      if constexpr (kGeo) score = geo_mixed(score, logg, __ldg(A.geo.user_logmax + u), A.geo.alpha);
       if (A.all_scores && jvalid) A.all_scores[(size_t)u * range + (j - A.poi_begin)] = score;
       const bool keep = jvalid && !(A.exclude && excluded);
       keys[KCAP + cell] = keep ? make_key(score, (int)j) : 0ull;
@@ -711,9 +723,10 @@ int launch_topk_merge_keys_multi(const unsigned long long* keys, unsigned long l
 
 int launch_fullrank_fp32(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& users, int64_t poi_begin,
                          int64_t poi_end, int k, int exclude, float* out_score, int32_t* out_id, float* all_scores,
-                         void* ws, size_t ws_bytes, cudaStream_t stream) {
+                         void* ws, size_t ws_bytes, cudaStream_t stream, const GeoMixArgs* geo) {
   if (users.n_users == 0 || poi_end <= poi_begin) return 0;
   FullrankArgs A;
+  A.geo = geo ? *geo : GeoMixArgs{};
   A.p = p;
   A.cat = cat;
   A.users = users;
@@ -729,10 +742,11 @@ int launch_fullrank_fp32(const NaisParams& p, const NaisCatalog& cat, const Nais
   if (A.n_splits > 1 && ws_bytes < (size_t)users.n_users * A.n_splits * k * sizeof(unsigned long long)) return NAIS_ERR_WORKSPACE;
   const size_t smem = fullrank_fp32_smem(p, A.stage_p, A.hc);
   if (smem > 227 * 1024) return NAIS_ERR_SHAPE;
-  cudaError_t e = cudaFuncSetAttribute(fullrank_fp32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  void (*kern)(const FullrankArgs) = geo ? fullrank_fp32_kernel<true> : fullrank_fp32_kernel<false>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
   dim3 grid(users.n_users, A.n_splits);
-  fullrank_fp32_kernel<<<grid, NT, smem, stream>>>(A);
+  kern<<<grid, NT, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   e = cudaGetLastError();
   if (e != cudaSuccess) return (int)e;

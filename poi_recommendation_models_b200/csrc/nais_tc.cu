@@ -473,6 +473,7 @@ struct MainArgs {
   int64_t max_chunks;             // chunk slots the operand image holds (users beyond it are truncated, never read out of bounds)
   int gate;                       // -1: one pass scores every user; 0 / 1: the SPLIT / MIX pass of NAIS_PREC_TC_AUTO
   const int* pass_flags;          // [2] raised by pack_users_kernel for every pass that has users (gate >= 0)
+  GeoMixArgs geo;                 // kGeo kernels: rank by the power-law mix (nais_fullrank_topk_geo_planned)
 };
 
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 512;" ::: "memory"); }
@@ -508,7 +509,10 @@ __device__ __forceinline__ unsigned long long warp_fold_top32(unsigned long long
 // immediate; the generic issuer spends ~15 instructions per MMA, which paces the kernel once a step is 9 MMAs) and the
 // specialised epilogue step loop (needs kSinglePart and kHch == 2).
 // kS: the static shape D = hid = kS of kFix 1 / 2 (64: the headline workload; 32: the small end of the C5 sweep).
-template <bool kSinglePart, int kHch, int kFix, int kS = 64>
+// kGeo (run-time-shape kernels only, kFix 0 / 4): every cell also adds its power-law term ln a + b ln max(0.01, d_km) to a
+// per-candidate log G partial (same exactly-once guard and `comb` combination as sumE / sumES, the h = j cell included), and the
+// item epilogue ranks by geo_mixed(score, log G, M_u).  Extra shared memory: geo_extra_smem.
+template <bool kSinglePart, int kHch, int kFix, int kS = 64, bool kGeo = false>
 __global__ void __launch_bounds__(THREADS, 1) fullrank_tc_kernel(const __grid_constant__ MainArgs A) {
   // kFix == 5 / 6: kFix 1 / 2 on CTA PAIRS (cta_group::2): the two CTAs of a cluster score the same user against two neighbouring
   // groups of candidate tiles with ONE M = 256 MMA per step — each supplies its 128 candidates (A) and HALF of the user's chunk (B)
@@ -520,6 +524,10 @@ __global__ void __launch_bounds__(THREADS, 1) fullrank_tc_kernel(const __grid_co
   // kFix == 3: D = hid = 128 (the reference's default, run.py:837-838) in SPLIT / MIX: the generic code paths below with the
   // shape constants known at compile time, so the K-part / K-step loops of the issuer unroll and its descriptors fold
   constexpr bool kD128 = kFix == 3;
+  static_assert(!kGeo || kFix == 0 || kFix == 4, "geo mode lives in the run-time-shape epilogue");
+  // `comb` arrays per partial set (sumE, sumES, excl [, log G]) and its tile stride: D > 64 aliases it on the 16 KB of A_ext + zero,
+  // where 4 arrays fit only at the tpc <= 2 those kernels run with
+  constexpr int kCombA = kGeo ? 4 : 3, kCombT = (kGeo && !kSinglePart) ? 2 : TPC;
   extern __shared__ __align__(128) unsigned char smem[];
   const Geo& g = A.g;
   unsigned char* sA = smem;
@@ -530,7 +538,7 @@ __global__ void __launch_bounds__(THREADS, 1) fullrank_tc_kernel(const __grid_co
   // item-end partial sums [3 partial sets][3 arrays][TPC][TM] = 13.5 KB.  D <= 64: private region.  D > 64 (smem is full):
   // ALIASES A_ext + zero (16 KB), only touched between the item-end barriers, then re-initialised.
   float* comb = kSinglePart ? reinterpret_cast<float*>(keys + SORTN) : reinterpret_cast<float*>(sE);
-  int* hm_id = reinterpret_cast<int*>(reinterpret_cast<unsigned char*>(keys + SORTN) + (kSinglePart ? 9 * TPC * TM * 4 : 0));  // [HMETA]
+  int* hm_id = reinterpret_cast<int*>(reinterpret_cast<unsigned char*>(keys + SORTN) + (kSinglePart ? 3 * kCombA * TPC * TM * 4 : 0));  // [HMETA]
   float* hm_la = reinterpret_cast<float*>(hm_id + HMETA);
   float* hm_lo = hm_la + HMETA;
   float* xch = hm_lo + HMETA;                                                   // [2][3][TM] partner-warp exchange (hch = 1; 3 senders when hsplit = 2)
@@ -922,26 +930,27 @@ __global__ void __launch_bounds__(THREADS, 1) fullrank_tc_kernel(const __grid_co
       epi_bar();
       for (int i = tid; i < H && i < HMETA; i += EPI_THREADS) {
         hm_id[i] = __ldg(A.users.items + hb + i);
-        hm_la[i] = geo ? __ldg(A.users.coords + 2 * (hb + i)) : 0.f;
-        hm_lo[i] = geo ? __ldg(A.users.coords + 2 * (hb + i) + 1) : 0.f;
+        hm_la[i] = (geo || kGeo) ? __ldg(A.users.coords + 2 * (hb + i)) : 0.f;
+        hm_lo[i] = (geo || kGeo) ? __ldg(A.users.coords + 2 * (hb + i) + 1) : 0.f;
         if constexpr (!kFastEpi)
-          if (g.km) hm_cos[i] = cosf((A.cat.center_lat + hm_la[i]) * 0.017453292519943295f);
+          if (g.km || kGeo) hm_cos[i] = cosf((A.cat.center_lat + hm_la[i]) * 0.017453292519943295f);
       }
       // candidates of this thread's row in the item's tiles
-      float clat[TPC], clon[TPC], ccos[TPC], sumE[TPC], sumES[TPC];
+      float clat[TPC], clon[TPC], ccos[TPC], sumE[TPC], sumES[TPC], sumL[TPC];
       int64_t jid[TPC];
       bool excl[TPC];
 #pragma unroll
       for (int t = 0; t < TPC; ++t) {
         jid[t] = t < tpc ? A.poi_begin + ((int64_t)grp * tpc + t) * TM + r : A.poi_end;
         const bool v = jid[t] < A.poi_end;
-        clat[t] = (v && geo) ? __ldg(A.cat.coords + 2 * (jid[t] - A.cat.row_base)) : 0.f;
-        clon[t] = (v && geo) ? __ldg(A.cat.coords + 2 * (jid[t] - A.cat.row_base) + 1) : 0.f;
+        clat[t] = (v && (geo || kGeo)) ? __ldg(A.cat.coords + 2 * (jid[t] - A.cat.row_base)) : 0.f;
+        clon[t] = (v && (geo || kGeo)) ? __ldg(A.cat.coords + 2 * (jid[t] - A.cat.row_base) + 1) : 0.f;
         ccos[t] = 1.f;
         if constexpr (!kFastEpi)
-          if (g.km) ccos[t] = cosf((A.cat.center_lat + clat[t]) * 0.017453292519943295f);
+          if (g.km || kGeo) ccos[t] = cosf((A.cat.center_lat + clat[t]) * 0.017453292519943295f);
         sumE[t] = 0.f;
         sumES[t] = 0.f;
+        sumL[t] = 0.f;
         excl[t] = false;
       }
       epi_bar();
@@ -1198,6 +1207,24 @@ __global__ void __launch_bounds__(THREADS, 1) fullrank_tc_kernel(const __grid_co
           const float a = (__uint_as_float(aux[1]) + asum) * sc.inv_sigma;
           if (h < H && (hch == 2 || hs == 0) && (hsplit == 1 || egrp == 0)) {
             const int64_t j = t == 0 ? jid[0] : (t == 1 ? jid[1] : jid[2]);
+            if constexpr (kGeo) {  // every cell once, the h = j cell included
+              float hla, hlo, hcs;
+              if (h < HMETA) {
+                hla = hm_la[h];
+                hlo = hm_lo[h];
+                hcs = hm_cos[h];
+              } else {
+                hla = __ldg(A.users.coords + 2 * (hb + h));
+                hlo = __ldg(A.users.coords + 2 * (hb + h) + 1);
+                hcs = cosf((A.cat.center_lat + hla) * 0.017453292519943295f);
+              }
+              const float cla = t == 0 ? clat[0] : (t == 1 ? clat[1] : clat[2]), clo = t == 0 ? clon[0] : (t == 1 ? clon[1] : clon[2]);
+              const float ccs = t == 0 ? ccos[0] : (t == 1 ? ccos[1] : ccos[2]);
+              const float lt = powerlaw_log_term(dist_km_f(cla, clo, hla, hlo, ccs, hcs), A.geo.ln_a, A.geo.b);
+              if (t == 0) sumL[0] += lt;
+              else if (t == 1) sumL[1] += lt;
+              else sumL[2] += lt;
+            }
             if ((int64_t)hist_id != j) {
               float a_km = a;
               if (g.km) {  // logit += dist_km * coefficient (haversine from centred coordinates, as the FP32 kernel forms it)
@@ -1236,27 +1263,32 @@ __global__ void __launch_bounds__(THREADS, 1) fullrank_tc_kernel(const __grid_co
       if (!kSinglePart) epi_bar();  // every group is past its last step: all MMAs are complete, A_ext + zero may hold `comb`
       if (part != 0) {
 #pragma unroll
-        for (int t2 = 0; t2 < TPC; ++t2) {
-          comb[((part - 1) * 3 + 0) * TPC * TM + t2 * TM + r] = sumE[t2];
-          comb[((part - 1) * 3 + 1) * TPC * TM + t2 * TM + r] = sumES[t2];
-          comb[((part - 1) * 3 + 2) * TPC * TM + t2 * TM + r] = excl[t2] ? 1.f : 0.f;
+        for (int t2 = 0; t2 < kCombT; ++t2) {
+          comb[((part - 1) * kCombA + 0) * kCombT * TM + t2 * TM + r] = sumE[t2];
+          comb[((part - 1) * kCombA + 1) * kCombT * TM + t2 * TM + r] = sumES[t2];
+          comb[((part - 1) * kCombA + 2) * kCombT * TM + t2 * TM + r] = excl[t2] ? 1.f : 0.f;
+          if constexpr (kGeo) comb[((part - 1) * kCombA + 3) * kCombT * TM + t2 * TM + r] = sumL[t2];
         }
       }
       epi_bar();
       if (part == 0) {
 #pragma unroll
         for (int t2 = 0; t2 < TPC; ++t2) {
-          float E = sumE[t2], ES = sumES[t2];
+          float E = sumE[t2], ES = sumES[t2], Lg = sumL[t2];
           bool ex = excl[t2];
+          if (t2 < kCombT) {  // (kCombT < TPC: tile t2 does not exist in this kernel)
 #pragma unroll
-          for (int q = 0; q < 3; ++q) {
-            E += comb[(q * 3 + 0) * TPC * TM + t2 * TM + r];
-            ES += comb[(q * 3 + 1) * TPC * TM + t2 * TM + r];
-            ex = ex || comb[(q * 3 + 2) * TPC * TM + t2 * TM + r] != 0.f;
+            for (int q = 0; q < 3; ++q) {
+              E += comb[(q * kCombA + 0) * kCombT * TM + t2 * TM + r];
+              ES += comb[(q * kCombA + 1) * kCombT * TM + t2 * TM + r];
+              ex = ex || comb[(q * kCombA + 2) * kCombT * TM + t2 * TM + r] != 0.f;
+              if constexpr (kGeo) Lg += comb[(q * kCombA + 3) * kCombT * TM + t2 * TM + r];
+            }
           }
           float score = ES / powf(E, beta);
           const bool valid = jid[t2] < A.poi_end;
           if (A.score_in && valid) score += A.score_in[(size_t)u * (A.poi_end - A.poi_begin) + (jid[t2] - A.poi_begin)];
+          if constexpr (kGeo) score = geo_mixed(score, Lg, __ldg(A.geo.user_logmax + u), A.geo.alpha);
           if (A.all_scores && valid) A.all_scores[(size_t)u * (A.poi_end - A.poi_begin) + (jid[t2] - A.poi_begin)] = score;
           kreg[t2] = (valid && !(A.exclude && ex)) ? make_key(score, (int)jid[t2]) : 0ull;
           if (!small_k) keys[t2 * TM + r] = kreg[t2];
@@ -1544,10 +1576,21 @@ static MainKernel pick_kernel(const tc::Geo& gg, bool generic) {
   return tc::fullrank_tc_kernel<false, 1, 0>;
 }
 
+// Geo re-ranking (MainArgs::geo) runs the run-time-shape kernels only, like NAIS_DIST_KM: the compile-time-shape and CTA-pair
+// kernels have no geo variant.  Extra shared memory: the fourth `comb` array of the D <= 64 kernels (private region) and the
+// staged cos(latitude) of the history items where NAIS_DIST_KM has not already reserved it.
+static MainKernel pick_geo_kernel(const tc::Geo& gg) {
+  if (gg.kp == 1) return gg.hch == 2 ? tc::fullrank_tc_kernel<true, 2, 0, 64, true> : tc::fullrank_tc_kernel<true, 1, 0, 64, true>;
+  if (gg.tpc == 1) return gg.hch == 2 ? tc::fullrank_tc_kernel<false, 2, 4, 64, true> : tc::fullrank_tc_kernel<false, 1, 4, 64, true>;
+  return gg.hch == 2 ? tc::fullrank_tc_kernel<false, 2, 0, 64, true> : tc::fullrank_tc_kernel<false, 1, 0, 64, true>;
+}
+static int geo_extra_smem(const tc::Geo& gg) { return (gg.kp == 1 ? 3 * tc::TPC * tc::TM * 4 : 0) + (gg.km ? 0 : tc::HMETA * 4); }
+
 // Per user batch: user operand image -> scoring pass(es) -> merge of the per-item lists.
 static int run_1(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& users, int64_t poi_begin, int64_t poi_end, int k,
                  int exclude, int precision, const void* plan, size_t plan_bytes, unsigned long long* out_keys, float* out_score,
-                 int32_t* out_id, float* all_scores, const float* score_in, bool merge, void* ws, size_t ws_bytes, cudaStream_t stream) {
+                 int32_t* out_id, float* all_scores, const float* score_in, bool merge, void* ws, size_t ws_bytes, cudaStream_t stream,
+                 const GeoMixArgs* geo = nullptr) {
   if (users.n_users == 0 || poi_end <= poi_begin) return 0;
   int sms;
   int rc = check_arch(sms);
@@ -1576,7 +1619,11 @@ static int run_1(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& u
   const bool generic = (precision & NAIS_PREC_FLAG_GENERIC) != 0;
   // CTA pairs need two co-scheduled SMs of a TPC with the kernel's shared memory each: asked once per device (a partitioned GPU may
   // not offer any); without them the one-CTA kernels run on the same plan (its candidate image is a superset)
-  bool use_pair = L.pair;
+  bool use_pair = L.pair && !geo;
+  if (geo) {
+    if (L.g.smem_bytes + geo_extra_smem(L.g) > 227 * 1024 || (L.two_pass && L.gs.smem_bytes + geo_extra_smem(L.gs) > 227 * 1024))
+      return NAIS_ERR_SHAPE;
+  }
   if (use_pair) {
     static int pair_ok[64];  // 0 unknown, 1 yes, -1 no
     int dev = 0;
@@ -1633,8 +1680,10 @@ static int run_1(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& u
     A.max_chunks = max_chunks;
     A.gate = gate;
     A.pass_flags = pass_flags;
-    MainKernel kern = pick_kernel(gg, generic);
-    cudaError_t e2 = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, gg.smem_bytes);
+    A.geo = geo ? *geo : GeoMixArgs{};
+    MainKernel kern = geo ? pick_geo_kernel(gg) : pick_kernel(gg, generic);
+    const int smem = gg.smem_bytes + (geo ? geo_extra_smem(gg) : 0);
+    cudaError_t e2 = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e2 != cudaSuccess) return (int)e2;
     if (gg.pair) {  // one cluster of two CTAs (the two SMs of a TPC) per pair item
       const int pairs = (int)(A.n_items < sms / 2 ? A.n_items : sms / 2);
@@ -1655,7 +1704,7 @@ static int run_1(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& u
       return e2 == cudaSuccess ? 0 : (int)e2;
     }
     const int grid = (int)(A.n_items < sms ? A.n_items : sms);
-    kern<<<grid, tc::THREADS, gg.smem_bytes, stream>>>(A);
+    kern<<<grid, tc::THREADS, smem, stream>>>(A);
     NAIS_COUNT_LAUNCH(1);
     e2 = cudaGetLastError();
     return e2 == cudaSuccess ? 0 : (int)e2;
@@ -1676,11 +1725,11 @@ static int run_1(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& u
 
 int fullrank_tc_run(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& users, int64_t poi_begin, int64_t poi_end, int k,
                     int exclude, int precision, const void* plan, size_t plan_bytes, unsigned long long* out_keys, float* out_score,
-                    int32_t* out_id, float* all_scores, void* ws, size_t ws_bytes, cudaStream_t stream) {
+                    int32_t* out_id, float* all_scores, void* ws, size_t ws_bytes, cudaStream_t stream, const GeoMixArgs* geo) {
   if (users.n_users == 0 || poi_end <= poi_begin) return 0;
   if (p.n_branch == 1)
     return run_1(p, cat, users, poi_begin, poi_end, k, exclude, precision, plan, plan_bytes, out_keys, out_score, out_id, all_scores,
-                 nullptr, true, ws, ws_bytes, stream);
+                 nullptr, true, ws, ws_bytes, stream, geo);
   const size_t sbytes = branch_scores_bytes(p, users.n_users, poi_begin, poi_end);
   if (!plan || ws_bytes < sbytes + 512) return NAIS_ERR_WORKSPACE;
   float* sbuf = reinterpret_cast<float*>(ws);  // running sum of the branch scores
@@ -1693,7 +1742,8 @@ int fullrank_tc_run(const NaisParams& p, const NaisCatalog& cat, const NaisUsers
     if (plan_bytes < off + b) return NAIS_ERR_WORKSPACE;
     const bool last = bi == p.n_branch - 1;
     const int rc = run_1(q, cat, users, poi_begin, poi_end, k, exclude, precision, reinterpret_cast<const unsigned char*>(plan) + off, b,
-                         out_keys, out_score, out_id, last ? all_scores : sbuf, bi ? sbuf : nullptr, last, rest, ws_bytes - sbytes, stream);
+                         out_keys, out_score, out_id, last ? all_scores : sbuf, bi ? sbuf : nullptr, last, rest, ws_bytes - sbytes, stream,
+                         last ? geo : nullptr);  // the mix needs the summed score: the last pass only
     if (rc) return rc;
     off += b;
   }
@@ -1711,7 +1761,7 @@ int launch_fullrank_tc(const NaisParams& p, const NaisCatalog& cat, const NaisUs
   int rc = fullrank_tc_prepare(p, cat, poi_begin, poi_end, precision, ws, plan_bytes, stream);
   if (rc) return rc;
   return fullrank_tc_run(p, cat, users, poi_begin, poi_end, k, exclude, precision, ws, plan_bytes, nullptr, out_score, out_id,
-                         all_scores, reinterpret_cast<unsigned char*>(ws) + plan_bytes, ws_bytes - plan_bytes, stream);
+                         all_scores, reinterpret_cast<unsigned char*>(ws) + plan_bytes, ws_bytes - plan_bytes, stream, nullptr);
 }
 
 }  // namespace nais

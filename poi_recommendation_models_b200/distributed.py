@@ -65,11 +65,17 @@ class ShardedRanker:
     CPU (tests/test_distributed_cpu.py); the defaults are the CUDA ops.  rank = user_slice * catalogue_shards + shard.
 
     local_topk(users, k, lo, hi, precision) -> keys [U, k] int64, or (score [U,k], id [U,k]) which is packed here
-    merge(keys [L, U, k]) -> (score [U, k], id [U, k])"""
+    merge(keys [L, U, k]) -> (score [U, k], id [U, k])
+
+    Geo re-ranking (`topk(..., geo=(a, b, alpha))`) adds one step before the local top-k: every rank takes the power-law
+    maximum M_u over its own range, and ONE all_reduce(MAX) of a [gu * per] vector — each rank fills only its own user slice,
+    -inf elsewhere — leaves every rank the maximum over the whole catalogue for the users it scores.
+    local_logmax(users, lo, hi, a, b) -> M [U] float32
+    local_topk(users, k, lo, hi, precision, geo: ops.GeoMix) -> as above, ranked by the mix"""
 
     def __init__(self, model, rank: int = 0, world: int = 1, local_topk: Optional[Callable] = None,
                  merge: Optional[Callable] = None, min_shard_pois: int = 32768, slice_users: Optional[Callable] = None,
-                 grid: Optional[Tuple[int, int]] = None):
+                 grid: Optional[Tuple[int, int]] = None, local_logmax: Optional[Callable] = None):
         self.model, self.rank, self.world = model, rank, world
         self.n = model.item_num
         self.gc, self.gu = grid if grid is not None else grid_shape(self.n, world, min_shard_pois)
@@ -78,15 +84,31 @@ class ShardedRanker:
         self.rc, self.ru = rank % self.gc, rank // self.gc
         self.lo, self.hi = shard_range(self.n, self.rc, self.gc)
         self._local = local_topk or self._cuda_local
+        self._logmax = local_logmax or self._cuda_logmax
         self._merge = merge or _merge_cuda
         self._slice = slice_users or (lambda users, u0, u1: users.slice(u0, u1))
         self.events = []
 
-    def _cuda_local(self, users, k, lo, hi, precision):
+    def _cuda_local(self, users, k, lo, hi, precision, geo=None):
         m = self.model
         plan = m.ranking_plan(precision, lo, hi)  # built on the first batch, reused while the weights stand
         return ops.fullrank_topk(m.variant, float(m.beta), m._params(), m._catalog, users, k, lo, hi, True, plan.precision, plan,
-                                 return_keys=self.world > 1)  # one GPU: the merge kernel writes score / id itself
+                                 return_keys=self.world > 1, geo=geo)  # one GPU: the merge kernel writes score / id itself
+
+    def _cuda_logmax(self, users, lo, hi, a, b):
+        return ops.powerlaw_logmax(self.model._catalog, users, a, b, lo, hi, True)
+
+    def _global_logmax(self, users, n_users: int, a: float, b: float) -> torch.Tensor:
+        """M_u of this rank's users over the whole catalogue: local maxima, then one all_reduce(MAX) among the ranks that
+        score the same users (one vector over every slice; a rank leaves the slices of other ranks at -inf)."""
+        m = self._logmax(users, self.lo, self.hi, a, b)
+        if self.world == 1:
+            return m
+        u0, u1, per = self.user_range(n_users)
+        full = torch.full((self.gu * per,), float("-inf"), dtype=torch.float32, device=m.device)
+        full[self.ru * per:self.ru * per + (u1 - u0)] = m
+        dist.all_reduce(full, op=dist.ReduceOp.MAX)
+        return full[self.ru * per:self.ru * per + (u1 - u0)].contiguous()
 
     def kernel_name(self, precision: str) -> str:
         return {"fp32": "fullrank_fp32_kernel"}.get(precision, "fullrank_tc_kernel")
@@ -110,14 +132,19 @@ class ShardedRanker:
         u0 = min(n_users, self.ru * per)
         return u0, min(n_users, u0 + per), per
 
-    def _score_and_exchange(self, users, n_users: int, k: int, precision: str, timed: bool):
+    def _score_and_exchange(self, users, n_users: int, k: int, precision: str, timed: bool, geo=None):
         """`users` = this rank's slice.  Local fused scoring + top-k, then ONE all-gather of the key lists and the
         on-device merge / unpack; every rank returns the lists of the whole batch [n_users, k]."""
         u0, u1, per = self.user_range(n_users)
         if timed:
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-        keys = self._local(users, k, self.lo, self.hi, precision)
+        if geo is None:
+            keys = self._local(users, k, self.lo, self.hi, precision)
+        else:
+            ga, gb, galpha = (float(x) for x in geo)
+            logmax = self._global_logmax(users, n_users, ga, gb)
+            keys = self._local(users, k, self.lo, self.hi, precision, ops.GeoMix(ga, gb, galpha, logmax))
         if timed:
             b.record()
             self.events = [(a, b)]
@@ -136,14 +163,15 @@ class ShardedRanker:
         outs = [self._merge(g[s * self.gc:(s + 1) * self.gc]) for s in range(self.gu)]  # one [gc, per, k] block per slice
         return torch.cat([o[0] for o in outs])[:n_users], torch.cat([o[1] for o in outs])[:n_users]
 
-    def topk(self, users, k: int, precision: str = "auto"):
-        """`users`: the whole batch (DeviceUsers), resident on every rank."""
+    def topk(self, users, k: int, precision: str = "auto", geo: Optional[Tuple[float, float, float]] = None):
+        """`users`: the whole batch (DeviceUsers), resident on every rank.  `geo` = (a, b, alpha): rank by the power-law
+        mix of `powerlaw.fused_rerank_topk` (the scores returned are the mixed values)."""
         timed = torch.cuda.is_available() and users.offsets.is_cuda
         n_users = getattr(users, "n_users", None)
         if self.gu > 1:
             u0, u1, _ = self.user_range(n_users)
             users = self._slice(users, u0, u1)
-        return self._score_and_exchange(users, n_users, k, precision, timed)
+        return self._score_and_exchange(users, n_users, k, precision, timed, geo)
 
     def topk_host(self, indptr: torch.Tensor, items: torch.Tensor, k: int, precision: str = "auto"):
         """End-to-end call: pinned host CSR -> device (only this rank's user slice), rank, top-k lists of the whole batch

@@ -794,13 +794,44 @@ def fullrank_prepare(variant: str, beta: float, P: Dict[str, torch.Tensor], cat:
     return _LAST_TC_PLAN[0]
 
 
+@dataclass
+class GeoMix:
+    """Power-law geo re-ranking of a full-rank call (include/nais_b200.h NaisGeoMix): rank by
+    (1 - alpha) * sigmoid(score) + alpha * exp(log G - M_u), log G = sum_h ln(a * max(0.01, d_km)^b).  `logmax` [U] float32 on
+    the device holds M_u over the whole ranked catalogue (`powerlaw_logmax`, max-combined across shards)."""
+    a: float
+    b: float
+    alpha: float
+    logmax: torch.Tensor
+
+    def slice(self, u0: int, u1: int) -> "GeoMix":
+        return GeoMix(self.a, self.b, self.alpha, self.logmax[u0:u1])
+
+
+def powerlaw_logmax(cat: DeviceCatalog, users: DeviceUsers, a: float, b: float, poi_begin: int = 0, poi_end: Optional[int] = None,
+                    exclude_history: bool = True) -> torch.Tensor:
+    """M_u = max_j log G(u, j) over [poi_begin, poi_end) (minus the history when `exclude_history`) [U] float32, -inf for a user
+    without candidates (nais_powerlaw_logmax; bit-identical to the maximum of powerlaw.log_scores, no [U, N] buffer)."""
+    dev = _need_cuda(users.offsets, cat.coords)
+    lib = _lib.load()
+    poi_end = cat.row_base + cat.n_rows if poi_end is None else poi_end
+    out = torch.empty(users.n_users, device=dev, dtype=torch.float32)
+    with torch.cuda.device(dev):
+        c, u = _structs(cat, users)
+        _lib.check(lib.nais_powerlaw_logmax(C.byref(c), C.byref(u), poi_begin, poi_end, float(a), float(b), int(exclude_history),
+                                            out.data_ptr(), _stream()), "nais_powerlaw_logmax")
+    return out
+
+
 def fullrank_topk(variant: str, beta: float, P: Dict[str, torch.Tensor], cat: DeviceCatalog, users: DeviceUsers, k: int,
                   poi_begin: int = 0, poi_end: Optional[int] = None, exclude_history: bool = True,
-                  precision: str = "fp32", plan: Optional[FullrankPlan] = None, return_keys: bool = False):
+                  precision: str = "fp32", plan: Optional[FullrankPlan] = None, return_keys: bool = False,
+                  geo: Optional[GeoMix] = None):
     """(score[U,k] pre-sigmoid descending, id[U,k] int32 global POI ids; -inf / -1 padding) — or, with `return_keys`, the
     packed ranking keys [U,k] int64 (bit pattern of the uint64 keys `topk_merge_keys` consumes).  `plan`: a
     `fullrank_prepare` result for the same weights / range / precision; without one the constants are recomputed by this
-    call (`nais_fullrank_topk`)."""
+    call (`nais_fullrank_topk`).  `geo`: rank by the power-law mix instead (`nais_fullrank_topk_geo_planned`, always planned);
+    the score is then the mixed value, not a pre-sigmoid score."""
     dev = _need_cuda(users.offsets, users.items, users.region, users.coords, cat.region, cat.coords, *P.values())
     lib = _lib.load()
     keep: List[torch.Tensor] = []
@@ -813,7 +844,7 @@ def fullrank_topk(variant: str, beta: float, P: Dict[str, torch.Tensor], cat: De
             precision = plan.precision
         precision = resolve_precision(lib, p, precision, dev)
         prec = PRECISIONS[precision]
-        planned = plan is not None or return_keys
+        planned = plan is not None or return_keys or geo is not None
         if planned:
             ws_bytes = lib.nais_fullrank_planned_workspace_bytes(C.byref(p), users.n_users, users.nnz, poi_begin, poi_end, k, prec)
         else:
@@ -822,7 +853,9 @@ def fullrank_topk(variant: str, beta: float, P: Dict[str, torch.Tensor], cat: De
             n_slices = min(users.n_users, -(-ws_bytes // WORKSPACE_LIMIT_BYTES))
             step = -(-users.n_users // n_slices)
             parts = [fullrank_topk(variant, beta, P, cat, users.slice(u0, min(users.n_users, u0 + step)), k, poi_begin, poi_end,
-                                   exclude_history, precision, plan, return_keys) for u0 in range(0, users.n_users, step)]
+                                   exclude_history, precision, plan, return_keys,
+                                   None if geo is None else geo.slice(u0, min(users.n_users, u0 + step)))
+                     for u0 in range(0, users.n_users, step)]
             if return_keys:
                 return torch.cat(parts)
             return torch.cat([a for a, _ in parts]), torch.cat([b for _, b in parts])
@@ -837,7 +870,16 @@ def fullrank_topk(variant: str, beta: float, P: Dict[str, torch.Tensor], cat: De
             out_k = None
             out_s = torch.empty(users.n_users, k, device=dev, dtype=torch.float32)
             out_i = torch.empty(users.n_users, k, device=dev, dtype=torch.int32)
-        if planned:
+        if geo is not None:
+            if geo.logmax.numel() != users.n_users or geo.logmax.device != dev or geo.logmax.dtype != torch.float32:
+                raise ValueError("geo.logmax must be a float32 [n_users] tensor on the users' device")
+            lm = geo.logmax.contiguous()
+            g = _lib.NaisGeoMix(float(geo.a), float(geo.b), float(geo.alpha), lm.data_ptr())
+            _lib.check(lib.nais_fullrank_topk_geo_planned(C.byref(p), C.byref(c), C.byref(u), poi_begin, poi_end, k,
+                                                          int(exclude_history), prec, _ptr(plan.buf), plan.nbytes, C.byref(g),
+                                                          _ptr(out_k), _ptr(out_s), _ptr(out_i), ws.data_ptr(), ws_bytes, _stream()),
+                       "nais_fullrank_topk_geo_planned")
+        elif planned:
             _lib.check(lib.nais_fullrank_topk_planned(C.byref(p), C.byref(c), C.byref(u), poi_begin, poi_end, k, int(exclude_history),
                                                       prec, _ptr(plan.buf), plan.nbytes, _ptr(out_k), _ptr(out_s), _ptr(out_i),
                                                       ws.data_ptr(), ws_bytes, _stream()), "nais_fullrank_topk_planned")

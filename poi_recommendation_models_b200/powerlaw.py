@@ -6,8 +6,12 @@
     normalize + (1 - alpha) * prediction + alpha * G   run.py:55-59, 523-546 (the re-ranking the reference keeps commented out)
 
 `PowerLaw` mirrors the reference class (same attributes, same random draws, same fitted a, b to ~1e-12; the pair loop
-and the gradient sums are vectorised).  `rerank_topk` is the fused device path: attention scores of the whole catalogue
-(`nais_fullrank_scores`), log G from `nais_powerlaw_logscore`, normalisation by the per-user maximum, mix, top-k.
+and the gradient sums are vectorised).  `fused_rerank_topk` is the device path: the per-user maximum of log G in one pass
+(`nais_powerlaw_logmax`), then the mix and its top-k inside the full-rank kernel against the model's ranking plan
+(`nais_fullrank_topk_geo_planned`) — no [users, N] buffer.  `rerank_topk` is the earlier composed path (whole-catalogue
+scores, log G and the mix materialised per slice of users, torch.topk); it stays as the comparison path.  On one B200 the
+composed path is the faster of the two today (profiles/r3_geo_rerank.json, DESIGN.md §4.1); the fused one needs no
+[users, N] memory and range-shards (distributed.ShardedRanker.topk(geo=...)).
 """
 from __future__ import annotations
 
@@ -143,3 +147,23 @@ def rerank_topk(model, users, k: int, a: float, b: float, alpha: float, precisio
         mixed[rows, hist] = float("-inf")
     val, idx = torch.topk(mixed, k, dim=1)
     return val, idx
+
+
+@torch.no_grad()
+def fused_rerank_topk(model, users, k: int, a: float, b: float, alpha: float, precision: str = "auto",
+                      exclude_history: bool = True) -> Tuple[torch.Tensor, torch.Tensor]:
+    """`rerank_topk` in two device passes and no [users, N] buffer: M_u = max_j log G over the candidates
+    (`ops.powerlaw_logmax`), then the full-rank kernel forms (1 - alpha) * sigmoid(score) + alpha * exp(log G - M_u) per
+    candidate and keeps its block top-k by that value (score descending, then id ascending), against `model.ranking_plan`.
+    Returns (mixed score [U,k] float32, ids [U,k] int64; -inf / -1 padding).  The model needs a catalogue with coordinates
+    (`set_catalog(..., coords=...)`), whatever its own distance input is."""
+    if not isinstance(users, ops.DeviceUsers):
+        users = model.make_users(*users)
+    cat = model._catalog
+    if cat is None or cat.coords is None or users.coords is None:
+        raise RuntimeError("geo re-ranking needs catalogue coordinates: call set_catalog(..., coords=...) first")
+    plan = model.ranking_plan(precision)
+    logmax = ops.powerlaw_logmax(cat, users, a, b, 0, model.item_num, exclude_history)
+    s, i = ops.fullrank_topk(model.variant, float(model.beta), model._params(), cat, users, k, 0, model.item_num, exclude_history,
+                             plan.precision, plan, geo=ops.GeoMix(float(a), float(b), float(alpha), logmax))
+    return s, i.to(torch.int64)
