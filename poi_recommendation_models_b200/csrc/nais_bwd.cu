@@ -907,13 +907,6 @@ int launch_rows_adagrad(const int32_t* keys, const float* rows, int64_t n, int w
 // ---------------------------------------------------------------------------------------------------------------------
 static inline size_t align_up(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
 
-struct BwdLayout {
-  size_t dq, dp, part, kin[3], vin[3], kout[3], vout[3], cub[3], pkey[3], pstart[3], prows[3], total;
-  int64_t n_chunks;
-  int grid, stride;
-  size_t cub_bytes;
-};
-
 static int bwd_grid() { return 148 * 2; }
 
 // lists: 0 = history ids (B*H entries), 1 = target ids (B), 2 = region ids of both (B*H + B)
@@ -950,7 +943,6 @@ static BwdLayout bwd_layout(const NaisParams& p, const NaisPairs& b) {
   cub::DeviceRadixSort::SortPairs(nullptr, cb, (const int*)nullptr, (int*)nullptr, (const uint32_t*)nullptr,
                                   (uint32_t*)nullptr, (int)(n_max > 0x7fffffff ? 0x7fffffff : n_max));
   L.cub_bytes = cb;
-  L.n_chunks = (n_max + SEG_CHUNK - 1) / SEG_CHUNK;
   const int wmax = w_poi > w_reg ? w_poi : w_reg;
   for (int i = 0; i < 3; ++i) {  // the three lists are sorted and reduced concurrently (side streams): private scratch each
     const int64_t nch = (n_of[i] + SEG_CHUNK - 1) / SEG_CHUNK;
@@ -973,15 +965,18 @@ size_t pairs_bwd_workspace_bytes(const NaisParams& p, const NaisPairs& b) { retu
 // sorts and their segment reduces are latency-bound launches that underfill the GPU one at a time (ncu launch list,
 // profiles/r2_launches_train_c3.csv: 29 us to sort 8 192 target ids, 27 us to reduce them), so lists 1 and 2 run on two side
 // streams forked from / joined to the caller's stream with events.  One pool per device, created on first use; the mutex is
-// held while a call ENQUEUES its work (cudaStreamWaitEvent binds to the record that precedes it at call time).
+// held while a PairsBwd step ENQUEUES its work (cudaStreamWaitEvent binds to the record that precedes it at call time).  Every event
+// a step waits for is recorded in that step, except `sorted0`, which `finish` waits for after an earlier `sort` released the mutex
+// (one host thread per GPU, include/nais_b200.h).
 struct SideStreams {
-  cudaStream_t s[3] = {nullptr, nullptr, nullptr};  // [0], [1]: lists 1, 2; [2]: the long list's sort when it is forked ahead (BWD_SORTS), then param_reduce
+  cudaStream_t s[3] = {nullptr, nullptr, nullptr};  // [0], [1]: lists 1, 2; [2]: list 0's sort when PairsBwd::sort forks it, then param_reduce
   cudaEvent_t fork = nullptr, join[2] = {nullptr, nullptr}, sorted0 = nullptr, pjoin = nullptr;  // pjoin: param_reduce (+ dense Adagrad) on s[2]
   bool ok = false;
 };
 static std::mutex g_side_mu;
-static SideStreams* side_streams() {  // (g_side_mu held)
+static SideStreams* side_streams() {
   static SideStreams pool[64];
+  std::lock_guard<std::mutex> side_lock(g_side_mu);
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
   SideStreams& S = pool[dev];
@@ -1010,169 +1005,162 @@ static int launch_bwd_tile(const BwdArgs& A, int D, int grid, cudaStream_t strea
   return (int)cudaGetLastError();
 }
 
-// `phase`: see BwdPhase (the forward of the autograd path ends with BWD_JOIN_SORTS).  The split phases and the fused optimizer take
-// pairs_fused_layout (disentangled: each id list belongs to one branch, so a row-sparse step per list IS the dense step); branch 0
-// sorts lists 0 / 1, branch 1 list 2.  `dense`: one DenseAdagradLaunch per branch, each enqueued behind that branch's param_reduce —
-// branch 1's holds embed_distance, whose gradient is complete only after branch 1's param_reduce (both branches read it).
-int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score_parts, const float* row_sum,
-                     const unsigned long long* act_mask, const float* dscore, const NaisGrads& g, const NaisAdagrad* opt, void* ws,
-                     size_t ws_bytes, cudaStream_t stream, BwdPhase phase, const DenseAdagradLaunch* dense) {
+// `split` and the fused optimizer take pairs_fused_layout (disentangled: each id list belongs to one branch, so a row-sparse step
+// per list IS the dense step); branch 0 sorts lists 0 / 1, branch 1 list 2.
+int PairsBwd::open(const NaisParams& p_, const NaisPairs& b_, const NaisGrads& g_, const NaisAdagrad* opt_, const float* score_parts_,
+                   const float* row_sum_, const unsigned long long* act_mask_, const float* dscore_, void* ws, size_t ws_bytes, bool split) {
+  p = p_, b = b_, g = g_, opt = opt_, base = reinterpret_cast<char*>(ws);
+  score_parts = score_parts_, row_sum = row_sum_, act_mask = act_mask_, dscore = dscore_;
   if (pairs_n_cells(b) + b.B >= 0x7fffffffLL) return NAIS_ERR_SHAPE;
-  if ((phase != BWD_ALL || opt) && !pairs_fused_layout(p)) return NAIS_ERR_MODE;
-  const BwdLayout L = bwd_layout(p, b);
+  if ((split || opt) && !pairs_fused_layout(p)) return NAIS_ERR_MODE;
+  L = bwd_layout(p, b);
   if (ws_bytes < L.total) return NAIS_ERR_WORKSPACE;
-  char* base = reinterpret_cast<char*>(ws);
-  int dense_rc = 0;
-  std::lock_guard<std::mutex> side_lock(g_side_mu);
-  SideStreams* side = side_streams();
+  side = side_streams();
   if (!side) return (int)cudaErrorUnknown;
-  // list t runs on: 0 -> the caller's stream, 1 / 2 -> side streams
-  auto stream_of = [&](int t) { return t == 0 ? stream : side->s[t - 1]; };
-  const int lanes = p.dist_mode == NAIS_DIST_LATLON ? 2 : 0;
-  const int64_t n_cells = pairs_n_cells(b);
-  const int64_t n_of[3] = {n_cells, b.B, n_cells + b.B};
-  auto I = [&](size_t off) { return reinterpret_cast<int*>(base + off); };
-  auto U = [&](size_t off) { return reinterpret_cast<uint32_t*>(base + off); };
-
+  n_of[0] = pairs_n_cells(b), n_of[1] = b.B, n_of[2] = n_of[0] + b.B;
   for (int bi = 0; bi < p.n_branch; ++bi) {
     const NaisBranch& br = p.branch[bi];
-    const int D = br.w_poi + br.w_reg;
-    if (D > 128 || p.hid > 128) return NAIS_ERR_SHAPE;  // backward tiles: D, hid <= 128 in this version
+    if (br.w_poi + br.w_reg > 128 || p.hid > 128) return NAIS_ERR_SHAPE;  // backward tiles: D, hid <= 128 in this version
     if (pairs_n_tiles(b) < 1) return 0;
     if (p.pairs_precision == NAIS_PAIRS_TC && !pairs_tc_bwd_supported(p, b)) return NAIS_ERR_SHAPE;
-    // the tcgen05 dropout backward takes the mask from the forward's act_mask (it regenerates nothing)
-    const bool tile_phase = phase != BWD_SORTS && phase != BWD_JOIN_SORTS;
-    if (p.pairs_precision == NAIS_PAIRS_TC && p.dropout_p > 0.f && !act_mask && tile_phase) return NAIS_ERR_NULL;
+    // the tcgen05 dropout backward takes the mask from the forward's act_mask (it regenerates nothing); a call that only sorts
+    // (no dscore) runs no tile kernel
+    if (p.pairs_precision == NAIS_PAIRS_TC && p.dropout_p > 0.f && !act_mask && dscore) return NAIS_ERR_NULL;
     // a table is processed if it has a gradient destination or a fused-optimizer state
-    const bool want[3] = {br.w_poi > 0 && (g.hist_poi[bi] || (opt && opt->sum_hist_poi[bi])),
-                          br.w_poi > 0 && (g.tgt_poi[bi] || (opt && opt->sum_tgt_poi[bi])),
-                          br.w_reg > 0 && (g.reg[bi] || (opt && opt->sum_reg[bi]))};
-    // ---- 1. sort the ids (they do not depend on the gradients; stable radix sort: equal ids keep cell order) ----------------
-    if ((phase == BWD_ALL || phase == BWD_SORTS) && (want[0] || want[1] || want[2])) {
-      const int64_t n_thr = n_cells > b.B ? n_cells : b.B;
-      make_keys_kernel<<<(unsigned)((n_thr + 255) / 256), 256, 0, stream>>>(
-          b, p.item_num, p.region_num, want[0] ? I(L.kin[0]) : nullptr, U(L.vin[0]), want[1] ? I(L.kin[1]) : nullptr, U(L.vin[1]),
-          want[2] ? I(L.kin[2]) : nullptr, U(L.vin[2]));
-      NAIS_COUNT_LAUNCH(1);
-      cudaEventRecord(side->fork, stream);
-      for (int t = 2; t >= 0; --t) {  // (the caller's stream last: the side streams are busy while it sorts the long list)
-        if (!want[t]) continue;
-        cudaStream_t sort_stream = t ? side->s[t - 1] : (phase == BWD_SORTS ? side->s[2] : stream);
-        if (sort_stream != stream) cudaStreamWaitEvent(sort_stream, side->fork, 0);
-        const int n_rows = t == 2 ? p.region_num : p.item_num;
-        int bits = 1;  // keys are 0 .. n_rows (n_rows = the "drop" key of an out-of-range id)
-        while ((1ll << bits) <= n_rows && bits < 31) ++bits;
-        size_t cb = L.cub_bytes;
-        cub::DeviceRadixSort::SortPairs(base + L.cub[t], cb, I(L.kin[t]), I(L.kout[t]), U(L.vin[t]), U(L.vout[t]), (int)n_of[t], 0, bits,
-                                        sort_stream);
-        if (phase == BWD_SORTS && t == 0) cudaEventRecord(side->sorted0, side->s[2]);
-      }
+    want[bi][0] = br.w_poi > 0 && (g.hist_poi[bi] || (opt && opt->sum_hist_poi[bi]));
+    want[bi][1] = br.w_poi > 0 && (g.tgt_poi[bi] || (opt && opt->sum_tgt_poi[bi]));
+    want[bi][2] = br.w_reg > 0 && (g.reg[bi] || (opt && opt->sum_reg[bi]));
+  }
+  n_branch = p.n_branch;
+  return 0;
+}
+
+// The ids do not depend on the gradients; stable radix sort: equal ids keep cell order.
+void PairsBwd::sort(int bi, cudaStream_t stream, bool fork_long) const {
+  const bool* w = want[bi];
+  if (!w[0] && !w[1] && !w[2]) return;
+  std::lock_guard<std::mutex> side_lock(g_side_mu);
+  const int64_t n_thr = n_of[0] > b.B ? n_of[0] : b.B;
+  make_keys_kernel<<<(unsigned)((n_thr + 255) / 256), 256, 0, stream>>>(b, p.item_num, p.region_num, w[0] ? I(L.kin[0]) : nullptr,
+                                                                        U(L.vin[0]), w[1] ? I(L.kin[1]) : nullptr, U(L.vin[1]),
+                                                                        w[2] ? I(L.kin[2]) : nullptr, U(L.vin[2]));
+  NAIS_COUNT_LAUNCH(1);
+  cudaEventRecord(side->fork, stream);
+  for (int t = 2; t >= 0; --t) {  // (the caller's stream last: the side streams are busy while it sorts the long list)
+    if (!w[t]) continue;
+    cudaStream_t sort_stream = t ? side->s[t - 1] : (fork_long ? side->s[2] : stream);
+    if (sort_stream != stream) cudaStreamWaitEvent(sort_stream, side->fork, 0);
+    const int n_rows = t == 2 ? p.region_num : p.item_num;
+    int bits = 1;  // keys are 0 .. n_rows (n_rows = the "drop" key of an out-of-range id)
+    while ((1ll << bits) <= n_rows && bits < 31) ++bits;
+    size_t cb = L.cub_bytes;
+    cub::DeviceRadixSort::SortPairs(base + L.cub[t], cb, I(L.kin[t]), I(L.kout[t]), U(L.vin[t]), U(L.vout[t]), (int)n_of[t], 0, bits,
+                                    sort_stream);
+    if (fork_long && t == 0) cudaEventRecord(side->sorted0, side->s[2]);
+  }
+}
+
+int PairsBwd::join_sorts(cudaStream_t stream) const {
+  std::lock_guard<std::mutex> side_lock(g_side_mu);
+  for (int bi = 0; bi < n_branch; ++bi)
+    for (int t = 0; t < 3; ++t) {
+      if (!want[bi][t]) continue;
+      cudaEvent_t ev = t ? side->join[t - 1] : side->sorted0;
+      cudaEventRecord(ev, t ? side->s[t - 1] : side->s[2]);
+      cudaStreamWaitEvent(stream, ev, 0);
     }
-    if (phase == BWD_JOIN_SORTS) {
-      for (int t = 0; t < 3; ++t) {
-        if (!want[t]) continue;
-        cudaEvent_t ev = t ? side->join[t - 1] : side->sorted0;
-        cudaEventRecord(ev, t ? side->s[t - 1] : side->s[2]);
-        cudaStreamWaitEvent(stream, ev, 0);
-      }
-    }
-    if (phase == BWD_SORTS || phase == BWD_JOIN_SORTS) continue;
-    // ---- 2. the tile kernel ------------------------------------------------------------------------------------------------
-    BwdArgs A;
-    A.p = p;
-    A.b = b;
-    A.bi = bi;
-    A.parts = score_parts + (size_t)bi * b.B;
-    A.row_sum = row_sum + (size_t)bi * b.B;
-    A.dscore = dscore;
-    A.act_mask = (p.n_branch == 1 && p.hid <= 64) ? act_mask : nullptr;
-    A.ws_dq = (want[0] || want[2]) ? reinterpret_cast<float*>(base + L.dq) : nullptr;
-    A.ws_dp = (want[1] || want[2]) ? reinterpret_cast<float*>(base + L.dp) : nullptr;
-    A.ws_part = reinterpret_cast<float*>(base + L.part);
-    A.part_stride = L.stride;
-    A.n_items = pairs_n_tiles(b);
-    int grid = (int)(A.n_items < L.grid ? A.n_items : L.grid);
-    int rc;
-    const int nkb = p.hid <= 64 ? 1 : 2, db = D <= 64 ? 1 : 2;
-    A.bad = bad_index_flag();
-    A.drop_inv = p.dropout_p > 0.f ? 1.f / (1.f - p.dropout_p) : 1.f;
-    const bool tc_ok = pairs_tc_bwd_supported(p, b) && (p.dropout_p <= 0.f || A.act_mask);  // (else the FP32 kernel regenerates the mask)
-    if (p.pairs_precision != NAIS_PAIRS_FP32 && tc_ok) rc = launch_pairs_bwd_tc(A, D, grid, stream);  // tcgen05 (bf16 two-term splits)
-    else if (nkb == 1 && db == 1) rc = launch_bwd_tile<1, 1>(A, D, grid, stream);
-    else if (nkb == 1) rc = launch_bwd_tile<1, 2>(A, D, grid, stream);
-    else if (db == 1) rc = launch_bwd_tile<2, 1>(A, D, grid, stream);
-    else rc = launch_bwd_tile<2, 2>(A, D, grid, stream);
-    if (rc) {  // (launch failure: rejoin the side streams before the caller may release the workspace)
-      for (int t = 1; t < 3; ++t)
-        if (want[t]) {
-          cudaEventRecord(side->join[t - 1], side->s[t - 1]);
-          cudaStreamWaitEvent(stream, side->join[t - 1], 0);
-        }
-      return rc;
-    }
-    // ---- 3. embedding rows: gather the contribution rows in key order ------------------------------------------------------------
-    auto dest = [&](float* grad, const float* param, float* sum, const int32_t* remap) {
-      SegOut o;
-      o.out = grad;
-      o.param = (opt && sum) ? const_cast<float*>(param) : nullptr;
-      o.sum = sum;
-      o.lr = opt ? opt->lr : 0.f;
-      o.eps = opt ? opt->eps : 0.f;
-      o.remap = remap;
-      return o;
-    };
-    auto seg = [&](int t, int off, int w, int n_rows, SegOut out) {
-      SegRows R;
-      R.dq = t == 1 ? A.ws_dp : A.ws_dq;  // the target list's sources are plain row indices into dp
-      R.dp = A.ws_dp;
-      R.n_cells = t == 1 ? n_of[1] : n_cells;
-      R.D = D;
-      R.off = off;
-      launch_segment_reduce(I(L.kout[t]), U(L.vout[t]), n_of[t], R, w, n_rows, out, I(L.pkey[t]), I(L.pstart[t]),
-                            reinterpret_cast<float*>(base + L.prows[t]), stream_of(t));
-    };
-    // fork again: the side streams (still ordered after their own sorts) wait for the tile kernel, reduce their list, and join
-    cudaEventRecord(side->fork, stream);
+  return (int)cudaGetLastError();
+}
+
+// `dense`: this branch's DenseAdagradLaunch (or NULL), enqueued behind its param_reduce — branch 1's holds embed_distance, whose
+// gradient is complete only after branch 1's param_reduce (both branches read it).
+int PairsBwd::finish(int bi, cudaStream_t stream, bool wait_sorted0, const DenseAdagradLaunch* dense) const {
+  const bool* w = want[bi];
+  const NaisBranch& br = p.branch[bi];
+  const int D = br.w_poi + br.w_reg, lanes = p.dist_mode == NAIS_DIST_LATLON ? 2 : 0;
+  std::lock_guard<std::mutex> side_lock(g_side_mu);
+  // ---- the tile kernel ----------------------------------------------------------------------------------------------------
+  BwdArgs A;
+  A.p = p;
+  A.b = b;
+  A.bi = bi;
+  A.parts = score_parts + (size_t)bi * b.B;
+  A.row_sum = row_sum + (size_t)bi * b.B;
+  A.dscore = dscore;
+  A.act_mask = (p.n_branch == 1 && p.hid <= 64) ? act_mask : nullptr;
+  A.ws_dq = (w[0] || w[2]) ? reinterpret_cast<float*>(base + L.dq) : nullptr;
+  A.ws_dp = (w[1] || w[2]) ? reinterpret_cast<float*>(base + L.dp) : nullptr;
+  A.ws_part = reinterpret_cast<float*>(base + L.part);
+  A.part_stride = L.stride;
+  A.n_items = pairs_n_tiles(b);
+  int grid = (int)(A.n_items < L.grid ? A.n_items : L.grid);
+  int rc;
+  const int nkb = p.hid <= 64 ? 1 : 2, db = D <= 64 ? 1 : 2;
+  A.bad = bad_index_flag();
+  A.drop_inv = p.dropout_p > 0.f ? 1.f / (1.f - p.dropout_p) : 1.f;
+  const bool tc_ok = pairs_tc_bwd_supported(p, b) && (p.dropout_p <= 0.f || A.act_mask);  // (else the FP32 kernel regenerates the mask)
+  if (p.pairs_precision != NAIS_PAIRS_FP32 && tc_ok) rc = launch_pairs_bwd_tc(A, D, grid, stream);  // tcgen05 (bf16 two-term splits)
+  else if (nkb == 1 && db == 1) rc = launch_bwd_tile<1, 1>(A, D, grid, stream);
+  else if (nkb == 1) rc = launch_bwd_tile<1, 2>(A, D, grid, stream);
+  else if (db == 1) rc = launch_bwd_tile<2, 1>(A, D, grid, stream);
+  else rc = launch_bwd_tile<2, 2>(A, D, grid, stream);
+  auto join_lists = [&] {  // `stream` waits for the side streams of lists 1 / 2
     for (int t = 1; t < 3; ++t)
-      if (want[t]) cudaStreamWaitEvent(side->s[t - 1], side->fork, 0);
-    // the per-CTA parameter partials -> w1 / b1 / w2 / distance-layer gradients (and the dense Adagrad step behind them) on the
-    // third side stream, idle since the long list's sort: next to the three lists' reduces instead of in front of one of them
-    cudaStream_t pstream = side->s[2];
-    cudaStreamWaitEvent(pstream, side->fork, 0);
-    {
-      const int n = p.hid * (D + lanes) + 2 * p.hid + 7;
-      param_reduce_kernel<<<(n + 255) / 256, 256, 0, pstream>>>(
-          A.ws_part, grid, L.stride, p.hid, D, lanes, g.w1[bi], g.b1[bi], g.w2[bi], bi == 0 ? g.dist_w : nullptr,
-          bi == 0 ? g.dist_b : nullptr, p.dist_mode == NAIS_DIST_KM ? g.dist_embed : nullptr, D, bi > 0);
-      NAIS_COUNT_LAUNCH(1);
-      // the one-call training step's dense Adagrad of these tensors needs nothing else: right behind them, next to the table reduces
-      if (dense) {
-        const DenseAdagradLaunch& da = dense[bi];
-        const int rd = launch_dense_adagrad(da.param, da.sum, da.grad, da.n, da.lr, da.eps, pstream);
-        if (rd) dense_rc = rd;
-      }
-      cudaEventRecord(side->pjoin, pstream);
-    }
-    if (phase == BWD_AFTER_SORTS && want[0]) cudaStreamWaitEvent(stream, side->sorted0, 0);  // the long list was sorted on a side stream
-    if (want[0]) seg(0, 0, br.w_poi, p.item_num, dest(g.hist_poi[bi], br.hist_poi, opt ? opt->sum_hist_poi[bi] : nullptr, g.remap_hist_poi[bi]));
-    if (want[1]) seg(1, 0, br.w_poi, p.item_num, dest(g.tgt_poi[bi], br.tgt_poi, opt ? opt->sum_tgt_poi[bi] : nullptr, g.remap_tgt_poi[bi]));
-    // (history-side and target-side region rows are one table in every variant: hist_reg == tgt_reg)
-    if (want[2]) seg(2, br.w_poi, br.w_reg, p.region_num, dest(g.reg[bi], br.hist_reg, opt ? opt->sum_reg[bi] : nullptr, g.remap_reg[bi]));
-    for (int t = 1; t < 3; ++t)
-      if (want[t]) {
+      if (w[t]) {
         cudaEventRecord(side->join[t - 1], side->s[t - 1]);
         cudaStreamWaitEvent(stream, side->join[t - 1], 0);
       }
-    cudaStreamWaitEvent(stream, side->pjoin, 0);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-    if (dense_rc) return dense_rc;
+  };
+  if (rc) {  // (launch failure: rejoin the side streams before the caller may release the workspace)
+    join_lists();
+    return rc;
   }
-  if (phase == BWD_SORTS || phase == BWD_JOIN_SORTS) {
-    cudaError_t e1 = cudaGetLastError();
-    return e1 == cudaSuccess ? 0 : (int)e1;
-  }
-  return 0;
+  // ---- embedding rows: gather the contribution rows in key order --------------------------------------------------------------
+  auto dest = [&](float* grad, const float* param, float* sum, const int32_t* remap) {
+    SegOut o;
+    o.out = grad;
+    o.param = (opt && sum) ? const_cast<float*>(param) : nullptr;
+    o.sum = sum;
+    o.lr = opt ? opt->lr : 0.f;
+    o.eps = opt ? opt->eps : 0.f;
+    o.remap = remap;
+    return o;
+  };
+  auto seg = [&](int t, int off, int width, int n_rows, SegOut out) {  // list t runs on: 0 -> the caller's stream, 1 / 2 -> side streams
+    SegRows R;
+    R.dq = t == 1 ? A.ws_dp : A.ws_dq;  // the target list's sources are plain row indices into dp
+    R.dp = A.ws_dp;
+    R.n_cells = t == 1 ? n_of[1] : n_of[0];
+    R.D = D;
+    R.off = off;
+    launch_segment_reduce(I(L.kout[t]), U(L.vout[t]), n_of[t], R, width, n_rows, out, I(L.pkey[t]), I(L.pstart[t]),
+                          reinterpret_cast<float*>(base + L.prows[t]), t == 0 ? stream : side->s[t - 1]);
+  };
+  // fork again: the side streams (still ordered after their own sorts) wait for the tile kernel, reduce their list, and join
+  cudaEventRecord(side->fork, stream);
+  for (int t = 1; t < 3; ++t)
+    if (w[t]) cudaStreamWaitEvent(side->s[t - 1], side->fork, 0);
+  // the per-CTA parameter partials -> w1 / b1 / w2 / distance-layer gradients (and the dense Adagrad step behind them) on the
+  // third side stream, idle since the long list's sort: next to the three lists' reduces instead of in front of one of them
+  cudaStream_t pstream = side->s[2];
+  cudaStreamWaitEvent(pstream, side->fork, 0);
+  const int n = p.hid * (D + lanes) + 2 * p.hid + 7;
+  param_reduce_kernel<<<(n + 255) / 256, 256, 0, pstream>>>(
+      A.ws_part, grid, L.stride, p.hid, D, lanes, g.w1[bi], g.b1[bi], g.w2[bi], bi == 0 ? g.dist_w : nullptr,
+      bi == 0 ? g.dist_b : nullptr, p.dist_mode == NAIS_DIST_KM ? g.dist_embed : nullptr, D, bi > 0);
+  NAIS_COUNT_LAUNCH(1);
+  // the one-call training step's dense Adagrad of these tensors needs nothing else: right behind them, next to the table reduces
+  const int dense_rc = dense ? launch_dense_adagrad(dense->param, dense->sum, dense->grad, dense->n, dense->lr, dense->eps, pstream) : 0;
+  cudaEventRecord(side->pjoin, pstream);
+  if (wait_sorted0 && w[0]) cudaStreamWaitEvent(stream, side->sorted0, 0);  // the long list was sorted on a side stream
+  if (w[0]) seg(0, 0, br.w_poi, p.item_num, dest(g.hist_poi[bi], br.hist_poi, opt ? opt->sum_hist_poi[bi] : nullptr, g.remap_hist_poi[bi]));
+  if (w[1]) seg(1, 0, br.w_poi, p.item_num, dest(g.tgt_poi[bi], br.tgt_poi, opt ? opt->sum_tgt_poi[bi] : nullptr, g.remap_tgt_poi[bi]));
+  // (history-side and target-side region rows are one table in every variant: hist_reg == tgt_reg)
+  if (w[2]) seg(2, br.w_poi, br.w_reg, p.region_num, dest(g.reg[bi], br.hist_reg, opt ? opt->sum_reg[bi] : nullptr, g.remap_reg[bi]));
+  join_lists();
+  cudaStreamWaitEvent(stream, side->pjoin, 0);
+  cudaError_t e = cudaGetLastError();
+  return e != cudaSuccess ? (int)e : dense_rc;
 }
 
 }  // namespace nais

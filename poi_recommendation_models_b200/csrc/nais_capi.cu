@@ -21,10 +21,7 @@ int launch_topk_merge_keys_multi(const unsigned long long* keys, unsigned long l
 int merge_scratch_lists(int n_lists, int k);
 int choose_splits(int n_users, int64_t range);
 // nais_bwd.cu
-size_t pairs_bwd_workspace_bytes(const NaisParams& p, const NaisPairs& b);
-int launch_pairs_bwd(const NaisParams& p, const NaisPairs& b, const float* score_parts, const float* row_sum,
-                     const unsigned long long* act_mask, const float* dscore, const NaisGrads& g, const NaisAdagrad* opt, void* ws,
-                     size_t ws_bytes, cudaStream_t stream, BwdPhase phase = BWD_ALL, const DenseAdagradLaunch* dense = nullptr);
+size_t pairs_bwd_workspace_bytes(const NaisParams& p, const NaisPairs& b);  // (the backward's steps: nais_common.cuh PairsBwd)
 bool pairs_tc_bwd_supported(const NaisParams& p, const NaisPairs& b);
 size_t rows_adagrad_workspace_bytes(int64_t n, int w);
 int launch_rows_adagrad(const int32_t* keys, const float* rows, int64_t n, int w, int n_rows, float* grad_out, float* param, float* sum,
@@ -348,20 +345,48 @@ size_t nais_pairs_backward_workspace_bytes(const NaisParams* p, const NaisPairs*
   return pairs_bwd_workspace_bytes(*p, *batch);
 }
 
-int nais_pairs_backward(const NaisParams* p, const NaisPairs* batch, const float* score_parts, const float* row_sum,
-                        const uint64_t* act_mask, const float* dscore, const NaisGrads* grads, void* workspace,
-                        size_t workspace_bytes, nais_stream_t stream) {
+// The checks every backward-type entry point makes, in this order: the first failing one decides the code.  0 also when B == 0,
+// where the caller has nothing to do.  `grads`: the NaisGrads (and the fused optimizer's NaisAdagrad) are given; `one_branch`: the
+// presorting pair takes one branch only; `opt`: the fused optimizer's state; `inputs`: the entry point's other arrays are given.
+static int check_backward_call(const NaisParams* p, const NaisPairs* batch, bool grads, bool one_branch, const NaisAdagrad* opt,
+                               bool inputs, const void* workspace, size_t workspace_bytes) {
   int rc = check_params(p);
   if (rc) return rc;
   rc = check_pairs(p, batch);
   if (rc) return rc;
   if (!grads) return NAIS_ERR_NULL;
+  if ((one_branch && p->n_branch != 1) || (opt && (!pairs_fused_layout(*p) || !(opt->lr >= 0.f) || !(opt->eps >= 0.f)))) return NAIS_ERR_MODE;
   if (batch->B == 0) return 0;
-  if (!score_parts || !row_sum || !dscore || !workspace) return NAIS_ERR_NULL;
+  if (!inputs || !workspace) return NAIS_ERR_NULL;
   if (!aligned16(workspace)) return NAIS_ERR_ALIGN;
   if (workspace_bytes < pairs_bwd_workspace_bytes(*p, *batch)) return NAIS_ERR_WORKSPACE;
-  return launch_pairs_bwd(*p, *batch, score_parts, row_sum, reinterpret_cast<const unsigned long long*>(act_mask), dscore, *grads,
-                          nullptr, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+  return 0;
+}
+
+// The backward of nais_pairs_backward, of nais_pairs_backward_adagrad (the fused optimizer `opt`) and of
+// nais_pairs_backward_presorted (one branch, on lists sorted and joined by nais_pairs_forward_presort: finish only).  Sort, then
+// finish, one branch at a time: two branches of the general layout may share a list, whose workspace buffers then serve one after
+// the other.
+static int backward_call(const NaisParams* p, const NaisPairs* batch, const float* score_parts, const float* row_sum,
+                         const uint64_t* act_mask, const float* dscore, const NaisGrads* grads, bool grads_given,
+                         const NaisAdagrad* opt, bool presorted, void* workspace, size_t workspace_bytes, nais_stream_t stream) {
+  int rc = check_backward_call(p, batch, grads_given, presorted, opt, score_parts && row_sum && dscore, workspace, workspace_bytes);
+  if (rc || batch->B == 0) return rc;
+  PairsBwd bwd;
+  rc = bwd.open(*p, *batch, *grads, opt, score_parts, row_sum, reinterpret_cast<const unsigned long long*>(act_mask), dscore,
+                workspace, workspace_bytes, presorted);
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  for (int bi = 0; bi < bwd.n_branch && !rc; ++bi) {
+    if (!presorted) bwd.sort(bi, st, false);
+    rc = bwd.finish(bi, st, false, nullptr);
+  }
+  return rc;
+}
+
+int nais_pairs_backward(const NaisParams* p, const NaisPairs* batch, const float* score_parts, const float* row_sum,
+                        const uint64_t* act_mask, const float* dscore, const NaisGrads* grads, void* workspace,
+                        size_t workspace_bytes, nais_stream_t stream) {
+  return backward_call(p, batch, score_parts, row_sum, act_mask, dscore, grads, grads, nullptr, false, workspace, workspace_bytes, stream);
 }
 
 // Training forward of the autograd path: the coming backward's id sorts are forked onto the side streams, the forward kernel runs
@@ -369,63 +394,34 @@ int nais_pairs_backward(const NaisParams* p, const NaisPairs* batch, const float
 int nais_pairs_forward_presort(const NaisParams* p, const NaisPairs* batch, const NaisGrads* grads, float* score, float* row_sum,
                                float* score_parts, uint64_t* act_mask, void* bwd_workspace, size_t bwd_workspace_bytes,
                                nais_stream_t stream) {
-  int rc = check_params(p);
-  if (rc) return rc;
-  rc = check_pairs(p, batch);
-  if (rc) return rc;
-  if (!grads) return NAIS_ERR_NULL;
-  if (p->n_branch != 1) return NAIS_ERR_MODE;
-  if (batch->B && !score) return NAIS_ERR_NULL;
-  if (batch->B == 0) return 0;
-  if (!bwd_workspace) return NAIS_ERR_NULL;
-  if (!aligned16(bwd_workspace)) return NAIS_ERR_ALIGN;
-  if (bwd_workspace_bytes < pairs_bwd_workspace_bytes(*p, *batch)) return NAIS_ERR_WORKSPACE;
+  int rc = check_backward_call(p, batch, grads, true, nullptr, score, bwd_workspace, bwd_workspace_bytes);
+  if (rc || batch->B == 0) return rc;
   bool tc = false;
   rc = choose_pairs_fwd(*p, *batch, &tc);
+  PairsBwd bwd;
+  if (!rc) rc = bwd.open(*p, *batch, *grads, nullptr, nullptr, nullptr, nullptr, nullptr, bwd_workspace, bwd_workspace_bytes, true);
   if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, *grads, nullptr, bwd_workspace, bwd_workspace_bytes, st, BWD_SORTS);
+  for (int bi = 0; bi < bwd.n_branch; ++bi) bwd.sort(bi, st, true);
+  rc = (int)cudaGetLastError();
   if (rc) return rc;
   rc = launch_chosen_fwd(tc, *p, *batch, score, row_sum, score_parts, reinterpret_cast<unsigned long long*>(act_mask), st);
   // (also after a failed forward launch: the caller may release the workspace as soon as this returns)
-  const int rj = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, *grads, nullptr, bwd_workspace, bwd_workspace_bytes, st,
-                                  BWD_JOIN_SORTS);
+  const int rj = bwd.join_sorts(st);
   return rc ? rc : rj;
 }
 
 int nais_pairs_backward_presorted(const NaisParams* p, const NaisPairs* batch, const float* score_parts, const float* row_sum,
                                   const uint64_t* act_mask, const float* dscore, const NaisGrads* grads, void* workspace,
                                   size_t workspace_bytes, nais_stream_t stream) {
-  int rc = check_params(p);
-  if (rc) return rc;
-  rc = check_pairs(p, batch);
-  if (rc) return rc;
-  if (!grads) return NAIS_ERR_NULL;
-  if (p->n_branch != 1) return NAIS_ERR_MODE;
-  if (batch->B == 0) return 0;
-  if (!score_parts || !row_sum || !dscore || !workspace) return NAIS_ERR_NULL;
-  if (!aligned16(workspace)) return NAIS_ERR_ALIGN;
-  if (workspace_bytes < pairs_bwd_workspace_bytes(*p, *batch)) return NAIS_ERR_WORKSPACE;
-  return launch_pairs_bwd(*p, *batch, score_parts, row_sum, reinterpret_cast<const unsigned long long*>(act_mask), dscore, *grads,
-                          nullptr, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), BWD_AFTER_JOIN);
+  return backward_call(p, batch, score_parts, row_sum, act_mask, dscore, grads, grads, nullptr, true, workspace, workspace_bytes, stream);
 }
 
 int nais_pairs_backward_adagrad(const NaisParams* p, const NaisPairs* batch, const float* score_parts, const float* row_sum,
                                 const uint64_t* act_mask, const float* dscore, const NaisGrads* grads, const NaisAdagrad* opt,
                                 void* workspace, size_t workspace_bytes, nais_stream_t stream) {
-  int rc = check_params(p);
-  if (rc) return rc;
-  rc = check_pairs(p, batch);
-  if (rc) return rc;
-  if (!grads || !opt) return NAIS_ERR_NULL;
-  if (!pairs_fused_layout(*p)) return NAIS_ERR_MODE;
-  if (!(opt->lr >= 0.f) || !(opt->eps >= 0.f)) return NAIS_ERR_MODE;
-  if (batch->B == 0) return 0;
-  if (!score_parts || !row_sum || !dscore || !workspace) return NAIS_ERR_NULL;
-  if (!aligned16(workspace)) return NAIS_ERR_ALIGN;
-  if (workspace_bytes < pairs_bwd_workspace_bytes(*p, *batch)) return NAIS_ERR_WORKSPACE;
-  return launch_pairs_bwd(*p, *batch, score_parts, row_sum, reinterpret_cast<const unsigned long long*>(act_mask), dscore, *grads,
-                          opt, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+  return backward_call(p, batch, score_parts, row_sum, act_mask, dscore, grads, grads && opt, opt, false, workspace, workspace_bytes,
+                       stream);
 }
 
 // ---- nais_pairs_train_step: forward -> sigmoid + BCE -> backward (tables stepped in the segment reduce) -> dense Adagrad ----------
@@ -480,15 +476,82 @@ static int check_train_state(const NaisParams* p, const NaisAdagrad* tables, con
   return 0;
 }
 
-// What one train_step_impl call enqueues: the whole step; only the id sorts of its backward (on the side streams, joined to `st`:
-// nais_train_users runs them for the NEXT user on its preparation stream); or the step on lists sorted by a STEP_SORTS call (same
-// arguments).
-enum StepPart { STEP_ALL = 0, STEP_SORTS = 1, STEP_AFTER_SORTS = 2 };
+// One optimizer step in its workspace (arguments already checked): the forward's kernel choice, the backward's context with the
+// gradient scratch of the MLP / distance layer (which also tells the backward which lists it needs), and per branch the dense
+// Adagrad of those tensors.  That Adagrad rides behind the kernel that finishes their gradients, next to the table reduces: one
+// launch less on the step's chain of dependent launches.  Two branches: branch 1's also steps row 0 of embed_distance, whose
+// gradient both branches' param_reduce add up.
+struct TrainStep {
+  TrainStepLayout L;
+  char* base;
+  bool fwd_tc = false;
+  unsigned long long* mask;
+  DenseAdagradLaunch da[2];
+  PairsBwd bwd;
+  float* f(size_t off) const { return reinterpret_cast<float*>(base + off); }
+};
 
-// the launches of one optimizer step (arguments already checked)
-static int train_step_impl(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
-                           const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace,
-                           size_t workspace_bytes, cudaStream_t st, StepPart part = STEP_ALL);
+static int open_train_step(TrainStep& s, const NaisParams* p, const NaisPairs* batch, const NaisAdagrad* tables,
+                           const NaisDenseAdagrad* dense, void* workspace, size_t workspace_bytes) {
+  const TrainStepLayout& L = s.L = train_step_layout(*p, *batch);
+  if (workspace_bytes < L.total) return NAIS_ERR_WORKSPACE;
+  s.base = reinterpret_cast<char*>(workspace);
+  NaisGrads g = {};
+  for (int bi = 0; bi < p->n_branch; ++bi) {
+    g.w1[bi] = s.f(L.gw1[bi]);
+    g.b1[bi] = s.f(L.gb1[bi]);
+    g.w2[bi] = s.f(L.gw2[bi]);
+  }
+  if (p->dist_mode == NAIS_DIST_LATLON) {
+    g.dist_w = s.f(L.gdw);
+    g.dist_b = s.f(L.gdb);
+  }
+  if (p->dist_mode == NAIS_DIST_KM) g.dist_embed = s.f(L.gde);
+  const NaisBranch& br = p->branch[0];
+  const int lanes = p->dist_mode == NAIS_DIST_LATLON ? 2 : 0, ldw = br.w_poi + br.w_reg + lanes;
+  s.da[0] = {{const_cast<float*>(br.w1), const_cast<float*>(br.b1), const_cast<float*>(br.w2),
+              lanes ? const_cast<float*>(p->dist_w) : nullptr, lanes ? const_cast<float*>(p->dist_b) : nullptr},
+             {dense->sum_w1, dense->sum_b1, dense->sum_w2, dense->sum_dist_w, dense->sum_dist_b},
+             {g.w1[0], g.b1[0], g.w2[0], g.dist_w, g.dist_b},
+             {p->hid * ldw, p->hid, p->hid, 4, 2},
+             dense->lr, dense->eps};
+  if (p->n_branch == 2) {
+    const NaisBranch& r = p->branch[1];
+    const bool km = p->dist_mode == NAIS_DIST_KM;
+    s.da[1] = {{const_cast<float*>(r.w1), const_cast<float*>(r.b1), const_cast<float*>(r.w2), km ? const_cast<float*>(p->dist_embed) : nullptr,
+                nullptr},
+               {dense->sum_region_w1, dense->sum_region_b1, dense->sum_region_w2, dense->sum_dist_embed, nullptr},
+               {g.w1[1], g.b1[1], g.w2[1], g.dist_embed, nullptr},
+               {p->hid * (r.w_poi + r.w_reg), p->hid, p->hid, r.w_poi + r.w_reg, 0},
+               dense->lr, dense->eps};
+  }
+  const int rc = choose_pairs_fwd(*p, *batch, &s.fwd_tc);
+  if (rc) return rc;
+  s.mask = (s.fwd_tc && p->hid <= 64) ? reinterpret_cast<unsigned long long*>(s.base + L.mask) : nullptr;
+  return s.bwd.open(*p, *batch, g, tables, s.f(L.parts), s.f(L.row_sum), s.mask, s.f(L.dscore), s.base + L.bwd, workspace_bytes - L.bwd,
+                    true);
+}
+
+// The backward's id sorts depend on the batch only: forked onto the side streams, they run next to what `st` runs after them.
+static int train_step_sorts(const TrainStep& s, cudaStream_t st) {
+  for (int bi = 0; bi < s.bwd.n_branch; ++bi) s.bwd.sort(bi, st, true);
+  return (int)cudaGetLastError();
+}
+
+// forward -> sigmoid + BCE -> backward (MLP / distance-layer gradients to scratch, tables stepped in place).  wait_sorted0: the
+// lists were sorted by this step's train_step_sorts and not joined since.
+static int train_step_rest(const TrainStep& s, const float* label, const float* row_weight, float* loss, float* score_out,
+                           cudaStream_t st, bool wait_sorted0) {
+  int rc = launch_chosen_fwd(s.fwd_tc, s.bwd.p, s.bwd.b, s.f(s.L.score), s.f(s.L.row_sum), s.f(s.L.parts), s.mask, st);
+  if (rc) return rc;
+  if (score_out) {
+    cudaError_t e = cudaMemcpyAsync(score_out, s.f(s.L.score), (size_t)s.bwd.b.B * 4, cudaMemcpyDeviceToDevice, st);
+    if (e != cudaSuccess) return (int)e;
+  }
+  rc = launch_bce_dscore(s.f(s.L.score), label, row_weight, s.bwd.b.B, s.f(s.L.dscore), loss, st);
+  for (int bi = 0; bi < s.bwd.n_branch && !rc; ++bi) rc = s.bwd.finish(bi, st, wait_sorted0, &s.da[bi]);
+  return rc;
+}
 
 int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
                           const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace,
@@ -503,76 +566,11 @@ int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, const flo
   if (batch->B == 0) return 0;
   if (!label || !workspace) return NAIS_ERR_NULL;
   if (!aligned16(workspace)) return NAIS_ERR_ALIGN;
-  return train_step_impl(p, batch, label, row_weight, tables, dense, loss, score_out, workspace, workspace_bytes,
-                         static_cast<cudaStream_t>(stream));
-}
-
-static int train_step_impl(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
-                           const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace,
-                           size_t workspace_bytes, cudaStream_t st, StepPart part) {
-  int rc;
-  const TrainStepLayout L = train_step_layout(*p, *batch);
-  if (workspace_bytes < L.total) return NAIS_ERR_WORKSPACE;
-  char* base = reinterpret_cast<char*>(workspace);
-  auto F = [&](size_t off) { return reinterpret_cast<float*>(base + off); };
-  // the gradient scratch of the MLP / distance layer (also tells the backward which lists it needs)
-  NaisGrads g;
-  memset(&g, 0, sizeof(g));
-  for (int bi = 0; bi < p->n_branch; ++bi) {
-    g.w1[bi] = F(L.gw1[bi]);
-    g.b1[bi] = F(L.gb1[bi]);
-    g.w2[bi] = F(L.gw2[bi]);
-  }
-  if (p->dist_mode == NAIS_DIST_LATLON) {
-    g.dist_w = F(L.gdw);
-    g.dist_b = F(L.gdb);
-  }
-  if (p->dist_mode == NAIS_DIST_KM) g.dist_embed = F(L.gde);
-  // the id sorts of the backward depend on the batch only: forked onto side streams now, they run next to the forward
-  if (part != STEP_AFTER_SORTS) {
-    rc = launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, g, tables, base + L.bwd, workspace_bytes - L.bwd, st, BWD_SORTS);
-    if (rc) return rc;
-  }
-  if (part == STEP_SORTS)
-    return launch_pairs_bwd(*p, *batch, nullptr, nullptr, nullptr, nullptr, g, tables, base + L.bwd, workspace_bytes - L.bwd, st,
-                            BWD_JOIN_SORTS);
-  // forward
-  bool fwd_tc = false;
-  rc = choose_pairs_fwd(*p, *batch, &fwd_tc);
-  if (rc) return rc;
-  unsigned long long* mask = (fwd_tc && p->hid <= 64) ? reinterpret_cast<unsigned long long*>(base + L.mask) : nullptr;
-  rc = launch_chosen_fwd(fwd_tc, *p, *batch, F(L.score), F(L.row_sum), F(L.parts), mask, st);
-  if (rc) return rc;
-  if (score_out) {
-    cudaError_t e = cudaMemcpyAsync(score_out, F(L.score), (size_t)batch->B * 4, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) return (int)e;
-  }
-  rc = launch_bce_dscore(F(L.score), label, row_weight, batch->B, F(L.dscore), loss, st);
-  if (rc) return rc;
-  // backward: MLP / distance-layer gradients to scratch, tables stepped in place
-  // (the dense Adagrad of the MLP / distance-layer tensors rides behind the kernel that finishes their gradients, next to the
-  // table reduces: one launch less on the step's chain of dependent launches)
-  // (two branches: branch 1's launch also steps row 0 of embed_distance, whose gradient both branches' param_reduce add up)
-  const NaisBranch& br = p->branch[0];
-  const int lanes = p->dist_mode == NAIS_DIST_LATLON ? 2 : 0, ldw = br.w_poi + br.w_reg + lanes;
-  DenseAdagradLaunch da[2] = {{{const_cast<float*>(br.w1), const_cast<float*>(br.b1), const_cast<float*>(br.w2),
-                                lanes ? const_cast<float*>(p->dist_w) : nullptr, lanes ? const_cast<float*>(p->dist_b) : nullptr},
-                               {dense->sum_w1, dense->sum_b1, dense->sum_w2, dense->sum_dist_w, dense->sum_dist_b},
-                               {g.w1[0], g.b1[0], g.w2[0], g.dist_w, g.dist_b},
-                               {p->hid * ldw, p->hid, p->hid, 4, 2},
-                               dense->lr, dense->eps}};
-  if (p->n_branch == 2) {
-    const NaisBranch& r = p->branch[1];
-    const bool km = p->dist_mode == NAIS_DIST_KM;
-    da[1] = {{const_cast<float*>(r.w1), const_cast<float*>(r.b1), const_cast<float*>(r.w2), km ? const_cast<float*>(p->dist_embed) : nullptr,
-              nullptr},
-             {dense->sum_region_w1, dense->sum_region_b1, dense->sum_region_w2, dense->sum_dist_embed, nullptr},
-             {g.w1[1], g.b1[1], g.w2[1], g.dist_embed, nullptr},
-             {p->hid * (r.w_poi + r.w_reg), p->hid, p->hid, r.w_poi + r.w_reg, 0},
-             dense->lr, dense->eps};
-  }
-  return launch_pairs_bwd(*p, *batch, F(L.parts), F(L.row_sum), mask, F(L.dscore), g, tables, base + L.bwd, workspace_bytes - L.bwd, st,
-                          part == STEP_AFTER_SORTS ? BWD_AFTER_JOIN : BWD_AFTER_SORTS, da);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  TrainStep s;
+  rc = open_train_step(s, p, batch, tables, dense, workspace, workspace_bytes);
+  if (!rc) rc = train_step_sorts(s, st);
+  return rc ? rc : train_step_rest(s, label, row_weight, loss, score_out, st, true);
 }
 
 // ---- nais_train_users: the reference's one-user-per-step schedule, a list of users per call ---------------------------------------
@@ -767,8 +765,10 @@ int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, in
                                 need_co ? poi_coords : nullptr, seed + (uint64_t)u, H, const_cast<int64_t*>(ub.b.tgt),
                                 reinterpret_cast<float*>(base + L.label), need_reg ? const_cast<int64_t*>(ub.b.treg) : nullptr,
                                 need_co ? const_cast<float*>(ub.b.tgt_coords) : nullptr, ps);
-    if (r) return r;
-    return train_step_impl(p, &ub.b, ub.label, nullptr, tables, dense, nullptr, nullptr, ub.step, L.total - L.step, ps, STEP_SORTS);
+    TrainStep s;  // the step's id sorts, joined to the preparation stream (the step waits for `prepared`)
+    if (!r) r = open_train_step(s, p, &ub.b, tables, dense, ub.step, L.total - L.step);
+    if (!r) r = train_step_sorts(s, ps);
+    return r ? r : s.bwd.join_sorts(ps);
   };
   // users with a history, in order; the others only get a zero loss
   int next = 0;
@@ -806,7 +806,9 @@ int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, in
     NaisParams pu = *p;  // (the id sorts of the preparation depend on the batch only, not on the dropout seed)
     if (p->dropout_p > 0.f) pu.dropout_seed = host_dropout_seeds[cur];
     cudaStreamWaitEvent(st, prepared[cur_slot], 0);
-    rc = train_step_impl(&pu, &ub.b, ub.label, nullptr, tables, dense, losses + cur, nullptr, ub.step, L.total - L.step, st, STEP_AFTER_SORTS);
+    TrainStep s;  // the rest of the step, on the lists the preparation sorted
+    rc = open_train_step(s, &pu, &ub.b, tables, dense, ub.step, L.total - L.step);
+    if (!rc) rc = train_step_rest(s, ub.label, nullptr, losses + cur, nullptr, st, false);
     if (rc) return bail(rc);
     cudaEventRecord(stepped[cur_slot], st);
     ++done;

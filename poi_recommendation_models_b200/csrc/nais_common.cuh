@@ -52,7 +52,7 @@ struct SmemAttrOnce {
   }
 };
 
-// The dense Adagrad step of the MLP / distance-layer tensors (nais_pairs_train_step), as launch_pairs_bwd enqueues it right behind
+// The dense Adagrad step of the MLP / distance-layer tensors (nais_pairs_train_step), as PairsBwd::finish enqueues it right behind
 // the kernel that finishes their gradients: w1, b1, w2, dist_w, dist_b (NULL param = absent).
 struct DenseAdagradLaunch {
   float* param[5];
@@ -62,14 +62,43 @@ struct DenseAdagradLaunch {
   float lr, eps;
 };
 
-// What one launch_pairs_bwd call enqueues (nais_bwd.cu).  The id sorts depend on the batch only, so a caller may fork them ahead:
-enum BwdPhase : int {
-  BWD_ALL = 0,         // the whole backward
-  BWD_SORTS = 1,       // only the id sorts, ALL of them on side streams (the one-call training step forks them before its forward)
-  BWD_AFTER_SORTS = 2, // the rest, on lists sorted by a BWD_SORTS call (same p, b, g, opt, ws)
-  BWD_AFTER_JOIN = 3,  // BWD_AFTER_SORTS after a BWD_JOIN_SORTS (no wait of its own for the long list)
-  BWD_JOIN_SORTS = 4,  // join the sort streams of a BWD_SORTS call to `stream` (so that nothing enqueued on `stream` later — or
-                       // the caller's allocator — can overtake the sorts)
+// Byte offsets of the pair backward's workspace (nais_bwd.cu bwd_layout)
+struct BwdLayout {
+  size_t dq, dp, part, kin[3], vin[3], kout[3], vout[3], cub[3], pkey[3], pstart[3], prows[3], cub_bytes, total;
+  int grid, stride;
+};
+
+// One call's pair backward (nais_bwd.cu): `open` makes every argument check, three steps enqueue the work:
+//   sort        for branch bi < n_branch: make_keys and the stable radix sorts of the branch's id lists: lists 1 / 2 on side
+//               streams 0 / 1, list 0 on `stream` or, with fork_long, on side stream 2, which then records `sorted0`;
+//   join_sorts  `stream` waits for every branch's sorts, so that nothing enqueued on it later — nor the caller's allocator — can
+//               overtake them;
+//   finish      for branch bi: the tile kernel, param_reduce (+ `dense`) on side stream 2, the three segment reduces and the
+//               joins.  wait_sorted0: list 0 was sorted with fork_long and not joined since.
+// The sorts depend on the batch only.  The one-call backward sorts and finishes one branch at a time; `split` callers run every
+// sort ahead of their forward and every finish after it, which needs each id list to belong to one branch (pairs_fused_layout).
+struct SideStreams;
+struct PairsBwd {
+  NaisParams p;  // (copies of the call's structs)
+  NaisPairs b;
+  NaisGrads g;
+  const NaisAdagrad* opt;
+  const float *score_parts, *row_sum, *dscore;  // the finish step's inputs (NULL: the call only sorts)
+  const unsigned long long* act_mask;
+  BwdLayout L;
+  char* base;  // the workspace
+  SideStreams* side;
+  int64_t n_of[3];   // entries of the lists: 0 = history ids (B*H), 1 = target ids (B), 2 = region ids of both (B*H + B)
+  int n_branch = 0;  // branches the steps process: 0 when the batch has no tiles
+  bool want[2][3];   // per branch, the lists it processes
+
+  int open(const NaisParams& p, const NaisPairs& b, const NaisGrads& g, const NaisAdagrad* opt, const float* score_parts,
+           const float* row_sum, const unsigned long long* act_mask, const float* dscore, void* ws, size_t ws_bytes, bool split);
+  void sort(int bi, cudaStream_t stream, bool fork_long) const;
+  int join_sorts(cudaStream_t stream) const;
+  int finish(int bi, cudaStream_t stream, bool wait_sorted0, const DenseAdagradLaunch* dense) const;
+  int* I(size_t off) const { return reinterpret_cast<int*>(base + off); }  // workspace words at a byte offset
+  uint32_t* U(size_t off) const { return reinterpret_cast<uint32_t*>(base + off); }
 };
 
 // Device address (current device) of the library's 4-byte bad-index word (nais_capi.cu); every launcher passes it to its kernel.

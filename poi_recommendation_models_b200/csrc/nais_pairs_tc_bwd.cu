@@ -981,7 +981,7 @@ bool pairs_tc_bwd_supported(const NaisParams& p, const NaisPairs& b) {
 }
 
 // grid <= 2 CTAs per SM (256 TMEM columns each); every CTA owns at least one tile (the caller passes min(n_items, grid)).  With
-// dropout A.act_mask must be the forward's pattern (launch_pairs_bwd runs the FP32 kernel instead when it is NULL).
+// dropout A.act_mask must be the forward's pattern (PairsBwd::finish runs the FP32 kernel instead when it is NULL).
 int launch_pairs_bwd_tc(const BwdArgs& A, int D, int grid, cudaStream_t stream) {
   if (A.p.dropout_p > 0.f) return A.act_mask ? ptcb::launch_shape<true>(A, D, grid, stream) : NAIS_ERR_NULL;
   return ptcb::launch_shape<false>(A, D, grid, stream);
