@@ -644,7 +644,7 @@ __global__ void segment_reduce_pass1_kernel(const int* __restrict__ keys, const 
   for (int q = 0; q < NQ; ++q) acc[q] = 0.f;
   int key = __shfl_sync(0xffffffffu, k0, 0), run_a = 0;  // the open run: its key and first entry
   auto flush = [&](int b) {                               // the open run ends before entry b
-    if (key >= n_rows) return;                            // ids outside the table (make_keys_kernel) are dropped
+    if ((unsigned)key >= (unsigned)n_rows) return;        // ids outside [0, n_rows) (make_keys_kernel's n_rows) are dropped
     const bool left = run_a == 0 && key == key_before, right = b == cnt && key == key_after;
     if (!left && !right) {
 #pragma unroll
@@ -685,7 +685,7 @@ __global__ void segment_reduce_pass1_kernel(const int* __restrict__ keys, const 
       fkey[u] = -1;
       if (j < cnt) {
         if (j > 0 && ((starts >> j) & 1ull)) {
-          if (kOpt && key < n_rows && !(run_a == 0 && key == key_before)) {
+          if (kOpt && (unsigned)key < (unsigned)n_rows && !(run_a == 0 && key == key_before)) {
             fkey[u] = key;
 #pragma unroll
             for (int q = 0; q < NQ; ++q) facc[u][q] = acc[q];

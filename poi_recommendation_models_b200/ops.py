@@ -560,14 +560,20 @@ def pairs_backward_compact(variant: str, beta: float, P: Dict[str, torch.Tensor]
 
 def rows_adagrad(keys: torch.Tensor, rows: torch.Tensor, param: torch.Tensor, state_sum: torch.Tensor, lr: float, eps: float) -> None:
     """nais_rows_adagrad: one row-sparse Adagrad step on `param` / `state_sum` (in place) from key-ordered (id, gradient row) pairs;
-    equal ids are summed first, in list order (deterministic)."""
+    equal ids are summed first, in list order (deterministic).  Ids outside [0, param rows) are skipped."""
+    n, w = rows.shape
+    if keys.dim() != 1 or keys.shape[0] != n:
+        raise RuntimeError(f"rows_adagrad: keys must be 1-D with one id per row ({n}); got {tuple(keys.shape)}")
+    if param.dim() != 2 or param.shape[1] != w or state_sum.shape != param.shape:
+        raise RuntimeError(f"rows_adagrad: param and its state must be [rows, {w}]; got {tuple(param.shape)} and {tuple(state_sum.shape)}")
     dev = _need_cuda(keys, rows, param, state_sum)
     lib = _lib.load()
-    n, w = rows.shape
     if not (param.is_contiguous() and state_sum.is_contiguous() and param.dtype == torch.float32 and state_sum.dtype == torch.float32):
         raise RuntimeError("rows_adagrad: param and its state must be contiguous float32")
     with torch.cuda.device(dev):
-        k32 = keys.to(torch.int32).contiguous()
+        # (clamped before the int32 cast: an id >= 2**31 or >= 2**32 stays out of range instead of wrapping onto a real row; the
+        # clamp is monotone, so the list stays in key order)
+        k32 = keys.clamp(-1, param.shape[0]).to(torch.int32).contiguous()
         r = _f32(rows)
         ws_bytes = lib.nais_rows_adagrad_workspace_bytes(n, w)
         ws = torch.empty(max(ws_bytes, 16), device=dev, dtype=torch.uint8)

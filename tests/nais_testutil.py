@@ -72,6 +72,74 @@ def oracle_user_scores(sd, variant, beta, coords, region, history, cand, dtype=t
     return s.numpy(), scale.numpy()
 
 
+SEG_CHUNK = 64  # entries per pass-1 chunk of the sorted-segment reduce (csrc/nais_bwd.cu)
+
+
+def segment_reduce_ref(keys, rows, n_rows):
+    """The embedding-gradient segment reduce of csrc/nais_bwd.cu restated in float32, in its documented summation order, so
+    it must equal the kernel bit for bit: every maximal run of equal keys is split at multiples of SEG_CHUNK into pieces; a
+    piece is 0.f + r[a] + r[a+1] + ... in entry order; a run's gradient is its first piece plus the following pieces, added in
+    chunk order.  Runs whose key is outside [0, n_rows) are dropped.  keys [n] ascending, rows [n, w] float32.
+    Returns (ids int64 [runs], grads float32 [runs, w]) of the kept runs, ids ascending."""
+    keys = np.asarray(keys, dtype=np.int64)
+    rows = np.asarray(rows, dtype=np.float32)
+    n, w = rows.shape
+    assert keys.shape == (n,) and (n == 0 or np.all(np.diff(keys) >= 0)), "keys must be ascending, one per row"
+    if n == 0:
+        return np.zeros(0, np.int64), np.zeros((0, w), np.float32)
+    idx = np.arange(n)
+    run_start = np.ones(n, bool)
+    run_start[1:] = keys[1:] != keys[:-1]
+    piece_start = run_start | (idx % SEG_CHUNK == 0)
+    piece = np.cumsum(piece_start) - 1                       # piece of each entry
+    first = idx[piece_start]                                 # first entry of each piece
+    pos = idx - first[piece]                                 # position inside the piece (< SEG_CHUNK)
+    acc = np.zeros((len(first), w), np.float32)
+    for p in range(int(pos.max()) + 1):                      # one entry per piece per step: no repeated index in a step
+        sel = pos == p
+        acc[piece[sel]] += rows[sel]
+    run_of_piece = np.cumsum(run_start[first]) - 1
+    run_first_piece = np.flatnonzero(run_start[first])
+    k_in_run = np.arange(len(first)) - run_first_piece[run_of_piece]
+    g = acc[run_first_piece].copy()
+    for k in range(1, int(k_in_run.max()) + 1):
+        sel = k_in_run == k
+        g[run_of_piece[sel]] += acc[sel]
+    ids = keys[run_start]
+    keep = (ids >= 0) & (ids < n_rows)
+    return ids[keep], g[keep]
+
+
+def fmaf32(a, b, c):
+    """fmaf(a, b, c) on float32 arrays, rounded once like the device instruction: a*b is exact in float64, the float64 two-sum
+    of a*b and c is exact, and where rounding that sum to float32 falls on a tie the residual decides the direction."""
+    a, b, c = (np.asarray(x, dtype=np.float32) for x in (a, b, c))
+    ab = a.astype(np.float64) * b.astype(np.float64)
+    cd = c.astype(np.float64)
+    t = ab + cd
+    bb = t - ab
+    err = (ab - (t - bb)) + (cd - bb)
+    r = t.astype(np.float32)
+    rd = r.astype(np.float64)
+    with np.errstate(invalid="ignore"):
+        other = np.nextafter(r, np.where(t > rd, np.float32(np.inf), np.float32(-np.inf)).astype(np.float32))
+        tie = (rd != t) & ((rd + other.astype(np.float64)) * 0.5 == t)
+        # on a tie, the exact value t + err lies on err's side: take the float32 neighbour on that side
+        flip = tie & (err != 0) & (np.sign(err) != np.sign(rd - t))
+    return np.where(flip, other, r).astype(np.float32)
+
+
+def rows_adagrad_ref(param, state_sum, g, lr, eps):
+    """The row-sparse Adagrad step of the segment reduce (csrc/nais_bwd.cu seg_store) in float32:
+    s2 = fmaf(g, g, s);  p - (lr * g) / (sqrt(s2) + eps).  Returns (param, sum).  (torch.optim.Adagrad computes
+    p + (-lr) * (g / d), which can differ from this by one ulp.)"""
+    g = np.asarray(g, dtype=np.float32)
+    s2 = fmaf32(g, g, state_sum)
+    lr, eps = np.float32(lr), np.float32(eps)
+    p = np.asarray(param, dtype=np.float32) - (lr * g) / (np.sqrt(s2) + eps)
+    return p.astype(np.float32), s2
+
+
 def lists_equal_outside_ties(got_ids, got_scores, ref_scores_by_id, k, tol=TOL):
     """got list must be a valid top-k of ref scores: every listed id's ref score >= (k-th best ref score) - tie tol,
     and the ref order is respected outside tie groups."""
