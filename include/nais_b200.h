@@ -324,6 +324,24 @@ NAIS_API int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, 
                                    const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score,
                                    void* workspace, size_t workspace_bytes, nais_stream_t stream);
 
+/* nais_pairs_train_step with the pairwise BPR loss -log sigmoid(s+ - s-) instead of BCE (the batch's `label` is not read).  The B
+ * rows come in groups of G = 1 + num_neg consecutive rows: row g*G is the positive, rows g*G + 1 .. g*G + num_neg its negatives —
+ * the order nais_sample_batch writes.  With d_gj = score[g*G] - score[g*G + j]:
+ *   loss = sum_g w_g sum_{j=1..num_neg} softplus(-d_gj),  w_g = group_weight[g], or 1 / (n_groups * num_neg) when group_weight is
+ *   NULL (the mean over pairs: -logsigmoid(d).mean());  softplus(-d) = max(-d, 0) + log1p(exp(-|d|)), finite for any score.
+ *   dL/dscore[g*G + j] = w_g sigma(-d_gj) (torch's log_sigmoid backward form), dL/dscore[g*G] = -sum_j w_g sigma(-d_gj), j ascending.
+ * The loss is summed by one CTA in a fixed order (deterministic, no atomics).  group_weight = 1 / (pairs of the user of g) makes a
+ * segmented multi-user step the sum of the per-user mean BPR losses.  Optimizer, workspace (nais_pairs_train_step_workspace_bytes)
+ * and outputs as nais_pairs_train_step.  bpr NULL is NAIS_ERR_NULL; num_neg < 1 or B % (1 + num_neg) != 0 is NAIS_ERR_SHAPE. */
+typedef struct NaisBprLoss {
+  int32_t num_neg;           /* >= 1: rows in groups of 1 + num_neg, positive first */
+  int32_t reserved0;
+  const float* group_weight; /* [B / (1 + num_neg)] device, or NULL = mean over pairs */
+} NaisBprLoss;
+NAIS_API int nais_pairs_train_step_bpr(const NaisParams* p, const NaisPairs* batch, const NaisBprLoss* bpr, const NaisAdagrad* tables,
+                                       const NaisDenseAdagrad* dense, float* loss, float* score, void* workspace, size_t workspace_bytes,
+                                       nais_stream_t stream);
+
 /* The reference's training schedule — ONE optimizer step per user (run.py:227-255) — for a list of users in one call: per user,
  * nais_sample_batch over his history (every positive + num_ng negatives each, labels [1, 0..0]: batches.py:67-108) and
  * nais_pairs_train_step with the batch-mean BCE, enqueued back to back with no host work in between but the launches (~15 per
@@ -360,6 +378,15 @@ NAIS_API int nais_train_users_dropout(const NaisParams* p, const int64_t* host_i
                                       const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* losses, void* workspace,
                                       size_t workspace_bytes, float center_lat, float center_lon, const uint64_t* host_dropout_seeds,
                                       nais_stream_t stream);
+/* nais_train_users_dropout with the BPR loss of nais_pairs_train_step_bpr: per user, the sampler (seed + user id) draws num_ng
+ * negatives for each positive, and one optimizer step takes the mean BPR loss over the user's H * num_ng (positive, negative)
+ * pairs.  losses[i] is that mean (0 for a user without history).  Workspace: nais_train_users_workspace_bytes; preparation one
+ * user ahead, streams and dropout seeds as nais_train_users_dropout.  num_ng < 1 is NAIS_ERR_SHAPE. */
+NAIS_API int nais_train_users_bpr(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
+                                  const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region, const float* poi_coords,
+                                  const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables,
+                                  const NaisDenseAdagrad* dense, float* losses, void* workspace, size_t workspace_bytes, float center_lat,
+                                  float center_lon, const uint64_t* host_dropout_seeds, nais_stream_t stream);
 
 /* Workspace for nais_fullrank_topk / nais_fullrank_scores: n_users and nnz = offsets[n_users] are host-known. */
 NAIS_API size_t nais_fullrank_workspace_bytes(const NaisParams* p, int32_t n_users, int64_t nnz, int64_t poi_begin,

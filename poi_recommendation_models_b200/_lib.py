@@ -61,6 +61,10 @@ class NaisDenseAdagrad(C.Structure):
                 ("sum_region_w2", C.c_void_p), ("sum_dist_embed", C.c_void_p)]
 
 
+class NaisBprLoss(C.Structure):
+    _fields_ = [("num_neg", C.c_int32), ("reserved0", C.c_int32), ("group_weight", C.c_void_p)]
+
+
 class NaisCatalog(C.Structure):
     _fields_ = [("region", C.c_void_p), ("coords", C.c_void_p), ("row_base", C.c_int64), ("n_rows", C.c_int64),
                 ("center_lat", C.c_float), ("center_lon", C.c_float)]
@@ -87,6 +91,8 @@ SYMBOLS = {
     "nais_pairs_train_step_workspace_bytes": (C.c_size_t, [C.POINTER(NaisParams), C.POINTER(NaisPairs)]),
     "nais_pairs_train_step": (C.c_int, [C.POINTER(NaisParams), C.POINTER(NaisPairs), C.c_void_p, C.c_void_p, C.POINTER(NaisAdagrad),
                                         C.POINTER(NaisDenseAdagrad), C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "nais_pairs_train_step_bpr": (C.c_int, [C.POINTER(NaisParams), C.POINTER(NaisPairs), C.POINTER(NaisBprLoss), C.POINTER(NaisAdagrad),
+                                            C.POINTER(NaisDenseAdagrad), C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "nais_train_users_workspace_bytes": (C.c_size_t, [C.POINTER(NaisParams), C.c_int32, C.c_int32]),
     "nais_train_users": (C.c_int, [C.POINTER(NaisParams), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_int32, C.c_int32, C.c_uint64, C.POINTER(NaisAdagrad), C.POINTER(NaisDenseAdagrad),
@@ -99,6 +105,10 @@ SYMBOLS = {
                                            C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_uint64, C.POINTER(NaisAdagrad),
                                            C.POINTER(NaisDenseAdagrad), C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float,
                                            C.c_void_p, C.c_void_p]),
+    "nais_train_users_bpr": (C.c_int, [C.POINTER(NaisParams), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_uint64, C.POINTER(NaisAdagrad),
+                                       C.POINTER(NaisDenseAdagrad), C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float,
+                                       C.c_void_p, C.c_void_p]),
     "nais_rows_adagrad_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32]),
     "nais_rows_adagrad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_float, C.c_float, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -836,6 +836,52 @@ int launch_bce_dscore(const float* score, const float* label, const float* row_w
   return (int)cudaGetLastError();
 }
 
+// nais_pairs_train_step_bpr (include/nais_b200.h): the BPR loss -log sigmoid(s+ - s-) on rows in groups of G = 1 + num_neg
+// (positive first), one CTA, the fixed reduction tree of bce_dscore_kernel (deterministic loss).  d = s[gG] - s[gG + j];
+// loss = sum_g w_g sum_j softplus(-d) with softplus(-d) = max(-d, 0) + log1p(exp(-|d|)) (finite for any |d|); its derivative
+// sigma(-d) in the form of torch's log_sigmoid backward: z = exp(-|d|), z / (1 + z) for d >= 0, 1 - z / (1 + z) for d < 0.
+// dscore[negative j] = w_g sigma(-d_j); dscore[positive] = -sum_j w_g sigma(-d_j), summed over j ascending.
+__global__ void __launch_bounds__(1024, 1) bpr_dscore_kernel(const float* __restrict__ score, const float* __restrict__ group_weight,
+                                                              int64_t n_groups, int num_neg, float* __restrict__ dscore,
+                                                              float* __restrict__ loss) {
+  __shared__ float red[32];
+  const int G = num_neg + 1;
+  const float wmean = 1.f / (float)(n_groups * num_neg);
+  float acc = 0.f;
+  for (int64_t g = threadIdx.x; g < n_groups; g += blockDim.x) {
+    const float* s = score + g * G;
+    float* ds = dscore + g * G;
+    const float sp = s[0], w = group_weight ? group_weight[g] : wmean;
+    float dpos = 0.f;
+    for (int j = 1; j < G; ++j) {
+      const float d = sp - s[j];
+      const float z = expf(-fabsf(d));
+      acc = fmaf(w, fmaxf(-d, 0.f) + log1pf(z), acc);
+      const float q = z / (1.f + z);
+      const float gj = w * (d >= 0.f ? q : 1.f - q);
+      ds[j] = gj;
+      dpos -= gj;
+    }
+    ds[0] = dpos;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    float v = threadIdx.x < (blockDim.x >> 5) ? red[threadIdx.x] : 0.f;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (threadIdx.x == 0) *loss = v;
+  }
+}
+int launch_bpr_dscore(const float* score, const float* group_weight, int64_t B, int num_neg, float* dscore, float* loss,
+                      cudaStream_t stream) {
+  bpr_dscore_kernel<<<1, 1024, 0, stream>>>(score, group_weight, B / (num_neg + 1), num_neg, dscore, loss);
+  NAIS_COUNT_LAUNCH(1);
+  return (int)cudaGetLastError();
+}
+
 // dense Adagrad of up to 5 small tensors in one launch (torch.optim.Adagrad, weight_decay = lr_decay = 0)
 struct DenseAdagradArgs {
   float* param[5];

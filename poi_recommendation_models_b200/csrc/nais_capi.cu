@@ -50,6 +50,8 @@ int launch_sample_batch(const int64_t* seg_offsets, const int64_t* hist, int n_s
 bool pairs_tc_supported(const NaisParams& p, const NaisPairs& b);
 int launch_bce_dscore(const float* score, const float* label, const float* row_weight, int64_t B, float* dscore, float* loss,
                       cudaStream_t stream);
+int launch_bpr_dscore(const float* score, const float* group_weight, int64_t B, int num_neg, float* dscore, float* loss,
+                      cudaStream_t stream);
 int launch_dense_adagrad(float* const* param, float* const* sum, const float* const* grad, const int* n, float lr, float eps,
                          cudaStream_t stream);
 int launch_pairs_fwd_tc(const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts,
@@ -538,39 +540,64 @@ static int train_step_sorts(const TrainStep& s, cudaStream_t st) {
   return (int)cudaGetLastError();
 }
 
-// forward -> sigmoid + BCE -> backward (MLP / distance-layer gradients to scratch, tables stepped in place).  wait_sorted0: the
-// lists were sorted by this step's train_step_sorts and not joined since.
-static int train_step_rest(const TrainStep& s, const float* label, const float* row_weight, float* loss, float* score_out,
-                           cudaStream_t st, bool wait_sorted0) {
+// The loss a training step takes on its [B] scores: sigmoid + BCE on `label` (weights `row_weight`, NULL = batch mean), or, with
+// bpr_num_neg > 0, BPR over groups of 1 + bpr_num_neg rows (weights `group_weight`, NULL = mean over pairs).
+struct StepLoss {
+  const float* label;
+  const float* row_weight;
+  int bpr_num_neg;
+  const float* group_weight;
+};
+
+// forward -> loss -> backward (MLP / distance-layer gradients to scratch, tables stepped in place).  wait_sorted0: the lists were
+// sorted by this step's train_step_sorts and not joined since.
+static int train_step_rest(const TrainStep& s, const StepLoss& sl, float* loss, float* score_out, cudaStream_t st, bool wait_sorted0) {
   int rc = launch_chosen_fwd(s.fwd_tc, s.bwd.p, s.bwd.b, s.f(s.L.score), s.f(s.L.row_sum), s.f(s.L.parts), s.mask, st);
   if (rc) return rc;
   if (score_out) {
     cudaError_t e = cudaMemcpyAsync(score_out, s.f(s.L.score), (size_t)s.bwd.b.B * 4, cudaMemcpyDeviceToDevice, st);
     if (e != cudaSuccess) return (int)e;
   }
-  rc = launch_bce_dscore(s.f(s.L.score), label, row_weight, s.bwd.b.B, s.f(s.L.dscore), loss, st);
+  rc = sl.bpr_num_neg > 0 ? launch_bpr_dscore(s.f(s.L.score), sl.group_weight, s.bwd.b.B, sl.bpr_num_neg, s.f(s.L.dscore), loss, st)
+                          : launch_bce_dscore(s.f(s.L.score), sl.label, sl.row_weight, s.bwd.b.B, s.f(s.L.dscore), loss, st);
   for (int bi = 0; bi < s.bwd.n_branch && !rc; ++bi) rc = s.bwd.finish(bi, st, wait_sorted0, &s.da[bi]);
   return rc;
 }
 
-int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
-                          const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace,
-                          size_t workspace_bytes, nais_stream_t stream) {
+// nais_pairs_train_step / nais_pairs_train_step_bpr: `bpr` NULL = the BCE step on `label`.
+static int pairs_train_step(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
+                            const NaisBprLoss* bpr, const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss,
+                            float* score_out, void* workspace, size_t workspace_bytes, nais_stream_t stream) {
   int rc = check_params(p);
   if (rc) return rc;
   rc = check_pairs(p, batch);
   if (rc) return rc;
+  if (bpr && (bpr->num_neg < 1 || batch->B % (1 + (int64_t)bpr->num_neg) != 0)) return NAIS_ERR_SHAPE;
   if (!loss) return NAIS_ERR_NULL;
   rc = check_train_state(p, tables, dense);
   if (rc) return rc;
   if (batch->B == 0) return 0;
-  if (!label || !workspace) return NAIS_ERR_NULL;
+  if ((!bpr && !label) || !workspace) return NAIS_ERR_NULL;
   if (!aligned16(workspace)) return NAIS_ERR_ALIGN;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   TrainStep s;
   rc = open_train_step(s, p, batch, tables, dense, workspace, workspace_bytes);
   if (!rc) rc = train_step_sorts(s, st);
-  return rc ? rc : train_step_rest(s, label, row_weight, loss, score_out, st, true);
+  const StepLoss sl = {label, row_weight, bpr ? bpr->num_neg : 0, bpr ? bpr->group_weight : nullptr};
+  return rc ? rc : train_step_rest(s, sl, loss, score_out, st, true);
+}
+
+int nais_pairs_train_step(const NaisParams* p, const NaisPairs* batch, const float* label, const float* row_weight,
+                          const NaisAdagrad* tables, const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace,
+                          size_t workspace_bytes, nais_stream_t stream) {
+  return pairs_train_step(p, batch, label, row_weight, nullptr, tables, dense, loss, score_out, workspace, workspace_bytes, stream);
+}
+
+int nais_pairs_train_step_bpr(const NaisParams* p, const NaisPairs* batch, const NaisBprLoss* bpr, const NaisAdagrad* tables,
+                              const NaisDenseAdagrad* dense, float* loss, float* score_out, void* workspace, size_t workspace_bytes,
+                              nais_stream_t stream) {
+  if (!bpr) return NAIS_ERR_NULL;
+  return pairs_train_step(p, batch, nullptr, nullptr, bpr, tables, dense, loss, score_out, workspace, workspace_bytes, stream);
 }
 
 // ---- nais_train_users: the reference's one-user-per-step schedule, a list of users per call ---------------------------------------
@@ -660,16 +687,18 @@ int nais_train_users_centred(const NaisParams* p, const int64_t* host_indptr, in
                                   num_ng, seed, tables, dense, losses, workspace, workspace_bytes, center_lat, center_lon, nullptr, stream);
 }
 
-int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
-                             const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region, const float* poi_coords,
-                             const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables,
-                             const NaisDenseAdagrad* dense, float* losses, void* workspace, size_t workspace_bytes, float center_lat,
-                             float center_lon, const uint64_t* host_dropout_seeds, nais_stream_t stream) {
+// The body of nais_train_users_dropout (bpr = false: the batch-mean BCE per user) and nais_train_users_bpr (the mean BPR loss over
+// the user's H * num_ng pairs: groups of 1 + num_ng rows, as the sampler writes them).
+static int train_users(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices, const int64_t* entry_region,
+                       const float* entry_coords, const int32_t* poi_region, const float* poi_coords, const int64_t* host_users,
+                       int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables, const NaisDenseAdagrad* dense,
+                       float* losses, void* workspace, size_t workspace_bytes, float center_lat, float center_lon,
+                       const uint64_t* host_dropout_seeds, bool bpr, nais_stream_t stream) {
   int rc = check_params(p);
   if (rc) return rc;
   rc = check_train_state(p, tables, dense);
   if (rc) return rc;
-  if (n_users < 0 || num_ng < 0) return NAIS_ERR_SHAPE;
+  if (n_users < 0 || num_ng < (bpr ? 1 : 0)) return NAIS_ERR_SHAPE;
   if (p->dropout_p > 0.f && !host_dropout_seeds) return NAIS_ERR_NULL;
   if (n_users == 0) return 0;
   if (!host_indptr || !indices || !host_users || !losses || !workspace) return NAIS_ERR_NULL;
@@ -693,7 +722,7 @@ int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, in
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // One user per optimizer step is a chain of small dependent launches (GPU latency, not throughput).  What depends on the batch
   // only — the segment structure, the sampler and the id sorts of the backward — is enqueued one user AHEAD on a library-owned
-  // preparation stream into the other half of the workspace; the step itself (forward, BCE, backward on the sorted lists, Adagrad)
+  // preparation stream into the other half of the workspace; the step itself (forward, loss, backward on the sorted lists, Adagrad)
   // stays on the caller's stream.  Same kernels on the same inputs in the same order per user: results do not change.
   cudaStream_t ps = prep_stream();
   if (!ps) return (int)cudaErrorUnknown;
@@ -808,7 +837,8 @@ int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, in
     cudaStreamWaitEvent(st, prepared[cur_slot], 0);
     TrainStep s;  // the rest of the step, on the lists the preparation sorted
     rc = open_train_step(s, &pu, &ub.b, tables, dense, ub.step, L.total - L.step);
-    if (!rc) rc = train_step_rest(s, ub.label, nullptr, losses + cur, nullptr, st, false);
+    const StepLoss sl = {ub.label, nullptr, bpr ? num_ng : 0, nullptr};
+    if (!rc) rc = train_step_rest(s, sl, losses + cur, nullptr, st, false);
     if (rc) return bail(rc);
     cudaEventRecord(stepped[cur_slot], st);
     ++done;
@@ -816,6 +846,24 @@ int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, in
   cudaError_t e = cudaGetLastError();
   release();
   return e == cudaSuccess ? 0 : (int)e;
+}
+
+int nais_train_users_dropout(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
+                             const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region, const float* poi_coords,
+                             const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables,
+                             const NaisDenseAdagrad* dense, float* losses, void* workspace, size_t workspace_bytes, float center_lat,
+                             float center_lon, const uint64_t* host_dropout_seeds, nais_stream_t stream) {
+  return train_users(p, host_indptr, n_rows, indices, entry_region, entry_coords, poi_region, poi_coords, host_users, n_users, num_ng, seed,
+                     tables, dense, losses, workspace, workspace_bytes, center_lat, center_lon, host_dropout_seeds, false, stream);
+}
+
+int nais_train_users_bpr(const NaisParams* p, const int64_t* host_indptr, int64_t n_rows, const int64_t* indices,
+                         const int64_t* entry_region, const float* entry_coords, const int32_t* poi_region, const float* poi_coords,
+                         const int64_t* host_users, int32_t n_users, int32_t num_ng, uint64_t seed, const NaisAdagrad* tables,
+                         const NaisDenseAdagrad* dense, float* losses, void* workspace, size_t workspace_bytes, float center_lat,
+                         float center_lon, const uint64_t* host_dropout_seeds, nais_stream_t stream) {
+  return train_users(p, host_indptr, n_rows, indices, entry_region, entry_coords, poi_region, poi_coords, host_users, n_users, num_ng, seed,
+                     tables, dense, losses, workspace, workspace_bytes, center_lat, center_lon, host_dropout_seeds, true, stream);
 }
 
 static int check_fullrank(const NaisParams* p, const NaisCatalog* cat, const NaisUsers* users, int64_t poi_begin,

@@ -90,20 +90,12 @@ class _NAISBase(nn.Module):
         return ops.pairs_score(self.variant, float(self.beta), tuple(P.values()), batch, None, None, None, None, drop_p, seed,
                                getattr(self, "pairs_precision", "auto"))
 
-    def fused_adagrad_step(self, optimizer: torch.optim.Adagrad, label, hist, tgt=None, hreg=None, treg=None, aux=None,
-                           row_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """One training step of run.py:248-254 (`zero_grad -> forward -> BCELoss -> backward -> Adagrad.step`) with the
-        embedding tables stepped by the row-sparse Adagrad fused into the backward's segment reduce: no dense
-        [N, D/2] gradient is zero-filled, written or read, and only the touched rows of the tables and of the optimizer's
-        `state['sum']` move.  With the reference's `weight_decay = 0` (run.py:833) this IS the dense step (SURVEY.md §7
-        'Dense Adagrad semantic'); other settings raise.  The MLP / dist-layer parameters go through `optimizer.step()` as
-        usual.  Returns the loss (same value `loss_func(forward(...), label)` gives).  `hist` may be an ops.SegmentedPairs
-        (many users in one step; tgt / hreg / treg / aux then stay None).  Every class takes the one-call path, the two-branch
-        disentangled one included (its embed_distance moves in row 0, the only row its forward reads).  `row_weight` [B]: the loss becomes
-        sum_b row_weight[b] * BCE_b instead of the batch mean — e.g. 1 / rows(user of b) makes a multi-user step the sum of the
-        reference's per-user mean losses (run.py:251)."""
+    def _fused_step_state(self, optimizer: torch.optim.Adagrad, what: str):
+        """What a fused optimizer step needs from `optimizer`: (P, the tables' state['sum'], their shared lr / eps, the param groups
+        of the MLP / dist-layer tensors, whether the whole step can be one library call: plain Adagrad with one lr / eps on those
+        tensors, float32 parameters and a pairs_precision name).  Raises unless the tables take the row-sparse Adagrad step."""
         if not isinstance(optimizer, torch.optim.Adagrad):
-            raise RuntimeError("fused_adagrad_step needs torch.optim.Adagrad (run.py:225)")
+            raise RuntimeError(f"{what} needs torch.optim.Adagrad (run.py:225)")
         P = self._params()
         group_of = {id(p): g for g in optimizer.param_groups for p in g["params"]}
         sums, lr, eps = {}, None, None
@@ -119,16 +111,32 @@ class _NAISBase(nn.Module):
                 raise RuntimeError("embedding tables must share lr / eps")
             lr, eps = g["lr"], g["eps"]
             sums[name] = optimizer.state[P[name]]["sum"]
+        dgroups = [group_of.get(id(t)) for n, t in P.items() if n not in ops._TABLES]
+        one_call = (getattr(self, "one_call", True) and isinstance(getattr(self, "pairs_precision", "auto"), str)
+                    and all(g is not None for g in dgroups)
+                    and all(g["weight_decay"] == 0 and g["lr_decay"] == 0 and not g.get("maximize", False) for g in dgroups)
+                    and len({(g["lr"], g["eps"]) for g in dgroups}) == 1 and all(t.dtype == torch.float32 for t in P.values()))
+        return P, sums, lr, eps, dgroups, one_call
+
+    def fused_adagrad_step(self, optimizer: torch.optim.Adagrad, label, hist, tgt=None, hreg=None, treg=None, aux=None,
+                           row_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """One training step of run.py:248-254 (`zero_grad -> forward -> BCELoss -> backward -> Adagrad.step`) with the
+        embedding tables stepped by the row-sparse Adagrad fused into the backward's segment reduce: no dense
+        [N, D/2] gradient is zero-filled, written or read, and only the touched rows of the tables and of the optimizer's
+        `state['sum']` move.  With the reference's `weight_decay = 0` (run.py:833) this IS the dense step (SURVEY.md §7
+        'Dense Adagrad semantic'); other settings raise.  The MLP / dist-layer parameters go through `optimizer.step()` as
+        usual.  Returns the loss (same value `loss_func(forward(...), label)` gives).  `hist` may be an ops.SegmentedPairs
+        (many users in one step; tgt / hreg / treg / aux then stay None).  Every class takes the one-call path, the two-branch
+        disentangled one included (its embed_distance moves in row 0, the only row its forward reads).  `row_weight` [B]: the loss becomes
+        sum_b row_weight[b] * BCE_b instead of the batch mean — e.g. 1 / rows(user of b) makes a multi-user step the sum of the
+        reference's per-user mean losses (run.py:251)."""
+        P, sums, lr, eps, dgroups, one_call = self._fused_step_state(optimizer, "fused_adagrad_step")
         pp = getattr(self, "pairs_precision", "auto")
         drop = (*self._draw_dropout(), pp)
         # ---- everything in one library call (nais_pairs_train_step) when the step is the reference's: mean / row-weighted BCE,
         # plain Adagrad on every parameter.  `one_call=False` on the model keeps the op-by-op path below (the parity tests compare).
         dense = {n: t for n, t in P.items() if n not in ops._TABLES}
-        dgroups = [group_of.get(id(t)) for t in dense.values()]
-        if (getattr(self, "one_call", True) and isinstance(pp, str) and type(self.loss_func) is nn.BCELoss
-                and self.loss_func.reduction == "mean" and self.loss_func.weight is None and all(g is not None for g in dgroups)
-                and all(g["weight_decay"] == 0 and g["lr_decay"] == 0 and not g.get("maximize", False) for g in dgroups)
-                and len({(g["lr"], g["eps"]) for g in dgroups}) == 1 and all(t.dtype == torch.float32 for t in P.values())):
+        if (one_call and type(self.loss_func) is nn.BCELoss and self.loss_func.reduction == "mean" and self.loss_func.weight is None):
             optimizer.zero_grad(set_to_none=True)
             dsum = {n: optimizer.state[t]["sum"] for n, t in dense.items()}
             loss, _ = ops.pairs_train_step(self.variant, float(self.beta), P, sums, dsum, lr, eps, dgroups[0]["lr"], dgroups[0]["eps"],
@@ -155,7 +163,44 @@ class _NAISBase(nn.Module):
         self._plan_epoch = getattr(self, "_plan_epoch", 0) + 1  # the kernel stepped the tables behind torch's version counters
         return loss.detach()
 
-    def train_users(self, optimizer: torch.optim.Adagrad, batcher, uids, negative_num: int, seed: int = 0) -> torch.Tensor:
+    def fused_bpr_step(self, optimizer: torch.optim.Adagrad, hist, tgt=None, hreg=None, treg=None, aux=None, num_neg: int = 1,
+                       group_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """One BPR training step — `zero_grad -> forward -> -logsigmoid(s+ - s-).mean() -> backward -> Adagrad.step` — in one library
+        call (nais_pairs_train_step_bpr), with the tables stepped by the row-sparse Adagrad of `fused_adagrad_step` (same optimizer
+        preconditions).  The batch's rows come in groups of 1 + num_neg, the positive first: a (user, pos, neg) triple is a group of
+        two rows, and the batches of DeviceBatcher.batch / multi_user_batch are groups of 1 + negative_num as they stand (their
+        labels are not needed).  `hist` may be an ops.SegmentedPairs.  `group_weight` [n_groups]: the loss becomes
+        sum_g group_weight[g] * sum_j -logsigmoid(s_g - s_gj) instead of the mean over pairs — 1 / pairs(user of g) makes a
+        multi-user step the sum of the per-user mean losses.  Returns the loss."""
+        P, sums, lr, eps, dgroups, one_call = self._fused_step_state(optimizer, "fused_bpr_step")
+        drop = (*self._draw_dropout(), getattr(self, "pairs_precision", "auto"))
+        optimizer.zero_grad(set_to_none=True)
+        if one_call:  # `one_call=False` on the model keeps the op-by-op path below (the parity tests compare)
+            dense = {n: t for n, t in P.items() if n not in ops._TABLES}
+            dsum = {n: optimizer.state[t]["sum"] for n, t in dense.items()}
+            loss, _ = ops.pairs_train_step_bpr(self.variant, float(self.beta), P, sums, dsum, lr, eps, dgroups[0]["lr"], dgroups[0]["eps"],
+                                               num_neg, hist, tgt, hreg, treg, aux, group_weight, drop)
+            for t in P.values():
+                optimizer.state[t]["step"] += 1
+            self._plan_epoch = getattr(self, "_plan_epoch", 0) + 1
+            return loss[0]
+        with torch.no_grad():
+            score, row_sum, parts, mask = ops.pairs_forward_raw(self.variant, float(self.beta), P, hist, tgt, hreg, treg, aux, drop)
+        s = score.detach().requires_grad_(True)  # dL/dscore through torch's own logsigmoid on the [n_groups, 1 + num_neg] view
+        v = s.view(-1, num_neg + 1)
+        nll = -nn.functional.logsigmoid(v[:, :1] - v[:, 1:])
+        loss = nll.mean() if group_weight is None else (nll * group_weight[:, None]).sum()
+        loss.backward()
+        with torch.no_grad():
+            G = ops.pairs_backward_adagrad(self.variant, float(self.beta), P, sums, lr, eps, hist, tgt, hreg, treg, aux, row_sum,
+                                           parts, s.grad, drop, act_mask=mask)
+        for name, grad in G.items():
+            P[name].grad = grad.to(P[name].dtype)
+        optimizer.step()  # the tables have no .grad: torch skips them
+        self._plan_epoch = getattr(self, "_plan_epoch", 0) + 1
+        return loss.detach()
+
+    def train_users(self, optimizer: torch.optim.Adagrad, batcher, uids, negative_num: int, seed: int = 0, loss: str = "bce") -> torch.Tensor:
         """The inner loop of `train_NAIS_region_distance` (run.py:227-255) — for every user: sample `negative_num` negatives per
         positive, forward, BCELoss, backward, Adagrad step — for a whole list of users in ONE library call (`nais_train_users`):
         the same optimizer steps in the same order as `for u in uids: fused_adagrad_step(optimizer, *batcher.multi_user_batch([u],
@@ -163,10 +208,14 @@ class _NAISBase(nn.Module):
         train matrix.  Every class, the disentangled one included.  In train mode the dropout classes draw one mask seed per
         user with a history, in list order, as `torch.randint(0, 2**62, (n_steps,))`: torch's CPU generator gives the values of
         n_steps single draws, so under the same `torch.manual_seed` the steps are the loop's.  Returns the per-user losses
-        [len(uids)] on the device."""
+        [len(uids)] on the device.  `loss="bpr"`: the same schedule with the BPR loss (nais_train_users_bpr) — per user the mean
+        -logsigmoid(s+ - s-) over his positives x negative_num negatives, the loop of `fused_bpr_step(optimizer,
+        batcher.multi_user_batch([u], negative_num, seed + u), num_neg=negative_num)`, bit for bit."""
         if not isinstance(optimizer, torch.optim.Adagrad):
             raise RuntimeError("train_users needs torch.optim.Adagrad (run.py:225)")
-        if type(self.loss_func) is not nn.BCELoss or self.loss_func.reduction != "mean":
+        if loss not in ("bce", "bpr"):
+            raise ValueError(f"train_users: loss must be 'bce' or 'bpr', not {loss!r}")
+        if loss == "bce" and (type(self.loss_func) is not nn.BCELoss or self.loss_func.reduction != "mean"):
             raise RuntimeError("train_users: the reference's mean BCELoss")
         P = self._params()
         group_of = {id(p): g for g in optimizer.param_groups for p in g["params"]}
@@ -194,7 +243,7 @@ class _NAISBase(nn.Module):
                                  batcher.entry_region if has_reg else None, batcher.entry_coords if has_co else None,
                                  batcher.region32 if has_reg else None, batcher.coords32 if has_co else None, uids, negative_num, seed,
                                  getattr(self, "pairs_precision", "auto") if isinstance(getattr(self, "pairs_precision", "auto"), str) else "auto",
-                                 center=batcher.center, dropout_p=drop_p, dropout_seeds=drop_seeds)
+                                 center=batcher.center, dropout_p=drop_p, dropout_seeds=drop_seeds, loss=loss)
         for t in P.values():
             optimizer.state[t]["step"] += n_steps
         self._plan_epoch = getattr(self, "_plan_epoch", 0) + 1

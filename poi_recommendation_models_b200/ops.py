@@ -620,18 +620,45 @@ def pairs_train_step(variant: str, beta: float, P: Dict[str, torch.Tensor], tabl
     return loss, score
 
 
+def pairs_train_step_bpr(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sums: Dict[str, torch.Tensor],
+                         dense_sums: Dict[str, torch.Tensor], lr_tables: float, eps_tables: float, lr_dense: float, eps_dense: float,
+                         num_neg: int, hist, tgt=None, hreg=None, treg=None, aux=None, group_weight: Optional[torch.Tensor] = None,
+                         drop=(0.0, 0, "auto"), want_score: bool = False):
+    """nais_pairs_train_step_bpr: `pairs_train_step` with the BPR loss -log sigmoid(s+ - s-) in ONE library call.  The rows come in
+    groups of 1 + num_neg (positive first: the order of DeviceBatcher.batch / multi_user_batch); the loss is the mean over the
+    (positive, negative) pairs, or sum_g group_weight[g] * sum_j softplus(s_g,j - s_g,0) with `group_weight` [n_groups].  Updates
+    `P` and the optimizer sums in place.  Returns (loss [1] on the device, pre-sigmoid scores [B] or None)."""
+    dev = _need_cuda(hist, tgt, group_weight, *P.values())
+    with _PairCall(dev, variant, beta, P, drop[2], drop, (hist, tgt, hreg, treg, aux)) as c:
+        o = _adagrad_struct(variant, P, table_sums, lr_tables, eps_tables, tables=True)
+        d = _adagrad_struct(variant, P, dense_sums, lr_dense, eps_dense, tables=False)
+        gw = None if group_weight is None else _f32(group_weight)
+        if gw is not None and gw.numel() * (num_neg + 1) != int(c.b.B):
+            raise RuntimeError(f"pairs_train_step_bpr: one group weight per group of {num_neg + 1} rows")
+        bpr = _lib.NaisBprLoss(int(num_neg), 0, _ptr(gw))
+        ws_bytes = c.query("nais_pairs_train_step_workspace_bytes")
+        loss = torch.empty(1, device=dev, dtype=torch.float32)
+        score = torch.empty(int(c.b.B), device=dev, dtype=torch.float32) if want_score else None
+        c.launch("nais_pairs_train_step_bpr", C.byref(bpr), C.byref(o), C.byref(d), loss.data_ptr(), _ptr(score), ws_bytes=ws_bytes)
+    return loss, score
+
+
 def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sums, dense_sums, lr_tables, eps_tables, lr_dense,
                 eps_dense, host_indptr, indices: torch.Tensor, entry_region: Optional[torch.Tensor],
                 entry_coords: Optional[torch.Tensor], poi_region: Optional[torch.Tensor], poi_coords: Optional[torch.Tensor],
                 users, num_ng: int, seed: int, pairs_precision: str = "auto", center: Tuple[float, float] = (0.0, 0.0),
-                dropout_p: float = 0.0, dropout_seeds=None) -> torch.Tensor:
+                dropout_p: float = 0.0, dropout_seeds=None, loss: str = "bce") -> torch.Tensor:
     """nais_train_users: the reference's schedule, one optimizer step per user (run.py:227-255), for a list of users in ONE library
     call — per user the device sampler over his CSR slice + the one-call training step, ~15 launches and no host work in between.
     `host_indptr` / `users`: numpy int64 (host).  `center`: the (lat, lon) subtracted from `entry_coords` / `poi_coords`.
     `dropout_p > 0`: train-mode dropout, the step of users[i] with mask seed `dropout_seeds[i]` (host, one per user; entries of
-    users without a history are ignored).  Updates every tensor of `P` and the optimizer sums in place; returns the per-user
-    losses [n] (device)."""
+    users without a history are ignored).  `loss`: "bce" (the reference's batch-mean BCE) or "bpr" (nais_train_users_bpr: the mean
+    BPR loss over the user's positive / negative pairs).  Updates every tensor of `P` and the optimizer sums in place; returns the
+    per-user losses [n] (device)."""
     import numpy as np
+    entry = {"bce": "nais_train_users_dropout", "bpr": "nais_train_users_bpr"}.get(loss)
+    if entry is None:
+        raise ValueError(f"train_users: loss must be 'bce' or 'bpr', not {loss!r}")
     dev = _need_cuda(indices, entry_region, entry_coords, poi_region, poi_coords, *P.values())
     hp = np.ascontiguousarray(np.asarray(host_indptr, dtype=np.int64))
     hu = np.ascontiguousarray(np.asarray(users, dtype=np.int64))
@@ -653,7 +680,7 @@ def train_users(variant: str, beta: float, P: Dict[str, torch.Tensor], table_sum
         pc = None if poi_coords is None else _f32(poi_coords)
         max_hist = int((hp[hu + 1] - hp[hu]).max()) if hu.size else 0
         losses = torch.empty(max(hu.size, 1), device=dev, dtype=torch.float32)
-        c.launch("nais_train_users_dropout", hp.ctypes.data, int(hp.size) - 1, indices.data_ptr(), _ptr(er), _ptr(ec), _ptr(pr), _ptr(pc),
+        c.launch(entry, hp.ctypes.data, int(hp.size) - 1, indices.data_ptr(), _ptr(er), _ptr(ec), _ptr(pr), _ptr(pc),
                  hu.ctypes.data, int(hu.size), int(num_ng), int(seed) & (2 ** 64 - 1), C.byref(o), C.byref(d), losses.data_ptr(),
                  ws_bytes=c.query("nais_train_users_workspace_bytes", max(max_hist, 1), int(num_ng)),
                  tail=(float(center[0]), float(center[1]), None if ds is None else ds.ctypes.data))
