@@ -8,7 +8,10 @@ against the fused one.  Prints one JSON line (with the GPU's name and power limi
   step   C3-sized multi-user step (13 users x 128 history items x 5 rows per item = 8,320 rows, 40,000 POIs): autograd on the
          dense layout + torch.optim.Adagrad, vs model.fused_adagrad_step on the segmented batch.
 
-    python examples/train_disentangled.py [--users 1083] [--out profiles/r3_train_disentangled.json]
+  --pairs-precision picks the pair kernels (model.pairs_precision: "auto" = tcgen05 where the shape has them, "fp32" = the FP32
+  CUDA-core kernels); a comma list runs each in turn, --repeats times, alternating, and the line holds one entry per run.
+
+    python examples/train_disentangled.py [--users 1083] [--pairs-precision fp32,auto --repeats 2] [--out profiles/....json]
 """
 import argparse
 import json
@@ -34,11 +37,12 @@ def gpu_info():
     return {"name": name.strip() or torch.cuda.get_device_name(0), "power_limit": power.strip()}
 
 
-def new_model(N, R, sd=None):
+def new_model(N, R, pairs_precision, sd=None):
     torch.manual_seed(0)
     m = M.NAIS_region_distance_disentangled_Embedding(N, D, HID, BETA, R, 1).cuda().train()
     if sd is not None:
         m.load_state_dict(sd)
+    m.pairs_precision = pairs_precision
     return m, torch.optim.Adagrad(m.parameters(), lr=LR)
 
 
@@ -50,11 +54,11 @@ def timed(fn):
     return time.perf_counter() - t0
 
 
-def epoch(users, pois):
+def epoch(users, pois, pairs_precision):
     data = synthetic.make_checkins(users, pois, seed=0, hist_len=None, max_hist=100, min_hist=5, median_hist=30)
     bt = PB.DeviceBatcher(data.train_csr(), data.region, data.coords, device="cuda", seed=0)
     order = np.random.default_rng(0).permutation(users)
-    m_ref, o_ref = new_model(pois, data.region_num)
+    m_ref, o_ref = new_model(pois, data.region_num, pairs_precision)
     sd0 = {k: v.detach().clone() for k, v in m_ref.state_dict().items()}
 
     def today():
@@ -65,7 +69,7 @@ def epoch(users, pois):
             m_ref.loss_func(m_ref(h, t, hr, tr, km), lab).backward()
             o_ref.step()
 
-    m_new, o_new = new_model(pois, data.region_num, sd0)
+    m_new, o_new = new_model(pois, data.region_num, pairs_precision, sd0)
     losses = []
     t_today = timed(today)
     t_fused = timed(lambda: losses.append(m_new.train_users(o_new, bt, order, NUM_NG, seed=1)))
@@ -74,7 +78,7 @@ def epoch(users, pois):
             "train_users_mean_loss": float(losses[0].mean())}
 
 
-def multi_user_step(reps=20, warmup=3):
+def multi_user_step(pairs_precision, reps=20, warmup=3):
     N, H, U = 40000, 128, 13
     data = synthetic.make_checkins(U, N, seed=1, hist_len=H)
     bt = PB.DeviceBatcher(data.train_csr(), data.region, data.coords, device="cuda", seed=0)
@@ -84,8 +88,8 @@ def multi_user_step(reps=20, warmup=3):
     h, t = torch.from_numpy(hist).cuda(), b.tgt
     reg = torch.from_numpy(data.region).cuda()
     km = PB.dist_km_pairs(data.coords, tgt, hist, device="cuda")
-    m_dense, o_dense = new_model(N, data.region_num)
-    m_fused, o_fused = new_model(N, data.region_num, m_dense.state_dict())
+    m_dense, o_dense = new_model(N, data.region_num, pairs_precision)
+    m_fused, o_fused = new_model(N, data.region_num, pairs_precision, m_dense.state_dict())
 
     def dense_step():
         o_dense.zero_grad()
@@ -107,12 +111,22 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--users", type=int, default=1083)
     ap.add_argument("--pois", type=int, default=38333)
+    ap.add_argument("--pairs-precision", default="auto", help='"auto", "fp32", "tc", or a comma list run in turn')
+    ap.add_argument("--repeats", type=int, default=1, help="rounds over the --pairs-precision list")
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r3_train_disentangled.json"))
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("needs a CUDA device")
-    line = {"gpu": gpu_info(), "model": "NAIS_region_distance_disentangled_Embedding D=hid=64", "epoch_c1": epoch(args.users, args.pois),
-            "step_c3": multi_user_step()}
+    names = args.pairs_precision.split(",")
+    line = {"gpu": gpu_info(), "model": "NAIS_region_distance_disentangled_Embedding D=hid=64"}
+    runs = []
+    for r in range(args.repeats):
+        for pp in names:
+            runs.append({"pairs_precision": pp, "round": r, "epoch_c1": epoch(args.users, args.pois, pp), "step_c3": multi_user_step(pp)})
+    if len(runs) == 1:
+        line.update(runs[0])
+    else:
+        line["runs"] = runs
     s = json.dumps(line)
     print(s)
     if args.out:

@@ -216,17 +216,20 @@ NAIS_API int nais_pairs_dispatch(const NaisParams* p, const NaisPairs* batch, in
 
 /* score[b] = attention_network(pairs)  (pre-sigmoid, model.py:246-297).  Saved for backward (each may be NULL):
  * row_sum[n_branch,B] = sum_h E_bh, score_parts[n_branch,B] = per-branch score (their sum over branches is score),
- * act_mask[cells] = the ReLU pattern of attn_layer1: bit k of word `cell` (b*H + h dense; NaisPairs) is set iff hidden unit k of
- * that cell was active (t_k > 0) — with dropout, active AND kept.  act_mask is written only by the tcgen05 forward with
- * hid <= 64 (nais_pairs_dispatch: fwd_tc); the tcgen05 backward then takes the unit-step of ReLU from it instead of thresholding
- * its own recomputed t (bf16 two-term splits: ~1e-5 relative, enough to flip a unit that sits on the kink and move a gradient by
- * one cell's whole contribution).  With dropout the tcgen05 backward NEEDS it: it draws no mask of its own. */
+ * act_mask[n_branch, cells] = the ReLU pattern of attn_layer1 (of branch bi's first layer from word bi*cells on): bit k of word
+ * `cell` (b*H + h dense; NaisPairs) is set iff hidden unit k of that cell was active (t_k > 0) — with dropout, active AND kept.
+ * act_mask is written only by the tcgen05 forward with hid <= 64 (nais_pairs_dispatch: fwd_tc).  One branch: [cells], as
+ * before; the disentangled two branches run the tcgen05 kernels too and write both patterns.  The tcgen05 backward then takes the
+ * unit-step of ReLU from it instead of thresholding its own recomputed t (bf16 two-term splits: ~1e-5 relative, enough to flip a
+ * unit that sits on the kink and move a gradient by one cell's whole contribution).  With dropout the tcgen05 backward NEEDS it:
+ * it draws no mask of its own. */
 NAIS_API int nais_pairs_forward(const NaisParams* p, const NaisPairs* batch, float* score, float* row_sum, float* score_parts,
                        uint64_t* act_mask, nais_stream_t stream);
 
 NAIS_API size_t nais_pairs_backward_workspace_bytes(const NaisParams* p, const NaisPairs* batch);
 /* Given dscore[B] = dL/dscore, write every parameter gradient.  score_parts / row_sum / act_mask are the forward's outputs
- * (act_mask: NULL unless the tcgen05 forward wrote it; required by the tcgen05 backward with dropout, see nais_pairs_dispatch).
+ * (act_mask: [n_branch, cells] as nais_pairs_forward writes it, branch bi's backward reads words bi*cells ..; NULL unless the
+ * tcgen05 forward wrote it; required by the tcgen05 backward with dropout, see nais_pairs_dispatch).
  * Streams: everything is ordered after the work already in `stream`, and `stream` is ordered after everything this call
  * enqueues, as for any other entry point — but the sort + reduce of the target-id and region-id lists and the reduce of the
  * per-CTA MLP-gradient partials run on three streams the library creates once per device (forked from / joined to `stream`

@@ -1133,7 +1133,7 @@ int PairsBwd::finish(int bi, cudaStream_t stream, bool wait_sorted0, const Dense
   A.parts = score_parts + (size_t)bi * b.B;
   A.row_sum = row_sum + (size_t)bi * b.B;
   A.dscore = dscore;
-  A.act_mask = (p.n_branch == 1 && p.hid <= 64) ? act_mask : nullptr;
+  A.act_mask = (p.hid <= 64 && act_mask) ? act_mask + (size_t)bi * n_of[0] : nullptr;  // [n_branch, cells]: this branch's pattern
   A.ws_dq = (w[0] || w[2]) ? reinterpret_cast<float*>(base + L.dq) : nullptr;
   A.ws_dp = (w[1] || w[2]) ? reinterpret_cast<float*>(base + L.dp) : nullptr;
   A.ws_part = reinterpret_cast<float*>(base + L.part);

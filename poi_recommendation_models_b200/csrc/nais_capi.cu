@@ -441,7 +441,7 @@ TrainStepLayout train_step_layout(const NaisParams& p, const NaisPairs& b) {
   L.row_sum = o, o += ts_al((size_t)p.n_branch * B * 4);
   L.parts = o, o += ts_al((size_t)p.n_branch * B * 4);
   L.dscore = o, o += ts_al((size_t)B * 4);
-  L.mask = o, o += ts_al((size_t)cells * 8);
+  L.mask = o, o += ts_al((size_t)p.n_branch * cells * 8);  // [n_branch, cells] ReLU patterns of the tcgen05 forward
   for (int bi = 0; bi < 2; ++bi) {  // per-branch MLP gradient scratch (branch 1: the disentangled layout's region MLP)
     const NaisBranch& br = p.branch[bi];
     const int ldw = br.w_poi + br.w_reg + lanes;

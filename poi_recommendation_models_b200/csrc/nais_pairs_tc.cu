@@ -1,7 +1,11 @@
 // Pair forward (model.py:246-297) with the attention-MLP contraction on tcgen05 — the default of nais_pairs_forward
-// (NaisParams::pairs_precision = NAIS_PAIRS_AUTO) for one branch, D in {16, 32, 48, 64}, hid <= 128 (multiple of 16), lat/lon or
-// no distance mode; everything else runs the FP32 kernel (nais_fp32.cu).  Train-mode dropout is a compile-time parameter (kDrop): the
-// epilogue draws the keep bits of NaisParams::dropout_seed (the FP32 kernels' mask, bit for bit) and saves "active and kept" in act_mask.
+// (NaisParams::pairs_precision = NAIS_PAIRS_AUTO) for one branch with lat/lon or no distance mode, and for the disentangled two
+// branches (nais_pairs_tile.cuh) with no distance mode or NAIS_DIST_KM; D in {16, 32, 48, 64} per branch, hid <= 128 (multiple of
+// 16); everything else runs the FP32 kernel (nais_fp32.cu).  Train-mode dropout is a compile-time parameter (kDrop): the epilogue
+// draws the keep bits of NaisParams::dropout_seed (the FP32 kernels' mask, bit for bit) and saves "active and kept" in act_mask.
+// The haversine-km logit term is another (kKm): a += km * sum_d embed_distance[0, d], added once per cell.  Two branches run one
+// launch each on a one-branch view of the parameters; the second adds its branch score to `score` (kAcc), so score = s0 + s1 as in
+// the FP32 kernel.
 //
 // A training row has its own history, so unlike full-rank scoring there is no per-user operand to reuse: the GEMM is
 //     T[cell, k] = sum_d X[cell, d] * W[k, d],      X[cell, :] = q_cell (.) p_row       (M = 128 cells, N = hid, K = D)
@@ -32,7 +36,7 @@ struct Args {
   float* score;    // [B]
   float* row_sum;  // [B] or NULL
   float* parts;    // [B] or NULL
-  unsigned long long* act_mask;  // [cells] ReLU pattern per cell (hid <= 64) or NULL
+  unsigned long long* act_mask;  // [cells] ReLU pattern per cell of this branch (hid <= 64) or NULL
   uint32_t tmem_cols;
   int* bad;  // the library's bad-index word (nais_common.cuh)
   uint32_t drop_thresh;  // dropout: dropout_threshold(dropout_p) and 1 / (1 - dropout_p) (kernel parameters: read from the constant bank)
@@ -49,7 +53,7 @@ __device__ __forceinline__ float pow2_scale(float amax, int target_exp) {
   return ldexpf(1.f, k);
 }
 
-template <int D, bool kDrop>
+template <int D, bool kDrop, bool kKm, bool kAcc>
 __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(const __grid_constant__ Args A) {
   extern __shared__ __align__(128) uint8_t smem[];
   const NaisParams& p = A.p;
@@ -113,6 +117,8 @@ __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(cons
   const uint32_t tmem = *tslot;
   const uint32_t tlane = tmem + ((uint32_t)(warp * 32) << 16);  // warp w owns TMEM lanes 32w .. 32w+31
   const bool vec4 = rows_vec4(br, 4);
+  float kmc = 0.f;  // kKm: sum_d embed_distance[0, d]
+  if constexpr (kKm) kmc = km_coef0(p, D);
 
   const int64_t n_items = pairs_n_tiles(A.b);
   uint32_t phase = 0;
@@ -147,7 +153,7 @@ __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(cons
       const int64_t hidx = valid ? T.hist0 + r * T.hist_rs + h : 0;       // history arrays
       // ---- build this cell's row of X -------------------------------------------------------------------------------------
       float x[D];
-      float ssum = 0.f, amax = 0.f, g0 = 0.f, g1 = 0.f;
+      float ssum = 0.f, amax = 0.f, g0 = 0.f, g1 = 0.f, km = 0.f;
       bool live = false;  // valid and not masked (history item != target)
       int it32 = 0, rg32 = 0;  // POI / region id of this cell (ids fit int32: item_num is int32); row 0 for padding cells
       if (valid) {
@@ -223,6 +229,7 @@ __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(cons
           g0 = sigmoidf_exact(fmaf(l1, __ldg(p.dist_w + 1), fmaf(l0, __ldg(p.dist_w + 0), __ldg(p.dist_b + 0))));
           g1 = sigmoidf_exact(fmaf(l1, __ldg(p.dist_w + 3), fmaf(l0, __ldg(p.dist_w + 2), __ldg(p.dist_b + 1))));
         }
+        if constexpr (kKm) km = pair_km(A.b, cidx, hidx, row0 + r);
         live = A.b.hist[hidx] != A.b.tgt[row0 + r];
       } else {
 #pragma unroll
@@ -283,6 +290,7 @@ __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(cons
         if (c0 < 32) act_lo |= bits << c0;
         else if (c0 < 64) act_hi |= bits << (c0 - 32);
       }
+      if constexpr (kKm) a += __fmul_rn(km, kmc);  // (the product rounded on its own, as the FP32 kernel adds it)
       if (A.act_mask && valid) A.act_mask[cidx] = ((unsigned long long)act_hi << 32) | act_lo;
       tc_fence_before();  // TMEM reads ordered before the barrier that precedes the next tile's MMAs
       float e = 0.f, es = 0.f;
@@ -316,7 +324,7 @@ __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(cons
     if (tid < nrows) {
       const float S = row_e[tid];
       const float sc = row_es[tid] / powf(S, p.beta);
-      A.score[row0 + tid] = sc;
+      A.score[row0 + tid] = kAcc ? A.score[row0 + tid] + sc : sc;
       if (A.row_sum) A.row_sum[row0 + tid] = S;
       if (A.parts) A.parts[row0 + tid] = sc;
     }
@@ -351,7 +359,7 @@ __device__ unsigned long long g_phase_clk[16];
 #define NAIS_PH(i)
 #endif
 
-template <bool kDrop>
+template <bool kDrop, bool kKm, bool kAcc>
 __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_constant__ Args A) {
   constexpr int D = 64, HIDC = 64, KC = D / 8, A_PLANE = KC * PT * 16, W_PLANE = KC * HIDC * 16;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -378,7 +386,7 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
   long long* m_hreg = m_hist + PT2;                              // [PT2] its region id
   long long* m_psid = m_hreg + PT2;                              // [PT2] target POI / region id behind this thread's 16 B of `ps`
   long long* m_tgt = m_psid + PT2;                               // [PMAXROWS] target POI id of each row (live mask)
-  float2* m_ll = reinterpret_cast<float2*>(m_tgt + PMAXROWS);    // [PT] |dlat|,|dlon| of the cell, or the history item's coordinates
+  float2* m_ll = reinterpret_cast<float2*>(m_tgt + PMAXROWS);    // [PT] |dlat|,|dlon| (kKm: .x = km) of the cell, or the history item's coordinates
   float2* m_tco = m_ll + PT;                                     // [PMAXROWS] target coordinates (segmented layout)
   uint64_t* bar = reinterpret_cast<uint64_t*>(m_tco + PMAXROWS);
   uint32_t* tslot = reinterpret_cast<uint32_t*>(bar + 1);
@@ -422,6 +430,8 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
   const uint32_t tmem = *tslot;
   const uint32_t tlane = tmem + ((uint32_t)(qd * 32) << 16);
   uint8_t* stg = stg_all + (size_t)(warp * 32) * STG_STRIDE;
+  float kmc = 0.f;  // kKm: sum_d embed_distance[0, d]
+  if constexpr (kKm) kmc = km_coef0(p, D);
 
   // ---- the input pipeline.  ncu + per-phase clocks on the unpipelined kernel (profiles/r2_phase_clocks_before.txt): 41 % of a
   // tile's time was exposed load latency in a dependent chain (target id -> target row; history id -> history row).  Now the
@@ -436,9 +446,14 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
       cp_async8(m_hist + tid, A.b.hist + c.hidx);
       if (br.w_reg) cp_async8(m_hreg + tid, A.b.hreg + c.hidx);
       if (lanes && half == 0) cp_async8(m_ll + cell, A.b.aux ? A.b.aux + c.cidx * 2 : A.b.hist_coords + c.hidx * 2);
+      if (kKm && half == 0) {  // the dense layout's km, or the history item's coordinates (where the lat/lon lanes stage theirs)
+        if (A.b.aux) cp_async4(m_ll + cell, A.b.aux + c.cidx);
+        else cp_async8(m_ll + cell, A.b.hist_coords + c.hidx * 2);
+      }
     }
     if (tid < Tn.nrows) cp_async8(m_tgt + tid, A.b.tgt + Tn.row0 + tid);
-    if (lanes && !A.b.aux && tid >= 32 && tid < 32 + Tn.nrows) cp_async8(m_tco + (tid - 32), A.b.tgt_coords + (Tn.row0 + tid - 32) * 2);
+    if ((lanes || kKm) && !A.b.aux && tid >= 32 && tid < 32 + Tn.nrows)
+      cp_async8(m_tco + (tid - 32), A.b.tgt_coords + (Tn.row0 + tid - 32) * 2);
     if (chn == 0 && tid * 4 < Tn.nrows * D) {
       const int r = (tid * 4) / D, d = tid * 4 - r * D;
       cp_async8(m_psid + tid, (d < br.w_poi ? A.b.tgt : A.b.treg) + Tn.row0 + r);
@@ -492,7 +507,7 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
     NAIS_PH(1)
     // ---- this half of the cell's row of X -----------------------------------------------------------------------------------
     float x[32];
-    float g0 = 0.f, g1 = 0.f, ssum = 0.f, amax = 0.f;
+    float g0 = 0.f, g1 = 0.f, ssum = 0.f, amax = 0.f, km = 0.f;
     bool live = false;
     if (valid) {
 #pragma unroll
@@ -521,6 +536,14 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
         l1 *= p.dist_scale;
         g0 = sigmoidf_exact(fmaf(l1, __ldg(p.dist_w + 1), fmaf(l0, __ldg(p.dist_w + 0), __ldg(p.dist_b + 0))));
         g1 = sigmoidf_exact(fmaf(l1, __ldg(p.dist_w + 3), fmaf(l0, __ldg(p.dist_w + 2), __ldg(p.dist_b + 1))));
+      }
+      if (kKm && half == 0) {  // (pair_km: the same dist_km_f call on the same coordinates)
+        const float2 hl = m_ll[cell];
+        km = hl.x;
+        if (!A.b.aux) {
+          const float2 tc = m_tco[r];
+          km = coords_km(A.b, tc.x, tc.y, hl.x, hl.y);
+        }
       }
       live = m_hist[tid] != m_tgt[r];
     } else {
@@ -606,6 +629,7 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
     NAIS_PH(7)
     if (half == 0) {
       a = apart[cell] + apart[PT + cell];
+      if constexpr (kKm) a += __fmul_rn(km, kmc);  // the halves meet at the logit; the km term once per cell
       if (A.act_mask && valid) A.act_mask[c.cidx] = ((unsigned long long)abits[cell] << 32) | bits;
       float e = 0.f, es = 0.f;
       if (live) {  // masked cells stay exactly 0 even if exp overflows (reference: exp_A * mask, then * history)
@@ -641,7 +665,7 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
           row_es[rr] = ses;
         } else {
           const float sc = ses / powf(se, p.beta);
-          A.score[row0 + rr] = sc;
+          A.score[row0 + rr] = kAcc ? A.score[row0 + rr] + sc : sc;
           if (A.row_sum) A.row_sum[row0 + rr] = se;
           if (A.parts) A.parts[row0 + rr] = sc;
         }
@@ -658,14 +682,14 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
   if (warp == 0) tmem_dealloc(tmem, 64u);
 }
 
-template <bool kDrop>
+template <bool kDrop, bool kKm, bool kAcc>
 static int launch2(const Args& A, int64_t n_items, int sms, cudaStream_t stream) {
   constexpr int D = 64, HIDC = 64;
   const size_t smem = 2 * (size_t)(D / 8) * PT * 16 + 2 * (size_t)(D / 8) * HIDC * 16 +
                       4096 + (4 * (size_t)HIDC + 2 * PMAXROWS * D + 2 * PT + 2 * PMAXROWS + 8 + 6 * PT + PT) * 4 +
                       (3 * (size_t)PT2 + PMAXROWS) * 8 + ((size_t)PT + PMAXROWS) * 8 + 16;
   static SmemAttrOnce attr;
-  cudaError_t e = attr(pairs_fwd_tc2_kernel<kDrop>, smem, true);
+  cudaError_t e = attr(pairs_fwd_tc2_kernel<kDrop, kKm, kAcc>, smem, true);
   if (e != cudaSuccess) return (int)e;
   int per_sm = 3;
   const int by_smem = (int)((227 * 1024) / (smem + 1024));
@@ -673,18 +697,18 @@ static int launch2(const Args& A, int64_t n_items, int sms, cudaStream_t stream)
   if (per_sm < 1) return NAIS_ERR_SHAPE;
   const int64_t cap = (int64_t)sms * per_sm;
   const int grid = (int)(n_items < cap ? n_items : cap);
-  pairs_fwd_tc2_kernel<kDrop><<<grid, PT2, smem, stream>>>(A);
+  pairs_fwd_tc2_kernel<kDrop, kKm, kAcc><<<grid, PT2, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
 
-template <int D, bool kDrop>
+template <int D, bool kDrop, bool kKm, bool kAcc>
 static int launch(const Args& A, int hid, int64_t n_items, int sms, cudaStream_t stream) {
   const size_t smem = 2 * (size_t)(D / 8) * PT * 16 + 2 * (size_t)(D / 8) * hid * 16 +
                       (4 * (size_t)hid + PMAXROWS * D + 2 * PT + 2 * PMAXROWS + 8) * 4 + 16 + (size_t)PT * STG_STRIDE;
-  cudaError_t e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return (int)e;
   // Persistent grid: as many CTAs as can be co-resident — the kernel's register budget (3 per SM for D = 64, else 4), shared
   // memory, and TMEM (tmem_cols of the SM's 512 columns per CTA; a CTA beyond that would simply wait in tcgen05.alloc).
@@ -695,57 +719,77 @@ static int launch(const Args& A, int hid, int64_t n_items, int sms, cudaStream_t
   if (per_sm < 1) return NAIS_ERR_SHAPE;
   const int64_t cap = (int64_t)sms * per_sm;
   const int grid = (int)(n_items < cap ? n_items : cap);
-  pairs_fwd_tc_kernel<D, kDrop><<<grid, PT, smem, stream>>>(A);
+  pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc><<<grid, PT, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
 
 // `two`: two threads per cell (D = hid = 64, a cell's 32-column halves each lie in one table)
-template <bool kDrop>
+template <bool kDrop, bool kKm, bool kAcc>
 static int launch_shape(const Args& A, int D, bool two, int64_t n_items, int sms, cudaStream_t stream) {
-  if (two) return launch2<kDrop>(A, n_items, sms, stream);
+  if (two) return launch2<kDrop, kKm, kAcc>(A, n_items, sms, stream);
   switch (D) {
-    case 16: return launch<16, kDrop>(A, A.p.hid, n_items, sms, stream);
-    case 32: return launch<32, kDrop>(A, A.p.hid, n_items, sms, stream);
-    case 48: return launch<48, kDrop>(A, A.p.hid, n_items, sms, stream);
-    case 64: return launch<64, kDrop>(A, A.p.hid, n_items, sms, stream);
+    case 16: return launch<16, kDrop, kKm, kAcc>(A, A.p.hid, n_items, sms, stream);
+    case 32: return launch<32, kDrop, kKm, kAcc>(A, A.p.hid, n_items, sms, stream);
+    case 48: return launch<48, kDrop, kKm, kAcc>(A, A.p.hid, n_items, sms, stream);
+    case 64: return launch<64, kDrop, kKm, kAcc>(A, A.p.hid, n_items, sms, stream);
     default: return NAIS_ERR_SHAPE;
   }
 }
 
 }  // namespace ptc
 
+// One branch (lat/lon or no distance mode, dropout or not), or the disentangled two (no distance mode or km, no dropout: the
+// disentangled model has none).
 bool pairs_tc_supported(const NaisParams& p, const NaisPairs& b) {
-  if (p.n_branch != 1 || b.B < 1) return false;
-  const int D = p.branch[0].w_poi + p.branch[0].w_reg;
-  if (D != 16 && D != 32 && D != 48 && D != 64) return false;
+  if (b.B < 1) return false;
+  const bool two = pairs_disentangled(p);
+  if (p.n_branch != 1 && !two) return false;
+  if (p.dist_mode == NAIS_DIST_KM && !two) return false;
+  if (two && p.dropout_p > 0.f) return false;
+  for (int bi = 0; bi < p.n_branch; ++bi) {
+    const int D = p.branch[bi].w_poi + p.branch[bi].w_reg;
+    if (D != 16 && D != 32 && D != 48 && D != 64) return false;
+  }
   if (p.hid < 16 || p.hid > 128 || (p.hid & 15)) return false;
-  if (p.dist_mode == NAIS_DIST_KM) return false;
   return true;
 }
 
+// row_sum / parts are [n_branch, B] and act_mask [n_branch, cells] (each may be NULL); branch bi writes its slice
 int launch_pairs_fwd_tc(const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts,
                         unsigned long long* act_mask, cudaStream_t stream) {
   const DeviceInfo di = device_info();
   if (di.major != 10) return NAIS_ERR_ARCH;
   const int sms = di.sms;
-  ptc::Args A;
-  A.p = p;
-  A.b = b;
-  A.score = score;
-  A.row_sum = row_sum;
-  A.parts = parts;
-  A.act_mask = p.hid <= 64 ? act_mask : nullptr;
-  A.bad = bad_index_flag();
-  A.drop_thresh = p.dropout_p > 0.f ? dropout_threshold(p.dropout_p) : 0u;
-  A.drop_inv = p.dropout_p > 0.f ? 1.f / (1.f - p.dropout_p) : 1.f;
-  A.tmem_cols = p.hid <= 32 ? 32u : (p.hid <= 64 ? 64u : 128u);
   const int64_t n_items = pairs_n_tiles(b);
   if (n_items < 1) return 0;
-  const int D = p.branch[0].w_poi + p.branch[0].w_reg;
-  const bool two = D == 64 && p.hid == 64 && rows_vec4(p.branch[0], 4) && pair_gather_uniform(p.branch[0]);
-  if (p.dropout_p > 0.f) return ptc::launch_shape<true>(A, D, two, n_items, sms, stream);
-  return ptc::launch_shape<false>(A, D, two, n_items, sms, stream);
+  const bool km = p.dist_mode == NAIS_DIST_KM;
+  for (int bi = 0; bi < p.n_branch; ++bi) {
+    ptc::Args A;
+    A.p = p;
+    A.p.n_branch = 1;  // the kernels read branch 0: a one-branch view of branch bi
+    A.p.branch[0] = p.branch[bi];
+    A.b = b;
+    A.score = score;
+    A.row_sum = row_sum ? row_sum + (size_t)bi * b.B : nullptr;
+    A.parts = parts ? parts + (size_t)bi * b.B : nullptr;
+    A.act_mask = (p.hid <= 64 && act_mask) ? act_mask + (size_t)bi * pairs_n_cells(b) : nullptr;
+    A.bad = bad_index_flag();
+    A.drop_thresh = p.dropout_p > 0.f ? dropout_threshold(p.dropout_p) : 0u;
+    A.drop_inv = p.dropout_p > 0.f ? 1.f / (1.f - p.dropout_p) : 1.f;
+    A.tmem_cols = p.hid <= 32 ? 32u : (p.hid <= 64 ? 64u : 128u);
+    const NaisBranch& br = p.branch[bi];
+    const int D = br.w_poi + br.w_reg;
+    const bool two = D == 64 && p.hid == 64 && rows_vec4(br, 4) && pair_gather_uniform(br);
+    int rc;
+    if (p.dropout_p > 0.f) rc = ptc::launch_shape<true, false, false>(A, D, two, n_items, sms, stream);  // (one branch only)
+    else if (km) rc = bi ? ptc::launch_shape<false, true, true>(A, D, two, n_items, sms, stream)
+                         : ptc::launch_shape<false, true, false>(A, D, two, n_items, sms, stream);
+    else rc = bi ? ptc::launch_shape<false, false, true>(A, D, two, n_items, sms, stream)
+                 : ptc::launch_shape<false, false, false>(A, D, two, n_items, sms, stream);
+    if (rc) return rc;
+  }
+  return 0;
 }
 
 }  // namespace nais

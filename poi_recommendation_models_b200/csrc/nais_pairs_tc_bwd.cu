@@ -1,6 +1,9 @@
 // Backward of the pair scorer with all three contractions on tcgen05 — the default of nais_pairs_backward[_adagrad]
-// (NaisParams::pairs_precision = NAIS_PAIRS_AUTO) for one branch, hidden_size = 64, D in {32, 64}, lat/lon or no distance mode,
-// 16-byte aligned table rows; everything else runs the FP32 kernel (nais_bwd.cu).  Train-mode dropout (kDrop) draws nothing: with
+// (NaisParams::pairs_precision = NAIS_PAIRS_AUTO) for one branch with lat/lon or no distance mode and for the disentangled two
+// branches with no distance mode or NAIS_DIST_KM (one launch per branch, BwdArgs::bi), hidden_size = 64, D in {32, 64}, 16-byte
+// aligned table rows; everything else runs the FP32 kernel (nais_bwd.cu).  The km logit term is a compile-time mode (kKm): the
+// recomputed logit adds km * sum_d embed_distance[0, d], and each CTA sums da * km over its cells in a fixed order into the partial
+// slot of the FP32 kernel (no atomics).  Train-mode dropout (kDrop) draws nothing: with
 // m = the forward's saved "active and kept" bit, relu(drop(t)) = m relu(t) / (1-p), so m gives the recomputed logit, the dw2 term
 // and dt = m da v / (1-p) — the dropout backward needs act_mask (without it the FP32 kernel runs, which regenerates the mask).
 // It writes the SAME workspace as pairs_bwd_kernel (dq rows, dp rows, one parameter partial per CTA), so the deterministic
@@ -92,7 +95,7 @@ __device__ __forceinline__ void gather_segment(const NaisBranch& br, int it32, i
   __syncwarp();
 }
 
-template <int D, bool kDrop>
+template <int D, bool kDrop, bool kKm>
 __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_constant__ BwdArgs A) {
   static_assert(D == 32 || D == 64, "segments of 32");
   extern __shared__ __align__(128) uint8_t smem[];
@@ -144,6 +147,8 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
   uint8_t* stg = sDT + (size_t)(warp * 32) * STG_STRIDE;
 
   float pd[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // dist_w[4], dist_b[2] partials of this thread's cells
+  float pkm = 0.f, kmc = 0.f;                    // kKm: sum of da * km over this thread's cells; sum_d embed_distance[0, d]
+  if constexpr (kKm) kmc = km_coef0(p, D);
   float dv_acc[2] = {0.f, 0.f};                  // dw2 partial of hidden units dv_k0, dv_k0 + 1 over this warp's cells
   const int dv_k0 = 32 * ((lane >> 4) & 1) + 16 * ((lane >> 3) & 1) + 8 * ((lane >> 2) & 1) + 4 * ((lane >> 1) & 1) + 2 * (lane & 1);
   uint32_t phase = 0, dw_started = 0;
@@ -182,12 +187,13 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
       const int64_t cidx = valid ? T.cell0 + r * (int64_t)H + h : 0;  // per-cell arrays
       const int64_t hidx = valid ? T.hist0 + r * T.hist_rs + h : 0;   // history arrays
       int it32 = 0, rg32 = 0;
-      float l0r = 0.f, l1r = 0.f;
+      float l0r = 0.f, l1r = 0.f, km = 0.f;
       bool live = false;
       if (valid) {
         it32 = checked_id(A.b.hist[hidx], p.item_num, A.bad);
         rg32 = br.w_reg ? checked_id(A.b.hreg[hidx], p.region_num, A.bad) : 0;
         if (lanes) pair_latlon(A.b, cidx, hidx, row0 + r, l0r, l1r);
+        if constexpr (kKm) km = pair_km(A.b, cidx, hidx, row0 + r);
         live = A.b.hist[hidx] != A.b.tgt[row0 + r];
       }
       float g0 = 0.f, g1 = 0.f;
@@ -259,6 +265,7 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
         }
       }
       if constexpr (kDrop) a *= A.drop_inv;
+      if constexpr (kKm) a += __fmul_rn(km, kmc);
       float dav = 0.f, gwv = 0.f;
       if (live) {
         const float S = rowv[r], sc = rowv[BWD_MAXROWS + r], G = rowv[2 * BWD_MAXROWS + r], Sb = rowv[3 * BWD_MAXROWS + r];
@@ -267,6 +274,7 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
         dav = G * (w * ssum - p.beta * (e / S) * sc);
         gwv = G * w;
       }
+      if constexpr (kKm) pkm = fmaf(dav, km, pkm);  // d logit / d embed_distance[0, d] = km for every d
       if constexpr (kDrop) dav *= A.drop_inv;  // d relu(drop(t)) / dt = m / (1-p)
       // unit step of ReLU: the forward's saved pattern when there is one (its t is accurate to ~2e-7; this kernel's recomputed t,
       // from bf16 two-term splits, only to ~1e-5 — a unit on the kink would flip and move the gradients by this cell's whole term)
@@ -430,8 +438,8 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
   dvs[warp * HID + dv_k0] = dv_acc[0];
   dvs[warp * HID + dv_k0 + 1] = dv_acc[1];
 #pragma unroll
-  for (int q = 0; q < 6; ++q) {
-    float v = pd[q];
+  for (int q = 0; q < (kKm ? 7 : 6); ++q) {
+    float v = q < 6 ? pd[q] : pkm;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     if (lane == 0) red[q * 4 + warp] = v;
@@ -439,7 +447,8 @@ __global__ void __launch_bounds__(PT, 2) pairs_bwd_tc_kernel(const __grid_consta
   tc_fence_before();
   __syncthreads();
   if (tid < HID) part[HID * ldw + HID + tid] = dvs[tid] + dvs[HID + tid] + dvs[2 * HID + tid] + dvs[3 * HID + tid];
-  if (tid < 7) part[HID * ldw + 2 * HID + tid] = tid < 6 ? red[tid * 4] + red[tid * 4 + 1] + red[tid * 4 + 2] + red[tid * 4 + 3] : 0.f;
+  if (tid < 7)
+    part[HID * ldw + 2 * HID + tid] = (tid < 6 || kKm) ? red[tid * 4] + red[tid * 4 + 1] + red[tid * 4 + 2] + red[tid * 4 + 3] : 0.f;
   if (warp == 0) tmem_dealloc(tmem, TMEM_COLS);
 }
 
@@ -471,7 +480,7 @@ __device__ unsigned long long g_phase_clk[16];
 #define NAIS_PH(i)
 #endif
 
-template <bool kDrop>
+template <bool kDrop, bool kKm>
 __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_constant__ BwdArgs A) {
   constexpr int D = 64;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -499,7 +508,7 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
   unsigned long long* m_mask = reinterpret_cast<unsigned long long*>(m_hreg + PT);  // [PT] ReLU pattern     (half 1)
   long long* m_psid = reinterpret_cast<long long*>(m_mask + PT);    // [PT2] id behind this thread's 16 B of `ps` (private)
   long long* m_tgt = m_psid + PT2;                                  // [BWD_MAXROWS] target POI id of each row (live mask)
-  float2* m_ll = reinterpret_cast<float2*>(m_tgt + BWD_MAXROWS);    // [PT] |dlat|,|dlon| or the history item's coordinates (half 0)
+  float2* m_ll = reinterpret_cast<float2*>(m_tgt + BWD_MAXROWS);    // [PT] |dlat|,|dlon| (kKm: .x = km) or the history item's coordinates (half 0)
   float2* m_tco = m_ll + PT;                                        // [BWD_MAXROWS] target coordinates (segmented layout)
   float* m_rowv = reinterpret_cast<float*>(m_tco + BWD_MAXROWS);    // [3][BWD_MAXROWS] S, score, dscore of each row
   uint64_t* bar = reinterpret_cast<uint64_t*>(m_rowv + 4 * BWD_MAXROWS);
@@ -548,13 +557,18 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
       if (half == 0) {
         cp_async8(m_hist + cell, A.b.hist + c.hidx);
         if (lanes) cp_async8(m_ll + cell, A.b.aux ? A.b.aux + c.cidx * 2 : A.b.hist_coords + c.hidx * 2);
+        if (kKm) {  // the dense layout's km, or the history item's coordinates (where the lat/lon lanes stage theirs)
+          if (A.b.aux) cp_async4(m_ll + cell, A.b.aux + c.cidx);
+          else cp_async8(m_ll + cell, A.b.hist_coords + c.hidx * 2);
+        }
       } else {
         if (br.w_reg) cp_async8(m_hreg + cell, A.b.hreg + c.hidx);
         if (A.act_mask) cp_async8(m_mask + cell, A.act_mask + c.cidx);
       }
     }
     if (tid < Tn.nrows) cp_async8(m_tgt + tid, A.b.tgt + Tn.row0 + tid);
-    if (lanes && !A.b.aux && tid >= 32 && tid < 32 + Tn.nrows) cp_async8(m_tco + (tid - 32), A.b.tgt_coords + (Tn.row0 + tid - 32) * 2);
+    if ((lanes || kKm) && !A.b.aux && tid >= 32 && tid < 32 + Tn.nrows)
+      cp_async8(m_tco + (tid - 32), A.b.tgt_coords + (Tn.row0 + tid - 32) * 2);
     if (chn == 0) {
       if (tid >= 64 && tid < 64 + Tn.nrows) {
         const int rr = tid - 64;
@@ -586,6 +600,8 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
   };
 
   float pd[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // dist_w[4], dist_b[2] partials (this thread's hidden units of its cells)
+  float pkm = 0.f, kmc = 0.f;                    // kKm: sum of da * km over this thread's cells (half 0); sum_d embed_distance[0, d]
+  if constexpr (kKm) kmc = km_coef0(p, D);
   float dv_acc = 0.f;                            // dw2 partial of hidden unit s0 + lane over this warp's cells
   uint32_t phase = 0, dw_started = 0;
   int64_t item = blockIdx.x;  // (the launch gives every CTA at least one tile)
@@ -625,7 +641,7 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
       rowv[3 * BWD_MAXROWS + tid] = powf(S, p.beta);
     }
     int it32 = 0, rg32 = 0;
-    float l0r = 0.f, l1r = 0.f, g0 = 0.f, g1 = 0.f;
+    float l0r = 0.f, l1r = 0.f, g0 = 0.f, g1 = 0.f, km = 0.f;
     bool live = false;
     uint32_t am32 = 0u;
     if (valid) {
@@ -644,6 +660,14 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
         const float a0 = l0r * p.dist_scale, a1 = l1r * p.dist_scale;
         g0 = sigmoidf_exact(fmaf(a1, __ldg(p.dist_w + 1), fmaf(a0, __ldg(p.dist_w + 0), __ldg(p.dist_b + 0))));
         g1 = sigmoidf_exact(fmaf(a1, __ldg(p.dist_w + 3), fmaf(a0, __ldg(p.dist_w + 2), __ldg(p.dist_b + 1))));
+      }
+      if (kKm) {  // both threads of the cell form the same km (pair_km: the same dist_km_f call on the same coordinates)
+        const float2 hl = m_ll[cell];
+        km = hl.x;
+        if (!A.b.aux) {
+          const float2 tc = m_tco[r];
+          km = coords_km(A.b, tc.x, tc.y, hl.x, hl.y);
+        }
       }
       live = hid64 != m_tgt[r];
       if (A.act_mask) am32 = (uint32_t)(m_mask[cell] >> s0);  // this half's 32 hidden units
@@ -722,7 +746,8 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
     }
     asm volatile("bar.sync %0, 64;" ::"r"(1 + qd) : "memory");  // the two warps of this lane quarter exchange their halves of a
     NAIS_PH(5)
-    const float a = asum[cell] + asum[PT + cell];
+    float a = asum[cell] + asum[PT + cell];
+    if constexpr (kKm) a += __fmul_rn(km, kmc);
     float dav = 0.f, gwv = 0.f;
     if (live) {
       const float S = rowv[r], sc = rowv[BWD_MAXROWS + r], G = rowv[2 * BWD_MAXROWS + r], Sb = rowv[3 * BWD_MAXROWS + r];
@@ -731,6 +756,7 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
       dav = G * (w * ssum - p.beta * (e / S) * sc);
       gwv = G * w;
     }
+    if constexpr (kKm) pkm = half == 0 ? fmaf(dav, km, pkm) : 0.f;
     if constexpr (kDrop) dav *= A.drop_inv;  // d relu(drop(t)) / dt = m / (1-p)
     const bool have_mask = kDrop || A.act_mask != nullptr;
     float dg0 = 0.f, dg1 = 0.f;
@@ -913,8 +939,8 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
   }
   dvs[qd * HID + s0 + lane] = dv_acc;
 #pragma unroll
-  for (int q = 0; q < 6; ++q) {
-    float v = pd[q];
+  for (int q = 0; q < (kKm ? 7 : 6); ++q) {
+    float v = q < 6 ? pd[q] : pkm;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     if (lane == 0) red[q * 8 + warp] = v;
@@ -924,14 +950,14 @@ __global__ void __launch_bounds__(PT2, 2) pairs_bwd_tc2_kernel(const __grid_cons
   if (tid < HID) part[HID * ldw + HID + tid] = dvs[tid] + dvs[HID + tid] + dvs[2 * HID + tid] + dvs[3 * HID + tid];
   if (tid < 7) {
     float v = 0.f;
-    if (tid < 6)
+    if (tid < 6 || kKm)
       for (int w = 0; w < 8; ++w) v += red[tid * 8 + w];
     part[HID * ldw + 2 * HID + tid] = v;
   }
   if (warp == 0) tmem_dealloc(tmem, TMEM_COLS);
 }
 
-template <bool kDrop>
+template <bool kDrop, bool kKm>
 static int launch2(const BwdArgs& A, int grid, cudaStream_t stream) {
   constexpr int D = 64;
   constexpr size_t dt_region = (8 * 32 * STG_STRIDE > 2 * (HID / 8) * PT * 16) ? 8 * 32 * STG_STRIDE : 2 * (HID / 8) * PT * 16;
@@ -940,51 +966,57 @@ static int launch2(const BwdArgs& A, int grid, cudaStream_t stream) {
                           (3 * (size_t)PT + PT2 + BWD_MAXROWS) * 8 + ((size_t)PT + BWD_MAXROWS) * 8 + 4 * BWD_MAXROWS * 4 + 16;
   static_assert(2 * (smem + 1024) <= 228 * 1024, "two CTAs per SM");
   static SmemAttrOnce attr;
-  cudaError_t e = attr(pairs_bwd_tc2_kernel<kDrop>, smem, true);
+  cudaError_t e = attr(pairs_bwd_tc2_kernel<kDrop, kKm>, smem, true);
   if (e != cudaSuccess) return (int)e;
-  pairs_bwd_tc2_kernel<kDrop><<<grid, PT2, smem, stream>>>(A);
+  pairs_bwd_tc2_kernel<kDrop, kKm><<<grid, PT2, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
 
-template <int D, bool kDrop>
+template <int D, bool kDrop, bool kKm>
 static int launch(const BwdArgs& A, int grid, cudaStream_t stream) {
   constexpr size_t smem = 2 * (size_t)(D / 8 + 1) * PT * 16 + 2 * (size_t)(D / 8) * HID * 16 + 2 * (size_t)(HID / 8) * PT * 16 +
                           (4 * HID + 2 * BWD_MAXROWS * D + 4 * BWD_MAXROWS + 4 * HID + 32) * 4 + 16;
-  cudaError_t e = cudaFuncSetAttribute(pairs_bwd_tc_kernel<D, kDrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(pairs_bwd_tc_kernel<D, kDrop, kKm>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  e = cudaFuncSetAttribute(pairs_bwd_tc_kernel<D, kDrop>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  e = cudaFuncSetAttribute(pairs_bwd_tc_kernel<D, kDrop, kKm>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return (int)e;
-  pairs_bwd_tc_kernel<D, kDrop><<<grid, PT, smem, stream>>>(A);
+  pairs_bwd_tc_kernel<D, kDrop, kKm><<<grid, PT, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
 
 // D = 64: two threads per cell when each 32-column half of a row lies in one table (every shipped model class)
-template <bool kDrop>
+template <bool kDrop, bool kKm>
 static int launch_shape(const BwdArgs& A, int D, int grid, cudaStream_t stream) {
-  if (D == 32) return launch<32, kDrop>(A, grid, stream);
-  return pair_gather_uniform(A.p.branch[A.bi]) ? launch2<kDrop>(A, grid, stream) : launch<64, kDrop>(A, grid, stream);
+  if (D == 32) return launch<32, kDrop, kKm>(A, grid, stream);
+  return pair_gather_uniform(A.p.branch[A.bi]) ? launch2<kDrop, kKm>(A, grid, stream) : launch<64, kDrop, kKm>(A, grid, stream);
 }
 
 }  // namespace ptcb
 
+// One branch (lat/lon or no distance mode, dropout or not), or the disentangled two (no distance mode or km, no dropout)
 bool pairs_tc_bwd_supported(const NaisParams& p, const NaisPairs& b) {
-  if (p.n_branch != 1 || b.B < 1 || p.hid != ptcb::HID) return false;
-  const NaisBranch& br = p.branch[0];
-  const int D = br.w_poi + br.w_reg;
-  if (D != 32 && D != 64) return false;
-  if (p.dist_mode == NAIS_DIST_KM) return false;
-  if (!rows_vec4(br, 4)) return false;
-  (void)b;
+  if (b.B < 1 || p.hid != ptcb::HID) return false;
+  const bool two = pairs_disentangled(p);
+  if (p.n_branch != 1 && !two) return false;
+  if (p.dist_mode == NAIS_DIST_KM && !two) return false;
+  if (two && p.dropout_p > 0.f) return false;
+  for (int bi = 0; bi < p.n_branch; ++bi) {
+    const NaisBranch& br = p.branch[bi];
+    const int D = br.w_poi + br.w_reg;
+    if (D != 32 && D != 64) return false;
+    if (!rows_vec4(br, 4)) return false;
+  }
   return device_info().major == 10;
 }
 
 // grid <= 2 CTAs per SM (256 TMEM columns each); every CTA owns at least one tile (the caller passes min(n_items, grid)).  With
 // dropout A.act_mask must be the forward's pattern (PairsBwd::finish runs the FP32 kernel instead when it is NULL).
 int launch_pairs_bwd_tc(const BwdArgs& A, int D, int grid, cudaStream_t stream) {
-  if (A.p.dropout_p > 0.f) return A.act_mask ? ptcb::launch_shape<true>(A, D, grid, stream) : NAIS_ERR_NULL;
-  return ptcb::launch_shape<false>(A, D, grid, stream);
+  if (A.p.dropout_p > 0.f) return A.act_mask ? ptcb::launch_shape<true, false>(A, D, grid, stream) : NAIS_ERR_NULL;
+  if (A.p.dist_mode == NAIS_DIST_KM) return ptcb::launch_shape<false, true>(A, D, grid, stream);
+  return ptcb::launch_shape<false, false>(A, D, grid, stream);
 }
 
 }  // namespace nais

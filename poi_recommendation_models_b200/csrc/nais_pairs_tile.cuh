@@ -85,12 +85,21 @@ __device__ __forceinline__ void pair_latlon(const NaisPairs& b, int64_t cidx, in
 
 // dist_km of one cell (NAIS_DIST_KM): the dense layout reads the tensor the caller built (powerLaw.dist, model.py:497-504), the
 // segmented layout forms the haversine distance from the centred fp32 coordinates like the full-rank path (nais_fp32.cu)
+__device__ __forceinline__ float coords_km(const NaisPairs& b, float tla, float tlo, float hla, float hlo) {
+  const float d2r = 0.017453292519943295f;
+  return dist_km_f(tla, tlo, hla, hlo, cosf((b.center_lat + tla) * d2r), cosf((b.center_lat + hla) * d2r));
+}
 __device__ __forceinline__ float pair_km(const NaisPairs& b, int64_t cidx, int64_t hidx, int64_t row) {
   if (b.aux) return __ldg(b.aux + cidx);
   const float tla = __ldg(b.tgt_coords + row * 2), tlo = __ldg(b.tgt_coords + row * 2 + 1);
   const float hla = __ldg(b.hist_coords + hidx * 2), hlo = __ldg(b.hist_coords + hidx * 2 + 1);
-  const float d2r = 0.017453292519943295f;
-  return dist_km_f(tla, tlo, hla, hlo, cosf((b.center_lat + tla) * d2r), cosf((b.center_lat + hla) * d2r));
+  return coords_km(b, tla, tlo, hla, hlo);
+}
+// the coefficient of the km logit term, sum_d embed_distance[0, d], in the order of the FP32 kernels (km_coef, nais_fp32.cu)
+__device__ __forceinline__ float km_coef0(const NaisParams& p, int D) {
+  float c = 0.f;
+  for (int d = 0; d < D; ++d) c += __ldg(p.dist_embed + d);
+  return c;
 }
 
 // ---- software pipelining of a tile's inputs (the two-threads-per-cell tcgen05 pair kernels): Ampere-style cp.async into shared

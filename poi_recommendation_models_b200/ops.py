@@ -403,10 +403,15 @@ class _PairCall:
         return ws
 
 
+def act_mask_words(p: NaisParams, b: NaisPairs) -> int:
+    """Words of the act_mask nais_pairs_forward writes for (p, b): [n_branch, cells] (include/nais_b200.h)."""
+    return p.n_branch * (b.n_cells if b.seg_offsets else b.B * b.H)
+
+
 def _forward_launch(c: _PairCall, want_mask: bool = True, presort: bool = False):
     """nais_pairs_forward -> (score, row_sum, parts, act_mask, presorted workspace): act_mask is the ReLU pattern the tcgen05
-    forward saves for the tcgen05 backward (int64 [cells]; with dropout "active and kept"; None when the FP32 forward runs or
-    hid > 64).  With `presort`
+    forward saves for the tcgen05 backward (int64 [n_branch * cells], branch bi's from bi * cells; with dropout "active and
+    kept"; None when the FP32 forward runs or hid > 64).  With `presort`
     (one-branch variants) the call is nais_pairs_forward_presort and the last element is the backward workspace holding the
     sorted id lists for nais_pairs_backward_presorted; else None."""
     p, b, dev = c.p, c.b, c.dev
@@ -415,8 +420,8 @@ def _forward_launch(c: _PairCall, want_mask: bool = True, presort: bool = False)
     row_sum = torch.empty(p.n_branch, B, device=dev, dtype=torch.float32)
     parts = torch.empty(p.n_branch, B, device=dev, dtype=torch.float32)
     mask = None
-    if want_mask and B and p.n_branch == 1 and p.hid <= 64 and pairs_dispatch(p, b)[0]:
-        mask = torch.empty(b.n_cells if b.seg_offsets else B * b.H, device=dev, dtype=torch.int64)
+    if want_mask and B and p.hid <= 64 and pairs_dispatch(p, b)[0]:
+        mask = torch.empty(act_mask_words(p, b), device=dev, dtype=torch.int64)
     outs = (score.data_ptr(), row_sum.data_ptr(), parts.data_ptr(), _ptr(mask))
     # (the backward tiles exist for D, hid <= 128: a wider forward-only shape keeps the plain call)
     if presort and B and p.n_branch == 1 and p.hid <= 128 and p.branch[0].w_poi + p.branch[0].w_reg <= 128:
