@@ -226,6 +226,27 @@ NAIS_API int nais_pairs_dispatch(const NaisParams* p, const NaisPairs* batch, in
 NAIS_API int nais_pairs_forward(const NaisParams* p, const NaisPairs* batch, float* score, float* row_sum, float* score_parts,
                        uint64_t* act_mask, nais_stream_t stream);
 
+/* Explanations: which history items a pair score is made of (NAIS's attention, per cell).  For row r (a history and target j),
+ * branch b (0, or 0 and 1 for the disentangled model) and history position h:
+ *   E_bh = exp(a_bh) * [hist_h != j]     exactly the forward's, no max-shift
+ *   S_b  = sum_h E_bh                    the forward's row_sum
+ *   s_bh                                 the forward's similarity
+ *   pi_bh = E_bh / S_b                   attention share: sums to 1 over h
+ *   c_h  = sum_b E_bh * s_bh / S_b^beta  contribution: sums over h to the row's pre-sigmoid score
+ * (position h is the same history item in both branches of the disentangled model: its POI in branch 0, its region in branch 1).
+ * Per row, the m positions with the largest c_h are written in descending order, ties by ascending position (the ranking key of
+ * nais_fullrank_topk): out_pos [B,m] indexes the row's own history — hist[b, pos] dense, hist[seg_offsets[s] + pos] segmented —
+ * out_contrib [B,m] holds c_h and out_attn [n_branch,B,m] (optional) pi_bh.  A masked cell (history id == target id, read from
+ * the ids) is never selected; a row with fewer than m selectable cells is padded with pos -1, contrib -inf, attn 0.  score [B]
+ * (optional) is the pre-sigmoid score, bit-identical to nais_pairs_forward's for the same inputs.
+ * Both layouts; the kernels of nais_pairs_forward (NaisParams::pairs_precision, nais_pairs_dispatch: fwd_tc), each storing every
+ * cell's E and E*s in the workspace, then one warp per row selects.  Deterministic.  Argument errors before any CUDA call: m
+ * outside [1, 32] -> NAIS_ERR_SHAPE, dropout_p > 0 -> NAIS_ERR_MODE (inference only), out_pos / out_contrib NULL -> NAIS_ERR_NULL,
+ * workspace_bytes < nais_pairs_explain_workspace_bytes -> NAIS_ERR_WORKSPACE. */
+NAIS_API size_t nais_pairs_explain_workspace_bytes(const NaisParams* p, const NaisPairs* batch);
+NAIS_API int nais_pairs_explain(const NaisParams* p, const NaisPairs* batch, int32_t m, float* score, int32_t* out_pos,
+                                float* out_contrib, float* out_attn, void* workspace, size_t workspace_bytes, nais_stream_t stream);
+
 NAIS_API size_t nais_pairs_backward_workspace_bytes(const NaisParams* p, const NaisPairs* batch);
 /* Given dscore[B] = dL/dscore, write every parameter gradient.  score_parts / row_sum / act_mask are the forward's outputs
  * (act_mask: [n_branch, cells] as nais_pairs_forward writes it, branch bi's backward reads words bi*cells ..; NULL unless the

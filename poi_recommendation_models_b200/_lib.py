@@ -87,6 +87,9 @@ SYMBOLS = {
     "nais_pairs_dispatch": (C.c_int, [C.POINTER(NaisParams), C.POINTER(NaisPairs), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "nais_pairs_forward": (C.c_int, [C.POINTER(NaisParams), C.POINTER(NaisPairs), C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_void_p]),
+    "nais_pairs_explain_workspace_bytes": (C.c_size_t, [C.POINTER(NaisParams), C.POINTER(NaisPairs)]),
+    "nais_pairs_explain": (C.c_int, [C.POINTER(NaisParams), C.POINTER(NaisPairs), C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "nais_pairs_backward_workspace_bytes": (C.c_size_t, [C.POINTER(NaisParams), C.POINTER(NaisPairs)]),
     "nais_pairs_train_step_workspace_bytes": (C.c_size_t, [C.POINTER(NaisParams), C.POINTER(NaisPairs)]),
     "nais_pairs_train_step": (C.c_int, [C.POINTER(NaisParams), C.POINTER(NaisPairs), C.c_void_p, C.c_void_p, C.POINTER(NaisAdagrad),

@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libnais_b200.so")
-SOURCES = ["nais_capi.cu", "nais_fp32.cu", "nais_bwd.cu", "nais_tc.cu", "nais_pairs_tc.cu", "nais_pairs_tc_bwd.cu", "nais_sampler.cu"]
+SOURCES = ["nais_capi.cu", "nais_fp32.cu", "nais_bwd.cu", "nais_tc.cu", "nais_pairs_tc.cu", "nais_pairs_tc_bwd.cu", "nais_sampler.cu", "nais_explain.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-I", os.path.join(ROOT, "include"), "-I", CSRC]
 

@@ -9,7 +9,8 @@
 
 namespace nais {
 // nais_fp32.cu
-int launch_pairs_fwd(const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts, cudaStream_t stream);
+int launch_pairs_fwd(const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts, cudaStream_t stream,
+                     float* cell_e = nullptr, float* cell_es = nullptr);
 int launch_fullrank_fp32(const NaisParams& p, const NaisCatalog& cat, const NaisUsers& users, int64_t poi_begin,
                          int64_t poi_end, int k, int exclude, float* out_score, int32_t* out_id, float* all_scores,
                          void* ws, size_t ws_bytes, cudaStream_t stream, const GeoMixArgs* geo = nullptr);
@@ -55,7 +56,10 @@ int launch_bpr_dscore(const float* score, const float* group_weight, int64_t B, 
 int launch_dense_adagrad(float* const* param, float* const* sum, const float* const* grad, const int* n, float lr, float eps,
                          cudaStream_t stream);
 int launch_pairs_fwd_tc(const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts,
-                        unsigned long long* act_mask, cudaStream_t stream);
+                        unsigned long long* act_mask, cudaStream_t stream, float* cell_e = nullptr, float* cell_es = nullptr);
+// nais_explain.cu
+int launch_explain_select(const NaisParams& p, const NaisPairs& b, int m, const float* cell_e, const float* cell_es,
+                          const float* row_sum, int32_t* out_pos, float* out_contrib, float* out_attn, cudaStream_t stream);
 }  // namespace nais
 
 namespace nais {
@@ -340,6 +344,55 @@ int nais_pairs_forward(const NaisParams* p, const NaisPairs* batch, float* score
   if (rc) return rc;
   return launch_chosen_fwd(tc, *p, *batch, score, row_sum, score_parts, reinterpret_cast<unsigned long long*>(act_mask),
                            static_cast<cudaStream_t>(stream));
+}
+
+// Workspace of nais_pairs_explain: cell_e, cell_es [n_branch, cells], row_sum [n_branch, B] and the score [B] of a caller that
+// passes none, each 256-byte aligned.  Host-known sizes only.
+struct ExplainLayout {
+  size_t cell_e, cell_es, row_sum, score, total;
+};
+static ExplainLayout explain_layout(const NaisParams& p, const NaisPairs& b) {
+  auto up = [](size_t n) { return (n + 255) & ~(size_t)255; };
+  const size_t cells = (size_t)p.n_branch * (size_t)pairs_n_cells(b) * sizeof(float);
+  ExplainLayout L;
+  L.cell_e = 0;
+  L.cell_es = L.cell_e + up(cells);
+  L.row_sum = L.cell_es + up(cells);
+  L.score = L.row_sum + up((size_t)p.n_branch * b.B * sizeof(float));
+  L.total = L.score + up((size_t)b.B * sizeof(float));
+  return L;
+}
+
+size_t nais_pairs_explain_workspace_bytes(const NaisParams* p, const NaisPairs* batch) {
+  if (check_params(p) || check_pairs(p, batch) || batch->B == 0) return 0;
+  return explain_layout(*p, *batch).total;
+}
+
+int nais_pairs_explain(const NaisParams* p, const NaisPairs* batch, int32_t m, float* score, int32_t* out_pos, float* out_contrib,
+                       float* out_attn, void* workspace, size_t workspace_bytes, nais_stream_t stream) {
+  int rc = check_params(p);
+  if (rc) return rc;
+  rc = check_pairs(p, batch);
+  if (rc) return rc;
+  if (m < 1 || m > 32) return NAIS_ERR_SHAPE;
+  if (p->dropout_p > 0.f) return NAIS_ERR_MODE;  // explanations are inference: no dropout
+  if (batch->B == 0) return 0;
+  if (!out_pos || !out_contrib) return NAIS_ERR_NULL;
+  const ExplainLayout L = explain_layout(*p, *batch);
+  if (workspace_bytes < L.total) return NAIS_ERR_WORKSPACE;
+  if (!workspace) return NAIS_ERR_NULL;
+  char* ws = static_cast<char*>(workspace);
+  float *cell_e = reinterpret_cast<float*>(ws + L.cell_e), *cell_es = reinterpret_cast<float*>(ws + L.cell_es);
+  float* row_sum = reinterpret_cast<float*>(ws + L.row_sum);
+  if (!score) score = reinterpret_cast<float*>(ws + L.score);
+  bool tc = false;
+  rc = choose_pairs_fwd(*p, *batch, &tc);  // the forward nais_pairs_forward runs for (p, batch), with the per-cell terms stored
+  if (rc) return rc;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  rc = tc ? launch_pairs_fwd_tc(*p, *batch, score, row_sum, nullptr, nullptr, st, cell_e, cell_es)
+          : launch_pairs_fwd(*p, *batch, score, row_sum, nullptr, st, cell_e, cell_es);
+  if (rc) return rc;
+  return launch_explain_select(*p, *batch, m, cell_e, cell_es, row_sum, out_pos, out_contrib, out_attn, st);
 }
 
 size_t nais_pairs_backward_workspace_bytes(const NaisParams* p, const NaisPairs* batch) {

@@ -163,6 +163,31 @@ __device__ __forceinline__ void bitonic_sort_desc(unsigned long long* buf, int n
   }
 }
 
+// Register top-k of a warp (full-rank block top-k, pair explanations).  32 keys, one per lane -> sorted descending across the lanes (bitonic network on shuffles)
+__device__ __forceinline__ unsigned long long warp_sort_desc(unsigned long long v, int lane) {
+#pragma unroll
+  for (int k = 2; k <= 32; k <<= 1) {
+#pragma unroll
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, j);
+      const bool desc = k == 32 || (lane & k) == 0, lower = (lane & j) == 0;
+      v = (lower == desc) ? (v > o ? v : o) : (v < o ? v : o);
+    }
+  }
+  return v;
+}
+// two descending rows -> the best 32 of both, descending
+__device__ __forceinline__ unsigned long long warp_fold_top32(unsigned long long a, unsigned long long b, int lane) {
+  const unsigned long long br = __shfl_sync(0xffffffffu, b, 31 - lane);
+  unsigned long long v = a > br ? a : br;
+#pragma unroll
+  for (int j = 16; j > 0; j >>= 1) {
+    const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, j);
+    v = ((lane & j) == 0) ? (v > o ? v : o) : (v < o ? v : o);
+  }
+  return v;
+}
+
 // Dropout keep-mask (see NaisParams::dropout_p): counter-based, so forward and backward regenerate the same mask.
 __host__ __device__ __forceinline__ uint32_t dropout_bits(uint64_t seed, uint64_t idx) {
   uint64_t z = seed + idx * 0x9E3779B97F4A7C15ull;

@@ -181,10 +181,14 @@ struct PairsFwdArgs {
   float* row_sum;  // [n_branch,B] or NULL
   float* parts;    // [n_branch,B] per-branch score or NULL
   int* bad;        // the library's bad-index word (nais_common.cuh)
+  float* cell_e;   // kCells: [n_branch, cells] masked exp E of every cell (nais_pairs_explain), indexed like act_mask
+  float* cell_es;  // kCells: [n_branch, cells] E * similarity
 };
 
 constexpr int MAXROWS = PAIR_MAXROWS;  // rows (targets) sharing one 128-cell tile when H is small
 
+// kCells: also store every cell's e and e * s (the per-history-item terms of the score) for nais_pairs_explain
+template <bool kCells>
 __global__ void __launch_bounds__(NT, 2) pairs_fwd_kernel(const __grid_constant__ PairsFwdArgs A) {
   extern __shared__ __align__(16) float smem[];
   const NaisParams& p = A.p;
@@ -316,6 +320,13 @@ __global__ void __launch_bounds__(NT, 2) pairs_fwd_kernel(const __grid_constant_
         }
         red_e[cell] = e;
         red_es[cell] = es;
+        if constexpr (kCells) {
+          if (valid) {
+            const size_t ci = (size_t)bi * pairs_n_cells(A.b) + cidx;
+            A.cell_e[ci] = e;
+            A.cell_es[ci] = es;
+          }
+        }
       }
       __syncthreads();
       // row reductions: warp w handles rows w, w+8, ...
@@ -587,7 +598,7 @@ static int max_D(const NaisParams& p) {
 }
 
 int launch_pairs_fwd(const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts,
-                     cudaStream_t stream) {
+                     cudaStream_t stream, float* cell_e, float* cell_es) {
   if (b.B == 0) return 0;
   PairsFwdArgs A;
   A.p = p;
@@ -596,15 +607,20 @@ int launch_pairs_fwd(const NaisParams& p, const NaisPairs& b, float* score, floa
   A.row_sum = row_sum;
   A.parts = parts;
   A.bad = bad_index_flag();
+  A.cell_e = cell_e;
+  A.cell_es = cell_es;
+  const bool cells = cell_e && cell_es;
   const int D = max_D(p);
   const size_t smem = (tile_smem_floats(D) + (size_t)MAXROWS * D + 2 * TC + 2 * MAXROWS) * sizeof(float);
   if (smem > 227 * 1024) return NAIS_ERR_SHAPE;
-  cudaError_t e = cudaFuncSetAttribute(pairs_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cells ? cudaFuncSetAttribute(pairs_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                        : cudaFuncSetAttribute(pairs_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
   int64_t grid = pairs_n_tiles(b);
   if (grid < 1) return 0;
   if (grid > 148 * 4) grid = 148 * 4;
-  pairs_fwd_kernel<<<(unsigned)grid, NT, smem, stream>>>(A);
+  if (cells) pairs_fwd_kernel<true><<<(unsigned)grid, NT, smem, stream>>>(A);
+  else pairs_fwd_kernel<false><<<(unsigned)grid, NT, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }

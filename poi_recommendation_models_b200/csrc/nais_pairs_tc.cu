@@ -41,6 +41,8 @@ struct Args {
   int* bad;  // the library's bad-index word (nais_common.cuh)
   uint32_t drop_thresh;  // dropout: dropout_threshold(dropout_p) and 1 / (1 - dropout_p) (kernel parameters: read from the constant bank)
   float drop_inv;
+  float* cell_e;   // kCells: [cells] masked exp E of every cell of this branch (nais_pairs_explain), indexed like act_mask
+  float* cell_es;  // kCells: [cells] E * similarity
 };
 
 __device__ __forceinline__ float pow2_scale(float amax, int target_exp) {
@@ -53,7 +55,8 @@ __device__ __forceinline__ float pow2_scale(float amax, int target_exp) {
   return ldexpf(1.f, k);
 }
 
-template <int D, bool kDrop, bool kKm, bool kAcc>
+// kCells (instantiated with kDrop = false only): also store every cell's e and e * s for nais_pairs_explain
+template <int D, bool kDrop, bool kKm, bool kAcc, bool kCells>
 __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(const __grid_constant__ Args A) {
   extern __shared__ __align__(128) uint8_t smem[];
   const NaisParams& p = A.p;
@@ -300,6 +303,12 @@ __global__ void __launch_bounds__(PT, (D > 48) ? 3 : 4) pairs_fwd_tc_kernel(cons
       }
       red_e[tid] = e;
       red_es[tid] = es;
+      if constexpr (kCells) {
+        if (valid) {
+          A.cell_e[cidx] = e;
+          A.cell_es[cidx] = es;
+        }
+      }
       __syncthreads();
       for (int rr = warp; rr < ((H <= PT) ? nrows : 1); rr += PT / 32) {
         const int c0 = (H <= PT) ? rr * H : 0;
@@ -359,7 +368,7 @@ __device__ unsigned long long g_phase_clk[16];
 #define NAIS_PH(i)
 #endif
 
-template <bool kDrop, bool kKm, bool kAcc>
+template <bool kDrop, bool kKm, bool kAcc, bool kCells>
 __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_constant__ Args A) {
   constexpr int D = 64, HIDC = 64, KC = D / 8, A_PLANE = KC * PT * 16, W_PLANE = KC * HIDC * 16;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -638,6 +647,12 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
       }
       red_e[cell] = e;
       red_es[cell] = es;
+      if constexpr (kCells) {
+        if (valid) {
+          A.cell_e[c.cidx] = e;
+          A.cell_es[c.cidx] = es;
+        }
+      }
     }
     __syncthreads();  // (d)
     NAIS_PH(8)
@@ -682,14 +697,14 @@ __global__ void __launch_bounds__(PT2, 3) pairs_fwd_tc2_kernel(const __grid_cons
   if (warp == 0) tmem_dealloc(tmem, 64u);
 }
 
-template <bool kDrop, bool kKm, bool kAcc>
+template <bool kDrop, bool kKm, bool kAcc, bool kCells>
 static int launch2(const Args& A, int64_t n_items, int sms, cudaStream_t stream) {
   constexpr int D = 64, HIDC = 64;
   const size_t smem = 2 * (size_t)(D / 8) * PT * 16 + 2 * (size_t)(D / 8) * HIDC * 16 +
                       4096 + (4 * (size_t)HIDC + 2 * PMAXROWS * D + 2 * PT + 2 * PMAXROWS + 8 + 6 * PT + PT) * 4 +
                       (3 * (size_t)PT2 + PMAXROWS) * 8 + ((size_t)PT + PMAXROWS) * 8 + 16;
   static SmemAttrOnce attr;
-  cudaError_t e = attr(pairs_fwd_tc2_kernel<kDrop, kKm, kAcc>, smem, true);
+  cudaError_t e = attr(pairs_fwd_tc2_kernel<kDrop, kKm, kAcc, kCells>, smem, true);
   if (e != cudaSuccess) return (int)e;
   int per_sm = 3;
   const int by_smem = (int)((227 * 1024) / (smem + 1024));
@@ -697,18 +712,18 @@ static int launch2(const Args& A, int64_t n_items, int sms, cudaStream_t stream)
   if (per_sm < 1) return NAIS_ERR_SHAPE;
   const int64_t cap = (int64_t)sms * per_sm;
   const int grid = (int)(n_items < cap ? n_items : cap);
-  pairs_fwd_tc2_kernel<kDrop, kKm, kAcc><<<grid, PT2, smem, stream>>>(A);
+  pairs_fwd_tc2_kernel<kDrop, kKm, kAcc, kCells><<<grid, PT2, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
 
-template <int D, bool kDrop, bool kKm, bool kAcc>
+template <int D, bool kDrop, bool kKm, bool kAcc, bool kCells>
 static int launch(const Args& A, int hid, int64_t n_items, int sms, cudaStream_t stream) {
   const size_t smem = 2 * (size_t)(D / 8) * PT * 16 + 2 * (size_t)(D / 8) * hid * 16 +
                       (4 * (size_t)hid + PMAXROWS * D + 2 * PT + 2 * PMAXROWS + 8) * 4 + 16 + (size_t)PT * STG_STRIDE;
-  cudaError_t e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc, kCells>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  e = cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc, kCells>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return (int)e;
   // Persistent grid: as many CTAs as can be co-resident — the kernel's register budget (3 per SM for D = 64, else 4), shared
   // memory, and TMEM (tmem_cols of the SM's 512 columns per CTA; a CTA beyond that would simply wait in tcgen05.alloc).
@@ -719,20 +734,20 @@ static int launch(const Args& A, int hid, int64_t n_items, int sms, cudaStream_t
   if (per_sm < 1) return NAIS_ERR_SHAPE;
   const int64_t cap = (int64_t)sms * per_sm;
   const int grid = (int)(n_items < cap ? n_items : cap);
-  pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc><<<grid, PT, smem, stream>>>(A);
+  pairs_fwd_tc_kernel<D, kDrop, kKm, kAcc, kCells><<<grid, PT, smem, stream>>>(A);
   NAIS_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
 
 // `two`: two threads per cell (D = hid = 64, a cell's 32-column halves each lie in one table)
-template <bool kDrop, bool kKm, bool kAcc>
+template <bool kDrop, bool kKm, bool kAcc, bool kCells = false>
 static int launch_shape(const Args& A, int D, bool two, int64_t n_items, int sms, cudaStream_t stream) {
-  if (two) return launch2<kDrop, kKm, kAcc>(A, n_items, sms, stream);
+  if (two) return launch2<kDrop, kKm, kAcc, kCells>(A, n_items, sms, stream);
   switch (D) {
-    case 16: return launch<16, kDrop, kKm, kAcc>(A, A.p.hid, n_items, sms, stream);
-    case 32: return launch<32, kDrop, kKm, kAcc>(A, A.p.hid, n_items, sms, stream);
-    case 48: return launch<48, kDrop, kKm, kAcc>(A, A.p.hid, n_items, sms, stream);
-    case 64: return launch<64, kDrop, kKm, kAcc>(A, A.p.hid, n_items, sms, stream);
+    case 16: return launch<16, kDrop, kKm, kAcc, kCells>(A, A.p.hid, n_items, sms, stream);
+    case 32: return launch<32, kDrop, kKm, kAcc, kCells>(A, A.p.hid, n_items, sms, stream);
+    case 48: return launch<48, kDrop, kKm, kAcc, kCells>(A, A.p.hid, n_items, sms, stream);
+    case 64: return launch<64, kDrop, kKm, kAcc, kCells>(A, A.p.hid, n_items, sms, stream);
     default: return NAIS_ERR_SHAPE;
   }
 }
@@ -755,15 +770,18 @@ bool pairs_tc_supported(const NaisParams& p, const NaisPairs& b) {
   return true;
 }
 
-// row_sum / parts are [n_branch, B] and act_mask [n_branch, cells] (each may be NULL); branch bi writes its slice
+// row_sum / parts are [n_branch, B], act_mask and cell_e / cell_es [n_branch, cells] (each may be NULL); branch bi writes its
+// slice.  cell_e and cell_es (nais_pairs_explain) run the kCells kernels; they are never given with dropout.
 int launch_pairs_fwd_tc(const NaisParams& p, const NaisPairs& b, float* score, float* row_sum, float* parts,
-                        unsigned long long* act_mask, cudaStream_t stream) {
+                        unsigned long long* act_mask, cudaStream_t stream, float* cell_e, float* cell_es) {
   const DeviceInfo di = device_info();
   if (di.major != 10) return NAIS_ERR_ARCH;
   const int sms = di.sms;
   const int64_t n_items = pairs_n_tiles(b);
   if (n_items < 1) return 0;
   const bool km = p.dist_mode == NAIS_DIST_KM;
+  const bool cells = cell_e && cell_es;
+  if (cells && p.dropout_p > 0.f) return NAIS_ERR_MODE;
   for (int bi = 0; bi < p.n_branch; ++bi) {
     ptc::Args A;
     A.p = p;
@@ -778,11 +796,17 @@ int launch_pairs_fwd_tc(const NaisParams& p, const NaisPairs& b, float* score, f
     A.drop_thresh = p.dropout_p > 0.f ? dropout_threshold(p.dropout_p) : 0u;
     A.drop_inv = p.dropout_p > 0.f ? 1.f / (1.f - p.dropout_p) : 1.f;
     A.tmem_cols = p.hid <= 32 ? 32u : (p.hid <= 64 ? 64u : 128u);
+    A.cell_e = cells ? cell_e + (size_t)bi * pairs_n_cells(b) : nullptr;
+    A.cell_es = cells ? cell_es + (size_t)bi * pairs_n_cells(b) : nullptr;
     const NaisBranch& br = p.branch[bi];
     const int D = br.w_poi + br.w_reg;
     const bool two = D == 64 && p.hid == 64 && rows_vec4(br, 4) && pair_gather_uniform(br);
     int rc;
-    if (p.dropout_p > 0.f) rc = ptc::launch_shape<true, false, false>(A, D, two, n_items, sms, stream);  // (one branch only)
+    if (cells) rc = km ? (bi ? ptc::launch_shape<false, true, true, true>(A, D, two, n_items, sms, stream)
+                             : ptc::launch_shape<false, true, false, true>(A, D, two, n_items, sms, stream))
+                       : (bi ? ptc::launch_shape<false, false, true, true>(A, D, two, n_items, sms, stream)
+                             : ptc::launch_shape<false, false, false, true>(A, D, two, n_items, sms, stream));
+    else if (p.dropout_p > 0.f) rc = ptc::launch_shape<true, false, false>(A, D, two, n_items, sms, stream);  // (one branch only)
     else if (km) rc = bi ? ptc::launch_shape<false, true, true>(A, D, two, n_items, sms, stream)
                          : ptc::launch_shape<false, true, false>(A, D, two, n_items, sms, stream);
     else rc = bi ? ptc::launch_shape<false, false, true>(A, D, two, n_items, sms, stream)

@@ -479,31 +479,6 @@ struct MainArgs {
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 512;" ::: "memory"); }
 
 // kSinglePart: D <= 64, a B stage holds a whole chunk (kp == 1).  kHch: history items per MMA step (2: hid <= 64, 1: hid 96/128).
-// 32 keys, one per lane -> sorted descending across the lanes (bitonic network on shuffles)
-__device__ __forceinline__ unsigned long long warp_sort_desc(unsigned long long v, int lane) {
-#pragma unroll
-  for (int k = 2; k <= 32; k <<= 1) {
-#pragma unroll
-    for (int j = k >> 1; j > 0; j >>= 1) {
-      const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, j);
-      const bool desc = k == 32 || (lane & k) == 0, lower = (lane & j) == 0;
-      v = (lower == desc) ? (v > o ? v : o) : (v < o ? v : o);
-    }
-  }
-  return v;
-}
-// two descending rows -> the best 32 of both, descending
-__device__ __forceinline__ unsigned long long warp_fold_top32(unsigned long long a, unsigned long long b, int lane) {
-  const unsigned long long br = __shfl_sync(0xffffffffu, b, 31 - lane);
-  unsigned long long v = a > br ? a : br;
-#pragma unroll
-  for (int j = 16; j > 0; j >>= 1) {
-    const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, j);
-    v = ((lane & j) == 0) ? (v > o ? v : o) : (v < o ? v : o);
-  }
-  return v;
-}
-
 // kFix: 0 = generic (every shape is a run-time value); 1 / 2 = the D = hid = 64 shape of the headline workload in SPLIT / MIX
 // precision with every tile constant known at compile time: a fully unrolled MMA issue sequence (descriptor = base +
 // immediate; the generic issuer spends ~15 instructions per MMA, which paces the kernel once a step is 9 MMAs) and the

@@ -19,13 +19,22 @@ There is no CPU path: calling a model whose parameters or inputs are not on a CU
 """
 from __future__ import annotations
 
-from typing import Dict, Optional, Sequence, Tuple
+from typing import Dict, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
 import torch.nn as nn
 
 from . import ops
+
+
+class Explanation(NamedTuple):
+    """`explain`'s result for a [U,k] list of recommended POIs, m explaining history items each (-1 / -inf / 0 padding)."""
+    score: torch.Tensor    # [U,k] pre-sigmoid score of (user, POI); NaN for a padded entry or a user without history
+    poi: torch.Tensor      # [U,k,m] int64 history POIs with the largest contributions, descending
+    pos: torch.Tensor      # [U,k,m] int64 their positions in the user's history (the CSR slice)
+    contrib: torch.Tensor  # [U,k,m] their contributions: over ALL history items they sum to `score`
+    attn: torch.Tensor     # [n_branch,U,k,m] their attention shares E_h / sum E per branch
 
 
 class _NAISBase(nn.Module):
@@ -340,6 +349,57 @@ class _NAISBase(nn.Module):
         s, i = ops.fullrank_topk(self.variant, float(self.beta), self._params(), self._catalog, users, k, poi_begin,
                                  poi_end, exclude_history, plan.precision, plan)
         return torch.sigmoid(s), i.to(torch.int64)
+
+    @torch.no_grad()
+    def explain(self, users, ids, m: int = 5, precision: str = "auto") -> Explanation:
+        """Why each recommended POI was recommended: for every (user u, POI j) of `ids` [U,k] (predict_topk's lists; -1 = padding),
+        the m history items h of u with the largest contribution c_h = sum_b E_bh s_bh / (sum_h' E_bh')^beta to the pre-sigmoid
+        score — which is exactly sum_h c_h — with their attention shares (include/nais_b200.h nais_pairs_explain).  `users`: the
+        DeviceUsers or (indptr, indices) pair the lists were ranked for.  One segmented pair batch (a segment per user, a row per
+        valid id; target regions and coordinates from set_catalog's catalogue), one library call; no dropout (inference), no
+        autograd.  `precision`: the pair kernels' "auto" / "fp32" / "tc".  Ids outside the catalogue are reported by
+        ops.check_indices like every pair call's."""
+        if self._catalog is None:
+            raise RuntimeError("call set_catalog(region, coords) first")
+        if not isinstance(users, ops.DeviceUsers):
+            users = self.make_users(*users)
+        cat, P = self._catalog, self._params()
+        dev = next(self.parameters()).device
+        ids = torch.as_tensor(ids, device=dev).to(torch.int64)
+        if ids.dim() != 2 or ids.shape[0] != users.n_users:
+            raise ValueError(f"ids must be [n_users, k] = [{users.n_users}, k]; got {tuple(ids.shape)}")
+        U, k = ids.shape
+        ho = np.asarray(users.host_offsets if users.host_offsets is not None else users.offsets.cpu().numpy(), dtype=np.int64)
+        H = np.diff(ho)
+        valid = (ids >= 0) & torch.as_tensor(H > 0, device=dev)[:, None]
+        st = ops.segment_structure(H, valid.sum(1).cpu().numpy(), dev)
+        flat = valid.reshape(-1).nonzero().squeeze(1)  # row-major: the rows of a user are contiguous, users in order
+        tgt = ids.reshape(-1)[flat]
+        has_reg = "embed_region.weight" in P
+        has_co = ops.VARIANT_DIST[self.variant][0] != ops.DIST_NONE
+        if (has_reg and (cat.region is None or users.region is None)) or (has_co and (cat.coords is None or users.coords is None)):
+            raise RuntimeError(f"explain: the {self.variant!r} model needs the catalogue's "
+                               + ("regions and coordinates" if has_reg and has_co else "regions" if has_reg else "coordinates"))
+        # catalogue rows of the targets: an id outside the table is gathered as row 0 here and reported by the kernel's id check
+        crow = (tgt - cat.row_base).clamp(0, max(cat.n_rows - 1, 0))
+        batch = ops.SegmentedPairs(
+            hist=users.items.to(torch.int64), hreg=users.region.to(torch.int64) if has_reg else None,
+            hist_coords=users.coords if has_co else None, tgt=tgt, treg=cat.region[crow].to(torch.int64) if has_reg else None,
+            tgt_coords=cat.coords[crow].contiguous() if has_co else None, label=None, seg_offsets=st["seg_offsets"],
+            row_offsets=st["row_offsets"], seg_cell_offsets=st["seg_cell_offsets"], tile_seg=st["tile_seg"], tile_row0=st["tile_row0"],
+            n_seg=st["n_seg"], B=st["B"], n_tiles=st["n_tiles"], n_cells=st["n_cells"], max_hist=st["max_hist"],
+            host_row_offsets=st["host_row_offsets"], center=cat.center)
+        score, pos, contrib, attn = ops.pairs_explain(self.variant, float(self.beta), P, batch, m=m, precision=precision)
+        nb = attn.shape[0]
+        o_score = torch.full((U * k,), float("nan"), device=dev)
+        o_pos = torch.full((U * k, m), -1, device=dev, dtype=torch.int64)
+        o_contrib = torch.full((U * k, m), float("-inf"), device=dev)
+        o_attn = torch.zeros(nb, U * k, m, device=dev)
+        o_score[flat], o_pos[flat], o_contrib[flat], o_attn[:, flat] = score, pos, contrib, attn
+        user = torch.arange(U, device=dev).repeat_interleave(k)
+        at = users.offsets[user][:, None] + o_pos.clamp(min=0)
+        poi = torch.where(o_pos >= 0, users.items.to(torch.int64)[at.clamp(max=max(users.nnz - 1, 0))] if users.nnz else o_pos, -1)
+        return Explanation(o_score.view(U, k), poi.view(U, k, m), o_pos.view(U, k, m), o_contrib.view(U, k, m), o_attn.view(nb, U, k, m))
 
 
 class NAIS_basic(_NAISBase):

@@ -701,6 +701,30 @@ def pairs_forward_raw(variant: str, beta: float, P: Dict[str, torch.Tensor], his
     return score, row_sum, parts, mask
 
 
+def pairs_explain(variant: str, beta: float, P: Dict[str, torch.Tensor], hist, tgt=None, hreg=None, treg=None, aux=None, m: int = 5,
+                  precision: str = "auto"):
+    """Why each pair scored what it did (nais_pairs_explain): (score [B] pre-sigmoid, bit-identical to the pair forward's; pos
+    [B,m] int64, the m history positions with the largest contribution c_h = sum_b E_bh s_bh / S_b^beta, descending, ties by
+    ascending position; contrib [B,m] those c_h (summed over all h they are the score); attn [n_branch,B,m] their attention
+    share E_bh / S_b).  Masked positions (history item == target) are never selected; rows with fewer than m selectable positions
+    are padded with pos -1, contrib -inf, attn 0.  `pos` indexes the row's own history: hist[b, pos], or for an ops.SegmentedPairs
+    `hist` the segment's slice of hist.hist.  `precision`: the pair forward's kernels ("auto", "fp32", "tc").  No dropout, no
+    autograd."""
+    dev = _need_cuda(hist, tgt, hreg, treg, aux, *P.values())
+    m = int(m)
+    if not 1 <= m <= 32:
+        raise ValueError(f"pairs_explain: m must be in [1, 32], got {m}")
+    with _PairCall(dev, variant, beta, P, precision, batch=(hist, tgt, hreg, treg, aux)) as c:
+        B, nb = int(c.b.B), int(c.p.n_branch)
+        score = torch.empty(B, device=dev, dtype=torch.float32)
+        pos = torch.empty(B, m, device=dev, dtype=torch.int32)
+        contrib = torch.empty(B, m, device=dev, dtype=torch.float32)
+        attn = torch.empty(nb, B, m, device=dev, dtype=torch.float32)
+        c.launch("nais_pairs_explain", m, score.data_ptr(), pos.data_ptr(), contrib.data_ptr(), attn.data_ptr(),
+                 ws_bytes=c.query("nais_pairs_explain_workspace_bytes"))
+    return score, pos.to(torch.int64), contrib, attn
+
+
 def dropout_keep_mask(seed: int, B: int, H: int, hid: int, p: float):
     """The keep-mask the kernels use for a dense [B,H] batch, on the host (numpy bool [B,H,hid]) — for tests / reproducing a step."""
     return dropout_keep_mask_cells(seed, B * H, hid, p).reshape(B, H, hid)
