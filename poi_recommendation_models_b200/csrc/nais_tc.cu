@@ -478,6 +478,26 @@ struct MainArgs {
 
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 512;" ::: "memory"); }
 
+// (p0, p1) += (|a|, |b|) as one packed add.rn.f32x2: ptxas folds the two fabsf into FADD2's |x| operand modifier, so a pair of
+// accumulator columns costs one issue slot instead of two.  Each half is an ordinary round-to-nearest fp32 add (no flush), so
+// the sums are bit-identical to the scalar `p0 += fabsf(a); p1 += fabsf(b);`.
+__device__ __forceinline__ void add_abs2(float& p0, float& p1, uint32_t a, uint32_t b) {
+  unsigned long long acc, val;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(acc) : "f"(p0), "f"(p1));
+  asm("mov.b64 %0, {%1, %2};" : "=l"(val) : "f"(fabsf(__uint_as_float(a))), "f"(fabsf(__uint_as_float(b))));
+  asm("add.rn.f32x2 %0, %0, %1;" : "+l"(acc) : "l"(val));
+  asm("mov.b64 {%0, %1}, %2;" : "=f"(p0), "=f"(p1) : "l"(acc));
+}
+// (p0, p1) = fma((|a|, |b|), (s0, s1), (p0, p1)) as one packed fma.rn.f32x2 (FFMA2, |x| folded): bit-identical to two fmaf
+__device__ __forceinline__ void fma_abs2(float& p0, float& p1, uint32_t a, uint32_t b, float s0, float s1) {
+  unsigned long long acc, val, sg;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(acc) : "f"(p0), "f"(p1));
+  asm("mov.b64 %0, {%1, %2};" : "=l"(val) : "f"(fabsf(__uint_as_float(a))), "f"(fabsf(__uint_as_float(b))));
+  asm("mov.b64 %0, {%1, %2};" : "=l"(sg) : "f"(s0), "f"(s1));
+  asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc) : "l"(val), "l"(sg));
+  asm("mov.b64 {%0, %1}, %2;" : "=f"(p0), "=f"(p1) : "l"(acc));
+}
+
 // kSinglePart: D <= 64, a B stage holds a whole chunk (kp == 1).  kHch: history items per MMA step (2: hid <= 64, 1: hid 96/128).
 // kFix: 0 = generic (every shape is a run-time value); 1 / 2 = the D = hid = 64 shape of the headline workload in SPLIT / MIX
 // precision with every tile constant known at compile time: a fully unrolled MMA issue sequence (descriptor = base +
@@ -933,7 +953,8 @@ __global__ void __launch_bounds__(THREADS, 1) fullrank_tc_kernel(const __grid_co
         // ---- specialised step loop: hid == 64, two history items per step, tpc == NBUF == 3 -----------------------------
         // Every step index is then (chunk, t) with buffer == t, so the t loop unrolls with compile-time TMEM / A_ext
         // addresses, the per-chunk history lookups leave the step body, and this group's acc_full parity is one bit that
-        // flips once per own chunk.  ~150 issue slots per warp-step instead of ~340 (the MIX mode is epilogue-issue bound).
+        // flips once per own chunk.  ~150 issue slots per warp-step instead of ~340 (the MIX mode is epilogue-issue bound); the |x| sums
+        // then run as packed pairs (add_abs2 / fma_abs2), 32 instead of 64 slots per warp-step.
         const unsigned char* ebase = sE + r * 16 + hs * 4;
         // A_ext of (chunk pc, tile t): 2 sigmoids -> hi/lo halves.  sAe / (1 + 2^z) = 1 / (1/sAe + 2^(z - log2 sAe))
         auto produce_f = [&](int t, bool on, float hla, float hlo, float cla, float clo) {
@@ -997,27 +1018,21 @@ __global__ void __launch_bounds__(THREADS, 1) fullrank_tc_kernel(const __grid_co
               if (b < nposb) {
 #pragma unroll
                 for (int i = 0; i < 16; i += 4) {
-                  p0 += fabsf(__uint_as_float(v[i]));
-                  p1 += fabsf(__uint_as_float(v[i + 1]));
-                  p2 += fabsf(__uint_as_float(v[i + 2]));
-                  p3 += fabsf(__uint_as_float(v[i + 3]));
+                  add_abs2(p0, p1, v[i], v[i + 1]);
+                  add_abs2(p2, p3, v[i + 2], v[i + 3]);
                 }
               } else if (b > nposb || nposm == 0) {
 #pragma unroll
                 for (int i = 0; i < 16; i += 4) {
-                  q0 += fabsf(__uint_as_float(v[i]));
-                  q1 += fabsf(__uint_as_float(v[i + 1]));
-                  q2 += fabsf(__uint_as_float(v[i + 2]));
-                  q3 += fabsf(__uint_as_float(v[i + 3]));
+                  add_abs2(q0, q1, v[i], v[i + 1]);
+                  add_abs2(q2, q3, v[i + 2], v[i + 3]);
                 }
               } else {  // the one block that holds both signs: signed FFMA with the +-1 vector kept in shared memory
 #pragma unroll
                 for (int i = 0; i < 16; i += 4) {
                   const float4 sg = *reinterpret_cast<const float4*>(sgn_mixed + i);
-                  p0 = fmaf(fabsf(__uint_as_float(v[i])), sg.x, p0);
-                  p1 = fmaf(fabsf(__uint_as_float(v[i + 1])), sg.y, p1);
-                  p2 = fmaf(fabsf(__uint_as_float(v[i + 2])), sg.z, p2);
-                  p3 = fmaf(fabsf(__uint_as_float(v[i + 3])), sg.w, p3);
+                  fma_abs2(p0, p1, v[i], v[i + 1], sg.x, sg.y);
+                  fma_abs2(p2, p3, v[i + 2], v[i + 3], sg.z, sg.w);
                 }
               }
             };
